@@ -8,6 +8,7 @@ collective).  The step runs as ONE CUDA graph (tgp_b200.GraphedStep: the dense p
 timed region holds no Python / allocator / launch overhead; the eager time is reported beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload all|c1|c2|c3|c4|c5]
+                    [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = graphs/s with inputs resident in HBM over exactly K timed steps;
 `long_run` repeats the measurement over a >= 100 ms region; `e2e` = the same metric through the public API from
@@ -16,6 +17,12 @@ pinned HOST buffers (edge list + features copied in every step, densified on the
 `kernels` = per-kernel time of one step (separate eager pass) and `host_gap_ms` = ms_per_step - their sum;
 `configs` = a measured entry (ms_per_step, roofline, ...) for every BASELINE.json config (C1..C5) that the
 launch can run; `cpu_baseline` = the CPU oracle (restated reference path) on a bounded sample.
+
+`--dump-outputs DIR` writes what the last timed step of the headline (dense) workload computed on rank 0 as
+DIR/<name>.npy in float32: the last level's pooled features `x_pool` and adjacency `adj_pool`, the `losses`
+([mincut, ortho, link, entropy], one row per level when there are several), and the gradients `grad_x` and `grad_s<i>`
+of X and of each level's assignment.  The inputs depend only on the workload and the rank, so two builds can be compared
+array for array.  Per-graph arrays are a fixed, seeded sample of the batch's graphs when all of them would exceed 64 MB.
 """
 from __future__ import annotations
 
@@ -36,6 +43,7 @@ for p in (ROOT, os.path.join(ROOT, "torch-geometric-pool_b200")):
 import torch  # noqa: E402
 
 METRIC = "coarsened graphs/s (Reduce+Connect fwd+bwd)"
+DUMP_BYTES = 64 * 10**6  # upper bound of what --dump-outputs writes
 
 DENSE = {
     "c2": dict(B=512, levels=[(256, 64)], F=128, dtype="f32", p=0.05, pooler="mincut", scaling="weak",
@@ -292,7 +300,21 @@ class DenseStep:
             outs.append(losses)
             grads.append(self.g_l)
         torch.autograd.backward([xl, al] + outs, [self.g_xp, self.g_ap] + grads)
-        return outs[0] if len(outs) == 1 else torch.stack(outs)
+        return xl, al, outs[0] if len(outs) == 1 else torch.stack(outs)
+
+    def outputs(self, step_out):
+        """What the caller of one step receives (`step_out` = what `run` returned; the gradients are read from X and S),
+        as float32 arrays for --dump-outputs.  Per-graph arrays keep a fixed, seeded sample of the graphs when all of
+        them would exceed DUMP_BYTES."""
+        xl, al, losses = step_out
+        per_graph = {"x_pool": xl, "adj_pool": al, "grad_x": self.x.grad}
+        per_graph.update({f"grad_s{i}": t.grad for i, t in enumerate(self.s)})
+        graph_bytes = sum(4 * t[0].numel() for t in per_graph.values())
+        n = min(self.B, (DUMP_BYTES - 4 * losses.numel()) // graph_bytes)
+        keep = torch.randperm(self.B, generator=torch.Generator().manual_seed(0))[:n].sort().values.to(xl.device)
+        out = {k: t.detach().index_select(0, keep).float() for k, t in per_graph.items()}
+        out["losses"] = losses.detach().float().clone()
+        return out
 
 
 def run_dense(ctx, name, headline):
@@ -323,6 +345,8 @@ def run_dense(ctx, name, headline):
                     graphed.replay()
                 torch.cuda.synchronize()
             ms = ctx.timed(graphed.replay, args.steps)
+            if args.dump_outputs:
+                out["_dump"] = st.outputs(graphed.outputs)
             long = ctx.long_run(graphed.replay)
             t_soak = time.perf_counter() + 0.3
             while time.perf_counter() < t_soak:
@@ -887,7 +911,12 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="all", choices=["all"] + sorted(DENSE) + sorted(SPARSE))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload in SPARSE):
+        ap.error("--dump-outputs writes the outputs of the dense headline step: --impl b200, --workload all, c2 or c3")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -898,6 +927,7 @@ def main():
     head_name = args.workload if args.workload in DENSE else "c2"
     configs = {}
     line = None
+    dump = None
 
     def attempt(name, fn):
         try:
@@ -927,6 +957,7 @@ def main():
             line["e2e"] = e2e
         configs[head_name] = {k: v for k, v in strip(head).items() if k not in ("kernels", "clocks")}
         configs[head_name]["config"] = config_of(head_name, world)
+        dump = head.get("_dump")
         del head
         torch.cuda.empty_cache()
     if args.workload == "all":
@@ -962,6 +993,12 @@ def main():
         if not args.no_cpu_baseline and world == 1 and args.workload in ("all",) + tuple(DENSE):
             line["cpu_baseline"] = cpu_baseline(DENSE[head_name])
         print(json.dumps(line), flush=True)
+        if dump is not None:
+            import numpy as np
+
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, t in dump.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), t.cpu().numpy())
     if ctx.dist is not None:
         ctx.dist.barrier()
         ctx.dist.destroy_process_group()
