@@ -250,10 +250,17 @@ int tgpb200_weight_norm_bwd(const int64_t* row, const float* w, const int64_t* b
  *                tgp/utils/losses.py:39-123, computed from the RAW product (tgp/poolers/mincut.py:226-237)
  *   loss_kind 2: losses[2] = link_pred_loss (one Frobenius norm over the batch, / link_div),
  *                losses[3] = entropy_loss (/ ent_div)   tgp/utils/losses.py:644-708, 476-500
+ *   loss_kind 3: DMoN (PyG DMoNPooling's losses), with d = adj 1, 2m = sum_i d_i, t = tr(S^T adj S) raw,
+ *                c = S^T d, e = S^T 1 per graph:  losses[0] = spectral = mean_b -(t - ||c||^2 / 2m) / 2m,
+ *                losses[1] = orthogonality_loss (as kind 1), losses[2] = cluster = mean_b ||e|| sqrt(K) / n_b - 1,
+ *                losses[3] = 0.  A graph with 2m = 0 gives a NaN spectral loss.  Needs adj.
  * adj [B,N,N], s [B,N,K], x [B,N,F] row-major of `dtype`; x may be NULL (connect only), adj may be NULL
  * (reduce only).  `saved` (tgpb200_dense_pool_saved_bytes) carries S^T A, S^T S, row statistics and the
  * per-graph loss terms from forward to backward; the backward also needs a scratch workspace.
  * grad_losses: 4 device floats (upstream gradients of losses[0..3]) or NULL.  grad_adj may be NULL.
+ * The _v2 entry points take `graph_nodes`: [B] device floats, the valid node count n_b of each graph (the cluster
+ * loss of kind 3 divides by it), or NULL for n_b = N.  It is read on the device only (no host synchronisation).
+ * The entry points without _v2 are the _v2 ones with graph_nodes = NULL.
  * ------------------------------------------------------------------------------------------ */
 size_t tgpb200_dense_pool_saved_bytes(int64_t B, int64_t N, int64_t K);
 size_t tgpb200_dense_pool_bwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int need_grad_adj);
@@ -266,6 +273,16 @@ int tgpb200_dense_pool_bwd(const void* adj, const void* s, const void* x, const 
                            int64_t F, int dtype, uint32_t flags, int loss_kind, float eps, float link_div,
                            float ent_div, void* grad_s, void* grad_x, void* grad_adj, void* saved, size_t saved_bytes,
                            void* workspace, size_t workspace_bytes, tgpb200_stream_t stream);
+int tgpb200_dense_pool_fwd_v2(const void* adj, const void* s, const void* x, int64_t B, int64_t N, int64_t K,
+                              int64_t F, int dtype, uint32_t flags, int loss_kind, float eps, float link_div,
+                              float ent_div, void* x_pool, void* adj_pool, float* losses, void* saved,
+                              size_t saved_bytes, tgpb200_stream_t stream, const float* graph_nodes);
+int tgpb200_dense_pool_bwd_v2(const void* adj, const void* s, const void* x, const void* grad_x_pool,
+                              const void* grad_adj_pool, const float* grad_losses, int64_t B, int64_t N, int64_t K,
+                              int64_t F, int dtype, uint32_t flags, int loss_kind, float eps, float link_div,
+                              float ent_div, void* grad_s, void* grad_x, void* grad_adj, void* saved,
+                              size_t saved_bytes, void* workspace, size_t workspace_bytes, tgpb200_stream_t stream,
+                              const float* graph_nodes);
 
 /* ------------------------------------------------------------------------------------------
  * Tensor-core batched product (tcgen05 / TMEM / TMA), the engine under the dense path; exported for tests

@@ -15,6 +15,6 @@ int dense_fwd_fused_ts(const float* A, const float* S, const float* X, int B, in
 // dense_bwd_fused.cu: fp32 backward in one launch -- W = A S stays in tensor memory and feeds dS; dX from the same pass.
 int dense_bwd_fused(const float* A, const float* S, const float* X, const float* Tt, const float* Gx, const float* Graw,
                     const float* Pm, int B, int N, int K, int F, const float* ew_S, const float* ew_d, const float* ew_coef,
-                    float eps, float* dS, float* dX, cudaStream_t stream);
+                    const float* ew_uv, float eps, float* dS, float* dX, cudaStream_t stream);
 }  // namespace tc
 }  // namespace tgp

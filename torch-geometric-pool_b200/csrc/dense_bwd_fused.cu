@@ -91,6 +91,7 @@ struct BwdParams {
   const float* S;      // element-wise terms (nullptr: none)
   const float* d;
   const float* coef;
+  const float* uv;     // [B, 2, K]: DMoN term d_i u_k + v_k of dS (nullptr: none)
   float eps;
   long long* dbg;
 };
@@ -336,7 +337,7 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
       // Element-wise gradient terms of dS (mincut denominator 2 c_den d_i S, entropy loss): this thread's row of S is
       // fetched NOW, asynchronously into shared memory, so that its latency sits behind the item's MMAs instead of in
       // the drain (loading it per chunk after the accumulators were ready cost 21 us of the 115 us kernel).
-      float dd = 0.f, c_ent = 0.f;
+      float dd = 0.f, c_ent = 0.f, di = 0.f;
       bool hook = false;
       const uint32_t hrow = hook0 + (uint32_t)(quad * 32 + lane) * (BNB * 4);
       if (!(TGPB200_ABL & 256) && P.S != nullptr && m < P.N) {
@@ -348,6 +349,7 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
           const float* srow = P.S + ((int64_t)b * P.N + m) * P.K;
           for (int j = 0; j * 4 < P.K; ++j) cp_async16(hrow + (uint32_t)((j ^ (lane & 7)) << 4), srow + j * 4);
         }
+        if (P.uv != nullptr) di = P.d[(int64_t)b * P.N + m];
       }
       cp_async_commit();
       mbar_wait(bar_tfull, (uint32_t)it & 1u);
@@ -382,6 +384,12 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
               }
             }
           }
+        }
+        if (is_ds && P.uv != nullptr) {  // DMoN: d_i u_k + v_k (per-graph vectors: every lane loads the same word)
+          const float* ub = P.uv + (int64_t)b * 2 * P.K + n0;
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (n0 + j < P.K) v[j] += fmaf(di, __ldg(ub + j), __ldg(ub + P.K + j));
         }
         // two staging tiles per warp: the store of the previous chunk may still be reading the other one
         const uint32_t stg = stg0 + (n_stored % kEpiBufs) * 4096u;
@@ -438,7 +446,7 @@ bool make_out_map(CUtensorMap* map, float* ptr, int64_t batch, int64_t rows, int
 // the one-product-per-launch chain.
 int dense_bwd_fused(const float* A, const float* S, const float* X, const float* Tt, const float* Gx, const float* Graw,
                     const float* Pm, int B, int N, int K, int F, const float* ew_S, const float* ew_d, const float* ew_coef,
-                    float eps, float* dS, float* dX, cudaStream_t stream) {
+                    const float* ew_uv, float eps, float* dS, float* dX, cudaStream_t stream) {
   {
     const char* e = getenv("TGPB200_BWD_FUSED");
     if (e && e[0] == '0') return TGPB200_ERR_UNSUPPORTED;
@@ -481,7 +489,7 @@ int dense_bwd_fused(const float* A, const float* S, const float* X, const float*
   if (!ok) return TGPB200_ERR_UNSUPPORTED;
   P.num_pairs = n;
   if (!make_out_map(&P.map_ds, dS, B, N, K) || !make_out_map(&P.map_dx, dX, B, N, F)) return TGPB200_ERR_UNSUPPORTED;
-  P.S = ew_S, P.d = ew_d, P.coef = ew_coef, P.eps = eps;
+  P.S = ew_S, P.d = ew_d, P.coef = ew_coef, P.uv = ew_S ? ew_uv : nullptr, P.eps = eps;
   P.stages = 5;
   {
     const char* e = getenv("TGPB200_BWD_STAGES");  // experiment: fewer shared-memory stages

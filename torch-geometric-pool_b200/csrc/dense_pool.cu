@@ -347,7 +347,7 @@ __device__ __forceinline__ void strip_sums4(int K, int r0, int r1, float* colred
 // ------------------------------------------------------------------------------------------
 // Per-graph epilogue (one cluster per graph): loss statistics from the RAW S^T A S and S^T S,
 // then post-processing (diag zero -> D^-1/2 A D^-1/2 -> / max|A|) exactly in ops.py:307-333 order.
-// stats[b] = {num, den, ||M||_F^2, ortho_b, ||A||_F^2, ent_b, maxnorm m, unused}
+// stats[b] = {num, den, ||M||_F^2, ortho_b, ||A||_F^2, ent_b, maxnorm m, 2m (DMoN only: k_dmon_stats)}
 // ------------------------------------------------------------------------------------------
 template <typename T, int V, bool STAGED>
 static __global__ void __launch_bounds__(512)
@@ -630,12 +630,84 @@ static __global__ void k_link_fix(const float* __restrict__ partial, int64_t n, 
   }
 }
 
+// DMoN statistics of graph b = blockIdx.x, one block per graph, fixed reduction order (no atomics):
+//   c = S^T d, e = S^T 1 (cvec / evec [B, K]), 2m = sum_i d_i with d = A 1 (k_row_stats / the fused forward),
+//   dst[b] = {2m, ||c||^2, ||e||^2, spectral_b, cluster_b, 0, 0, 0}, and stats[b][7] = 2m for k_graph_bwd.
+//   spectral_b = -(t - ||c||^2 / 2m) / 2m with t = tr(S^T A S) raw (stats[b][0]);  cluster_b = ||e|| sqrt(K) / n_b - 1.
+template <typename T>
+static __global__ void __launch_bounds__(256)
+    k_dmon_stats(const T* __restrict__ S, const float* __restrict__ d, const float* __restrict__ graph_nodes, int N,
+                 int K, float* __restrict__ stats, float* __restrict__ cvec, float* __restrict__ evec,
+                 float* __restrict__ dst) {
+  __shared__ float red[32];
+  __shared__ float colc[8][33], cole[8][33];
+  const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, w = t >> 5, nw = blockDim.x >> 5;
+  const T* Sb = S + (int64_t)b * N * K;
+  const float* db = d + (int64_t)b * N;
+  float cc = 0.f, ee = 0.f;
+  for (int c0 = 0; c0 < K; c0 += 32) {  // lane = column, warps stride over the rows (128-byte row segments)
+    const int k = c0 + lane;
+    float ac = 0.f, ae = 0.f;
+    if (k < K) {
+#pragma unroll 4
+      for (int i = w; i < N; i += nw) {
+        const float s = to_f32<T>(Sb[(int64_t)i * K + k]);
+        ac = fmaf(db[i], s, ac);
+        ae += s;
+      }
+    }
+    colc[w][lane] = ac, cole[w][lane] = ae;
+    __syncthreads();
+    if (w == 0 && k < K) {
+      float sc = 0.f, se = 0.f;
+      for (int q = 0; q < nw; ++q) sc += colc[q][lane], se += cole[q][lane];
+      cvec[(int64_t)b * K + k] = sc, evec[(int64_t)b * K + k] = se;
+      cc = fmaf(sc, sc, cc), ee = fmaf(se, se, ee);
+    }
+    __syncthreads();
+  }
+  float m = 0.f;
+  for (int i = t; i < N; i += blockDim.x) m += db[i];
+  m = block_sum(m, red);
+  cc = block_sum(cc, red);
+  ee = block_sum(ee, red);
+  if (t == 0) {
+    const float n = graph_nodes ? graph_nodes[b] : (float)N;
+    float* o = dst + (int64_t)b * 8;
+    o[0] = m, o[1] = cc, o[2] = ee;
+    o[3] = -(stats[(int64_t)b * 8 + 0] - cc / m) / m;  // 2m = 0 gives NaN, as the restated formula does
+    o[4] = sqrtf(ee) * sqrtf((float)K) / n - 1.f;
+    o[5] = o[6] = o[7] = 0.f;
+    stats[(int64_t)b * 8 + 7] = m;
+  }
+}
+
+// losses[0..3] = {spectral, ortho, cluster, 0} (means over the batch) for loss_kind 3; one block, fixed order.
+static __global__ void k_finalize_dmon(const float* __restrict__ stats, const float* __restrict__ dst, int B,
+                                       float* __restrict__ losses) {
+  __shared__ float red[32];
+  float spec = 0.f, ortho = 0.f, clus = 0.f;
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    spec += dst[(int64_t)b * 8 + 3];
+    ortho += stats[(int64_t)b * 8 + 3];
+    clus += dst[(int64_t)b * 8 + 4];
+  }
+  spec = block_sum(spec, red), ortho = block_sum(ortho, red), clus = block_sum(clus, red);
+  if (threadIdx.x == 0) {
+    losses[0] = spec / (float)B;
+    losses[1] = ortho / (float)B;
+    losses[2] = clus / (float)B;
+    losses[3] = 0.f, losses[4] = 0.f, losses[5] = 0.f;
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // Backward assembly (one cluster per graph, row strips as in the epilogue):
 //   Graw = d L / d (S^T A S) raw   from  Gpool (through max-norm, degree-norm, diag-zero) + trace terms
 //   P    = d L / d (S^T S) symmetrised:  dS += S P        (ortho + link ||M||^2 term)
 //   coef[b] = {c_den, c_a2, c_ent}  for the element-wise terms
-// gl = upstream grads of {cut, ortho, link, entropy} (device floats, already x coefficient).
+// gl = upstream grads of {cut, ortho, link, entropy} (device floats, already x coefficient); for loss_kind 3 (DMoN)
+// {spectral, ortho, cluster, -}: c_num and P here, the rest of the DMoN gradient in k_dmon_bwd.
 // ------------------------------------------------------------------------------------------
 template <typename T, int V, bool STAGED>
 static __global__ void __launch_bounds__(512)
@@ -704,6 +776,8 @@ static __global__ void __launch_bounds__(512)
     float cq = L > 0.f ? g_link / (2.f * L * link_div) : 0.f;  // dL/dq
     c_a2 = cq, c_num = -2.f * cq, c_m2 = cq;
     c_ent = g_ent / ent_div;
+  } else if (loss_kind == 3) {  // DMoN spectral loss through t = tr(S^T A S): -gamma / 2m on the diagonal
+    c_num = -g_cut / ((float)B * st[7]);
   }
   if (t == 0 && cl.rank == 0) {
     coef[b * 4 + 0] = c_den, coef[b * 4 + 1] = c_a2, coef[b * 4 + 2] = c_ent, coef[b * 4 + 3] = 0.f;
@@ -716,7 +790,7 @@ static __global__ void __launch_bounds__(512)
 
   // --- P = dL/dM + transpose  (M symmetric so both terms are symmetric)
   if (P && hasM) {
-    if (loss_kind == 1) {
+    if (loss_kind == 1 || loss_kind == 3) {  // orthogonality loss (MinCut and DMoN)
       const float nM = sqrtf(st[2]), rr = st[3], isk = 1.0f / sqrtf((float)K), inM = 1.0f / nM;
       // With U = M/nM - I/sqrt(K) and r = ||U||:  <U, M> = nM * <U, M/nM> = nM * r^2 / 2  (no extra reduction,
       // and no cancellation near perfect orthogonality).
@@ -861,21 +935,62 @@ static __global__ void __launch_bounds__(512)
   cl.sync();  // no CTA may retire while a peer can still read its shared memory
 }
 
-// dS += element-wise terms:  c_den * 2 d_i S_ik  +  c_ent * (-log(S+eps) - S/(S+eps)).
+// The rest of the DMoN gradient for graph b = blockIdx.x (one block per graph; gl = {g_s, g_o, g_c, -}, gamma = g_s / B):
+//   uv[b] = {u [K], v [K]}:  dS_ik += d_i u_k + v_k,  u = 2 gamma c / (2m)^2,  v = (g_c / B) sqrt(K) e / (n_b ||e||)
+//   rvec[b, i] (when dA is wanted):  dA_ij += r_i = gamma (2 (S c)_i / (2m)^2 + t / (2m)^2 - 2 ||c||^2 / (2m)^3)
+//   coef_r[b] = {1, 0, 0, 0}: k_da_elementwise then adds the row broadcast r_i (it reads r in place of ss).
+template <typename T>
+static __global__ void __launch_bounds__(256)
+    k_dmon_bwd(const T* __restrict__ S, const float* __restrict__ stats, const float* __restrict__ cvec,
+               const float* __restrict__ evec, const float* __restrict__ dst, const float* __restrict__ graph_nodes,
+               const float* __restrict__ gl, int B, int N, int K, float* __restrict__ uv, float* __restrict__ rvec,
+               float* __restrict__ coef_r) {
+  const int b = blockIdx.x, t = threadIdx.x;
+  const float* cb = cvec + (int64_t)b * K;
+  const float* ds = dst + (int64_t)b * 8;
+  const float m = ds[0], cc = ds[1], ne = sqrtf(ds[2]), tr = stats[(int64_t)b * 8 + 0];
+  const float gamma = gl ? gl[0] / (float)B : 0.f, gc = gl ? gl[2] / (float)B : 0.f;
+  const float n = graph_nodes ? graph_nodes[b] : (float)N;
+  const float im = 1.f / m, cu = 2.f * gamma * im * im;
+  const float cv = ne > 0.f ? gc * sqrtf((float)K) / (n * ne) : 0.f;
+  float* ub = uv + (int64_t)b * 2 * K;
+  for (int k = t; k < K; k += blockDim.x) {
+    ub[k] = cu * cb[k];
+    ub[K + k] = cv * evec[(int64_t)b * K + k];
+  }
+  if (t == 0) coef_r[b * 4 + 0] = 1.f, coef_r[b * 4 + 1] = 0.f, coef_r[b * 4 + 2] = 0.f, coef_r[b * 4 + 3] = 0.f;
+  if (!rvec) return;
+  const float r0 = gamma * (tr * im * im - 2.f * cc * im * im * im);
+  const int lane = t & 31, w = t >> 5, nw = blockDim.x >> 5;
+  const T* Sb = S + (int64_t)b * N * K;
+  for (int i = w; i < N; i += nw) {  // one warp per row: (S c)_i
+    float sc = 0.f;
+    for (int k = lane; k < K; k += 32) sc = fmaf(to_f32<T>(Sb[(int64_t)i * K + k]), cb[k], sc);
+    sc = warp_sum(sc);
+    if (lane == 0) rvec[(int64_t)b * N + i] = fmaf(cu, sc, r0);
+  }
+}
+
+// dS += element-wise terms:  c_den * 2 d_i S_ik  +  c_ent * (-log(S+eps) - S/(S+eps))  [+ d_i u_k + v_k, uv: DMoN].
 template <typename T>
 static __global__ void k_ds_elementwise(const T* __restrict__ S, const float* __restrict__ d,
-                                        const float* __restrict__ coef, int64_t total, int N, int K, float eps,
-                                        T* __restrict__ dS) {
+                                        const float* __restrict__ coef, const float* __restrict__ uv, int64_t total,
+                                        int N, int K, float eps, T* __restrict__ dS) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   int64_t row = i / K;
   int b = (int)(row / N);
   float c_den = coef[b * 4 + 0], c_ent = coef[b * 4 + 2];
-  if (c_den == 0.f && c_ent == 0.f) return;
+  if (c_den == 0.f && c_ent == 0.f && !uv) return;
   float s = to_f32<T>(S[i]);
   float v = to_f32<T>(dS[i]);
   if (c_den != 0.f) v += c_den * 2.f * d[row] * s;
   if (c_ent != 0.f) v += c_ent * (-logf(s + eps) - s / (s + eps));
+  if (uv) {
+    const int k = (int)(i - row * K);
+    const float* ub = uv + (int64_t)b * 2 * K;
+    v += fmaf(d[row], ub[k], ub[K + k]);
+  }
   dS[i] = from_f32<T>(v);
 }
 
@@ -1028,7 +1143,8 @@ static StripPlan strip_plan(int K, int nvec, int nstrips, int64_t elems_for_512 
 template <typename T>
 struct DensePlan {
   T* Tt;  // T = S^T A  [B, K, N]
-  float *Araw, *M, *d, *ss, *a2, *ent, *dvec, *stats, *losses;
+  float *Araw, *M, *d, *ss, *a2, *ent, *dvec, *stats, *losses, *link_partial;
+  float *dm_c, *dm_e, *dm_st;  // DMoN: c = S^T d, e = S^T 1 [B, K], per-graph terms [B, 8] (k_dmon_stats)
   int32_t* argmax;
   bool ok;
   DensePlan(Workspace& ws, int64_t B, int64_t N, int64_t K) {
@@ -1043,6 +1159,10 @@ struct DensePlan {
     stats = ws.take<float>((size_t)B * 8);
     losses = ws.take<float>(8);
     argmax = ws.take<int32_t>((size_t)B);
+    link_partial = ws.take<float>((size_t)B * ((N + 63) / 64) * ((N + 63) / 64));
+    dm_c = ws.take<float>((size_t)B * K);
+    dm_e = ws.take<float>((size_t)B * K);
+    dm_st = ws.take<float>((size_t)B * 8);
     ok = ws.ok;
   }
 };
@@ -1051,16 +1171,16 @@ static size_t dense_saved_bytes(int64_t B, int64_t N, int64_t K) {
   size_t f = sizeof(float);
   return align_up((size_t)B * K * N * f) + align_up((size_t)B * K * K * f) * 2 + align_up((size_t)B * N * f) * 4 +
          align_up((size_t)B * K * f) + align_up((size_t)B * 8 * f) + align_up(8 * f) + align_up((size_t)B * 4) +
-         align_up((size_t)B * ((N + 63) / 64) * ((N + 63) / 64) * f) + 4096;
+         align_up((size_t)B * ((N + 63) / 64) * ((N + 63) / 64) * f) + align_up((size_t)B * K * f) * 2 +
+         align_up((size_t)B * 8 * f) + 4096;
 }
 
 template <typename T>
 static int dense_fwd(const T* A, const T* S, const T* X, int B, int N, int K, int F, uint32_t flags, int loss_kind,
-                     float eps, float link_div, float ent_div, T* Xpool, T* Apool, float* losses_out, Workspace& saved,
-                     cudaStream_t st) {
+                     float eps, float link_div, float ent_div, const float* graph_nodes, T* Xpool, T* Apool,
+                     float* losses_out, Workspace& saved, cudaStream_t st) {
   DensePlan<T> pl(saved, B, N, K);
-  float* link_partial = saved.take<float>((size_t)B * ((N + 63) / 64) * ((N + 63) / 64));
-  if (!pl.ok || !saved.ok) return TGPB200_ERR_WORKSPACE;
+  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
   int rc;
   int64_t NK = (int64_t)N * K, NN = (int64_t)N * N, NF = (int64_t)N * F, KK = (int64_t)K * K, KF = (int64_t)K * F;
   const Mat Smn{S, NK, K, 1};  // S read with the node index as the contraction dim
@@ -1125,15 +1245,21 @@ static int dense_fwd(const T* A, const T* S, const T* X, int B, int N, int K, in
                    N, K, flags, eps, Apool, pl.dvec, pl.stats, pl.argmax, sp.rows_per, sp.rowp_floats);
     // fp32: the identity holds rtol 1e-5 down to q ~ 0.05 ||A||^2; bf16 (T stored in bf16, rtol 2e-2) down to 0.25
     const float link_tau = (loss_kind == 2 && A) ? (std::is_same<T, float>::value ? 0.05f : 0.25f) : 0.f;
-    launch("k_finalize_losses", k_finalize_losses, 1, 256, 0, st, pl.stats, B, eps, link_div, ent_div, link_tau,
-           pl.losses);
+    if (loss_kind == 3) {
+      launch("k_dmon_stats", k_dmon_stats<T>, (unsigned)B, 256, 0, st, S, pl.d, graph_nodes, N, K, pl.stats, pl.dm_c,
+             pl.dm_e, pl.dm_st);
+      launch("k_finalize_dmon", k_finalize_dmon, 1, 256, 0, st, pl.stats, pl.dm_st, B, pl.losses);
+    } else {
+      launch("k_finalize_losses", k_finalize_losses, 1, 256, 0, st, pl.stats, B, eps, link_div, ent_div, link_tau,
+             pl.losses);
+    }
     if (link_tau > 0.f) {
       const int tn = (N + 63) / 64;
       const int64_t total = (int64_t)tn * tn * B;
       const int64_t cap = (int64_t)tc::device_sm_count() * 8;
       launch("k_link_residual", k_link_residual<T>, (unsigned)(total < cap ? total : cap), 256, 0, st, A, S, N, K, tn, total,
-             pl.losses, link_partial);
-      launch("k_link_fix", k_link_fix, 1, 1024, 0, st, link_partial, (int64_t)B * tn * tn, link_div, pl.losses);
+             pl.losses, pl.link_partial);
+      launch("k_link_fix", k_link_fix, 1, 1024, 0, st, pl.link_partial, (int64_t)B * tn * tn, link_div, pl.losses);
     }
     if (losses_out) cudaMemcpyAsync(losses_out, pl.losses, 4 * sizeof(float), cudaMemcpyDeviceToDevice, st);
   }
@@ -1143,7 +1269,8 @@ static int dense_fwd(const T* A, const T* S, const T* X, int B, int N, int K, in
 template <typename T>
 static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const T* gApool, const float* gl, int B,
                      int N, int K, int F, uint32_t flags, int loss_kind, float eps, float link_div, float ent_div,
-                     T* dS_out, T* dX_out, T* dA_out, Workspace& saved, Workspace& ws, cudaStream_t st) {
+                     const float* graph_nodes, T* dS_out, T* dX_out, T* dA_out, Workspace& saved, Workspace& ws,
+                     cudaStream_t st) {
   DensePlan<T> pl(saved, B, N, K);
   if (!pl.ok) return TGPB200_ERR_WORKSPACE;
   int64_t NK = (int64_t)N * K, NN = (int64_t)N * N, NF = (int64_t)N * F, KK = (int64_t)K * K, KF = (int64_t)K * F;
@@ -1154,11 +1281,19 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
   T* U = ws.take<T>((size_t)B * NK);
   T* Gt = ws.take<T>((size_t)B * KK);  // Graw / P in the operand dtype (bf16 runs)
   T* Pt = ws.take<T>((size_t)B * KK);
+  float* uv = ws.take<float>((size_t)B * 2 * K);  // DMoN (k_dmon_bwd)
+  float* rvec = ws.take<float>((size_t)B * N);
+  float* coef_r = ws.take<float>((size_t)B * 4);
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   int rc;
   if (B == 0) return TGPB200_OK;
   const bool have_a = A != nullptr;
   const bool f32 = std::is_same<T, float>::value;
+  const bool dmon = loss_kind == 3 && have_a;
+  if (!dmon) uv = nullptr;
+  else
+    launch("k_dmon_bwd", k_dmon_bwd<T>, (unsigned)B, 256, 0, st, S, pl.stats, pl.dm_c, pl.dm_e,
+           pl.dm_st, graph_nodes, gl, B, N, K, uv, dA_out ? rvec : (float*)nullptr, coef_r);
   if (have_a) {
     const StripPlan sp = strip_plan(K, 4, 3);
     const bool v4 = K % 4 == 0 && aligned16(gApool);
@@ -1181,7 +1316,7 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
       // one launch: W = A S in tensor memory -> dS (all four products + element-wise terms) and dX
       const bool ew = loss_kind != 0;
       rc = tc::dense_bwd_fused(A, S, X, pl.Tt, gXpool, Graw, loss_kind != 0 ? P : (float*)nullptr, B, N, K, F,
-                               ew ? S : (const float*)nullptr, pl.d, coef, eps, dS_out, dX_out, st);
+                               ew ? S : (const float*)nullptr, pl.d, coef, uv, eps, dS_out, dX_out, st);
       if (rc == TGPB200_OK) fused_bwd = true;
       else if (rc != TGPB200_ERR_UNSUPPORTED) return rc;
     }
@@ -1210,7 +1345,9 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
     }
     if (n > 0) {
       EwHook hook;
-      if (have_a && loss_kind != 0) {
+      // DMoN's d_i u_k + v_k is left to k_ds_elementwise: carried in the engine's epilogue it cost the MinCut
+      // products of k_tc_gemm / k_tc_gemm_pair extra register spills
+      if (have_a && loss_kind != 0 && !dmon) {
         hook.S = S, hook.d = pl.d, hook.coef = coef, hook.eps = eps, hook.applied = &ew_done;
       }
       rc = mm<T, T>(B, N, K, n, kd, a, b, dS_out, NK, K, 1, st, hook, "k_tc_gemm:dS");
@@ -1221,7 +1358,7 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
   }
   if (have_a && loss_kind != 0 && !ew_done)
     launch("k_ds_elementwise", k_ds_elementwise<T>, (unsigned)ceil_div((int64_t)B * NK, 256), 256, 0, st, S, pl.d, coef,
-           (int64_t)B * NK, N, K, eps, dS_out);
+           (const float*)uv, (int64_t)B * NK, N, K, eps, dS_out);
   }  // !fused_bwd
   if (have_a && dA_out) {  // dA = (S Graw) S^T + element-wise terms
     rc = mm1<T, T>(B, N, K, K, Mat{S, NK, K, 0}, Mat{Gt, KK, K, 1}, U, NK, K, 1, st, "k_tc_gemm:U=SG");
@@ -1229,13 +1366,16 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
     rc = mm1<T, T>(B, N, N, K, Mat{U, NK, K, 0}, Mat{S, NK, K, 0}, dA_out, NN, N, 1, st, "k_tc_gemm:dA=USt");
     if (rc) return rc;
     if (loss_kind != 0) {
+      // MinCut: c_den * ss_i; DMoN: the row term r_i of k_dmon_bwd (coef_r = {1, 0, ..})
+      const float* row_term = dmon ? rvec : pl.ss;
+      const float* row_coef = dmon ? coef_r : coef;
       constexpr int V = 16 / sizeof(T);
       if (N % V == 0 && aligned16(A) && aligned16(dA_out))
         launch("k_da_elementwise", k_da_elementwise_vec<T>, (unsigned)ceil_div((int64_t)B * NN / V, 256), 256, 0, st, A,
-               pl.ss, coef, (int64_t)B * NN / V, N, dA_out);
+               row_term, row_coef, (int64_t)B * NN / V, N, dA_out);
       else
-        launch("k_da_elementwise", k_da_elementwise<T>, (unsigned)ceil_div((int64_t)B * NN, 256), 256, 0, st, A, pl.ss,
-               coef, (int64_t)B * NN, N, dA_out);
+        launch("k_da_elementwise", k_da_elementwise<T>, (unsigned)ceil_div((int64_t)B * NN, 256), 256, 0, st, A,
+               row_term, row_coef, (int64_t)B * NN, N, dA_out);
     }
   }
   return launch_status();
@@ -1252,7 +1392,8 @@ size_t tgpb200_dense_pool_saved_bytes(int64_t B, int64_t N, int64_t K) { return 
 size_t tgpb200_dense_pool_bwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int need_grad_adj) {
   size_t f = sizeof(float);
   (void)need_grad_adj;
-  return 4 * align_up((size_t)B * K * K * f) + align_up((size_t)B * 4 * f) + 2 * align_up((size_t)B * N * K * f) + 8192;
+  return 4 * align_up((size_t)B * K * K * f) + align_up((size_t)B * 4 * f) + 2 * align_up((size_t)B * N * K * f) +
+         align_up((size_t)B * 2 * K * f) + align_up((size_t)B * N * f) + align_up((size_t)B * 4 * f) + 8192;
 }
 
 // Batched product with the shape-general fallback (tensor-core engine when the operand layout satisfies the TMA
@@ -1278,23 +1419,56 @@ int tgpb200_bmm(const void* a, const void* b, void* out, int64_t batch, int64_t 
   return TGPB200_ERR_UNSUPPORTED;
 }
 
-int tgpb200_dense_pool_fwd(const void* adj, const void* s, const void* x, int64_t B, int64_t N, int64_t K, int64_t F,
-                           int dtype, uint32_t flags, int loss_kind, float eps, float link_div, float ent_div,
-                           void* x_pool, void* adj_pool, float* losses, void* saved, size_t saved_bytes,
-                           tgpb200_stream_t stream) {
+int tgpb200_dense_pool_fwd_v2(const void* adj, const void* s, const void* x, int64_t B, int64_t N, int64_t K,
+                              int64_t F, int dtype, uint32_t flags, int loss_kind, float eps, float link_div,
+                              float ent_div, void* x_pool, void* adj_pool, float* losses, void* saved,
+                              size_t saved_bytes, tgpb200_stream_t stream, const float* graph_nodes) {
   if (B < 0 || N < 0 || K < 0 || F < 0 || !s || !saved) return TGPB200_ERR_INVALID;
   if (B >= INT32_MAX || N >= 65536 || K >= 32768 || F >= INT32_MAX) return TGPB200_ERR_UNSUPPORTED;
-  if (loss_kind < 0 || loss_kind > 2 || (loss_kind != 0 && !adj)) return TGPB200_ERR_INVALID;
+  if (loss_kind < 0 || loss_kind > 3 || (loss_kind != 0 && !adj)) return TGPB200_ERR_INVALID;
   if (adj && !adj_pool) return TGPB200_ERR_INVALID;
   Workspace sv(saved, saved_bytes);
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == TGPB200_F32)
     return dense_fwd<float>((const float*)adj, (const float*)s, (const float*)x, (int)B, (int)N, (int)K, (int)F, flags,
-                            loss_kind, eps, link_div, ent_div, (float*)x_pool, (float*)adj_pool, losses, sv, st);
+                            loss_kind, eps, link_div, ent_div, graph_nodes, (float*)x_pool, (float*)adj_pool, losses,
+                            sv, st);
   if (dtype == TGPB200_BF16)
     return dense_fwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, (const __nv_bfloat16*)x, (int)B,
-                                    (int)N, (int)K, (int)F, flags, loss_kind, eps, link_div, ent_div,
+                                    (int)N, (int)K, (int)F, flags, loss_kind, eps, link_div, ent_div, graph_nodes,
                                     (__nv_bfloat16*)x_pool, (__nv_bfloat16*)adj_pool, losses, sv, st);
+  return TGPB200_ERR_UNSUPPORTED;
+}
+
+int tgpb200_dense_pool_fwd(const void* adj, const void* s, const void* x, int64_t B, int64_t N, int64_t K, int64_t F,
+                           int dtype, uint32_t flags, int loss_kind, float eps, float link_div, float ent_div,
+                           void* x_pool, void* adj_pool, float* losses, void* saved, size_t saved_bytes,
+                           tgpb200_stream_t stream) {
+  return tgpb200_dense_pool_fwd_v2(adj, s, x, B, N, K, F, dtype, flags, loss_kind, eps, link_div, ent_div, x_pool,
+                                   adj_pool, losses, saved, saved_bytes, stream, nullptr);
+}
+
+int tgpb200_dense_pool_bwd_v2(const void* adj, const void* s, const void* x, const void* grad_x_pool,
+                              const void* grad_adj_pool, const float* grad_losses, int64_t B, int64_t N, int64_t K,
+                              int64_t F, int dtype, uint32_t flags, int loss_kind, float eps, float link_div,
+                              float ent_div, void* grad_s, void* grad_x, void* grad_adj, void* saved,
+                              size_t saved_bytes, void* workspace, size_t workspace_bytes, tgpb200_stream_t stream,
+                              const float* graph_nodes) {
+  if (B < 0 || N < 0 || K < 0 || F < 0 || !s || !saved) return TGPB200_ERR_INVALID;
+  if (loss_kind < 0 || loss_kind > 3) return TGPB200_ERR_INVALID;
+  Workspace sv(saved, saved_bytes), ws(workspace, workspace_bytes);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == TGPB200_F32)
+    return dense_bwd<float>((const float*)adj, (const float*)s, (const float*)x, (const float*)grad_x_pool,
+                            (const float*)grad_adj_pool, grad_losses, (int)B, (int)N, (int)K, (int)F, flags, loss_kind,
+                            eps, link_div, ent_div, graph_nodes, (float*)grad_s, (float*)grad_x, (float*)grad_adj, sv,
+                            ws, st);
+  if (dtype == TGPB200_BF16)
+    return dense_bwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, (const __nv_bfloat16*)x,
+                                    (const __nv_bfloat16*)grad_x_pool, (const __nv_bfloat16*)grad_adj_pool,
+                                    grad_losses, (int)B, (int)N, (int)K, (int)F, flags, loss_kind, eps, link_div,
+                                    ent_div, graph_nodes, (__nv_bfloat16*)grad_s, (__nv_bfloat16*)grad_x,
+                                    (__nv_bfloat16*)grad_adj, sv, ws, st);
   return TGPB200_ERR_UNSUPPORTED;
 }
 
@@ -1303,21 +1477,9 @@ int tgpb200_dense_pool_bwd(const void* adj, const void* s, const void* x, const 
                            int64_t F, int dtype, uint32_t flags, int loss_kind, float eps, float link_div,
                            float ent_div, void* grad_s, void* grad_x, void* grad_adj, void* saved, size_t saved_bytes,
                            void* workspace, size_t workspace_bytes, tgpb200_stream_t stream) {
-  if (B < 0 || N < 0 || K < 0 || F < 0 || !s || !saved) return TGPB200_ERR_INVALID;
-  if (loss_kind < 0 || loss_kind > 2) return TGPB200_ERR_INVALID;
-  Workspace sv(saved, saved_bytes), ws(workspace, workspace_bytes);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == TGPB200_F32)
-    return dense_bwd<float>((const float*)adj, (const float*)s, (const float*)x, (const float*)grad_x_pool,
-                            (const float*)grad_adj_pool, grad_losses, (int)B, (int)N, (int)K, (int)F, flags, loss_kind,
-                            eps, link_div, ent_div, (float*)grad_s, (float*)grad_x, (float*)grad_adj, sv, ws, st);
-  if (dtype == TGPB200_BF16)
-    return dense_bwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, (const __nv_bfloat16*)x,
-                                    (const __nv_bfloat16*)grad_x_pool, (const __nv_bfloat16*)grad_adj_pool,
-                                    grad_losses, (int)B, (int)N, (int)K, (int)F, flags, loss_kind, eps, link_div,
-                                    ent_div, (__nv_bfloat16*)grad_s, (__nv_bfloat16*)grad_x, (__nv_bfloat16*)grad_adj,
-                                    sv, ws, st);
-  return TGPB200_ERR_UNSUPPORTED;
+  return tgpb200_dense_pool_bwd_v2(adj, s, x, grad_x_pool, grad_adj_pool, grad_losses, B, N, K, F, dtype, flags,
+                                   loss_kind, eps, link_div, ent_div, grad_s, grad_x, grad_adj, saved, saved_bytes,
+                                   workspace, workspace_bytes, stream, nullptr);
 }
 
 }  // extern "C"

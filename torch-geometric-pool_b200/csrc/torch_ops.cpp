@@ -48,13 +48,24 @@ Tensor workspace(size_t bytes, const Tensor& like) {
 // (x_pool, adj_pool, losses[4], saved) = fused S^T X, postprocess(S^T A S), auxiliary losses
 // tgp/reduce/base_reduce.py:158-161, tgp/connect/dense_conn.py:112-138,257-271, tgp/utils/ops.py:282-335,
 // tgp/utils/losses.py:39-123,476-500,644-708
+// graph_nodes (optional): [B] float32 valid-node counts n_b on the device (DMoN's cluster loss); absent means N.
+const float* graph_nodes_ptr(const OptTensor& graph_nodes, int64_t B) {
+  if (!graph_nodes.has_value() || !graph_nodes->defined()) return nullptr;
+  require_cuda(*graph_nodes, "graph_nodes");
+  TORCH_CHECK(graph_nodes->scalar_type() == at::kFloat, "tgp_b200: graph_nodes must be float32");
+  TORCH_CHECK(graph_nodes->dim() == 1 && graph_nodes->size(0) == B, "tgp_b200: graph_nodes must have shape [B] = [", B,
+              "], got ", graph_nodes->sizes());
+  return B > 0 ? graph_nodes->data_ptr<float>() : nullptr;
+}
+
 std::tuple<Tensor, Tensor, Tensor, Tensor> stas_fused(const OptTensor& x, const OptTensor& adj, const Tensor& s,
                                                       int64_t flags, int64_t loss_kind, double link_div,
-                                                      double ent_div) {
+                                                      double ent_div, const OptTensor& graph_nodes) {
   require_cuda(s, "s");
   TORCH_CHECK(s.dim() == 3, "stas_fused expects s of shape [B, N, K]");
   c10::cuda::CUDAGuard guard(s.device());
   const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
+  const float* gn = graph_nodes_ptr(graph_nodes, B);
   const bool has_x = x.has_value() && x->defined(), has_a = adj.has_value() && adj->defined();
   if (has_x) require_cuda(*x, "x");
   if (has_a) require_cuda(*adj, "adj");
@@ -63,10 +74,10 @@ std::tuple<Tensor, Tensor, Tensor, Tensor> stas_fused(const OptTensor& x, const 
   Tensor x_pool = at::empty({has_x ? B : 0, K, F}, s.options());
   Tensor adj_pool = at::empty({has_a ? B : 0, K, K}, s.options());
   Tensor losses = at::zeros({4}, s.options().dtype(at::kFloat));
-  check(tgpb200_dense_pool_fwd(ptr(adj), s.data_ptr(), ptr(x), B, N, K, F, dtype_code(s), (uint32_t)flags,
-                               (int)loss_kind, 1e-8f, (float)link_div, (float)ent_div,
-                               has_x ? x_pool.data_ptr() : nullptr, has_a ? adj_pool.data_ptr() : nullptr,
-                               losses.data_ptr<float>(), saved.data_ptr(), (size_t)saved.numel(), stream_of(s)),
+  check(tgpb200_dense_pool_fwd_v2(ptr(adj), s.data_ptr(), ptr(x), B, N, K, F, dtype_code(s), (uint32_t)flags,
+                                  (int)loss_kind, 1e-8f, (float)link_div, (float)ent_div,
+                                  has_x ? x_pool.data_ptr() : nullptr, has_a ? adj_pool.data_ptr() : nullptr,
+                                  losses.data_ptr<float>(), saved.data_ptr(), (size_t)saved.numel(), stream_of(s), gn),
         "stas_fused");
   return {x_pool, adj_pool, losses, saved};
 }
@@ -74,9 +85,11 @@ std::tuple<Tensor, Tensor, Tensor, Tensor> stas_fused(const OptTensor& x, const 
 std::tuple<Tensor, Tensor, Tensor> stas_fused_bwd(const OptTensor& x, const OptTensor& adj, const Tensor& s,
                                                   const Tensor& saved, const OptTensor& gx_pool,
                                                   const OptTensor& gadj_pool, const OptTensor& glosses, int64_t flags,
-                                                  int64_t loss_kind, double link_div, double ent_div, bool need_gadj) {
+                                                  int64_t loss_kind, double link_div, double ent_div, bool need_gadj,
+                                                  const OptTensor& graph_nodes) {
   c10::cuda::CUDAGuard guard(s.device());
   const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
+  const float* gn = graph_nodes_ptr(graph_nodes, B);
   const bool has_x = x.has_value() && x->defined(), has_a = adj.has_value() && adj->defined();
   const int64_t F = has_x ? x->size(-1) : 0;
   const bool want_gx = has_x && gx_pool.has_value() && gx_pool->defined();
@@ -88,11 +101,12 @@ std::tuple<Tensor, Tensor, Tensor> stas_fused_bwd(const OptTensor& x, const OptT
   Tensor gxp = want_gx ? gx_pool->contiguous() : Tensor();
   Tensor gap = (has_a && gadj_pool.has_value() && gadj_pool->defined()) ? gadj_pool->contiguous() : Tensor();
   Tensor gl = (glosses.has_value() && glosses->defined()) ? glosses->to(at::kFloat).contiguous() : Tensor();
-  check(tgpb200_dense_pool_bwd(ptr(adj), s.data_ptr(), ptr(x), ptr(gxp), ptr(gap),
-                               gl.defined() ? gl.data_ptr<float>() : nullptr, B, N, K, F, dtype_code(s), (uint32_t)flags,
-                               (int)loss_kind, 1e-8f, (float)link_div, (float)ent_div, gs.data_ptr(),
-                               want_gx ? gx.data_ptr() : nullptr, want_ga ? ga.data_ptr() : nullptr,
-                               saved.data_ptr(), (size_t)saved.numel(), ws.data_ptr(), (size_t)ws.numel(), stream_of(s)),
+  check(tgpb200_dense_pool_bwd_v2(ptr(adj), s.data_ptr(), ptr(x), ptr(gxp), ptr(gap),
+                                  gl.defined() ? gl.data_ptr<float>() : nullptr, B, N, K, F, dtype_code(s),
+                                  (uint32_t)flags, (int)loss_kind, 1e-8f, (float)link_div, (float)ent_div, gs.data_ptr(),
+                                  want_gx ? gx.data_ptr() : nullptr, want_ga ? ga.data_ptr() : nullptr,
+                                  saved.data_ptr(), (size_t)saved.numel(), ws.data_ptr(), (size_t)ws.numel(),
+                                  stream_of(s), gn),
         "stas_fused_bwd");
   return {gx, ga, gs};
 }
@@ -155,11 +169,11 @@ std::tuple<Tensor, Tensor> segment_reduce_bwd(const Tensor& x, const Tensor& nod
 }  // namespace
 
 TORCH_LIBRARY(tgp_b200, m) {
-  m.def("stas_fused(Tensor? x, Tensor? adj, Tensor s, int flags, int loss_kind, float link_div, float ent_div) -> "
-        "(Tensor, Tensor, Tensor, Tensor)");
+  m.def("stas_fused(Tensor? x, Tensor? adj, Tensor s, int flags, int loss_kind, float link_div, float ent_div, "
+        "Tensor? graph_nodes=None) -> (Tensor, Tensor, Tensor, Tensor)");
   m.def("stas_fused_bwd(Tensor? x, Tensor? adj, Tensor s, Tensor saved, Tensor? gx_pool, Tensor? gadj_pool, "
-        "Tensor? glosses, int flags, int loss_kind, float link_div, float ent_div, bool need_gadj) -> "
-        "(Tensor, Tensor, Tensor)");
+        "Tensor? glosses, int flags, int loss_kind, float link_div, float ent_div, bool need_gadj, "
+        "Tensor? graph_nodes=None) -> (Tensor, Tensor, Tensor)");
   m.def("build_csr(Tensor cluster_index, int num_clusters) -> (Tensor, Tensor)");
   m.def("segment_reduce(Tensor x, Tensor node_index, Tensor cluster_index, Tensor? weight, Tensor order, Tensor ptr, "
         "int num_clusters, int op) -> Tensor");

@@ -92,6 +92,15 @@ SIGNATURES = {
         _INT,
         [_P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _INT, _U32, _INT, _F, _F, _F, _P, _P, _P, _P, _SZ, _P, _SZ, _P],
     ),
+    "tgpb200_dense_pool_fwd_v2": (
+        _INT,
+        [_P, _P, _P, _I64, _I64, _I64, _I64, _INT, _U32, _INT, _F, _F, _F, _P, _P, _P, _P, _SZ, _P, _P],
+    ),
+    "tgpb200_dense_pool_bwd_v2": (
+        _INT,
+        [_P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _INT, _U32, _INT, _F, _F, _F, _P, _P, _P, _P, _SZ, _P, _SZ, _P,
+         _P],
+    ),
 }
 
 

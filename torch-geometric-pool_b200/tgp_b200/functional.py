@@ -297,7 +297,7 @@ def sparse_connect_padded(
 # --------------------------------------------------------------------------- #
 # Dense reduce + connect + losses
 # --------------------------------------------------------------------------- #
-LOSS_NONE, LOSS_MINCUT, LOSS_DIFFPOOL = 0, 1, 2
+LOSS_NONE, LOSS_MINCUT, LOSS_DIFFPOOL, LOSS_DMON = 0, 1, 2, 3
 
 
 def dense_flags(remove_self_loops: bool, degree_norm: bool, adj_transpose: bool, edge_weight_norm: bool) -> int:
@@ -321,21 +321,31 @@ def dense_pool(
     loss_kind: int = LOSS_NONE,
     link_div: float = 1.0,
     ent_div: float = 1.0,
+    graph_nodes: Optional[Tensor] = None,
 ):
     """Fused ``(S^T X, postprocess(S^T A S), losses[4])`` for batched dense inputs.
 
-    ``losses`` = ``[mincut, ortho, link, entropy]`` (unused entries are 0).
+    ``losses`` = ``[mincut, ortho, link, entropy]`` (unused entries are 0); with ``loss_kind=LOSS_DMON`` it is
+    ``[spectral, ortho, cluster, 0]``.  ``graph_nodes`` ([B], on the device): the number of valid nodes of each graph,
+    which DMoN's cluster loss divides by (``None``: every graph has N nodes).
     """
-    _require_cuda(x, adj, s)
+    _require_cuda(x, adj, s, graph_nodes)
     if s.dim() != 3:
         raise ValueError("dense_pool expects s of shape [B, N, K]")
+    if loss_kind == LOSS_DMON and adj is None:
+        raise ValueError("dense_pool: the DMoN losses need adj")
+    if graph_nodes is not None:
+        if graph_nodes.shape != (s.size(0),):
+            raise ValueError(f"dense_pool: graph_nodes must have shape [B] = [{s.size(0)}], got {list(graph_nodes.shape)}")
+        graph_nodes = graph_nodes.to(torch.float32).contiguous()
     s = s.contiguous()
     x = None if x is None else x.contiguous()
     adj = None if adj is None else adj.contiguous()
     if x is not None and x.dtype != s.dtype or adj is not None and adj.dtype != s.dtype:
         raise RuntimeError("tgp_b200.dense_pool: x, adj and s must share one dtype")
     flags = dense_flags(remove_self_loops, degree_norm, adj_transpose, edge_weight_norm)
-    x_pool, adj_pool, losses, _ = _T.stas_fused(x, adj, s, flags, loss_kind, float(link_div), float(ent_div))
+    x_pool, adj_pool, losses, _ = _T.stas_fused(x, adj, s, flags, loss_kind, float(link_div), float(ent_div),
+                                                graph_nodes)
     return (x_pool if x is not None else None), (adj_pool if adj is not None else None), losses
 
 

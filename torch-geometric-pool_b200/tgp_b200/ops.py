@@ -43,7 +43,7 @@ _T = torch.ops.tgp_b200
 # stas_fused: (x_pool, adj_pool, losses[4], saved) = fused S^T X, postprocess(S^T A S), auxiliary losses
 # --------------------------------------------------------------------------------------------------------------
 @torch.library.register_fake("tgp_b200::stas_fused")
-def _stas_fused_fake(x, adj, s, flags, loss_kind, link_div, ent_div):
+def _stas_fused_fake(x, adj, s, flags, loss_kind, link_div, ent_div, graph_nodes=None):
     B, N, K = s.shape
     F = x.size(-1) if x is not None else 0
     saved = L.load().tgpb200_dense_pool_saved_bytes(B, N, K)
@@ -52,24 +52,27 @@ def _stas_fused_fake(x, adj, s, flags, loss_kind, link_div, ent_div):
 
 
 @torch.library.register_fake("tgp_b200::stas_fused_bwd")
-def _stas_fused_bwd_fake(x, adj, s, saved, gx_pool, gadj_pool, glosses, flags, loss_kind, link_div, ent_div, need_gadj):
+def _stas_fused_bwd_fake(x, adj, s, saved, gx_pool, gadj_pool, glosses, flags, loss_kind, link_div, ent_div, need_gadj,
+                         graph_nodes=None):
     gx = torch.empty_like(x) if x is not None else s.new_empty((0,))
     ga = torch.empty_like(adj) if (adj is not None and need_gadj) else s.new_empty((0,))
     return gx, ga, torch.empty_like(s)
 
 
 def _stas_setup(ctx, inputs, output):
-    x, adj, s, flags, loss_kind, link_div, ent_div = inputs
-    ctx.save_for_backward(x, adj, s, output[3])
+    x, adj, s, flags, loss_kind, link_div, ent_div, graph_nodes = inputs
+    ctx.save_for_backward(x, adj, s, output[3], graph_nodes)
     ctx.cfg = (flags, loss_kind, link_div, ent_div)
     ctx.set_materialize_grads(False)
 
 
 def _stas_backward(ctx, gx_pool, gadj_pool, glosses, _gsaved):
-    x, adj, s, saved = ctx.saved_tensors
+    x, adj, s, saved, graph_nodes = ctx.saved_tensors
     need_adj = adj is not None and ctx.needs_input_grad[1]
-    gx, ga, gs = _T.stas_fused_bwd(x, adj, s, saved, gx_pool, gadj_pool, glosses, *ctx.cfg, need_adj)
-    return (gx if x is not None else None), (ga if need_adj else None), gs, None, None, None, None
+    gx, ga, gs = _T.stas_fused_bwd(x, adj, s, saved, gx_pool, gadj_pool, glosses, *ctx.cfg, need_adj, graph_nodes)
+    # one entry per argument the call passed (the dispatcher drops trailing arguments left at their default)
+    rest = (None,) * (len(ctx.needs_input_grad) - 3)
+    return ((gx if x is not None else None), (ga if need_adj else None), gs) + rest
 
 
 torch.library.register_autograd("tgp_b200::stas_fused", _stas_backward, setup_context=_stas_setup)

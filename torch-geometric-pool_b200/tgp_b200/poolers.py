@@ -1,6 +1,6 @@
 """Pooler-level orchestration of the path (what the pooler ``forward``s do after ``select``).
 
-``mincut_pool`` / ``diff_pool`` run reduce + connect + auxiliary losses + post-processing as ONE
+``mincut_pool`` / ``diff_pool`` / ``dmon_pool`` run reduce + connect + auxiliary losses + post-processing as ONE
 fused forward and ONE fused backward; ``topk_pool`` / ``cluster_pool`` chain the sparse reduce and
 the sparse connect.  ``patch_pooler`` installs the B200 operators on a reference pooler object.
 """
@@ -58,6 +58,33 @@ def diff_pool(
         link_div=float(adj.numel()) if normalize_loss else 1.0, ent_div=float(num_nodes),
     )
     loss = {"link_loss": losses[2] * link_loss_coeff, "entropy_loss": losses[3] * ent_loss_coeff}
+    return x_pool, adj_pool, loss
+
+
+def dmon_pool(
+    x: Tensor,
+    adj: Tensor,
+    s: Tensor,
+    mask: Optional[Tensor] = None,
+    spectral_loss_coeff: float = 1.0,
+    cluster_loss_coeff: float = 1.0,
+    ortho_loss_coeff: float = 1.0,
+    remove_self_loops: bool = True,
+    degree_norm: bool = True,
+    adj_transpose: bool = True,
+    edge_weight_norm: bool = False,
+) -> Tuple[Tensor, Tensor, Dict[str, Tensor]]:
+    """DMoNPooling.forward batched path after select: ``S^T X``, ``postprocess(S^T A S)`` and the spectral, cluster
+    and orthogonality losses of PyG's ``DMoNPooling`` (restated in ``tests/dmon_oracle.py``), all from the raw product.
+    ``mask`` [B, N] gives the valid node count of each graph (the cluster loss divides by it); it stays on the device.
+    No activation is applied to the pooled features."""
+    graph_nodes = None if mask is None else mask.sum(1).to(torch.float32)
+    x_pool, adj_pool, losses = F_.dense_pool(
+        x, adj, s, remove_self_loops=remove_self_loops, degree_norm=degree_norm, adj_transpose=adj_transpose,
+        edge_weight_norm=edge_weight_norm, loss_kind=F_.LOSS_DMON, graph_nodes=graph_nodes,
+    )
+    loss = {"spectral_loss": losses[0] * spectral_loss_coeff, "cluster_loss": losses[2] * cluster_loss_coeff,
+            "ortho_loss": losses[1] * ortho_loss_coeff}
     return x_pool, adj_pool, loss
 
 
@@ -131,6 +158,7 @@ def _pooling_output_cls():
         return PoolingOutput
 
 
+_DMON_COEFFS = ("spectral_loss_coeff", "cluster_loss_coeff", "ortho_loss_coeff")
 _AGGR_TO_OP = {"SumAggregation": "sum", "MeanAggregation": "mean", "MaxAggregation": "max", "MinAggregation": "min"}
 
 
@@ -150,7 +178,7 @@ def _reduce_op_of(reducer) -> Optional[str]:
 
 
 def _fused_dense_forward(pooler, kind: str):
-    """``forward`` of a batched ``MinCutPooling`` / ``DiffPool`` (tgp/poolers/mincut.py:210-258,
+    """``forward`` of a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` (tgp/poolers/mincut.py:210-258,
     tgp/poolers/diffpool.py:200-237) with reduce + connect + auxiliary losses + post-processing as ONE fused
     forward / backward; select, input densification, lifting and the unbatched mode stay the reference's."""
     ref_forward = pooler.forward
@@ -169,6 +197,9 @@ def _fused_dense_forward(pooler, kind: str):
                      edge_weight_norm=c.edge_weight_norm)
         if kind == "mincut":
             x_pool, adj_pool, loss = mincut_pool(x, adj, so.s, pooler.cut_loss_coeff, pooler.ortho_loss_coeff, **flags)
+        elif kind == "dmon":
+            x_pool, adj_pool, loss = dmon_pool(x, adj, so.s, mask, pooler.spectral_loss_coeff, pooler.cluster_loss_coeff,
+                                               pooler.ortho_loss_coeff, **flags)
         else:
             x_pool, adj_pool, loss = diff_pool(x, adj, so.s, num_nodes=1, link_loss_coeff=pooler.link_loss_coeff,
                                                ent_loss_coeff=1.0, normalize_loss=pooler.normalize_loss, **flags)
@@ -191,9 +222,10 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
       same ctor attributes (the poolers read them, tgp/poolers/mincut.py:233-236);
     * ``pooler.reducer``: ``BaseReduce`` / ``AggrReduce(sum | mean | max | min)`` -> ``B200Reduce`` with the SAME
       reduction; any other reducer (learned / order-statistic aggregators) is left in place.  ``reduce_op`` overrides;
-    * ``fuse_dense``: a batched ``MinCutPooling`` / ``DiffPool`` also gets the fused forward (reduce + connect +
-      losses + post-processing in one kernel chain) -- without it the patched pooler still calls the reference's
-      torch loss functions.
+    * ``fuse_dense``: a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` also gets the fused forward
+      (reduce + connect + losses + post-processing in one kernel chain) -- without it the patched pooler still calls
+      the reference's torch loss functions.  A ``DMoNPooling`` lacking one of ``spectral_loss_coeff``,
+      ``cluster_loss_coeff``, ``ortho_loss_coeff`` keeps the reference forward.
     """
     for attr in ("connector", "preconnector"):
         conn = getattr(pooler, attr, None)
@@ -211,7 +243,9 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
         op = reduce_op if reduce_op is not None else _reduce_op_of(reducer)
         if op is not None:
             pooler.reducer = B200Reduce(op)
-    kind = {"MinCutPooling": "mincut", "DiffPool": "diff"}.get(type(pooler).__name__)
+    kind = {"MinCutPooling": "mincut", "DiffPool": "diff", "DMoNPooling": "dmon"}.get(type(pooler).__name__)
+    if kind == "dmon" and not all(hasattr(pooler, a) for a in _DMON_COEFFS):
+        kind = None
     if fuse_dense and kind is not None and type(getattr(pooler, "connector", None)).__name__ == "B200DenseConnect":
         pooler.forward = _fused_dense_forward(pooler, kind)
     return pooler
