@@ -2,7 +2,7 @@
 
     python benchmarks/per_graph_kernels.py [c2|c3l1]
 
-TGPB200_STRIP_ELEMS = matrix elements per CTA (the cluster size follows), TGPB200_STRIP_STAGE=0 disables staging.
+TGPB200_STRIP_ELEMS = matrix elements per CTA (the cluster size follows).
 """
 import os
 import sys
@@ -37,11 +37,9 @@ def main():
                                        loss_kind=kind, ent_div=float(B * N))
         torch.autograd.backward([xp, ap, losses], [g_xp, g_ap, g_l])
 
-    for elems, stage in [(8192, 1), (8192, 0), (16384, 1), (16384, 0), (32768, 1), (32768, 0), (1 << 20, 0), (2048, 1),
-                         (4096, 1)]:
+    for elems in [2048, 4096, 8192, 16384, 32768, 1 << 20]:
         os.environ["TGPB200_STRIP_ELEMS"] = str(elems)
-        os.environ["TGPB200_STRIP_STAGE"] = str(stage)
-        row = [f"elems={elems:8d} stage={stage}"]
+        row = [f"elems={elems:8d}"]
         for kern in ("k_graph_epilogue", "k_graph_bwd"):
             for _ in range(3):
                 step()

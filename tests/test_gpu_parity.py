@@ -437,17 +437,19 @@ def test_dense_pool_fp32_vs_oracle(B, N, K, F, kind):
         close32(g_, e_, f"{kind} {n_}", rtol=1e-5 if not n_.startswith("grad") else 1e-4)
 
 
-@pytest.mark.parametrize("elems,stage", [(64, 1), (128, 0), (32768, 1), (600, 0)])
+@pytest.mark.parametrize("elems,self_loops", [(64, 1), (128, 0), (32768, 1), (600, 0)])
 @pytest.mark.parametrize("K", [6, 12, 32, 128])
-def test_dense_per_graph_kernels_all_strip_plans(monkeypatch, elems, stage, K):
+def test_dense_per_graph_kernels_all_strip_plans(monkeypatch, elems, self_loops, K):
     """The per-graph epilogue / backward kernels run as clusters of row strips; every plan (cluster size 1..8,
-    staged or not, scalar / 128-bit paths) must give the same answer as the float64 oracle for every flag set."""
+    scalar / 128-bit paths) must give the same answer as the float64 oracle for every flag set, with and without
+    weighted self loops in the input adjacency."""
     monkeypatch.setenv("TGPB200_STRIP_ELEMS", str(elems))
-    monkeypatch.setenv("TGPB200_STRIP_STAGE", str(stage))
     B, N, F = 3, 160, 32
     g = torch.Generator().manual_seed(1000 + K)
     a, s_raw, x = _dense_inputs(g, B, N, K, F)
-    a = a + torch.diag_embed(torch.rand(B, N, generator=g))  # self loops so that remove_self_loops matters
+    loops = torch.diag_embed(torch.rand(B, N, generator=g))
+    if self_loops:
+        a = a + loops
     gx = torch.randn(B, K, F, generator=g)
     ga = torch.randn(B, K, K, generator=g)
     ga = ga + ga.transpose(1, 2)

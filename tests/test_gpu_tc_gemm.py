@@ -45,20 +45,25 @@ def test_tc_gemm_fp32_3xtf32(a_mn, b_mn, B, M, N, Kd):
     assert err <= 2e-6 * scale * max(1.0, (Kd / 64) ** 0.5), f"3xTF32 error {err} vs scale {scale}"
 
 
-@pytest.mark.parametrize("ts", ["1", "0"])
+@pytest.mark.parametrize("tma_store", ["1", "0"])
 @pytest.mark.parametrize("a_mn", [False, True])
 @pytest.mark.parametrize("b_mn", [False, True])
 @pytest.mark.parametrize("B,M,N,Kd", [(2, 200, 40, 100), (3, 132, 72, 36), (1, 640, 320, 260), (300, 128, 64, 64)])
-def test_tc_gemm_fp32_ragged_shapes_both_engines(monkeypatch, ts, a_mn, b_mn, B, M, N, Kd):
+def test_tc_gemm_fp32_ragged_shapes_both_engines(tma_store, a_mn, b_mn, B, M, N, Kd):
     """fp32 products with ragged M / N / K (partial tiles, zero-filled TMA tails, several n-tiles, more tiles than
-    SMs) on the TMEM-operand engine and on the shared-memory engine."""
-    monkeypatch.setenv("TGPB200_GEMM_TS", ts)
+    SMs) on the TMEM-operand engine, through both of its epilogues: a plain row-major output leaves through the
+    TMA-store epilogue (tma_store "1"), an accumulated one through the register-store epilogue (tma_store "0")."""
     g = torch.Generator().manual_seed(5 * M + N + Kd)
     a = torch.randn((B, Kd, M) if a_mn else (B, M, Kd), generator=g).to(DEV)
     b = torch.randn((B, Kd, N) if b_mn else (B, N, Kd), generator=g).to(DEV)
-    out = _run(a, b, a_mn, b_mn, M, N, Kd)
     ref = _ref(a, b, a_mn, b_mn)
     scale = ref.abs().max().item()
+    if tma_store == "1":
+        out = _run(a, b, a_mn, b_mn, M, N, Kd)
+    else:
+        acc = torch.randn(B, M, N, generator=g).to(DEV)
+        out = _run(a, b, a_mn, b_mn, M, N, Kd, alpha=0.5, acc=acc)
+        ref = 0.5 * ref + acc.double()
     torch.testing.assert_close(out.double(), ref, rtol=1e-5, atol=1e-5 * scale)
 
 
@@ -92,26 +97,27 @@ def test_tc_gemm_bf16(a_mn, b_mn):
     torch.testing.assert_close(outb.double(), ref, rtol=2e-2, atol=2e-2)
 
 
-@pytest.mark.parametrize("pair", ["1", "0"])
+@pytest.mark.parametrize("out_bf16", ["1", "0"])
 @pytest.mark.parametrize("a_mn", [False, True])
 @pytest.mark.parametrize("b_mn", [False, True])
 @pytest.mark.parametrize("B,M,N,Kd", [(1, 256, 64, 64), (7, 512, 256, 128), (3, 384, 128, 200), (2, 200, 192, 64),
                                       (160, 256, 128, 64), (2, 1024, 512, 320)])
-def test_tc_gemm_bf16_cta_pairs(monkeypatch, pair, a_mn, b_mn, B, M, N, Kd):
-    """bf16 products with more than one 128-row tile run on CTA pairs (cta_group::2, 256-row tiles).  Ragged M / N,
-    several n-tiles, more pair tiles than SM pairs, and the single-CTA engine on the same inputs."""
+def test_tc_gemm_bf16_cta_pairs(out_bf16, a_mn, b_mn, B, M, N, Kd):
+    """bf16 products with more than one 128-row tile on the bf16 engine: ragged M / N, several n-tiles, more tiles
+    than SMs, with and without alpha / accumulation, into a bf16 (out_bf16 "1") or an fp32 output."""
     if (a_mn and M % 8) or (b_mn and N % 8):
         pytest.skip("MN-major rows must be 16-byte multiples")
-    monkeypatch.setenv("TGPB200_GEMM_PAIR", pair)
+    odt = torch.bfloat16 if out_bf16 == "1" else torch.float32
+    tol = dict(rtol=2e-2, atol=2e-2) if out_bf16 == "1" else dict(rtol=1e-5, atol=2e-4)
     g = torch.Generator().manual_seed(M + 3 * N + Kd)
     a = torch.randn((B, Kd, M) if a_mn else (B, M, Kd), generator=g).bfloat16().to(DEV)
     b = torch.randn((B, Kd, N) if b_mn else (B, N, Kd), generator=g).bfloat16().to(DEV)
-    out = _run(a, b, a_mn, b_mn, M, N, Kd)
+    out = _run(a, b, a_mn, b_mn, M, N, Kd, out_dtype=odt)
     ref = _ref(a, b, a_mn, b_mn)
-    torch.testing.assert_close(out.double(), ref, rtol=1e-5, atol=2e-4)
-    acc = torch.randn(B, M, N, generator=g).to(DEV)
-    out2 = _run(a, b, a_mn, b_mn, M, N, Kd, alpha=0.5, acc=acc)
-    torch.testing.assert_close(out2.double(), 0.5 * ref + acc.double(), rtol=1e-5, atol=2e-4)
+    torch.testing.assert_close(out.double(), ref, **tol)
+    acc = torch.randn(B, M, N, generator=g).to(DEV, odt)
+    out2 = _run(a, b, a_mn, b_mn, M, N, Kd, out_dtype=odt, alpha=0.5, acc=acc)
+    torch.testing.assert_close(out2.double(), 0.5 * ref + acc.double(), **tol)
 
 
 def test_tc_gemm_alpha_accumulate_and_transposed_output():

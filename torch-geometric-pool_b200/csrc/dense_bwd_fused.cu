@@ -491,10 +491,6 @@ int dense_bwd_fused(const float* A, const float* S, const float* X, const float*
   if (!make_out_map(&P.map_ds, dS, B, N, K) || !make_out_map(&P.map_dx, dX, B, N, F)) return TGPB200_ERR_UNSUPPORTED;
   P.S = ew_S, P.d = ew_d, P.coef = ew_coef, P.uv = ew_S ? ew_uv : nullptr, P.eps = eps;
   P.stages = 5;
-  {
-    const char* e = getenv("TGPB200_BWD_STAGES");  // experiment: fewer shared-memory stages
-    if (e && atoi(e) >= 2 && atoi(e) <= 5) P.stages = atoi(e);
-  }
   P.dbg = g_engine_dbg;
   static bool attr_set = false;
   if (!attr_set) {

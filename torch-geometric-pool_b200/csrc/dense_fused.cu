@@ -12,7 +12,6 @@
 // Every operand is MN-major (the contraction index i is the row of all three tensors): tiles are [BK = 16 nodes]
 // x [128-byte column blocks]; fp32 runs as 3xTF32 (hi/lo split in place, 32-byte-atom swizzle), bf16 as one pass.
 // Roles (320 threads): warp 0 TMA producer, warp 1 MMA issuer, warps 2-5 split + statistics, warps 6-9 epilogue.
-#include <stdlib.h>
 #include <string.h>
 
 #include "dense.cuh"
@@ -34,29 +33,18 @@ struct FusedParams {
   int nb_a, nb_x, nb_s;   // 128-byte column blocks per segment
   int t_a, t_x, t_s;      // 128-row MMA tiles per segment
   int stages, acc_bufs, blocked;
-  int groups;             // grouped form (K = 256, bf16): units per graph, each owning kGrpTiles M-tiles (0 = whole graph)
-  int a_groups;           // groups that hold A tiles (2: d / a2 are summed from two partial row sums)
   int concat;             // fp32: accumulators 2 BN wide, hi_a x [hi_s | lo_s] as ONE MMA (lo of S right behind S)
   uint32_t tmem_cols;
   float eps;
+  long long* dbg;         // optional timeline of block 0 (debug); ahead of Tt so that Tt / Xp stay 16-byte aligned
   void* Tt;               // [B, K, N]  operand dtype: T = S^T A
   void* Xp;               // [B, K, F]  operand dtype
   float* Mm;              // [B, K, K]
   float *d, *ss, *a2, *ent;  // [B, N]
-  long long* dbg;            // optional timeline of block 0 (debug)
 };
 
-// Grouped form (kGrp, bf16, K = 256): the 2 N/128 + F/128 + 2 accumulator tiles of a graph do not fit the 512 TMEM
-// columns, so a graph is split into units of kGrpTiles = 2 M-tiles (A column pairs, X column pairs, S); every unit
-// streams its own 256 M-side columns plus all of S (the N-side operand).  Consecutive units are the groups of one
-// graph, so S comes from HBM once and from L2 for the other units.  Row statistics: the S unit writes ss / ent, the
-// A units d / a2 (two A units per graph add their partial row sums with atomicAdd onto zero: two addends, so the
-// result does not depend on the order).
-constexpr int kGrpTiles = 2;
-
-template <bool kF32, bool kGrp = false>
+template <bool kF32>
 __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constant__ FusedParams P) {
-  static_assert(!(kF32 && kGrp), "the grouped form is bf16 only");
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   constexpr int ES = kF32 ? 4 : 2;
   constexpr int EPB = kStageRowBytes / ES;  // columns per 128-byte block
@@ -65,10 +53,8 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
   using T = typename std::conditional<kF32, float, __nv_bfloat16>::type;
 
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  constexpr int kGrpBlocks = kGrpTiles * (BM / EPB);  // M-side column blocks of a unit
-  const int nb = kGrp ? kGrpBlocks + P.nb_s : P.nb_a + P.nb_x + P.nb_s;
+  const int nb = P.nb_a + P.nb_x + P.nb_s;
   const uint32_t raw_bytes = (uint32_t)nb * kBlockBytes;
-  const int units = kGrp ? P.B * P.groups : P.B;
   const uint32_t stage_bytes = raw_bytes * (kF32 ? 2 : 1);
   const int stages = P.stages;
   // +4 blocks of slack: a partial last MMA tile reads (and ignores) up to 3 blocks past its segment
@@ -83,7 +69,7 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t smem_base = smem_u32(smem);
-  const int G = kGrp ? kGrpTiles : P.t_a + P.t_x + P.t_s;  // accumulator tiles of one unit
+  const int G = P.t_a + P.t_x + P.t_s;  // accumulator tiles of one graph
   const int BN = P.BN;
   const int kblocks = (P.N + FBK - 1) / FBK;
 
@@ -111,22 +97,14 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
       int s = 0;
       uint32_t ph = 0;
       int dbg_n = 0;
-      for (int u = blockIdx.x; u < units; u += gridDim.x) {
-        const int b = kGrp ? u / P.groups : u, q = kGrp ? u % P.groups : 0;
-        // grouped: segment of the unit and its first column block inside the segment
-        const int ag = P.a_groups, xg = P.t_x / kGrpTiles;
-        const CUtensorMap* gmap = q < ag ? &P.map_a : (q < ag + xg ? &P.map_x : &P.map_s);
-        const int gblk = (q < ag ? q : (q < ag + xg ? q - ag : 0)) * kGrpBlocks;
+      for (int b = blockIdx.x; b < P.B; b += gridDim.x) {
         for (int kb = 0; kb < kblocks; ++kb) {
           mbar_wait(bar_empty(s), ph ^ 1);
           if (P.dbg && blockIdx.x == 0 && dbg_n < 96) P.dbg[dbg_n * 8 + 0] = clock64();
           uint32_t dst = smem_base + (uint32_t)s * stage_bytes;
           mbar_arrive_expect_tx(bar_full(s), raw_bytes);
           const int k0 = kb * FBK;
-          if (kGrp) {  // two TMA instructions: the unit's M-side blocks, all of S
-            tma_load_4d(dst, gmap, bar_full(s), 0, k0, gblk, b);
-            tma_load_4d(dst + kGrpBlocks * kBlockBytes, &P.map_s, bar_full(s), 0, k0, 0, b);
-          } else if (P.blocked) {  // one TMA instruction per segment (4-D blocked maps)
+          if (P.blocked) {  // one TMA instruction per segment (4-D blocked maps)
             tma_load_4d(dst, &P.map_a, bar_full(s), 0, k0, 0, b);
             tma_load_4d(dst + P.nb_a * kBlockBytes, &P.map_x, bar_full(s), 0, k0, 0, b);
             tma_load_4d(dst + (P.nb_a + P.nb_x) * kBlockBytes, &P.map_s, bar_full(s), 0, k0, 0, b);
@@ -155,13 +133,12 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
       uint32_t tile_off[8];  // first column block of MMA tile g, in 16-byte units
 #pragma unroll
       for (int g = 0; g < 8; ++g) {
-        int blk = kGrp ? g * (BM / EPB)
-                       : (g < P.t_a ? g * (BM / EPB)
-                                    : (g < P.t_a + P.t_x ? P.nb_a + (g - P.t_a) * (BM / EPB)
-                                                         : P.nb_a + P.nb_x + (g - P.t_a - P.t_x) * (BM / EPB)));
+        int blk = g < P.t_a ? g * (BM / EPB)
+                            : (g < P.t_a + P.t_x ? P.nb_a + (g - P.t_a) * (BM / EPB)
+                                                 : P.nb_a + P.nb_x + (g - P.t_a - P.t_x) * (BM / EPB));
         tile_off[g] = (uint32_t)blk * (kBlockBytes >> 4);
       }
-      const uint32_t b_off = (uint32_t)(kGrp ? kGrpBlocks : P.nb_a + P.nb_x) * (kBlockBytes >> 4);
+      const uint32_t b_off = (uint32_t)(P.nb_a + P.nb_x) * (kBlockBytes >> 4);
       const uint32_t lo_off = raw_bytes >> 4, stage_off = stage_bytes >> 4;
       // concat mode: stage = [A | X | S | S lo | A lo | X lo]
       const uint32_t s_lo_off = (uint32_t)P.nb_s * (kBlockBytes >> 4), ax_lo_off = lo_off + s_lo_off;
@@ -171,7 +148,7 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
       uint32_t ph = 0;
       int it = 0;
       int dbg_m = 0;
-      for (int u = blockIdx.x; u < units; u += gridDim.x, ++it) {
+      for (int b = blockIdx.x; b < P.B; b += gridDim.x, ++it) {
         const int ab = P.acc_bufs == 2 ? (it & 1) : 0;
         const uint32_t aph = P.acc_bufs == 2 ? ((uint32_t)(it >> 1) & 1u) : ((uint32_t)it & 1u);
         mbar_wait(bar_tempty(ab), aph ^ 1);
@@ -228,10 +205,7 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
     int s = 0;
     uint32_t ph = 0;
     int dbg_s = 0;
-    for (int u = blockIdx.x; u < units; u += gridDim.x) {
-      const int b = kGrp ? u / P.groups : u, q = kGrp ? u % P.groups : 0;
-      // grouped: 0 = A unit (d, a2), 1 = X unit (nothing), 2 = S unit (ss, ent from the M-side copy of S)
-      const int gseg = q < P.a_groups ? 0 : (q < P.a_groups + P.t_x / kGrpTiles ? 1 : 2);
+    for (int b = blockIdx.x; b < P.B; b += gridDim.x) {
       for (int kb = 0; kb < kblocks; ++kb) {
         mbar_wait(bar_full(s), ph);
         if (P.dbg && blockIdx.x == 0 && t == 0 && dbg_s < 96) P.dbg[dbg_s * 8 + 5] = clock64();
@@ -294,14 +268,9 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
           if (blk + 2 <= b1) { batch(seg_tag, std::integral_constant<int, 2>{}, blk); blk += 2; }
           if (blk < b1) batch(seg_tag, std::integral_constant<int, 1>{}, blk);
         };
-        if (kGrp) {
-          if (gseg == 0) segment(std::integral_constant<int, 0>{}, 0, kGrpBlocks);
-          if (gseg == 2) segment(std::integral_constant<int, 2>{}, 0, kGrpBlocks);
-        } else {
-          segment(std::integral_constant<int, 0>{}, 0, P.nb_a);
-          segment(std::integral_constant<int, 1>{}, P.nb_a, P.nb_a + P.nb_x);
-          segment(std::integral_constant<int, 2>{}, P.nb_a + P.nb_x, nb);
-        }
+        segment(std::integral_constant<int, 0>{}, 0, P.nb_a);
+        segment(std::integral_constant<int, 1>{}, P.nb_a, P.nb_a + P.nb_x);
+        segment(std::integral_constant<int, 2>{}, P.nb_a + P.nb_x, nb);
         // the 8 lanes of a row (fixed lane group, fixed block order -> deterministic)
 #pragma unroll
         for (int o = 1; o < 8; o <<= 1) {
@@ -313,18 +282,7 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
         const int node = kb * FBK + r;
         if ((t & 7) == 0 && node < P.N) {
           const int64_t o = (int64_t)b * P.N + node;
-          if (!kGrp) {
-            P.d[o] = sd, P.a2[o] = sa2, P.ss[o] = s2, P.ent[o] = se;
-          } else if (gseg == 2) {
-            P.ss[o] = s2, P.ent[o] = se;
-          } else if (gseg == 0) {
-            if (P.a_groups == 1) {
-              P.d[o] = sd, P.a2[o] = sa2;
-            } else {  // two partial row sums onto zero: x + y == y + x, order-independent
-              atomicAdd(P.d + o, sd);
-              atomicAdd(P.a2 + o, sa2);
-            }
-          }
+          P.d[o] = sd, P.a2[o] = sa2, P.ss[o] = s2, P.ent[o] = se;
         }
         if (kF32) fence_proxy_async();
         mbar_arrive(bar_lo(s));
@@ -337,26 +295,23 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
     // ===================== epilogue =====================
     const int quad = warp & 3;
     int it = 0;
-    for (int u = blockIdx.x; u < units; u += gridDim.x, ++it) {
-      const int b = kGrp ? u / P.groups : u, q = kGrp ? u % P.groups : 0;
+    for (int b = blockIdx.x; b < P.B; b += gridDim.x, ++it) {
       const int ab = P.acc_bufs == 2 ? (it & 1) : 0;
       const uint32_t aph = P.acc_bufs == 2 ? ((uint32_t)(it >> 1) & 1u) : ((uint32_t)it & 1u);
       mbar_wait(bar_tfull(ab), aph);
       tc_fence_after();
       const int row = quad * 32 + lane;
-      for (int gl = 0; gl < G; ++gl) {
-        // grouped: the unit's local tile gl is tile q * kGrpTiles + gl of the graph (A tiles, X tiles, S tiles)
-        const int g = kGrp ? q * kGrpTiles + gl : gl;
+      for (int g = 0; g < G; ++g) {
         const int seg = g < P.t_a ? 0 : (g < P.t_a + P.t_x ? 1 : 2);
         const int m = (seg == 0 ? g : (seg == 1 ? g - P.t_a : g - P.t_a - P.t_x)) * BM + row;
         const int m_ext = seg == 0 ? P.N : (seg == 1 ? P.F : P.K);
         for (int c0 = 0; c0 < BN; c0 += 32) {
           float v[32];
           const int accw = P.concat ? 2 * BN : BN;
-          tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(ab * G * accw + gl * accw + c0), v);
+          tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(ab * G * accw + g * accw + c0), v);
           if (P.concat) {  // + hi x lo_s
             float v2[32];
-            tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(ab * G * accw + gl * accw + BN + c0), v2);
+            tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(ab * G * accw + g * accw + BN + c0), v2);
 #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] += v2[j];
           }
@@ -409,51 +364,10 @@ int dense_fwd_fused(const void* A, const void* S, const void* X, int B, int N, i
   P.t_a = (N + BM - 1) / BM, P.t_x = (F + BM - 1) / BM, P.t_s = (K + BM - 1) / BM;
   // every segment must start on an MMA-tile boundary of its own blocks: tiles are 128 columns = BM/epb blocks
   const int G = P.t_a + P.t_x + P.t_s;
-  if (G * P.BN > 512 || G > 8) {
-    // grouped form: K = 256 (two accumulator tiles fill the tensor memory), bf16, every segment a whole number of units
-    // Opt-in (TGPB200_FUSED_GROUPS=1): measured on C3 level 1 it moves 1.74 GB in 760 us (2.3 TB/s) against 539 us
-    // for the four launches it replaces (3.08 GB at 5.7 TB/s) -- the accumulators fill the tensor memory, so the
-    // strided epilogue of a unit cannot overlap the next unit's main loop.
-    static const bool grouped_on = [] { const char* e = getenv("TGPB200_FUSED_GROUPS"); return e && e[0] == '1'; }();
-    if (!grouped_on || !bf16 || K != 256 || N % (kGrpTiles * BM) || F % (kGrpTiles * BM) || P.t_a / kGrpTiles > 2)
-      return TGPB200_ERR_UNSUPPORTED;
-    const int gblocks = kGrpTiles * (BM / epb);
-    if (P.nb_s != gblocks) return TGPB200_ERR_UNSUPPORTED;  // the S unit loads S through the same 4-block box
-    P.a_groups = P.t_a / kGrpTiles;
-    P.groups = P.a_groups + P.t_x / kGrpTiles + 1;
-    P.acc_bufs = 1, P.concat = 0, P.blocked = 1, P.tmem_cols = 512;
-    const size_t stage_bytes = (size_t)(gblocks + P.nb_s) * kBlockBytes;
-    int stages = (int)((size_t)(210 * 1024) / stage_bytes);
-    if (stages > 12) stages = 12;
-    P.stages = stages;
-    P.eps = eps;
-    P.Tt = Tt, P.Xp = Xp, P.Mm = Mm, P.d = d, P.ss = ss, P.a2 = a2, P.ent = ent;
-    P.dbg = nullptr;
-    if (!make_map_blocked(&P.map_a, A, true, B, N, N, N, (int64_t)N * N, FBK, gblocks, false) ||
-        !make_map_blocked(&P.map_x, X, true, B, N, F, F, (int64_t)N * F, FBK, gblocks, false) ||
-        !make_map_blocked(&P.map_s, S, true, B, N, K, K, (int64_t)N * K, FBK, gblocks, false))
-      return TGPB200_ERR_UNSUPPORTED;
-    static bool grp_attr = false;
-    if (!grp_attr) {
-      grp_attr = true;
-      cudaFuncSetAttribute(k_dense_fwd_fused<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    }
-    const size_t smem = stage_bytes * stages + 4 * kBlockBytes + (3 * stages + 4) * 8 + 16 + 1024;
-    if (smem > 227 * 1024) return TGPB200_ERR_UNSUPPORTED;
-    if (P.a_groups == 2) {  // the two A units of a graph add their partial row sums
-      cudaMemsetAsync(d, 0, (size_t)B * N * sizeof(float), stream);
-      cudaMemsetAsync(a2, 0, (size_t)B * N * sizeof(float), stream);
-    }
-    const int sms = device_sm_count();
-    const int64_t units = (int64_t)B * P.groups;
-    launch("k_dense_fwd_fused_bf16_grouped", k_dense_fwd_fused<false, true>, (int)(units < sms ? units : sms), 320, smem,
-           stream, P);
-    return launch_status();
-  }
-  {
-    const char* e = getenv("TGPB200_FUSED_CONCAT");
-    P.concat = (!bf16 && K % 32 == 0 && P.BN == K && 2 * G * P.BN <= 512 && !(e && e[0] == '0')) ? 1 : 0;
-  }
+  // the accumulators of a graph must fit the 512 TMEM columns (K = 256 never does): otherwise the caller runs the
+  // per-product launches
+  if (G * P.BN > 512 || G > 8) return TGPB200_ERR_UNSUPPORTED;
+  P.concat = (!bf16 && K % 32 == 0 && P.BN == K && 2 * G * P.BN <= 512) ? 1 : 0;
   const int accw = P.concat ? 2 * P.BN : P.BN;
   P.acc_bufs = (2 * G * accw <= 512) ? 2 : 1;
   uint32_t cols = 32;
@@ -468,8 +382,7 @@ int dense_fwd_fused(const void* A, const void* S, const void* X, int B, int N, i
   P.Tt = Tt, P.Xp = Xp, P.Mm = Mm, P.d = d, P.ss = ss, P.a2 = a2, P.ent = ent;
   P.dbg = g_fused_dbg;
   const bool sw32 = !bf16;
-  const char* env = getenv("TGPB200_FUSED_BLOCKED");
-  P.blocked = (N % epb == 0 && F % epb == 0 && K % epb == 0 && P.nb_a <= 256 && !(env && env[0] == '0')) ? 1 : 0;
+  P.blocked = (N % epb == 0 && F % epb == 0 && K % epb == 0 && P.nb_a <= 256) ? 1 : 0;
   if (P.blocked) {
     if (!make_map_blocked(&P.map_a, A, bf16, B, N, N, N, (int64_t)N * N, FBK, P.nb_a, sw32) ||
         !make_map_blocked(&P.map_x, X, bf16, B, N, F, F, (int64_t)N * F, FBK, P.nb_x, sw32) ||

@@ -135,16 +135,6 @@ __device__ __forceinline__ void stv(T* p, const float (&a)[V]) {
     p[0] = from_f32<T>(a[0]);
   }
 }
-// strip copy global -> shared as fp32, several 128-bit loads in flight per thread
-template <int V, typename T>
-__device__ __forceinline__ void stage_strip(float* dst, const T* src, int cnt) {
-#pragma unroll 4
-  for (int i = threadIdx.x * V; i < cnt; i += blockDim.x * V) {
-    float a[V];
-    ldv<V, T>(src + i, a);
-    stv<V, float>(dst + i, a);
-  }
-}
 
 template <typename T, int V>
 static __global__ void k_row_stats(const T* __restrict__ A, const T* __restrict__ S, int64_t rows, int N, int K,
@@ -187,8 +177,8 @@ static __global__ void k_row_stats(const T* __restrict__ A, const T* __restrict_
 
 // ------------------------------------------------------------------------------------------
 // Per-graph kernels run as a thread-block CLUSTER per graph: CTA `rank` owns the row strip
-// [rank * rows_per, (rank + 1) * rows_per) of the [K, K] matrices (staged once in its shared memory), and the
-// graph-wide reductions are combined through distributed shared memory in a fixed order (bitwise reproducible).
+// [rank * rows_per, (rank + 1) * rows_per) of the [K, K] matrices, and the graph-wide
+// reductions are combined through distributed shared memory in a fixed order (bitwise reproducible).
 // A cluster of one CTA is the small-K case.
 // ------------------------------------------------------------------------------------------
 struct GraphCluster {
@@ -349,13 +339,13 @@ __device__ __forceinline__ void strip_sums4(int K, int r0, int r1, float* colred
 // then post-processing (diag zero -> D^-1/2 A D^-1/2 -> / max|A|) exactly in ops.py:307-333 order.
 // stats[b] = {num, den, ||M||_F^2, ortho_b, ||A||_F^2, ent_b, maxnorm m, 2m (DMoN only: k_dmon_stats)}
 // ------------------------------------------------------------------------------------------
-template <typename T, int V, bool STAGED>
+template <typename T, int V>
 static __global__ void __launch_bounds__(512)
     k_graph_epilogue(const float* __restrict__ Araw, const float* __restrict__ M, const float* __restrict__ d,
                      const float* __restrict__ ss, const float* __restrict__ a2, const float* __restrict__ ent, int N,
                      int K, uint32_t flags, float eps, T* __restrict__ Apool, float* __restrict__ dvec,
-                     float* __restrict__ stats, int32_t* __restrict__ argmax, int rows_per, int rowp_floats) {
-  // dq[K] (degree scale, all columns), part[K], rowp[rowp_floats]  (+ the two staged row strips)
+                     float* __restrict__ stats, int32_t* __restrict__ argmax, int rows_per) {
+  // dq[K] (degree scale, all columns), part[K], rowp[StripPlan::rowp_floats]
   extern __shared__ __align__(16) float sm[];
   __shared__ float red[32];
   __shared__ int redi[32];
@@ -372,15 +362,6 @@ static __global__ void __launch_bounds__(512)
   const float* Ar = hasA ? Araw + (int64_t)b * K * K + i0 : nullptr;
   const float* Mg = hasM ? M + (int64_t)b * K * K + i0 : nullptr;
   float* st = stats + (int64_t)b * 8;
-  if constexpr (STAGED) {  // the kernel is a chain of short passes over the same strip: keep it on chip
-    float* sA = sm + 2 * K + rowp_floats;
-    float* sM = sA + rows_per * K;
-    if (hasA) stage_strip<V, float>(sA, Ar, cnt);
-    if (hasM) stage_strip<V, float>(sM, Mg, cnt);
-    Ar = sA;  // unconditional: the later accesses compile to shared-memory loads
-    Mg = sM;
-    __syncthreads();
-  }
 
   const int kshift = (K & (K - 1)) == 0 ? __ffs(K) - 1 : -1;
   auto row_of = [&](int i) { return r0 + (kshift >= 0 ? (i >> kshift) : (i / K)); };  // i is strip-local
@@ -709,15 +690,15 @@ static __global__ void k_finalize_dmon(const float* __restrict__ stats, const fl
 // gl = upstream grads of {cut, ortho, link, entropy} (device floats, already x coefficient); for loss_kind 3 (DMoN)
 // {spectral, ortho, cluster, -}: c_num and P here, the rest of the DMoN gradient in k_dmon_bwd.
 // ------------------------------------------------------------------------------------------
-template <typename T, int V, bool STAGED>
+template <typename T, int V>
 static __global__ void __launch_bounds__(512)
     k_graph_bwd(const float* __restrict__ Araw, const float* __restrict__ M, const T* __restrict__ Gpool,
                 const float* __restrict__ dvec, const float* __restrict__ stats, const int32_t* __restrict__ argmax,
                 const float* __restrict__ gl, const float* __restrict__ losses, int B, int K, uint32_t flags,
                 int loss_kind, float eps, float link_div, float ent_div, float* __restrict__ Graw,
-                float* __restrict__ P, float* __restrict__ coef, int rows_per, int rowp_floats, T* __restrict__ Gt,
+                float* __restrict__ P, float* __restrict__ coef, int rows_per, T* __restrict__ Gt,
                 T* __restrict__ Pt) {
-  // dsq[K] = 1/d_v, part[K], tot[K] = rowdot + coldot, rowv[K], rowp[rowp_floats]  (+ three staged strips)
+  // dsq[K] = 1/d_v, part[K], tot[K] = rowdot + coldot, rowv[K], rowp[StripPlan::rowp_floats]
   extern __shared__ __align__(16) float sm[];
   __shared__ float red[32];
   __shared__ __align__(16) float colred[4 * 512];
@@ -736,25 +717,8 @@ static __global__ void __launch_bounds__(512)
   const float* Ar = Araw + (int64_t)b * K * K + i0;
   const float* Mb = hasM ? M + (int64_t)b * K * K + i0 : nullptr;
   const T* Gp = hasG ? Gpool + (int64_t)b * K * K + i0 : nullptr;
-  const float* Gs = nullptr;  // staged fp32 copy of the upstream gradient strip
-  if constexpr (STAGED) {
-    float* sA = sm + 4 * K + rowp_floats;
-    float* sM = sA + rows_per * K;
-    float* sG = sM + rows_per * K;
-    stage_strip<V, float>(sA, Ar, cnt);
-    if (hasM) stage_strip<V, float>(sM, Mb, cnt);
-    if (hasG) stage_strip<V, T>(sG, Gp, cnt);
-    Ar = sA;  // unconditional: the later accesses compile to shared-memory loads
-    Mb = sM;
-    Gs = sG;
-    __syncthreads();
-  }
-  auto gp = [&](int i) {
-    if constexpr (STAGED) return Gs[i]; else return to_f32<T>(Gp[i]);
-  };
-  auto gpv = [&](int i, float (&g)[V]) {
-    if constexpr (STAGED) ldv<V, float>(Gs + i, g); else ldv<V, T>(Gp + i, g);
-  };
+  auto gp = [&](int i) { return to_f32<T>(Gp[i]); };
+  auto gpv = [&](int i, float (&g)[V]) { ldv<V, T>(Gp + i, g); };
   auto outv = [&](T* ot, float* of, int i, const float (&v)[V]) {  // operand-dtype copy (bf16 runs) or fp32
     if (ot) stv<V, T>(ot + i, v); else stv<V, float>(of + i, v);
   };
@@ -864,7 +828,7 @@ static __global__ void __launch_bounds__(512)
       strip_sums4<true, true>(K, r0, r1, colred, rowp, part, rowv, [&](int i, int r, int c0, float (&p)[4]) {
         float av[4], gv[4];
         ldv<4, float>(Ar + i, av);
-        if constexpr (STAGED) ldv<4, float>(Gs + i, gv); else ldv<4, T>(Gp + i, gv);
+        ldv<4, T>(Gp + i, gv);
         const float ir = dsq[r];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
@@ -1109,34 +1073,25 @@ static int mm1(int batch, int M, int N, int kd, Mat A, Mat Bm, TC* out, int64_t 
   return mm<T, TC>(batch, M, N, 1, &kd, &A, &Bm, out, obs, ors, ocs, st, EwHook(), tag);
 }
 
-// How a per-graph kernel splits a [K, K] matrix over a cluster: R CTAs of `threads` threads, `rows_per` rows each;
-// the strips are staged in shared memory when `nvec` K-vectors plus `nstrips` strips fit.
+// How a per-graph kernel splits a [K, K] matrix over a cluster: R CTAs of `threads` threads, `rows_per` rows each,
+// with `nvec` K-vectors and the row partials in shared memory.
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 struct StripPlan {
-  int R, rows_per, threads, stage, rowp_floats;
+  int R, rows_per, threads, rowp_floats;
   size_t smem;
 };
-static StripPlan strip_plan(int K, int nvec, int nstrips, int64_t elems_for_512 = 2048) {
-  // tuning knobs (read per call; benchmarks/per_graph_kernels.py sweeps them)
+static StripPlan strip_plan(int K, int nvec, int64_t elems_for_512 = 2048) {
+  // elements per CTA (read per call; benchmarks/per_graph_kernels.py sweeps it)
   const char* e = getenv("TGPB200_STRIP_ELEMS");
   const int ev = e ? atoi(e) : 0;
   const int target = ev > 0 ? ev : 32768;  // measured best on B200 (K = 256: two CTAs per graph)
-  const char* es = getenv("TGPB200_STRIP_STAGE");
-  const bool allow_stage = es && es[0] == '1';  // staging measured no faster than L2-served re-reads
   StripPlan p;
   p.R = 1;
   while (p.R < 8 && ceil_div(K, p.R) * (int64_t)K > target) p.R *= 2;
   p.rows_per = (int)ceil_div(K, p.R);
   p.rowp_floats = (int)(ceil_div((int64_t)p.rows_per * (K >= 128 ? K / 128 : 1), 4) * 4);
-  const size_t vec = ((size_t)nvec * K + p.rowp_floats) * sizeof(float);
-  const size_t strips = (size_t)nstrips * p.rows_per * K * sizeof(float);
-  p.stage = allow_stage && vec + strips <= 160 * 1024;
-  p.smem = vec + (p.stage ? strips : 0);
-  {
-    const char* et = getenv("TGPB200_STRIP_THREADS");
-    const int tv = et ? atoi(et) : 0;
-    p.threads = (tv == 128 || tv == 256 || tv == 512) ? tv : ((int64_t)p.rows_per * K >= elems_for_512 ? 512 : 256);
-  }
+  p.smem = ((size_t)nvec * K + p.rowp_floats) * sizeof(float);
+  p.threads = (int64_t)p.rows_per * K >= elems_for_512 ? 512 : 256;
   return p;
 }
 
@@ -1235,14 +1190,13 @@ static int dense_fwd(const T* A, const T* S, const T* X, int B, int N, int K, in
   }
   if (B > 0) {
     // 256 threads up to 8 K elements per CTA: measured 16.6 vs 21.1 us on C2 (the backward kernel prefers 512)
-    const StripPlan sp = strip_plan(K, 2, 2, 8193);
+    const StripPlan sp = strip_plan(K, 2, 8193);
     const bool v4 = K % 4 == 0 && aligned16(Apool);
-    auto kern = sp.stage ? (v4 ? k_graph_epilogue<T, 4, true> : k_graph_epilogue<T, 1, true>)
-                         : (v4 ? k_graph_epilogue<T, 4, false> : k_graph_epilogue<T, 1, false>);
+    auto kern = v4 ? k_graph_epilogue<T, 4> : k_graph_epilogue<T, 1>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024);
     launch_cluster("k_graph_epilogue", kern, (unsigned)B * sp.R, sp.threads, sp.R, sp.smem, st,
                    A ? pl.Araw : (float*)nullptr, loss_kind != 0 ? pl.M : (float*)nullptr, pl.d, pl.ss, pl.a2, pl.ent,
-                   N, K, flags, eps, Apool, pl.dvec, pl.stats, pl.argmax, sp.rows_per, sp.rowp_floats);
+                   N, K, flags, eps, Apool, pl.dvec, pl.stats, pl.argmax, sp.rows_per);
     // fp32: the identity holds rtol 1e-5 down to q ~ 0.05 ||A||^2; bf16 (T stored in bf16, rtol 2e-2) down to 0.25
     const float link_tau = (loss_kind == 2 && A) ? (std::is_same<T, float>::value ? 0.05f : 0.25f) : 0.f;
     if (loss_kind == 3) {
@@ -1295,15 +1249,14 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
     launch("k_dmon_bwd", k_dmon_bwd<T>, (unsigned)B, 256, 0, st, S, pl.stats, pl.dm_c, pl.dm_e,
            pl.dm_st, graph_nodes, gl, B, N, K, uv, dA_out ? rvec : (float*)nullptr, coef_r);
   if (have_a) {
-    const StripPlan sp = strip_plan(K, 4, 3);
+    const StripPlan sp = strip_plan(K, 4);
     const bool v4 = K % 4 == 0 && aligned16(gApool);
-    auto kern = sp.stage ? (v4 ? k_graph_bwd<T, 4, true> : k_graph_bwd<T, 1, true>)
-                         : (v4 ? k_graph_bwd<T, 4, false> : k_graph_bwd<T, 1, false>);
+    auto kern = v4 ? k_graph_bwd<T, 4> : k_graph_bwd<T, 1>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024);
     launch_cluster("k_graph_bwd", kern, (unsigned)B * sp.R, sp.threads, sp.R, sp.smem, st, pl.Araw,
                    loss_kind != 0 ? pl.M : (float*)nullptr, gApool, pl.dvec, pl.stats, pl.argmax, gl, pl.losses, B, K,
                    flags, loss_kind, eps, link_div, ent_div, Graw, loss_kind != 0 ? P : (float*)nullptr, coef,
-                   sp.rows_per, sp.rowp_floats, f32 ? (T*)nullptr : Gt, (f32 || loss_kind == 0) ? (T*)nullptr : Pt);
+                   sp.rows_per, f32 ? (T*)nullptr : Gt, (f32 || loss_kind == 0) ? (T*)nullptr : Pt);
     if (f32) {
       Gt = reinterpret_cast<T*>(Graw);
       Pt = reinterpret_cast<T*>(P);
@@ -1346,7 +1299,7 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
     if (n > 0) {
       EwHook hook;
       // DMoN's d_i u_k + v_k is left to k_ds_elementwise: carried in the engine's epilogue it cost the MinCut
-      // products of k_tc_gemm / k_tc_gemm_pair extra register spills
+      // products of the bf16 engine extra register spills
       if (have_a && loss_kind != 0 && !dmon) {
         hook.S = S, hook.d = pl.d, hook.coef = coef, hook.eps = eps, hook.applied = &ew_done;
       }

@@ -10,7 +10,7 @@
 namespace tgp {
 
 // ------------------------------------------------------------------------------------------
-// Exclusive scan of int32 (n < 2^31).  reduce-then-scan over 4096-item tiles.
+// Exclusive scan of int32 (n < 2^31): one block for small inputs, a single pass over 4096-item tiles otherwise.
 // ------------------------------------------------------------------------------------------
 constexpr int kScanThreads = 256;
 constexpr int kScanItems = 16;
@@ -44,20 +44,6 @@ __device__ __forceinline__ int block_exclusive_scan_i(int v, int* smem /* >= 33 
   return base + inc - v;
 }
 
-static __global__ void k_scan_reduce(const int* __restrict__ in, int64_t n, int* __restrict__ tile_sums) {
-  __shared__ int red[33];
-  int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
-  int s = 0;
-#pragma unroll
-  for (int j = 0; j < kScanItems; ++j) {
-    int64_t i = base + j;
-    if (i < n) s += in[i];
-  }
-  int tot;
-  block_exclusive_scan_i(s, red, &tot);
-  if (threadIdx.x == 0) tile_sums[blockIdx.x] = tot;
-}
-
 // Single block: exclusive scan of tile_sums[nt] in place; optional totals.
 static __global__ void k_scan_spine(int* __restrict__ tile_sums, int nt, int* __restrict__ total32,
                                     int64_t* __restrict__ total64) {
@@ -78,30 +64,9 @@ static __global__ void k_scan_spine(int* __restrict__ tile_sums, int nt, int* __
   }
 }
 
-static __global__ void k_scan_down(const int* __restrict__ in, int* __restrict__ out, int64_t n,
-                                   const int* __restrict__ tile_offsets) {
-  __shared__ int red[33];
-  int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
-  int v[kScanItems];
-  int s = 0;
-#pragma unroll
-  for (int j = 0; j < kScanItems; ++j) {
-    int64_t i = base + j;
-    v[j] = i < n ? in[i] : 0;
-    s += v[j];
-  }
-  int ex = block_exclusive_scan_i(s, red, nullptr) + tile_offsets[blockIdx.x];
-#pragma unroll
-  for (int j = 0; j < kScanItems; ++j) {
-    int64_t i = base + j;
-    if (i < n) out[i] = ex;
-    ex += v[j];
-  }
-}
-
-// Small inputs (n <= kScanSmall): ONE block scans the whole array with a running carry -- one launch instead of three.
-// (The TopK step on 128 small graphs, BASELINE config 1, is a chain of ~20 launches of a few microseconds each; nine of
-// them were the three phases of three scans.)  Integer sums: the result is identical to the tiled path.
+// Small inputs (n <= kScanSmall): ONE block scans the whole array with a running carry -- one launch and no memset.
+// (The TopK step on 128 small graphs, BASELINE config 1, is a chain of ~20 launches of a few microseconds each.)
+// Integer sums: the result is identical to the tiled path.
 constexpr int kScanSmall = 32768;
 constexpr int kScanSmallItems = 8;
 static __global__ void __launch_bounds__(1024) k_scan_small(const int* __restrict__ in, int* __restrict__ out, int n,
@@ -134,7 +99,7 @@ static __global__ void __launch_bounds__(1024) k_scan_small(const int* __restric
 }
 
 // Large inputs: single-pass scan with decoupled look-back -- the input is read ONCE and there is one kernel (plus the
-// memset of the tile states) instead of three.  Tiles take a ticket, publish (flag, tile sum) packed in 64 bits and walk
+// memset of the tile states).  Tiles take a ticket, publish (flag, tile sum) packed in 64 bits and walk
 // back over the published aggregates until they meet an inclusive prefix (same protocol as k_compact_onepass).
 // tile_state ([tiles] uint64) and ticket (int) must be zero before the launch.  Sums are < 2^31 (contract of this scan).
 static __global__ void __launch_bounds__(kScanThreads)
@@ -220,7 +185,7 @@ static __global__ void __launch_bounds__(kScanThreads)
   }
 }
 
-// workspace: tile sums of the three-phase path, or tile states + ticket of the one-pass path (the larger of the two)
+// workspace: tile states + ticket of the one-pass path
 inline size_t scan_workspace_bytes(int64_t n) {
   return align_up(((size_t)ceil_div(n > 0 ? n : 1, kScanTile) + 2) * sizeof(unsigned long long));
 }
@@ -235,19 +200,9 @@ inline int exclusive_scan_i32(const int* in, int* out, int64_t n, int* total32, 
     launch("k_scan_small", k_scan_small, 1, 1024, 0, stream, in, out, (int)n, total32, total64);
     return launch_status();
   }
-  {
-    static const bool three_phase = [] { const char* e = getenv("TGPB200_SCAN_ONEPASS"); return e && e[0] == '0'; }();
-    if (!three_phase) {
-      cudaMemsetAsync(state, 0, ((size_t)nt + 2) * sizeof(unsigned long long), stream);
-      launch("k_scan_onepass", k_scan_onepass, nt, kScanThreads, 0, stream, in, out, n, state,
-             reinterpret_cast<int*>(state + nt), nt, total32, total64);
-      return launch_status();
-    }
-  }
-  int* sums = reinterpret_cast<int*>(state);
-  launch("k_scan_reduce", k_scan_reduce, nt, kScanThreads, 0, stream, in, n, sums);
-  launch("k_scan_spine", k_scan_spine, 1, 1024, 0, stream, sums, nt, total32, total64);
-  if (n > 0) launch("k_scan_down", k_scan_down, nt, kScanThreads, 0, stream, in, out, n, sums);
+  cudaMemsetAsync(state, 0, ((size_t)nt + 2) * sizeof(unsigned long long), stream);
+  launch("k_scan_onepass", k_scan_onepass, nt, kScanThreads, 0, stream, in, out, n, state,
+         reinterpret_cast<int*>(state + nt), nt, total32, total64);
   return launch_status();
 }
 
@@ -465,7 +420,7 @@ static int compact_onepass(Pred pred, Emit emit, int64_t n, int64_t* count_out, 
 }
 
 // ------------------------------------------------------------------------------------------
-// Stable LSD radix sort of (key, uint32 payload) pairs; 8, 10 or 11 bits per pass (fewest passes that cover the key).
+// Stable LSD radix sort of (key, uint32 payload) pairs, 8 bits per pass.
 // Pass = tile histogram -> scan of [bins][tiles] -> stable scatter (warp match ranking, smem-staged stores).
 // ------------------------------------------------------------------------------------------
 constexpr int kSortThreads = 256;
@@ -474,33 +429,18 @@ constexpr int kSortThreads = 256;
 #endif
 constexpr int kSortItems = TGPB200_SORT_ITEMS;
 constexpr int kSortTile = kSortThreads * kSortItems;
-constexpr int kSortMaxBins = 2048;
+constexpr int kSortMaxBins = 2048;  // histogram rows reserved per tile in the workspace (a pass uses kRadixBins)
 
-struct RadixPlan {
-  int bits;    // digit width
-  int passes;  // number of passes
-};
-inline RadixPlan radix_plan(int key_bits) {
-  if (key_bits < 1) key_bits = 1;
-  // Measured on B200 (20 M 39-bit keys): a 10-bit pass costs 1.55x an 8-bit pass (2 KB x 8 warp counters and
-  // the staging buffer halve the occupancy), so 4 x 10-bit passes lose to 5 x 8-bit passes.  8 bits it is; the
-  // wider instantiations stay available through TGPB200_RADIX_BITS for experiments.
-  RadixPlan p;
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("TGPB200_RADIX_BITS");
-    forced = e ? atoi(e) : 0;
-  }
-  p.bits = (forced == 10 || forced == 11) ? forced : 8;
-  p.passes = (key_bits + p.bits - 1) / p.bits;
-  return p;
-}
-inline int radix_passes(int key_bits) { return radix_plan(key_bits).passes; }
+// Measured on B200 (20 M 39-bit keys): a 10-bit pass costs 1.55x an 8-bit pass (2 KB x 8 warp counters and the staging
+// buffer halve the occupancy), so 4 x 10-bit passes lose to 5 x 8-bit passes.
+constexpr int kRadixBits = 8;
+constexpr int kRadixBins = 1 << kRadixBits;
+inline int radix_passes(int key_bits) { return key_bits < 1 ? 1 : (key_bits + kRadixBits - 1) / kRadixBits; }
 
-template <typename KeyT, int BITS>
+template <typename KeyT>
 static __global__ void k_radix_hist(const KeyT* __restrict__ keys, int64_t n, const int64_t* __restrict__ n_dev,
                                     int shift, int* __restrict__ tile_hist, int nt) {
-  constexpr int BINS = 1 << BITS;
+  constexpr int BINS = kRadixBins;
   __shared__ int h[BINS];
   if (n_dev) n = min(n, *n_dev);  // device-side count (capacity launch): tiles past it publish empty histograms
   for (int d = threadIdx.x; d < BINS; d += kSortThreads) h[d] = 0;
@@ -519,7 +459,7 @@ static __global__ void k_radix_hist(const KeyT* __restrict__ keys, int64_t n, co
 // __match_any_sync (stable inside the warp); per-digit counts are then prefixed over warps and digits.  The items
 // are first placed in shared memory in tile-local sorted order, so that the final global writes of a digit run are
 // consecutive (full-sector stores) instead of one scattered 8/12-byte write per item.
-template <typename KeyT, int BITS, bool kIota>
+template <typename KeyT, bool kIota>
 static __global__ void __launch_bounds__(kSortThreads)
     k_radix_scatter(const KeyT* __restrict__ keys_in, const uint32_t* __restrict__ vals_in,
                     KeyT* __restrict__ keys_out, uint32_t* __restrict__ vals_out, int64_t n,
@@ -527,7 +467,7 @@ static __global__ void __launch_bounds__(kSortThreads)
   constexpr int NW = kSortThreads / 32;
   if (n_dev) n = min(n, *n_dev);
   if ((int64_t)blockIdx.x * kSortTile >= n) return;
-  constexpr int BINS = 1 << BITS;
+  constexpr int BINS = kRadixBins;
   constexpr int DPT = BINS / kSortThreads;  // digits owned by one thread (consecutive)
   extern __shared__ __align__(16) unsigned char radix_smem[];
   KeyT* s_keys = reinterpret_cast<KeyT*>(radix_smem);                                     // [kSortTile]
@@ -623,9 +563,9 @@ static __global__ void __launch_bounds__(kSortThreads)
   }
 }
 
-template <typename KeyT, int BITS>
+template <typename KeyT>
 constexpr size_t radix_scatter_smem() {
-  return (sizeof(KeyT) + 4) * kSortTile + sizeof(int) * (kSortThreads / 32 + 2) * (1 << BITS);
+  return (sizeof(KeyT) + 4) * kSortTile + sizeof(int) * (kSortThreads / 32 + 2) * kRadixBins;
 }
 
 inline size_t radix_sort_workspace_bytes(int64_t n) {
@@ -636,31 +576,30 @@ inline size_t radix_sort_workspace_bytes(int64_t n) {
 // NOTE: internal linkage on purpose.  The kernels above are `static` (one copy per translation unit), so the
 // "attribute already set" flag below must be per translation unit too; an `inline` function would share one flag
 // across units and leave the other units' kernel copies without the > 48 KB shared-memory opt-in.
-template <typename KeyT, int BITS>
+template <typename KeyT>
 static int radix_pass(const KeyT* kin, const uint32_t* vin, KeyT* kout, uint32_t* vout, int64_t n,
                       const int64_t* n_dev, int shift, int* hist, int nt, Workspace& ws, cudaStream_t stream) {
-  constexpr int BINS = 1 << BITS;
   static bool smem_attr_set = false;  // per instantiation: > 48 KB dynamic shared memory needs the opt-in
   if (!smem_attr_set) {
     smem_attr_set = true;
-    cudaFuncSetAttribute(k_radix_scatter<KeyT, BITS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)radix_scatter_smem<KeyT, BITS>());
-    cudaFuncSetAttribute(k_radix_scatter<KeyT, BITS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)radix_scatter_smem<KeyT, BITS>());
+    cudaFuncSetAttribute(k_radix_scatter<KeyT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         (int)radix_scatter_smem<KeyT>());
+    cudaFuncSetAttribute(k_radix_scatter<KeyT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         (int)radix_scatter_smem<KeyT>());
   }
   if (nt == 1) {
     // one tile: the scatter kernel's own digit prefix is the global one -- one launch per pass instead of three
     hist = nullptr;
   } else {
-    launch("k_radix_hist", k_radix_hist<KeyT, BITS>, nt, kSortThreads, 0, stream, kin, n, n_dev, shift, hist, nt);
-    int rc = exclusive_scan_i32(hist, hist, (int64_t)nt * BINS, nullptr, nullptr, ws, stream);
+    launch("k_radix_hist", k_radix_hist<KeyT>, nt, kSortThreads, 0, stream, kin, n, n_dev, shift, hist, nt);
+    int rc = exclusive_scan_i32(hist, hist, (int64_t)nt * kRadixBins, nullptr, nullptr, ws, stream);
     if (rc != TGPB200_OK) return rc;
   }
   if (vin == nullptr)
-    launch("k_radix_scatter", k_radix_scatter<KeyT, BITS, true>, nt, kSortThreads, radix_scatter_smem<KeyT, BITS>(),
+    launch("k_radix_scatter", k_radix_scatter<KeyT, true>, nt, kSortThreads, radix_scatter_smem<KeyT>(),
            stream, kin, (const uint32_t*)nullptr, kout, vout, n, n_dev, shift, hist, nt);
   else
-    launch("k_radix_scatter", k_radix_scatter<KeyT, BITS, false>, nt, kSortThreads, radix_scatter_smem<KeyT, BITS>(),
+    launch("k_radix_scatter", k_radix_scatter<KeyT, false>, nt, kSortThreads, radix_scatter_smem<KeyT>(),
            stream, kin, vin, kout, vout, n, n_dev, shift, hist, nt);
   return TGPB200_OK;
 }
@@ -674,8 +613,8 @@ static int radix_sort_pairs(KeyT* keys0, uint32_t* vals0_or_null, uint32_t* vals
                             int64_t n, int key_bits, bool* result_in_1, Workspace& ws, cudaStream_t stream,
                             const int64_t* n_dev = nullptr) {
   int nt = (int)ceil_div(n > 0 ? n : 1, kSortTile);
-  const RadixPlan plan = radix_plan(key_bits);
-  int* hist = ws.take<int>((size_t)nt * (1 << plan.bits));
+  const int passes = radix_passes(key_bits);
+  int* hist = ws.take<int>((size_t)nt * kRadixBins);
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   size_t mark2 = ws.off;
   KeyT* kin = keys0;
@@ -683,13 +622,9 @@ static int radix_sort_pairs(KeyT* keys0, uint32_t* vals0_or_null, uint32_t* vals
   const uint32_t* vin = vals0_or_null;
   uint32_t* vout = vals1;
   bool in1 = false;
-  for (int p = 0; p < plan.passes; ++p) {
-    int shift = plan.bits * p;
+  for (int p = 0; p < passes; ++p) {
     ws.off = mark2;
-    int rc;
-    if (plan.bits == 8) rc = radix_pass<KeyT, 8>(kin, vin, kout, vout, n, n_dev, shift, hist, nt, ws, stream);
-    else if (plan.bits == 10) rc = radix_pass<KeyT, 10>(kin, vin, kout, vout, n, n_dev, shift, hist, nt, ws, stream);
-    else rc = radix_pass<KeyT, 11>(kin, vin, kout, vout, n, n_dev, shift, hist, nt, ws, stream);
+    int rc = radix_pass<KeyT>(kin, vin, kout, vout, n, n_dev, kRadixBits * p, hist, nt, ws, stream);
     if (rc != TGPB200_OK) return rc;
     in1 = !in1;
     KeyT* tk = kin;

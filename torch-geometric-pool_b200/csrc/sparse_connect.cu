@@ -28,11 +28,6 @@ static __global__ void k_build_table(const int64_t* __restrict__ node_index, int
 constexpr int kSmallNodes = 32768;
 constexpr int kSmallThreads = 1024;
 
-inline bool small_paths_enabled() {
-  static const bool on = [] { const char* e = getenv("TGPB200_SMALL_PATHS"); return !(e && e[0] == '0'); }();
-  return on;
-}
-
 static __global__ void __launch_bounds__(kSmallThreads)
     k_kept_init_small(const int64_t* __restrict__ node_index, int kept, int N, int32_t* __restrict__ table,
                       uint32_t* __restrict__ bits, unsigned long long* __restrict__ state, int state_words) {
@@ -868,7 +863,7 @@ int tgpb200_filter_relabel_onepass(const int64_t* row, const int64_t* col, const
   const size_t state_words = compact_onepass_state_words(E);
   unsigned long long* state = ws.take<unsigned long long>(state_words);
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
-  const bool small = small_paths_enabled() && N <= kSmallNodes && kept <= kSmallNodes && state_words <= 4096;
+  const bool small = N <= kSmallNodes && kept <= kSmallNodes && state_words <= 4096;
   if (small) {
     launch("k_kept_init_small", k_kept_init_small, 1, kSmallThreads, 0, st, node_index, (int)kept, (int)N, table, bits, state,
            (int)state_words);
@@ -906,7 +901,7 @@ int tgpb200_filter_relabel_bwd(const float* grad_out, const int32_t* src_edge, i
   if (E == 0) return TGPB200_OK;
   if (!grad_in || (num_out > 0 && (!grad_out || !src_edge))) return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
-  if (small_paths_enabled() && E <= kSmallNodes && num_out <= kSmallNodes) {  // zero fill + scatter as one launch
+  if (E <= kSmallNodes && num_out <= kSmallNodes) {  // zero fill + scatter as one launch
     launch("k_unfilter_small", k_unfilter_small, 1, kSmallThreads, 0, st, grad_out, src_edge, (int)num_out, num_out_dev, (int)E,
            grad_in);
     return launch_status();

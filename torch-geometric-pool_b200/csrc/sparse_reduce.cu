@@ -565,8 +565,7 @@ static int launch_bwd(const void* x, const int64_t* node_index, const int64_t* c
   bool vec = (F % W == 0) && Vec<OT>::N == W;
   int32_t* first = ws.take<int32_t>((size_t)(N > 0 ? N : 1));
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
-  static const bool small_path = [] { const char* e = getenv("TGPB200_SMALL_PATHS"); return !(e && e[0] == '0'); }();
-  if (small_path && N > 0 && N <= 32768 && nnz <= 32768) {
+  if (N > 0 && N <= 32768 && nnz <= 32768) {
     first = nullptr;  // the backward kernels search the (cache-resident) sorted node_index themselves: one launch less
   } else {
     cudaMemsetAsync(first, 0xff, (size_t)(N > 0 ? N : 1) * sizeof(int32_t), st);
@@ -633,8 +632,7 @@ int tgpb200_build_csr(const int64_t* cluster_index, int64_t nnz, int64_t K, int3
   uint32_t* valsA = ws.take<uint32_t>(n);
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (nnz > 0 && K == 0) return TGPB200_ERR_INVALID;
-  static const bool small_path = [] { const char* e = getenv("TGPB200_SMALL_PATHS"); return !(e && e[0] == '0'); }();
-  if (small_path && nnz <= kCsrSmallNnz && K <= kCsrSmallK) {
+  if (nnz <= kCsrSmallNnz && K <= kCsrSmallK) {
     launch("k_build_csr_small", k_build_csr_small, 1, kCsrSmallThreads, 0, st, cluster_index, (int)nnz, (int)K, order, ptr);
     return launch_status();
   }

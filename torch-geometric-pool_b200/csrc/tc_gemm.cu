@@ -265,23 +265,23 @@ __device__ __forceinline__ void store_chunk(const KernelParams& P, float (&v)[32
 constexpr int kThreads = 320;
 constexpr uint32_t kEpiStageBytes = 32 * 1024;  // 8 x 4 KB staging buffers of the TMA-store epilogue
 
-template <bool kF32>
+// bf16 engine: both operands in shared memory, one kind::f16 pass.
 __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__ KernelParams P) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  constexpr int ES = kF32 ? 4 : 2;           // operand element size
-  constexpr int EPB = kStageRowBytes / ES;   // elements per 128-byte line (= BK)
+  constexpr int EPB = kStageRowBytes / 2;    // bf16 elements per 128-byte line (= BK)
   constexpr int BK = EPB;
-  constexpr int UMMA_K = 32 / ES;            // 8 (tf32) or 16 (bf16): 32 bytes of K per instruction
+  constexpr int UMMA_K = 16;                 // 32 bytes of K per instruction
   constexpr int KSTEPS = BK / UMMA_K;        // 4
 
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const int BN = P.BN;
   const uint32_t a_bytes = BM * kStageRowBytes, b_bytes = (uint32_t)BN * kStageRowBytes;
-  const uint32_t stage_bytes = (a_bytes + b_bytes) * (kF32 ? 2 : 1);
+  const uint32_t stage_bytes = a_bytes + b_bytes;
   const int stages = P.stages;
   // [stages][stage_bytes] | epilogue staging (kEpiStageBytes, TMA stores) | barriers
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)stage_bytes * stages + kEpiStageBytes);
-  // barrier layout: full[stages], lo[stages], empty[stages], tmem_full[2], tmem_empty[2]
+  // barrier layout: full[stages], lo[stages], empty[stages], tmem_full[2], tmem_empty[2] -- the layout of
+  // k_tc_gemm_ts, which gemm() sizes the shared memory for; nothing here waits on lo[]
   const uint32_t bar_base = smem_u32(bars);
   auto bar_full = [&](int s) { return bar_base + 8u * s; };
   auto bar_lo = [&](int s) { return bar_base + 8u * (stages + s); };
@@ -301,7 +301,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(bar_tfull(i), 1);
-      mbar_init(bar_tempty(i), kF32 ? 128 : 256);
+      mbar_init(bar_tempty(i), 256);
     }
     fence_barrier_init();
   }
@@ -356,8 +356,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__
   } else if (warp == 1) {
     // ===================== MMA issuer: ONE elected thread runs the whole loop =====================
     // (electing per k-block and reconverging the warp afterwards costs ~150 cycles per iteration: mma_rate.cu, k_loop)
-    // instruction descriptor: c=F32 (1<<4), a/b format, a/b major, N>>3 at [17,23), M>>4 at [24,29)
-    const uint32_t fmt = kF32 ? 2u : 1u;  // TF32 : BF16
+    // instruction descriptor: c=F32 (1<<4), a/b format BF16 (1), a/b major, N>>3 at [17,23), M>>4 at [24,29)
     const uint32_t tm = __shfl_sync(kFull, tmem_base, 0);
     if (elect_one()) {
       int s = 0;
@@ -368,37 +367,25 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__
         uint32_t aph = (uint32_t)(it >> 1) & 1u;
         mbar_wait(bar_tempty(ab), aph ^ 1);
         tc_fence_after();
-        // fp32: the accumulator is 2 BN columns wide: [hi_a hi_b + lo_a hi_b | hi_a lo_b] (summed by the epilogue)
-        uint32_t d_tmem = tm + (uint32_t)(ab * (kF32 ? 2 * BN : BN));
+        uint32_t d_tmem = tm + (uint32_t)(ab * BN);
         uint32_t accum = 0;
         for (int p = 0; p < P.num_pairs; ++p) {
-          const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)P.a_mn[p] << 15) |
+          const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)P.a_mn[p] << 15) |
                                  ((uint32_t)P.b_mn[p] << 16) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-          // same with N = 2 BN: one instruction multiplies hi_a by [hi_b | lo_b] (the lo tile sits right behind the
-          // hi tile of B in shared memory): 3xTF32 as two instructions per k-step instead of three.
-          const uint32_t idesc2 = (idesc & ~(0x3fu << 17)) | ((uint32_t)((2 * BN) >> 3) << 17);
           const uint32_t a_lbo = P.a_mn[p] ? BK * kStageRowBytes : 16, b_lbo = P.b_mn[p] ? BK * kStageRowBytes : 16;
           const uint32_t a_step = P.a_mn[p] ? UMMA_K * kStageRowBytes : 32, b_step = P.b_mn[p] ? UMMA_K * kStageRowBytes : 32;
-          // fp32 MN-major tiles use 4-row (512 B) swizzle atoms, everything else 8-row (1024 B) atoms
-          const uint64_t desc_a0 = make_desc(smem_base, a_lbo, (kF32 && P.a_mn[p]) ? 512 : 1024, (kF32 && P.a_mn[p]) ? 1 : 2);
-          const uint64_t desc_b0 = make_desc(smem_base, b_lbo, (kF32 && P.b_mn[p]) ? 512 : 1024, (kF32 && P.b_mn[p]) ? 1 : 2);
+          const uint64_t desc_a0 = make_desc(smem_base, a_lbo, 1024, 2);
+          const uint64_t desc_b0 = make_desc(smem_base, b_lbo, 1024, 2);
           for (int kb = 0, nkb = (P.kd[p] + BK - 1) / BK; kb < nkb; ++kb) {
             mbar_wait(bar_full(s), ph);
-            if (kF32) mbar_wait(bar_lo(s), ph);
             tc_fence_after();
             // descriptors differ only in the 14-bit start-address field: build once per pair, then add offsets
             const uint32_t so = ((uint32_t)s * stage_bytes) >> 4;
             const uint64_t da0 = desc_a0 + so, db0 = desc_b0 + so + (a_bytes >> 4);
-            const uint32_t a_lo_off = (a_bytes + 2 * b_bytes) >> 4;  // stage = [A | B | B lo | A lo]
 #pragma unroll
             for (int kk = 0; kk < KSTEPS; ++kk) {
               const uint64_t da = da0 + (uint64_t)(kk * (a_step >> 4)), db = db0 + (uint64_t)(kk * (b_step >> 4));
-              if (kF32) {
-                umma<true>(d_tmem, da, db, idesc2, kk == 0 ? accum : 1u);  // hi_a x [hi_b | lo_b]
-                umma<true>(d_tmem, da + a_lo_off, db, idesc, 1u);          // lo_a x hi_b
-              } else {
-                umma<false>(d_tmem, da, db, idesc, kk == 0 ? accum : 1u);
-              }
+              umma<false>(d_tmem, da, db, idesc, kk == 0 ? accum : 1u);
             }
             umma_commit(bar_empty(s));
             accum = 1;
@@ -409,53 +396,13 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__
       }
     }
     __syncwarp();
-  } else if (kF32 && warp < 6) {
-    // ===================== operand split (fp32 only): lo = x - trunc_tf32(x) =====================
-    {
-      const int t = threadIdx.x - 64;  // 0..127
-      int s = 0;
-      uint32_t ph = 0;
-      const uint32_t raw_bytes = a_bytes + b_bytes;
-      for (int item = blockIdx.x; item < P.num_items; item += gridDim.x) {
-        for (int p = 0; p < P.num_pairs; ++p) {
-          for (int kb = 0, nkb = (P.kd[p] + BK - 1) / BK; kb < nkb; ++kb) {
-            mbar_wait(bar_full(s), ph);
-            // round-to-nearest split: hi = rna_tf32(x) overwrites the TMA tile in place, lo = x - hi goes next
-            // to it.  (The tensor core truncates its fp32 inputs to tf32; with a truncated hi the residual error
-            // is one-sided and adds up coherently over long sums, with a rounded hi it is ~2^-23 and zero-mean.)
-            // stage layout [A | B | B lo | A lo]: the lo tile of B directly follows its hi tile (N-concatenated operand)
-            const uint32_t raw = smem_base + (uint32_t)s * stage_bytes;
-            const uint32_t nvec = raw_bytes / 16;  // multiple of 512 (BM and BN are multiples of 64 rows)
-            const uint32_t a_vec = a_bytes / 16;   // multiple of 512 as well: a batch never straddles A and B
-            for (uint32_t i0 = t; i0 < nvec; i0 += 128 * 4) {
-              const uint32_t lo_delta = i0 < a_vec ? a_bytes + 2 * b_bytes : b_bytes;
-              float4 v[4];
-#pragma unroll
-              for (int u = 0; u < 4; ++u) v[u] = lds128(raw + (i0 + u * 128) * 16);
-#pragma unroll
-              for (int u = 0; u < 4; ++u) {
-                float4 h, r;
-                h.x = rna_tf32(v[u].x), h.y = rna_tf32(v[u].y), h.z = rna_tf32(v[u].z), h.w = rna_tf32(v[u].w);
-                r.x = v[u].x - h.x, r.y = v[u].y - h.y, r.z = v[u].z - h.z, r.w = v[u].w - h.w;
-                sts128(raw + (i0 + u * 128) * 16, h);
-                sts128(raw + lo_delta + (i0 + u * 128) * 16, r);
-              }
-            }
-            fence_proxy_async();
-            mbar_arrive(bar_lo(s));
-            if (++s == stages) { s = 0; ph ^= 1; }
-          }
-        }
-      }
-    }
   } else {
-    // ===================== epilogue: TMEM -> registers -> global =====================
-    // fp32: warps 6-9.  bf16 needs no split warps, so warps 2-5 join: each quadrant's two warps take alternate
-    // 32-column chunks (the fused element-wise epilogue of the backward is instruction-bound with four warps).
+    // ===================== epilogue (warps 2-9): TMEM -> registers -> global =====================
+    // Each quadrant's two warps take alternate 32-column chunks (the fused element-wise epilogue of the backward is
+    // instruction-bound with four warps); every warp owns one 4 KB staging buffer.
     const int quad = warp & 3;  // TMEM lane quadrant this warp may access
-    const int c_first = (!kF32 && warp < 6) ? 32 : 0, c_step = kF32 ? 32 : 64;
-    // fp32: four epilogue warps with two staging buffers each; bf16: eight warps with one
-    EpiStage es{smem_base + (uint32_t)stage_bytes * stages + (uint32_t)(kF32 ? (warp - 6) * 2 : (warp - 2)) * 4096u, 0};
+    const int c_first = warp < 6 ? 32 : 0, c_step = 64;
+    EpiStage es{smem_base + (uint32_t)stage_bytes * stages + (uint32_t)(warp - 2) * 4096u, 0};
     int it = 0;
     for (int item = blockIdx.x; item < P.num_items; item += gridDim.x, ++it) {
       int nt = item % P.n_tiles, mt = (item / P.n_tiles) % P.m_tiles, b = item / (P.n_tiles * P.m_tiles);
@@ -466,25 +413,18 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__
       const int64_t obase = (int64_t)b * P.out_bs + (int64_t)m * P.out_rs;
       // element-wise terms: coefficients of this row and the S values of the first chunk before the accumulators are
       // waited for, the values of chunk c + 1 while chunk c is processed
-      EwPre<kF32> ew, ew_next;
-      ew_item<kF32>(P, ew, b, m);
-      ew_load<kF32>(P, ew, b, m, nt * BN + c_first);
+      EwPre<false> ew, ew_next;
+      ew_item<false>(P, ew, b, m);
+      ew_load<false>(P, ew, b, m, nt * BN + c_first);
       mbar_wait(bar_tfull(ab), aph);
       tc_fence_after();
       for (int c0 = c_first; c0 < BN; c0 += c_step) {
         ew_next = ew;
-        if (c0 + c_step < BN) ew_load<kF32>(P, ew_next, b, m, nt * BN + c0 + c_step);
+        if (c0 + c_step < BN) ew_load<false>(P, ew_next, b, m, nt * BN + c0 + c_step);
         float v[32];
-        uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(ab * (kF32 ? 2 * BN : BN) + c0);
-        tmem_ld32(taddr, v);
-        if (kF32) {  // + hi_a x lo_b
-          float v2[32];
-          tmem_ld32(taddr + (uint32_t)BN, v2);
-#pragma unroll
-          for (int j = 0; j < 32; ++j) v[j] += v2[j];
-        }
+        tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(ab * BN + c0), v);
         const int n0 = nt * BN + c0;
-        if (n0 < P.N && m_base < P.M) store_chunk<kF32>(P, v, b, m_base, m, n0, obase, es, ew);  // warp-uniform test
+        if (n0 < P.N && m_base < P.M) store_chunk<false>(P, v, b, m_base, m, n0, obase, es, ew);  // warp-uniform test
         ew = ew_next;
       }
       tc_fence_before();
@@ -496,179 +436,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__
   tc_fence_before();
   __syncthreads();
   if (warp == 1) tmem_dealloc(tmem_base, P.tmem_cols);
-}
-
-// ------------------------------------------------------------------------------------------
-// bf16 engine on CTA pairs (tcgen05 cta_group::2): the two CTAs of a cluster compute ONE 256 x BN tile.  Each CTA
-// stages its own 128 rows of A and HALF of the B tile, so a B operand crosses L2 -> SM once per 256 output rows
-// instead of once per 128 (the batched products of the dense path are bound by exactly that traffic).
-//   * both CTAs run a TMA producer; every load signals the LEADER's full barrier (transaction bytes of both CTAs),
-//   * only the leader issues tcgen05.mma.cta_group::2; its commits are multicast to the empty / tmem-full barriers
-//     of both CTAs,
-//   * each CTA's eight epilogue warps drain the CTA's own 128 TMEM lanes and arrive on the leader's tmem-empty
-//     barrier (count 2 x 256).
-// P.m_tiles counts 256-row tiles here.
-// ------------------------------------------------------------------------------------------
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
-    k_tc_gemm_pair(const __grid_constant__ KernelParams P) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  constexpr int EPB = kStageRowBytes / 2;  // 64 bf16 per 128-byte line (= BK)
-  constexpr int BK = EPB;
-  constexpr int UMMA_K = 16;
-  constexpr int KSTEPS = BK / UMMA_K;
-
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  const int BN = P.BN, HN = BN / 2;
-  const uint32_t a_bytes = BM * kStageRowBytes, b_bytes = (uint32_t)HN * kStageRowBytes;  // per CTA
-  const uint32_t stage_bytes = a_bytes + b_bytes;
-  const int stages = P.stages;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)stage_bytes * stages);
-  const uint32_t bar_base = smem_u32(bars);
-  auto bar_full = [&](int s) { return bar_base + 8u * s; };
-  auto bar_empty = [&](int s) { return bar_base + 8u * (stages + s); };
-  auto bar_tfull = [&](int i) { return bar_base + 8u * (2 * stages + i); };
-  auto bar_tempty = [&](int i) { return bar_base + 8u * (2 * stages + 2 + i); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * stages + 4);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t smem_base = smem_u32(smem);
-  const uint32_t rank = cluster_ctarank();
-  const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < stages; ++s) {
-      mbar_init(bar_full(s), 1);   // the leader's producer expects the bytes of BOTH CTAs (used in the leader only)
-      mbar_init(bar_empty(s), 1);  // multicast commit
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(bar_tfull(i), 1);     // multicast commit
-      mbar_init(bar_tempty(i), 512);  // 2 CTAs x 8 epilogue warps (used in the leader only)
-    }
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc_pair(smem_u32(tmem_slot), P.tmem_cols);
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();  // the peer's barriers are initialised before any remote arrive / TMA signal
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  // (k-block counts come from the kernel parameters each time: a dynamically indexed local array lives in local
-  //  memory, and with 227 KB of the L1 carved out as shared memory those loads miss to L2 inside the hot loops)
-
-  if (warp == 0) {
-    // ===================== TMA producer (both CTAs) =====================
-    if (lane == 0) {
-      int s = 0;
-      uint32_t ph = 0;
-      for (int item = pair; item < P.num_items; item += npairs) {
-        int nt = item % P.n_tiles, mt = (item / P.n_tiles) % P.m_tiles, b = item / (P.n_tiles * P.m_tiles);
-        const int m0 = (mt * 2 + (int)rank) * BM, n0 = nt * BN + (int)rank * HN;
-        for (int p = 0; p < P.num_pairs; ++p) {
-          for (int kb = 0, nkb = (P.kd[p] + BK - 1) / BK; kb < nkb; ++kb) {
-            mbar_wait(bar_empty(s), ph ^ 1);
-            const uint32_t sa = smem_base + (uint32_t)s * stage_bytes, sb = sa + a_bytes;
-            const uint32_t lf = mapa_shared(bar_full(s), 0);
-            // A remote arrive.expect_tx per stage from the peer measured 2x slower end to end (cluster-scope release
-            // on the producer's critical path); the peer's bytes may land before the leader's expect_tx of the same
-            // phase (the transaction count goes negative transiently), never after the phase: the peer refills a
-            // stage only after the multicast commit that follows the phase's completion.
-            if (rank == 0) mbar_arrive_expect_tx(bar_full(s), 2 * (a_bytes + b_bytes));
-            const int k0 = kb * BK;
-            if (P.a_mn[p]) {
-              for (int blk = 0; blk < BM / EPB; ++blk)
-                tma_load_3d_pair(sa + blk * (BK * kStageRowBytes), &P.map_a[p], lf, m0 + blk * EPB, k0, b);
-            } else {
-              tma_load_3d_pair(sa, &P.map_a[p], lf, k0, m0, b);
-            }
-            if (P.b_mn[p]) {
-              for (int blk = 0; blk < HN / EPB; ++blk)
-                tma_load_3d_pair(sb + blk * (BK * kStageRowBytes), &P.map_b[p], lf, n0 + blk * EPB, k0, b);
-            } else {
-              tma_load_3d_pair(sb, &P.map_b[p], lf, k0, n0, b);  // box rows = BN / 2
-            }
-            if (++s == stages) { s = 0; ph ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer (leader CTA only; whole warp, one elected lane issues) =====================
-    if (rank == 0) {
-      const uint32_t tm = __shfl_sync(kFull, tmem_base, 0);
-      int s = 0;
-      uint32_t ph = 0;
-      int it = 0;
-      for (int item = pair; item < P.num_items; item += npairs, ++it) {
-        const int ab = it & 1;
-        const uint32_t aph = (uint32_t)(it >> 1) & 1u;
-        mbar_wait(bar_tempty(ab), aph ^ 1);
-        tc_fence_after();
-        const uint32_t d_tmem = tm + (uint32_t)(ab * BN);
-        uint32_t accum = 0;
-        for (int p = 0; p < P.num_pairs; ++p) {
-          // bf16 x bf16 -> f32, M = 256 over the pair, N = BN
-          const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)P.a_mn[p] << 15) |
-                                 ((uint32_t)P.b_mn[p] << 16) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-          const uint32_t a_lbo = P.a_mn[p] ? BK * kStageRowBytes : 16, b_lbo = P.b_mn[p] ? BK * kStageRowBytes : 16;
-          const uint32_t a_step = P.a_mn[p] ? UMMA_K * kStageRowBytes : 32, b_step = P.b_mn[p] ? UMMA_K * kStageRowBytes : 32;
-          const uint64_t desc_a0 = make_desc(smem_base, a_lbo, 1024, 2);
-          const uint64_t desc_b0 = make_desc(smem_base, b_lbo, 1024, 2);
-          for (int kb = 0, nkb = (P.kd[p] + BK - 1) / BK; kb < nkb; ++kb) {
-            mbar_wait(bar_full(s), ph);
-            tc_fence_after();
-            const uint32_t so = ((uint32_t)s * stage_bytes) >> 4;
-            const uint64_t da0 = desc_a0 + so, db0 = desc_b0 + so + (a_bytes >> 4);
-            if (elect_one()) {
-#pragma unroll
-              for (int kk = 0; kk < KSTEPS; ++kk)
-                umma_pair_bf16(d_tmem, da0 + (uint64_t)(kk * (a_step >> 4)), db0 + (uint64_t)(kk * (b_step >> 4)), idesc,
-                               kk == 0 ? accum : 1u);
-              umma_commit_pair(bar_empty(s));  // frees the stage in both CTAs
-            }
-            __syncwarp();
-            accum = 1;
-            if (++s == stages) { s = 0; ph ^= 1; }
-          }
-        }
-        if (elect_one()) umma_commit_pair(bar_tfull(ab));  // accumulator halves ready in both CTAs
-        __syncwarp();
-      }
-    }
-  } else {
-    // ===================== epilogue (both CTAs): own 128 TMEM lanes -> global =====================
-    const int quad = warp & 3;
-    const int c_first = warp < 6 ? 32 : 0;
-    EpiStage es{0u, 0};  // P.tma_out is never set for the pair engine
-    int it = 0;
-    for (int item = pair; item < P.num_items; item += npairs, ++it) {
-      int nt = item % P.n_tiles, mt = (item / P.n_tiles) % P.m_tiles, b = item / (P.n_tiles * P.m_tiles);
-      const int ab = it & 1;
-      const uint32_t aph = (uint32_t)(it >> 1) & 1u;
-      mbar_wait(bar_tfull(ab), aph);
-      tc_fence_after();
-      const int m_base = (mt * 2 + (int)rank) * BM + quad * 32;
-      const int m = m_base + lane;
-      const int64_t obase = (int64_t)b * P.out_bs + (int64_t)m * P.out_rs;
-      for (int c0 = c_first; c0 < BN; c0 += 64) {
-        float v[32];
-        tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(ab * BN + c0), v);
-        const int n0 = nt * BN + c0;
-        if (n0 >= P.N || m_base >= P.M) continue;  // warp-uniform
-        EwPre<false> ew;
-        ew_item<false>(P, ew, b, m);
-        ew_load<false>(P, ew, b, m, n0);
-        store_chunk<false>(P, v, b, m_base, m, n0, obase, es, ew);
-      }
-      tc_fence_before();
-      mbar_arrive_cluster(mapa_shared(bar_tempty(ab), 0));
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();  // both CTAs are done with TMEM and with each other's barriers
-  if (warp == 1) tmem_dealloc_pair(tmem_base, P.tmem_cols);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1090,32 +857,14 @@ int gemm(const GemmProblem& p, cudaStream_t stream) {
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
     if (num_sms <= 0) num_sms = 148;
-    cudaFuncSetAttribute(k_tc_gemm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    cudaFuncSetAttribute(k_tc_gemm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    cudaFuncSetAttribute(k_tc_gemm_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(k_tc_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     cudaFuncSetAttribute(k_tc_gemm_ts, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   }
   KernelParams P;
   memset(&P, 0, sizeof(P));
   const bool bf16 = p.in_bf16 != 0;
   P.BN = pick_bn(p);
-  // CTA pairs (cta_group::2, 256-row tiles) for bf16 products with at least two 128-row tiles per batch item.
-  // Opt-in (TGPB200_GEMM_PAIR=1): measured on B200 it is on par with the single-CTA engine for the batched products
-  // of the dense path (they run at ~5.3 TB/s of HBM traffic, i.e. they are HBM-bound, not L2->SM bound) and 8 %
-  // slower on a compute-bound 4096^3 product (1132 vs 1232 TFLOP/s; longer cross-CTA hand-off per stage).
-  bool pair = false;
-  {
-    const char* e = getenv("TGPB200_GEMM_PAIR");
-    pair = e && e[0] == '1' && bf16 && p.M > BM && P.BN >= 64 && num_sms >= 2;
-  }
-  for (int i = 0; i < p.num_pairs && pair; ++i)
-    if (p.b[i].mn_major && P.BN % 128 != 0) pair = false;  // each CTA needs whole 128-byte blocks of its half of B
-  bool ts = !bf16;  // fp32: A operand staged in tensor memory
-  {
-    const char* e = getenv("TGPB200_GEMM_TS");
-    if (e && e[0] == '0') ts = false;
-  }
-  const int tile_m = pair ? 2 * BM : BM;
+  const bool ts = !bf16;  // fp32: A operand staged in tensor memory (k_tc_gemm_ts)
   P.num_pairs = p.num_pairs;
   P.batch = p.batch, P.M = p.M, P.N = p.N;
   // Small per-item products (M, N <= 64: the [K, K] products of the pooled graphs) leave three quarters of a 128 x 128
@@ -1124,11 +873,11 @@ int gemm(const GemmProblem& p, cudaStream_t stream) {
   // their products (the off-diagonal blocks are computed and dropped: the MMA costs N/2 cycles either way).
   {
     const char* e = getenv("TGPB200_GEMM_PACK2");
-    P.pack2 = ts && !pair && !(e && e[0] == '0') && p.num_pairs == 1 && p.M <= 64 && p.N <= 64 && p.batch >= 2 &&
+    P.pack2 = ts && !(e && e[0] == '0') && p.num_pairs == 1 && p.M <= 64 && p.N <= 64 && p.batch >= 2 &&
               !p.a[0].mn_major && p.b[0].mn_major && p.ew_S == nullptr && p.out_col_stride == 1;
   }
   if (P.pack2) P.BN = 128;
-  P.m_tiles = (p.M + tile_m - 1) / tile_m, P.n_tiles = (p.N + P.BN - 1) / P.BN;
+  P.m_tiles = (p.M + BM - 1) / BM, P.n_tiles = (p.N + P.BN - 1) / P.BN;
   P.num_items = P.pack2 ? (p.batch + 1) / 2 : p.batch * P.m_tiles * P.n_tiles;
   for (int i = 0; i < p.num_pairs; ++i) {
     P.kd[i] = p.kd[i];
@@ -1138,19 +887,17 @@ int gemm(const GemmProblem& p, cudaStream_t stream) {
     } else if (!make_operand_map(&P.map_a[i], p.a[i], bf16, p.batch, p.M, p.kd[i], P.pack2 ? 64 : BM)) {
       return TGPB200_ERR_UNSUPPORTED;
     }
-    if (!make_operand_map(&P.map_b[i], p.b[i], bf16, p.batch, p.N, p.kd[i], pair ? P.BN / 2 : P.BN)) return TGPB200_ERR_UNSUPPORTED;
+    if (!make_operand_map(&P.map_b[i], p.b[i], bf16, p.batch, p.N, p.kd[i], P.BN)) return TGPB200_ERR_UNSUPPORTED;
   }
-  const size_t stage_bytes = pair ? (size_t)(BM + P.BN / 2) * kStageRowBytes
-                             : ts ? (size_t)(BM + 2 * P.BN) * kStageRowBytes
-                                  : (size_t)(BM + P.BN) * kStageRowBytes * (bf16 ? 1 : 2);
+  const size_t stage_bytes = (size_t)(BM + (ts ? 2 : 1) * P.BN) * kStageRowBytes;
   const size_t budget = 192 * 1024;  // + 32 KB of epilogue staging + barriers + alignment slack <= 227 KB
   int stages = (int)(budget / stage_bytes);
-  if (stages > (pair ? 8 : 6)) stages = pair ? 8 : 6;
+  if (stages > 6) stages = 6;
   if (stages < 2) return TGPB200_ERR_UNSUPPORTED;
   P.stages = stages;
   uint32_t cols = 32;
-  // shared-memory fp32 accumulators are 2 BN wide ([.. | hi_a lo_b]); the TMEM-operand form adds a 2 x 64 column ring
-  while (cols < (uint32_t)(ts ? 2 * P.BN + kTsSlots * kRingCols : (bf16 ? 2 : 4) * P.BN)) cols <<= 1;
+  // two BN-wide accumulators; the TMEM-operand engine adds its ring of operand slots
+  while (cols < (uint32_t)(2 * P.BN + (ts ? kTsSlots * kRingCols : 0))) cols <<= 1;
   P.tmem_cols = cols;
   P.out = p.out, P.out_bs = p.out_batch_stride, P.out_rs = p.out_row_stride, P.out_cs = p.out_col_stride;
   P.alpha = p.alpha, P.accumulate = p.accumulate, P.out_bf16 = p.out_bf16;
@@ -1164,12 +911,11 @@ int gemm(const GemmProblem& p, cudaStream_t stream) {
   // TMA-store epilogue: row-major destination, no read-modify-write, 16-byte aligned rows
   {
     const int oes = p.out_bf16 ? 2 : 4;
-    const char* e = getenv("TGPB200_GEMM_TMA_STORE");
     // staging tiles per epilogue warp: the fp32 engine's four warps own 8 KB each, the bf16 engine's eight warps 4 KB
     // each -- room for two 2 KB bf16 chunks, so a store can still read one while the next chunk is staged
     P.epi_bufs = bf16 ? (p.out_bf16 ? 2 : 1) : 2;
     P.tma_out = 0;
-    if (!(e && e[0] == '0') && !pair && p.out_col_stride == 1 && !p.accumulate && ((uintptr_t)p.out & 15) == 0 &&
+    if (p.out_col_stride == 1 && !p.accumulate && ((uintptr_t)p.out & 15) == 0 &&
         (p.out_row_stride * oes) % 16 == 0 && (p.out_batch_stride * oes) % 16 == 0 && p.out_row_stride >= p.N) {
       EncodeTiledFn fn = encode_fn();
       cuuint64_t dims[3] = {(cuuint64_t)p.N, (cuuint64_t)p.M, (cuuint64_t)p.batch};
@@ -1184,20 +930,12 @@ int gemm(const GemmProblem& p, cudaStream_t stream) {
     }
   }
   const size_t smem = stage_bytes * stages + kEpiStageBytes + (3 * stages + 4) * 8 + 16 + 1024;
-  if (pair) {
-    int npairs = P.num_items < num_sms / 2 ? P.num_items : num_sms / 2;
-    launch(p.tag ? p.tag : "k_tc_gemm_pair_bf16", k_tc_gemm_pair, 2 * npairs, kThreads, smem, stream, P);
-    return launch_status();
-  }
   int grid = P.num_items < num_sms ? P.num_items : num_sms;
   if (ts) {
     launch(p.tag ? p.tag : "k_tc_gemm_ts_3xtf32", k_tc_gemm_ts, grid, kThreadsTs, smem + 64, stream, P);
     return launch_status();
   }
-  if (bf16)
-    launch(p.tag ? p.tag : "k_tc_gemm_bf16", k_tc_gemm<false>, grid, kThreads, smem, stream, P);
-  else
-    launch(p.tag ? p.tag : "k_tc_gemm_3xtf32", k_tc_gemm<true>, grid, kThreads, smem, stream, P);
+  launch(p.tag ? p.tag : "k_tc_gemm_bf16", k_tc_gemm, grid, kThreads, smem, stream, P);
   return launch_status();
 }
 

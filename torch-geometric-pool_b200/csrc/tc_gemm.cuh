@@ -5,17 +5,16 @@
 // * operands arrive by TMA (cp.async.bulk.tensor, 128B swizzle) into a multi-stage shared-memory ring,
 // * one elected thread issues tcgen05.mma (cta_group::1, M = 128) with the accumulator in TMEM
 //   (double-buffered so the epilogue of tile t overlaps the main loop of tile t+1),
-// * fp32 inputs use the error-compensated 3xTF32 scheme (hi*hi + hi*lo + lo*hi, kind::tf32): four "split"
-//   warps rewrite each fp32 tile in shared memory as hi = rna_tf32(x) (in place) and lo = x - hi (next to it);
-//   bf16 inputs are a single kind::f16 pass,
+// * bf16 inputs are a single kind::f16 pass with both operands in shared memory (k_tc_gemm, 320 threads: warp 0 =
+//   TMA producer, warp 1 = MMA issuer + TMEM allocator, warps 2-9 = epilogue),
+// * fp32 inputs use the error-compensated 3xTF32 scheme (hi*hi + hi*lo + lo*hi, kind::tf32) with the A operand in
+//   tensor memory (k_tc_gemm_ts): "split" warps write hi = rna_tf32(x) and lo = x - hi of the A tile into TMEM and of
+//   the B tile into shared memory,
 // * either operand may be K-major or MN-major in global memory (no transposes are materialised),
 // * the epilogue reads TMEM with tcgen05.ld and writes fp32 or bf16 through swizzled shared-memory tiles and TMA
 //   stores when the output is row-contiguous and 16-byte aligned (per-thread stores with arbitrary strides otherwise).
 //
-// Warp roles (320 threads): warp 0 = TMA producer, warp 1 = MMA issuer + TMEM allocator (one elected thread runs the
-// issuing loop), warps 2-5 = operand split (fp32) / extra epilogue warps (bf16), warps 6-9 = epilogue.
-// (Eight split warps for fp32, data-parallel or as two groups on alternate stages, measured no faster: 53 us on the
-// C2-shaped products either way -- with operands in shared memory the engine sits on the shared-memory pipe.)
+// One elected thread of the MMA warp runs the whole issuing loop.
 #pragma once
 #include <cuda.h>
 

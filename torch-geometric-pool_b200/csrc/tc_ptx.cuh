@@ -124,58 +124,6 @@ __device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t desc_a, uint64_t 
         : "memory");
   }
 }
-// ------------------------------------------------------------------------------------------
-// CTA-pair (cta_group::2) variants: two CTAs of a cluster share one 256-row MMA tile.
-// ------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// shared::cluster address of the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
-}
-// TMA load into this CTA's shared memory that signals a barrier of the pair's leader CTA
-__device__ __forceinline__ void tma_load_3d_pair(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1,
-                                                 int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::
-          "r"(dst),
-      "l"(map), "r"(leader_bar), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t addr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(ncols) : "memory");
-}
-// arrive (once the issued MMAs have completed) on the barrier at this offset in both CTAs of the pair
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
-  asm volatile(
-      "{\n.reg .b16 m;\nmov.b16 m, 3;\n"
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], m;\n}\n" ::"r"(bar)
-      : "memory");
-}
-__device__ __forceinline__ void umma_pair_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                               uint32_t accum) {
-  asm volatile(
-      "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accum)
-      : "memory");
-}
 
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
   uint32_t r[32];
