@@ -35,45 +35,29 @@
 namespace tgp {
 namespace tc {
 
-extern long long* g_engine_dbg;
-
 namespace {
 
-// 4 epilogue warps keep the CTA at 448 threads: registers are allocated per 128 threads, so 576 threads are budgeted as
-// 640 (96 registers per thread, spills inside the pipeline loops) while 448 get 128 registers and no spill.
-#ifndef TGPB200_BWD_EPI_WARPS
-#define TGPB200_BWD_EPI_WARPS 4
-#endif
-// Ablation switches (timing experiments only, results are wrong when any bit is set): benchmarks/ablate_bwd.sh
-#ifndef TGPB200_ABL
-#define TGPB200_ABL 0
-#endif
-#ifndef TGPB200_BWD_CONCAT
-#define TGPB200_BWD_CONCAT 0
-#endif
-// Optional (TGPB200_BWD_CONCAT=1): 3xTF32 of the W / dS pairs as TWO instructions per k-step, hi_a x [hi_b | lo_b]
-// (N = 128: the lo tile of B directly follows its hi tile in shared memory) + lo_a x hi_b (N = 64), with 128-column
-// accumulators ([.. | hi_a lo_b], summed by whoever reads them).  Fewer instructions, but the wider accumulators leave
-// room for two operand slots only; measured equal to the three-instruction form, which keeps four slots.
-constexpr bool kConcat = TGPB200_BWD_CONCAT != 0;
 constexpr int kPairs = 7;
 constexpr int kGroups = 2;                 // split groups (k-block kc goes to group kc % kGroups)
 // TMEM operand ring: the slot of k-block kc is kc % kSlots.  A slot is recycled when the MMAs that read it have
 // RETIRED (tcgen05.commit -> mbarrier -> the split warps' wait): with as many slots as split groups that round trip
-// (~1.8 k cycles: benchmarks/ablate_bwd.sh, every stage of the pipeline emptied) bounds the kernel at one k-block per
+// (~1.8 k cycles, measured with every stage of the pipeline emptied) bounds the kernel at one k-block per
 // ~900 cycles whatever the k-block contains.  With more slots than groups the split warps never wait for it.
-constexpr int kSlots = kConcat ? 2 : 4;
+constexpr int kSlots = 4;
 static_assert(kSlots % kGroups == 0, "every operand slot must belong to ONE split group (its waiters see every phase)");
-constexpr int kEpiW = TGPB200_BWD_EPI_WARPS;  // epilogue warps (one or two per TMEM lane quadrant)
+// 4 epilogue warps (one per TMEM lane quadrant) keep the CTA at 448 threads: registers are allocated per 128 threads, so
+// 576 threads are budgeted as 640 (96 registers per thread, spills inside the pipeline loops) while 448 get 128
+// registers and no spill.
+constexpr int kEpiW = 4;
 constexpr int kThreadsBwd = 64 + kGroups * 128 + kEpiW * 32;
 constexpr int BK = 32, KSTEPS = 4;
 constexpr int BNB = 64;                    // MMA N of every pair
-constexpr uint32_t kAccW = kConcat ? 128 : 64;  // width of the W and dS accumulators
+constexpr uint32_t kAccW = 64;             // width of the W and dS accumulators
 constexpr uint32_t kColW = 0, kColS = kAccW, kColX = 2 * kAccW, kColRing = 2 * kAccW + 128, kRing = 64;
 static_assert(kColRing + kSlots * kRing <= 512, "tensor memory budget");
 constexpr uint32_t kABytes = BM * kStageRowBytes, kBBytes = BNB * kStageRowBytes;
 constexpr uint32_t kStage = kABytes + 2 * kBBytes;  // [A raw | B hi | B lo] = 32 KB
-constexpr uint32_t kEpiBufs = kEpiW == 4 ? 2 : 1;  // staging tiles per epilogue warp (32 KB in total)
+constexpr uint32_t kEpiBufs = 2;          // staging tiles per epilogue warp (32 KB in total)
 constexpr uint32_t kEpiBytes = kEpiW * kEpiBufs * 4096;
 // rows of S for the element-wise terms of dS: 128 rows x 64 columns fp32, prefetched with cp.async while the item's MMAs run
 constexpr uint32_t kHookBytes = BM * BNB * 4;
@@ -82,7 +66,7 @@ enum ASrc { kAKMajor = 0, kAMnPlain = 1, kATmem = 2 };
 
 struct BwdParams {
   CUtensorMap map_a[kPairs], map_b[kPairs];
-  int kd[kPairs], a_src[kPairs], b_mn[kPairs], b_n0[kPairs], first[kPairs], wide[kPairs];
+  int kd[kPairs], a_src[kPairs], b_mn[kPairs], b_n0[kPairs], first[kPairs];
   uint32_t acc_col[kPairs];
   int num_pairs;
   int batch, N, K, F;
@@ -93,7 +77,6 @@ struct BwdParams {
   const float* coef;
   const float* uv;     // [B, 2, K]: DMoN term d_i u_k + v_k of dS (nullptr: none)
   float eps;
-  long long* dbg;
 };
 
 __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid_constant__ BwdParams P) {
@@ -112,14 +95,6 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t smem_base = smem_u32(smem);
-  if (P.dbg && threadIdx.x == 0) {  // per-CTA start (global timer, ns) and SM id: rows 200.. of the debug buffer
-    unsigned long long t;
-    uint32_t smid;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    P.dbg[(200 + blockIdx.x) * 8 + 0] = (long long)t;
-    P.dbg[(200 + blockIdx.x) * 8 + 2] = (long long)smid;
-  }
 
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < stages; ++s) {
@@ -155,12 +130,9 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
           mbar_wait(bar_empty(s), ph ^ 1);
           const uint32_t sa = smem_base + (uint32_t)s * kStage, sb = sa + kABytes;
           const int k0 = kb * BK;
-          if ((TGPB200_ABL & 64) && elect_one()) mbar_arrive(bar_full(s));
-          if (!(TGPB200_ABL & 64) && elect_one()) {
-            const bool load_a = src != kATmem && !(TGPB200_ABL & 32);
-            mbar_arrive_expect_tx(bar_full(s), (load_a ? kABytes : 0u) + kBBytes);
-            if (!load_a) {
-            } else if (src == kAMnPlain) tma_load_3d(sa, &P.map_a[p], bar_full(s), m0, k0, b);      // [32 k][128 m], no swizzle
+          if (elect_one()) {
+            mbar_arrive_expect_tx(bar_full(s), (src != kATmem ? kABytes : 0u) + kBBytes);
+            if (src == kAMnPlain) tma_load_3d(sa, &P.map_a[p], bar_full(s), m0, k0, b);      // [32 k][128 m], no swizzle
             else if (src == kAKMajor) tma_load_3d(sa, &P.map_a[p], bar_full(s), k0, m0, b);  // [128 m][32 k], 128B swizzle
             if (P.b_mn[p]) {
               for (int blk = 0; blk < BNB / 32; ++blk)
@@ -195,34 +167,23 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
           const uint32_t b_lbo = P.b_mn[p] ? BK * kStageRowBytes : 16;
           const uint32_t b_step = P.b_mn[p] ? 8 * kStageRowBytes : 32;
           const uint64_t desc_b0 = make_desc(smem_base, b_lbo, P.b_mn[p] ? 512 : 1024, P.b_mn[p] ? 1 : 2);
-          const uint32_t idesc2 = (idesc & ~(0x3fu << 17)) | ((uint32_t)((2 * BNB) >> 3) << 17);
-          const bool wide = kConcat && P.wide[p] != 0;
           uint32_t accum = P.first[p] ? 0u : 1u;
           for (int kb = 0, nkb = (P.kd[p] + BK - 1) / BK; kb < nkb; ++kb, ++kc) {
-            if (P.dbg && blockIdx.x == 0 && kc < 128) P.dbg[kc * 8 + 7] = clock64();
             mbar_wait(bar_lo(s), ph);
-            if (P.dbg && blockIdx.x == 0 && kc < 128) P.dbg[kc * 8 + 5] = clock64();
-            if (!(TGPB200_ABL & 1024)) tc_fence_after();
+            tc_fence_after();
             const uint32_t ts = kc % (uint32_t)kSlots;
             const uint32_t a_stage = tm + kColRing + ts * kRing;
             const uint64_t db0 = desc_b0 + (uint64_t)(((uint32_t)s * kStage + kABytes) >> 4);
 #pragma unroll
-            for (int kk = 0; kk < ((TGPB200_ABL & 128) ? 0 : KSTEPS); ++kk) {
+            for (int kk = 0; kk < KSTEPS; ++kk) {
               const uint64_t db = db0 + (uint64_t)(kk * (b_step >> 4)), db_lo = db + (kBBytes >> 4);
               const uint32_t a_hi = a_stage + (uint32_t)(kk * 16), a_lo = a_hi + 8;
-              if (wide) {
-                umma_ts_tf32(d_tmem, a_hi, db, idesc2, kk == 0 ? accum : 1u);  // hi_a x [hi_b | lo_b]
-                umma_ts_tf32(d_tmem, a_lo, db, idesc, 1u);                     // lo_a x hi_b
-              } else {
-                umma_ts_tf32(d_tmem, a_lo, db, idesc, kk == 0 ? accum : 1u);
-                umma_ts_tf32(d_tmem, a_hi, db_lo, idesc, 1u);
-                umma_ts_tf32(d_tmem, a_hi, db, idesc, 1u);
-              }
+              umma_ts_tf32(d_tmem, a_lo, db, idesc, kk == 0 ? accum : 1u);
+              umma_ts_tf32(d_tmem, a_hi, db_lo, idesc, 1u);
+              umma_ts_tf32(d_tmem, a_hi, db, idesc, 1u);
             }
-            if (P.dbg && blockIdx.x == 0 && kc < 128) P.dbg[kc * 8 + 0] = clock64();
-            if (TGPB200_ABL & 4096) mbar_arrive(bar_empty(s)); else umma_commit(bar_empty(s));
-            if (TGPB200_ABL & 8192) mbar_arrive(bar_tfree(ts)); else umma_commit(bar_tfree(ts));
-            if (P.dbg && blockIdx.x == 0 && kc < 128) P.dbg[kc * 8 + 6] = clock64();
+            umma_commit(bar_empty(s));
+            umma_commit(bar_tfree(ts));
             accum = 1;
             if (++s == stages) { s = 0; ph ^= 1; }
           }
@@ -256,7 +217,7 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
           mbar_wait(bar_full(s), ph);
           const uint32_t sa = smem_base + (uint32_t)s * kStage, sb = sa + kABytes;
           // B: hi in place, lo behind it
-          for (uint32_t ch = t; ch < ((TGPB200_ABL & 1) ? 0u : kBBytes / 16); ch += 128) {
+          for (uint32_t ch = t; ch < kBBytes / 16; ch += 128) {
             const float4 v = lds128(sb + ch * 16);
             float4 h, l;
             h.x = rna_tf32(v.x), h.y = rna_tf32(v.y), h.z = rna_tf32(v.z), h.w = rna_tf32(v.w);
@@ -264,22 +225,13 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
             sts128(sb + ch * 16, h);
             sts128(sb + kBBytes + ch * 16, l);
           }
-          if (!(TGPB200_ABL & 2)) fence_proxy_async();
+          fence_proxy_async();
           // A: this thread's row, 32 k values
           float x[32];
-          if (TGPB200_ABL & 4) {
-#pragma unroll
-            for (int k = 0; k < 32; ++k) x[k] = (float)(k + lane);
-          } else if (src == kATmem) {
+          if (src == kATmem) {
             mbar_wait(bar_wfull, (uint32_t)it & 1u);
             tc_fence_after();
             tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + kColW + (uint32_t)(kb * BK), x);
-            if (kConcat) {
-              float x2[32];
-              tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + kColW + 64u + (uint32_t)(kb * BK), x2);
-#pragma unroll
-              for (int k = 0; k < 32; ++k) x[k] += x2[k];
-            }
           } else if (src == kAMnPlain) {
 #pragma unroll
             for (int k = 0; k < 32; ++k) x[k] = lds32(sa + (uint32_t)k * (BM * 4) + (uint32_t)m_local * 4);
@@ -291,12 +243,6 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
             }
           }
           const uint32_t slot = kc % (uint32_t)kSlots;
-          if (TGPB200_ABL & 16384) {  // skeleton experiment: nothing between the two barriers
-            __syncwarp();
-            if (lane == 0) mbar_arrive(bar_lo(s));
-            if (++s == stages) { s = 0; ph ^= 1; }
-            continue;
-          }
           mbar_wait(bar_tfree(slot), ((kc / (uint32_t)kSlots) & 1u) ^ 1u);
           tc_fence_after();
           const uint32_t a_stage = tmem_base + ((uint32_t)(q * 32) << 16) + kColRing + slot * kRing;
@@ -308,14 +254,12 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
               hi[i] = rna_tf32(x[kk * 8 + i]);
               lo[i] = x[kk * 8 + i] - hi[i];
             }
-            if (!(TGPB200_ABL & 8)) tmem_st16(a_stage + (uint32_t)(kk * 16), hi, lo);
-            else if (hi[0] == 123.456f && lo[7] == 3.f) P.dbg[0] = 1;  // keep the conversion alive
+            tmem_st16(a_stage + (uint32_t)(kk * 16), hi, lo);
           }
           tmem_st_wait();
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(bar_lo(s));  // 128 per-thread arrivals on one barrier word serialise
-          if (P.dbg && blockIdx.x == 0 && lane == 0 && kc < 128) P.dbg[kc * 8 + 1 + q] = clock64();
           if (++s == stages) { s = 0; ph ^= 1; }
         }
       }
@@ -323,8 +267,7 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
   } else {
     // ===================== epilogue: dS (+ element-wise terms) and dX through TMA stores =====================
     const int quad = warp & 3;
-    const int ew = warp - 2 - kGroups * 4;   // 0 .. 7
-    const int e2 = ew >> 2;                  // which of the quadrant's warps
+    const int ew = warp - 2 - kGroups * 4;   // 0 .. 3
     const uint32_t stg0 = smem_base + (uint32_t)kStage * stages + (uint32_t)ew * kEpiBufs * 4096u;
     uint32_t n_stored = 0;
     const uint32_t hook0 = smem_base + (uint32_t)kStage * stages + kEpiBytes;
@@ -340,7 +283,7 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
       float dd = 0.f, c_ent = 0.f, di = 0.f;
       bool hook = false;
       const uint32_t hrow = hook0 + (uint32_t)(quad * 32 + lane) * (BNB * 4);
-      if (!(TGPB200_ABL & 256) && P.S != nullptr && m < P.N) {
+      if (P.S != nullptr && m < P.N) {
         const float c_den = P.coef[b * 4 + 0];
         c_ent = P.coef[b * 4 + 2];
         hook = c_den != 0.f || c_ent != 0.f;
@@ -353,22 +296,14 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
       }
       cp_async_commit();
       mbar_wait(bar_tfull, (uint32_t)it & 1u);
-      if (P.dbg && blockIdx.x == 0 && ew == 0 && lane == 0 && it < 32) P.dbg[(128 + it) * 8 + 0] = clock64();
       tc_fence_after();
       cp_async_wait_all();
       __syncwarp();
-      for (int c = 0; c < ((TGPB200_ABL & 16) ? 0 : n_chunks); ++c) {
-        if (kEpiW == 8 && (c & 1) != e2) continue;
+      for (int c = 0; c < n_chunks; ++c) {
         const bool is_ds = c < 2;
         const int n0 = is_ds ? c * 32 : (c - 2) * 32;
         float v[32];
         tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (is_ds ? kColS : kColX) + (uint32_t)n0, v);
-        if (kConcat && is_ds) {  // + hi_a x lo_b
-          float v2[32];
-          tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + kColS + 64u + (uint32_t)n0, v2);
-#pragma unroll
-          for (int j = 0; j < 32; ++j) v[j] += v2[j];
-        }
         if (m_base >= P.N || n0 >= (is_ds ? P.K : P.F)) continue;  // warp-uniform
         if (is_ds && hook) {
 #pragma unroll
@@ -394,10 +329,7 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
         // two staging tiles per warp: the store of the previous chunk may still be reading the other one
         const uint32_t stg = stg0 + (n_stored % kEpiBufs) * 4096u;
         ++n_stored;
-        if (lane == 0) {
-          if (kEpiBufs == 2) tma_store_wait_read<1>();
-          else tma_store_wait_read<0>();
-        }
+        if (lane == 0) tma_store_wait_read<kEpiBufs - 1>();
         __syncwarp();
         const uint32_t row = stg + (uint32_t)lane * 128u;
 #pragma unroll
@@ -405,7 +337,7 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
           sts128(row + (uint32_t)((c4 ^ (lane & 7)) << 4), make_float4(v[4 * c4], v[4 * c4 + 1], v[4 * c4 + 2], v[4 * c4 + 3]));
         fence_proxy_async();
         __syncwarp();
-        if (lane == 0 && !(TGPB200_ABL & 512)) {
+        if (lane == 0) {
           tma_store_3d(is_ds ? &P.map_ds : &P.map_dx, stg, n0, m_base, b);
           tma_store_commit();
         }
@@ -413,18 +345,12 @@ __global__ void __launch_bounds__(kThreadsBwd, 1) k_dense_bwd_fused(const __grid
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_tempty);
-      if (P.dbg && blockIdx.x == 0 && ew == 0 && lane == 0 && it < 32) P.dbg[(128 + it) * 8 + 1] = clock64();
     }
     if (lane == 0) tma_store_wait_all();
   }
 
   tc_fence_before();
   __syncthreads();
-  if (P.dbg && threadIdx.x == 0) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    P.dbg[(200 + blockIdx.x) * 8 + 1] = (long long)t;
-  }
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
@@ -466,7 +392,6 @@ int dense_bwd_fused(const float* A, const float* S, const float* X, const float*
   bool ok = true;
   auto add = [&](int kd, int a_src, OperandDesc a, OperandDesc b, int b_n0, uint32_t acc, int first) {
     P.kd[n] = kd, P.a_src[n] = a_src, P.b_mn[n] = b.mn_major, P.b_n0[n] = b_n0, P.acc_col[n] = acc, P.first[n] = first;
-    P.wide[n] = acc != kColX && acc != kColX + (uint32_t)BNB;
     if (a_src == kAKMajor) ok = ok && make_operand_map(&P.map_a[n], a, false, B, N, kd, BM);
     else if (a_src == kAMnPlain) ok = ok && make_operand_map_mn_plain(&P.map_a[n], a, B, N, kd);
     // the N extent of a B operand is its full column / row count (b_n0 selects the 64-wide slice)
@@ -491,7 +416,6 @@ int dense_bwd_fused(const float* A, const float* S, const float* X, const float*
   if (!make_out_map(&P.map_ds, dS, B, N, K) || !make_out_map(&P.map_dx, dX, B, N, F)) return TGPB200_ERR_UNSUPPORTED;
   P.S = ew_S, P.d = ew_d, P.coef = ew_coef, P.uv = ew_S ? ew_uv : nullptr, P.eps = eps;
   P.stages = 5;
-  P.dbg = g_engine_dbg;
   static bool attr_set = false;
   if (!attr_set) {
     attr_set = true;

@@ -36,8 +36,8 @@ struct FusedParams {
   int concat;             // fp32: accumulators 2 BN wide, hi_a x [hi_s | lo_s] as ONE MMA (lo of S right behind S)
   uint32_t tmem_cols;
   float eps;
-  long long* dbg;         // optional timeline of block 0 (debug); ahead of Tt so that Tt / Xp stay 16-byte aligned
-  void* Tt;               // [B, K, N]  operand dtype: T = S^T A
+  // 16-byte aligned: the output pointers are fetched in 16-byte-aligned pairs (ss / a2 with one 128-bit load)
+  alignas(16) void* Tt;   // [B, K, N]  operand dtype: T = S^T A
   void* Xp;               // [B, K, F]  operand dtype
   float* Mm;              // [B, K, K]
   float *d, *ss, *a2, *ent;  // [B, N]
@@ -96,11 +96,9 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
     if (lane == 0) {
       int s = 0;
       uint32_t ph = 0;
-      int dbg_n = 0;
       for (int b = blockIdx.x; b < P.B; b += gridDim.x) {
         for (int kb = 0; kb < kblocks; ++kb) {
           mbar_wait(bar_empty(s), ph ^ 1);
-          if (P.dbg && blockIdx.x == 0 && dbg_n < 96) P.dbg[dbg_n * 8 + 0] = clock64();
           uint32_t dst = smem_base + (uint32_t)s * stage_bytes;
           mbar_arrive_expect_tx(bar_full(s), raw_bytes);
           const int k0 = kb * FBK;
@@ -113,8 +111,6 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
             for (int j = 0; j < P.nb_x; ++j, dst += kBlockBytes) tma_load_3d(dst, &P.map_x, bar_full(s), j * EPB, k0, b);
             for (int j = 0; j < P.nb_s; ++j, dst += kBlockBytes) tma_load_3d(dst, &P.map_s, bar_full(s), j * EPB, k0, b);
           }
-          if (P.dbg && blockIdx.x == 0 && dbg_n < 96) P.dbg[dbg_n * 8 + 1] = clock64();
-          ++dbg_n;
           if (++s == stages) { s = 0; ph ^= 1; }
         }
       }
@@ -147,7 +143,6 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
       int s = 0;
       uint32_t ph = 0;
       int it = 0;
-      int dbg_m = 0;
       for (int b = blockIdx.x; b < P.B; b += gridDim.x, ++it) {
         const int ab = P.acc_bufs == 2 ? (it & 1) : 0;
         const uint32_t aph = P.acc_bufs == 2 ? ((uint32_t)(it >> 1) & 1u) : ((uint32_t)it & 1u);
@@ -156,9 +151,7 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
         const uint32_t d0 = tm + (uint32_t)(ab * G * accw);
         for (int kb = 0; kb < kblocks; ++kb) {
           mbar_wait(bar_full(s), ph);
-          if (P.dbg && blockIdx.x == 0 && lane == 0 && dbg_m < 96) P.dbg[dbg_m * 8 + 2] = clock64();
           mbar_wait(bar_lo(s), ph);
-          if (P.dbg && blockIdx.x == 0 && lane == 0 && dbg_m < 96) P.dbg[dbg_m * 8 + 3] = clock64();
           tc_fence_after();
           const uint64_t dst = desc0 + (uint64_t)((uint32_t)s * stage_off);
           if (elect_one()) {
@@ -190,8 +183,6 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
           umma_commit(bar_empty(s));
           }
           __syncwarp();
-          if (P.dbg && blockIdx.x == 0 && lane == 0 && dbg_m < 96) P.dbg[dbg_m * 8 + 4] = clock64();
-          ++dbg_m;
           if (++s == stages) { s = 0; ph ^= 1; }
         }
         if (elect_one()) umma_commit(bar_tfull(ab));
@@ -204,11 +195,9 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
     const int r = t >> 3;             // node row inside the k-block (16 rows x 8 chunks = one 2 KB block)
     int s = 0;
     uint32_t ph = 0;
-    int dbg_s = 0;
     for (int b = blockIdx.x; b < P.B; b += gridDim.x) {
       for (int kb = 0; kb < kblocks; ++kb) {
         mbar_wait(bar_full(s), ph);
-        if (P.dbg && blockIdx.x == 0 && t == 0 && dbg_s < 96) P.dbg[dbg_s * 8 + 5] = clock64();
         const uint32_t st = smem_base + (uint32_t)s * stage_bytes + (uint32_t)t * 16;
         float sd = 0.f, sa2 = 0.f, s2 = 0.f, se = 0.f;
         constexpr int NV = 16 / ES;  // values per 16-byte chunk
@@ -286,8 +275,6 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
         }
         if (kF32) fence_proxy_async();
         mbar_arrive(bar_lo(s));
-        if (P.dbg && blockIdx.x == 0 && t == 0 && dbg_s < 96) P.dbg[dbg_s * 8 + 6] = clock64();
-        ++dbg_s;
         if (++s == stages) { s = 0; ph ^= 1; }
       }
     }
@@ -346,9 +333,6 @@ __global__ void __launch_bounds__(320, 1) k_dense_fwd_fused(const __grid_constan
   if (warp == 1) tmem_dealloc(tmem_base, P.tmem_cols);
 }
 
-long long* g_fused_dbg = nullptr;
-long long* g_engine_dbg = nullptr;
-
 // Returns TGPB200_ERR_UNSUPPORTED when the shape does not fit (the caller then uses the per-product path).
 int dense_fwd_fused(const void* A, const void* S, const void* X, int B, int N, int K, int F, bool bf16, float eps,
                     void* Tt, void* Xp, float* Mm, float* d, float* ss, float* a2, float* ent, cudaStream_t stream) {
@@ -380,7 +364,6 @@ int dense_fwd_fused(const void* A, const void* S, const void* X, int B, int N, i
   P.stages = stages;
   P.eps = eps;
   P.Tt = Tt, P.Xp = Xp, P.Mm = Mm, P.d = d, P.ss = ss, P.a2 = a2, P.ent = ent;
-  P.dbg = g_fused_dbg;
   const bool sw32 = !bf16;
   P.blocked = (N % epb == 0 && F % epb == 0 && K % epb == 0 && P.nb_a <= 256) ? 1 : 0;
   if (P.blocked) {
@@ -413,7 +396,3 @@ int dense_fwd_fused(const void* A, const void* S, const void* X, int B, int N, i
 
 }  // namespace tc
 }  // namespace tgp
-
-extern "C" void tgpb200_debug_fused_timeline(long long* p) { tgp::tc::g_fused_dbg = p; }
-// same for the engine / fused backward (k_tc_gemm_ts, k_dense_bwd_fused): [160][8] clock64 stamps of block 0
-extern "C" void tgpb200_debug_engine_timeline(long long* p) { tgp::tc::g_engine_dbg = p; }

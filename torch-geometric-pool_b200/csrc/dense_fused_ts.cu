@@ -29,8 +29,6 @@
 namespace tgp {
 namespace tc {
 
-extern long long* g_fused_dbg;  // optional clock64 timeline of block 0 (dense_fused.cu, benchmarks/fused_fwd_timeline.py)
-
 namespace {
 
 constexpr int TBK = 16;                              // nodes per k-block
@@ -50,10 +48,6 @@ constexpr int kSplitThreads = kSplitWarps * 32;         // per group
 constexpr int kEpiWarps = 8;                            // two per TMEM lane quadrant, alternate 32-column chunks
 constexpr int kTsThreads = 64 + kSplitGroups * kSplitThreads + kEpiWarps * 32;  // TMA, MMA, split groups, epilogue
 constexpr int kTpr = kEpiWarps * 32 / 16;               // statistics (epilogue warps): threads per node row
-// Ablation switches (timing experiments only; results are wrong when any bit is set): benchmarks/ablate_fwd.py
-#ifndef TGPB200_ABLF
-#define TGPB200_ABLF 0   // 1 no drain, 2 no statistics, 4 no B split, 8 no M-side staging, 16 no MMAs, 32 no TMA loads
-#endif
 constexpr int kACols = 32;                           // TMEM columns per (tile, k-block): 2 k-steps x (8 hi + 8 lo)
 
 struct TsParams {
@@ -70,8 +64,6 @@ struct TsParams {
   float* Xp;               // [B, K, F]
   float* Mm;               // [B, K, K]
   float *d, *ss, *a2, *ent;
-  long long* dbg;  // [96][8]: 0 tma issue, 1 tma issued, 2 mma ready-wait done, 3 -, 4 mma issued, 5 split start,
-                   //          6 split done, 7 split pass 1 done (TMEM ring wait starts), 3 TMEM ring wait done
 };
 
 __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __grid_constant__ TsParams P) {
@@ -124,15 +116,12 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
       int s = 0;
       uint32_t ph = 0;
       const uint32_t tx = (uint32_t)TBK * (P.N + P.F + P.K) * 4 + sb_bytes;
-      int dbg_n = 0;
       for (int b = blockIdx.x; b < P.B; b += gridDim.x) {
         for (int kb = 0; kb < kblocks; ++kb) {
           mbar_wait(bar_empty(s), ph ^ 1);
-          if (P.dbg && blockIdx.x == 0 && lane == 0 && dbg_n < 96) P.dbg[dbg_n * 8 + 0] = clock64();
           const uint32_t dst = smem_base + (uint32_t)s * stage_bytes;
           const int k0 = kb * TBK;
-          if ((TGPB200_ABLF & 32) && elect_one()) mbar_arrive(bar_full(s));
-          if (!(TGPB200_ABLF & 32) && elect_one()) {
+          if (elect_one()) {
             mbar_arrive_expect_tx(bar_full(s), tx);
             tma_load_3d(dst, &P.map_a, bar_full(s), 0, k0, b);
             tma_load_3d(dst + off_x, &P.map_x, bar_full(s), 0, k0, b);
@@ -140,8 +129,6 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
             for (int j = 0; j < P.nb_s; ++j) tma_load_3d(dst + off_sb + j * kSBlock, &P.map_sb, bar_full(s), j * 32, k0, b);
           }
           __syncwarp();
-          if (P.dbg && blockIdx.x == 0 && lane == 0 && dbg_n < 96) P.dbg[dbg_n * 8 + 1] = clock64();
-          ++dbg_n;
           if (++s == stages) { s = 0; ph ^= 1; }
         }
       }
@@ -164,13 +151,12 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
         tc_fence_after();
         for (int kb = 0; kb < kblocks; ++kb, ++kc) {
           mbar_wait(bar_ready(s), ph);
-          if (P.dbg && blockIdx.x == 0 && kc < 96) P.dbg[kc * 8 + 2] = clock64();
           tc_fence_after();
           const uint32_t ts = kc & 1u;
           const uint32_t a_stage = tm + a_cols0 + ts * (uint32_t)(G * kACols);
           const uint64_t db0 = desc0 + (uint64_t)(((uint32_t)s * stage_bytes + off_sb) >> 4);
 #pragma unroll
-          for (int kk = 0; kk < ((TGPB200_ABLF & 16) ? 0 : 2); ++kk) {
+          for (int kk = 0; kk < 2; ++kk) {
             const uint64_t db = db0 + (uint64_t)(kk * ((8 * kStageRowBytes) >> 4)), db_lo = db + (sb_bytes >> 4);
             const uint32_t acc0 = (kb > 0 || kk > 0) ? 1u : 0u;
             for (int g = 0; g < G; ++g) {
@@ -183,7 +169,6 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
           }
           umma_commit(bar_empty(s));    // the TMA producer may refill the shared-memory stage
           umma_commit(bar_tfree(ts));   // the split warps may overwrite the TMEM operand stage
-          if (P.dbg && blockIdx.x == 0 && kc < 96) P.dbg[kc * 8 + 4] = clock64();
           if (++s == stages) { s = 0; ph ^= 1; }
         }
         umma_commit(bar_tfull);
@@ -209,10 +194,9 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
           continue;
         }
         mbar_wait(bar_full(s), ph);
-        if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 96) P.dbg[kc * 8 + 5] = clock64();
         const uint32_t base = smem_base + (uint32_t)s * stage_bytes;
         // ---- pass 1b: hi / lo of the B operand (swizzled S blocks), in place + next to it
-        for (uint32_t ch = t; ch < ((TGPB200_ABLF & 4) ? 0u : (uint32_t)P.nb_s * 128); ch += kSplitThreads) {
+        for (uint32_t ch = t; ch < (uint32_t)P.nb_s * 128; ch += kSplitThreads) {
           const uint32_t a = base + off_sb + ch * 16;
           const float4 v = lds128(a);
           float4 h, l;
@@ -224,12 +208,10 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
         fence_proxy_async();
         // ---- pass 2: hi / lo of the M-side operand into the TMEM ring (lane = M row, 8 columns = 8 nodes)
         const uint32_t ts = kc & 1u;
-        if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 96) P.dbg[kc * 8 + 7] = clock64();
         mbar_wait(bar_tfree(ts), ((kc >> 1) & 1u) ^ 1u);
-        if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 96) P.dbg[kc * 8 + 3] = clock64();
         tc_fence_after();
         const uint32_t a_stage = tmem_base + ((uint32_t)(q * 32) << 16) + a_cols0 + ts * (uint32_t)(G * kACols);
-        for (int g = half; g < ((TGPB200_ABLF & 8) ? 0 : G); g += kSplitWarps / 4) {
+        for (int g = half; g < G; g += kSplitWarps / 4) {
           const int seg = g < P.t_a ? 0 : (g < P.t_a + P.t_x ? 1 : 2);
           const int m = (seg == 0 ? g : (seg == 1 ? g - P.t_a : g - P.t_a - P.t_x)) * BM + q * 32 + lane;
           const int ext = seg == 0 ? P.N : (seg == 1 ? P.F : P.K);
@@ -252,7 +234,6 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
         tmem_st_wait();
         tc_fence_before();
         mbar_arrive(bar_ready(s));
-        if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 96) P.dbg[kc * 8 + 6] = clock64();
         if (++s == stages) { s = 0; ph ^= 1; }
       }
     }
@@ -274,20 +255,18 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
         mbar_wait(bar_full(s), ph);
         const uint32_t base = smem_base + (uint32_t)s * stage_bytes;
         float sd = 0.f, sa2 = 0.f, s2 = 0.f, se = 0.f;
-        if (!(TGPB200_ABLF & 2)) {
-          const uint32_t ra = base + (uint32_t)r * P.N * 4;
-          for (int col = c16 * 4; col < P.N; col += 4 * kTpr) {
-            const float4 v = lds128(ra + col * 4);
-            sd += (v.x + v.y) + (v.z + v.w);
-            sa2 += fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, v.w * v.w)));
-          }
-          const uint32_t rs = base + off_s + (uint32_t)r * P.K * 4;
-          for (int col = c16 * 4; col < P.K; col += 4 * kTpr) {
-            const float4 v = lds128(rs + col * 4);
-            s2 += fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, v.w * v.w)));
-            se -= fmaf(v.x, __logf(v.x + P.eps),
-                       fmaf(v.y, __logf(v.y + P.eps), fmaf(v.z, __logf(v.z + P.eps), v.w * __logf(v.w + P.eps))));
-          }
+        const uint32_t ra = base + (uint32_t)r * P.N * 4;
+        for (int col = c16 * 4; col < P.N; col += 4 * kTpr) {
+          const float4 v = lds128(ra + col * 4);
+          sd += (v.x + v.y) + (v.z + v.w);
+          sa2 += fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, v.w * v.w)));
+        }
+        const uint32_t rs = base + off_s + (uint32_t)r * P.K * 4;
+        for (int col = c16 * 4; col < P.K; col += 4 * kTpr) {
+          const float4 v = lds128(rs + col * 4);
+          s2 += fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, v.w * v.w)));
+          se -= fmaf(v.x, __logf(v.x + P.eps),
+                     fmaf(v.y, __logf(v.y + P.eps), fmaf(v.z, __logf(v.z + P.eps), v.w * __logf(v.w + P.eps))));
         }
 #pragma unroll
         for (int o = 1; o < kTpr; o <<= 1) {
@@ -297,7 +276,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
           se += __shfl_xor_sync(kFull, se, o);
         }
         const int node = kb * TBK + r;
-        if (!(TGPB200_ABLF & 2) && c16 == 0 && node < P.N) {
+        if (c16 == 0 && node < P.N) {
           const int64_t o = (int64_t)b * P.N + node;
           P.d[o] = sd, P.a2[o] = sa2, P.ss[o] = s2, P.ent[o] = se;
         }
@@ -307,7 +286,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) k_dense_fwd_fused_ts(const __gr
       mbar_wait(bar_tfull, (uint32_t)it & 1u);
       tc_fence_after();
       int chunk = 0;
-      for (int g = 0; g < ((TGPB200_ABLF & 1) ? 0 : G); ++g) {
+      for (int g = 0; g < G; ++g) {
         const int seg = g < P.t_a ? 0 : (g < P.t_a + P.t_x ? 1 : 2);
         const int m0 = (seg == 0 ? g : (seg == 1 ? g - P.t_a : g - P.t_a - P.t_x)) * BM + quad * 32;  // warp-uniform
         const int m_ext = seg == 0 ? P.N : (seg == 1 ? P.F : P.K);
@@ -397,7 +376,6 @@ int dense_fwd_fused_ts(const float* A, const float* S, const float* X, int B, in
   P.stages = stages;
   P.eps = eps;
   P.Tt = Tt, P.Xp = Xp, P.Mm = Mm, P.d = d, P.ss = ss, P.a2 = a2, P.ent = ent;
-  P.dbg = g_fused_dbg;
   if (!make_map_rows(&P.map_a, A, B, N, N) || !make_map_rows(&P.map_x, X, B, N, F) || !make_map_rows(&P.map_s, S, B, N, K))
     return TGPB200_ERR_UNSUPPORTED;
   if (!make_map_3d(&P.map_sb, S, false, B, N, K, K, (int64_t)N * K, TBK, true)) return TGPB200_ERR_UNSUPPORTED;

@@ -181,9 +181,6 @@ static __global__ void k_tile_desc(const int32_t* __restrict__ tile_mlo, const i
 // at most kBkPer = kBkCap / kBkThreads entries, so every phase is a fixed, fully unrolled loop whose global loads
 // are all issued before the first one is consumed.  kPacked: coarse column and arrival index share one 32-bit rank
 // key (column < 2^21), so that the counting loop is one compare per element on 128-bit shared-memory reads.
-#ifndef TGPB200_ABLB
-#define TGPB200_ABLB 0  // timing experiments only: 1 no rank loop, 2 no run combination / output, 4 no column / cluster gathers
-#endif
 constexpr int kBkPer = kBkCap / kBkThreads;
 
 template <bool kPacked>
@@ -244,11 +241,11 @@ static __global__ void __launch_bounds__(kBkThreads) k_bucket_tiles(BucketArgs A
       }
     }
 #pragma unroll
-    for (int k = 0; k < kBkPer; ++k) q[k] = (e[k] >= 0 && !(TGPB200_ABLB & 4)) ? __ldg(A.col + e[k]) : 0;
+    for (int k = 0; k < kBkPer; ++k) q[k] = e[k] >= 0 ? __ldg(A.col + e[k]) : 0;
 #pragma unroll
     for (int k = 0; k < kBkPer; ++k) {
       if (q[k] < 0 || q[k] >= A.N) q[k] = 0;
-      q[k] = (e[k] >= 0 && !(TGPB200_ABLB & 4)) ? __ldg(A.cluster + q[k]) : (int64_t)((threadIdx.x * 7 + k) & 1023);
+      q[k] = e[k] >= 0 ? __ldg(A.cluster + q[k]) : (int64_t)((threadIdx.x * 7 + k) & 1023);
     }
 #pragma unroll
     for (int k = 0; k < kBkPer; ++k) {
@@ -271,9 +268,7 @@ static __global__ void __launch_bounds__(kBkThreads) k_bucket_tiles(BucketArgs A
     const int start = m_voff[rk], end = r_end[rk];
     int rank = 0;
     int q = start;
-    if (TGPB200_ABLB & 1) {
-      rank = j - start;
-    } else if (kPacked) {  // keys are unique (arrival index in the low bits); dummies (all ones) rank last, ties impossible
+    if (kPacked) {  // keys are unique (arrival index in the low bits); dummies (all ones) rank last, ties impossible
       // rank = keys below cc = row length - 1 (the entry itself) - keys above cc
       const uint32_t ncc = ~cc;
       uint32_t g0 = 0, g1 = 0;
@@ -295,7 +290,7 @@ static __global__ void __launch_bounds__(kBkThreads) k_bucket_tiles(BucketArgs A
   }
   __syncthreads();
   // run heads combine their members in arrival order; the first member's weight of every head is loaded up front
-  if (!(TGPB200_ABLB & 2)) {
+  {
     constexpr uint32_t kColMask = kPacked ? ~0x7ffu : ~0u;
     int64_t e0[kBkPer];
     float w0[kBkPer];

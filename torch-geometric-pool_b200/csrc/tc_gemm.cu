@@ -31,16 +31,14 @@ struct KernelParams {
   const float* ew_d;
   const float* ew_coef;
   float ew_eps;
-  long long* dbg;  // optional clock64 timeline of block 0 ([128][8], benchmarks/engine_timeline.py)
   // Row-major destinations leave through TMA stores: every epilogue warp stages its 32 x 32 chunk in shared memory
   // (swizzled, one row per lane) and one lane issues cp.async.bulk.tensor.  Writing the rows straight from the
   // registers costs 32 separate 128-byte lines per store instruction and kept the LSU busy for ~3 k cycles per
-  // 128 x 64 tile (benchmarks/engine_timeline.py), stalling the split warps that share it.
+  // 128 x 64 tile (measured with a cycle-counter timeline of the fp32 engine), stalling the split warps that share it.
   CUtensorMap map_out;
   int tma_out;       // 1: use map_out
   int epi_bufs;      // staging buffers per epilogue warp (1 or 2)
   int pack2;         // fp32 TMEM-operand engine: one 128 x 128 tile holds the products of TWO batch items with M, N <= 64
-  int abl;           // timing experiments (TGPB200_ABL_GEMM): 1 no B loads, 2 no A loads, 4 no element-wise terms, 8 no stores
 };
 
 // Staging state of one epilogue warp for the TMA-store path
@@ -48,13 +46,12 @@ struct EpiStage {
   uint32_t smem;  // first staging buffer of this warp (1024-byte aligned, 4 KB per buffer)
   int n;          // chunks staged so far
 };
-extern long long* g_engine_dbg;
 
 // Element-wise gradient terms of the dense backward (GemmProblem::ew_*), software-pipelined: the per-row coefficients
 // are loaded once per item BEFORE the wait for the accumulators, and the values of S that chunk c needs are loaded
 // while chunk c - 1 is processed.  Loaded per chunk after the accumulators were ready, the four dependent global
 // round trips (two coefficients, the degree, the row of S) made the epilogue of `dS` the bottleneck of that product
-// (C3: 553 -> 354 us without the terms; benchmarks: TGPB200_ABL_GEMM=4).
+// (C3: 553 -> 354 us for that product with the terms skipped).
 template <bool kF32>
 struct EwPre {
   float dd = 0.f, c_ent = 0.f;
@@ -65,7 +62,7 @@ struct EwPre {
 template <bool kF32>
 __device__ __forceinline__ void ew_item(const KernelParams& P, EwPre<kF32>& e, int b, int m) {
   e.on = false;
-  if (P.ew_S == nullptr || (P.abl & 4) || m >= P.M || P.out_cs != 1) return;
+  if (P.ew_S == nullptr || m >= P.M || P.out_cs != 1) return;
   const float c_den = P.ew_coef[b * 4 + 0];
   e.c_ent = P.ew_coef[b * 4 + 2];
   if (c_den == 0.f && e.c_ent == 0.f) return;
@@ -153,7 +150,6 @@ __device__ __forceinline__ void store_chunk(const KernelParams& P, float (&v)[32
   if (P.out_cs == 1) {
     const bool full = n0 + 32 <= P.N;
     ew_apply<kF32>(P, ew, v, b, m, n0);
-    if (P.abl & 8) return;
     if (P.tma_out) {
       // stage (lane = row of the chunk) with the swizzle of the output map, then one TMA store; rows >= M and
       // columns >= N are clipped by the map
@@ -329,23 +325,21 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_gemm(const __grid_constant__
             uint32_t sa = smem_base + (uint32_t)s * stage_bytes, sb = sa + a_bytes;
             int k0 = kb * BK;
             if (elect_one()) {
-            mbar_arrive_expect_tx(bar_full(s), ((P.abl & 2) ? 0u : a_bytes) + ((P.abl & 1) ? 0u : b_bytes));
-            // K-major: one box [rows x 128 B].  MN-major: one box [BK k-rows x 128 B] per 128-byte block of
-            // the MN extent, laid out block after block (the canonical UMMA MN-major SW128 layout, LBO = BK*128 B).
-            if (P.abl & 2) {
-            } else if (P.a_mn[p]) {
-              for (int blk = 0; blk < BM / EPB; ++blk)
-                tma_load_3d(sa + blk * (BK * kStageRowBytes), &P.map_a[p], bar_full(s), m0 + blk * EPB, k0, b);
-            } else {
-              tma_load_3d(sa, &P.map_a[p], bar_full(s), k0, m0, b);
-            }
-            if (P.abl & 1) {
-            } else if (P.b_mn[p]) {
-              for (int blk = 0; blk < BN / EPB; ++blk)
-                tma_load_3d(sb + blk * (BK * kStageRowBytes), &P.map_b[p], bar_full(s), n0 + blk * EPB, k0, b);
-            } else {
-              tma_load_3d(sb, &P.map_b[p], bar_full(s), k0, n0, b);
-            }
+              mbar_arrive_expect_tx(bar_full(s), a_bytes + b_bytes);
+              // K-major: one box [rows x 128 B].  MN-major: one box [BK k-rows x 128 B] per 128-byte block of
+              // the MN extent, laid out block after block (the canonical UMMA MN-major SW128 layout, LBO = BK*128 B).
+              if (P.a_mn[p]) {
+                for (int blk = 0; blk < BM / EPB; ++blk)
+                  tma_load_3d(sa + blk * (BK * kStageRowBytes), &P.map_a[p], bar_full(s), m0 + blk * EPB, k0, b);
+              } else {
+                tma_load_3d(sa, &P.map_a[p], bar_full(s), k0, m0, b);
+              }
+              if (P.b_mn[p]) {
+                for (int blk = 0; blk < BN / EPB; ++blk)
+                  tma_load_3d(sb + blk * (BK * kStageRowBytes), &P.map_b[p], bar_full(s), n0 + blk * EPB, k0, b);
+              } else {
+                tma_load_3d(sb, &P.map_b[p], bar_full(s), k0, n0, b);
+              }
             }
             __syncwarp();
             if (++s == stages) { s = 0; ph ^= 1; }
@@ -509,15 +503,12 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
     // ===================== TMA producer =====================
     int s = 0;
     uint32_t ph = 0;
-    int dbg_n = 0;
     for (int item = blockIdx.x; item < P.num_items; item += gridDim.x) {
       int nt = item % P.n_tiles, mt = (item / P.n_tiles) % P.m_tiles, b = item / (P.n_tiles * P.m_tiles);
       int m0 = mt * BM, n0 = nt * BN;
       for (int p = 0; p < P.num_pairs; ++p) {
         for (int kb = 0, nkb = (P.kd[p] + BK - 1) / BK; kb < nkb; ++kb) {
           mbar_wait(bar_empty(s), ph ^ 1);
-          if (P.dbg && blockIdx.x == 0 && lane == 0 && dbg_n < 128) P.dbg[dbg_n * 8 + 0] = clock64();
-          ++dbg_n;
           const uint32_t sa = smem_base + (uint32_t)s * stage_bytes, sb = sa + a_bytes;
           const int k0 = kb * BK;
           if (P.pack2) {
@@ -571,7 +562,6 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
           const uint64_t desc_b0 = make_desc(smem_base, b_lbo, P.b_mn[p] ? 512 : 1024, P.b_mn[p] ? 1 : 2);
           for (int kb = 0, nkb = (P.kd[p] + BK - 1) / BK; kb < nkb; ++kb, ++kc) {
             mbar_wait(bar_lo(s), ph);
-            if (P.dbg && blockIdx.x == 0 && kc < 128) P.dbg[kc * 8 + 5] = clock64();
             tc_fence_after();
             const uint32_t ts = kc % (uint32_t)kTsSlots;
             const uint32_t a_stage = tm + ring0 + ts * kRingCols;
@@ -586,7 +576,6 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
             }
             umma_commit(bar_empty(s));
             umma_commit(bar_tfree(ts));
-            if (P.dbg && blockIdx.x == 0 && kc < 128) P.dbg[kc * 8 + 6] = clock64();
             accum = 1;
             if (++s == stages) { s = 0; ph ^= 1; }
           }
@@ -615,7 +604,6 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
             continue;
           }
           mbar_wait(bar_full(s), ph);
-          if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 128) P.dbg[kc * 8 + 1] = clock64();
           const uint32_t sa = smem_base + (uint32_t)s * stage_bytes, sb = sa + a_bytes;
           // B: hi in place, lo behind it
           for (uint32_t ch = t; ch < b_bytes / 16; ch += 128) {
@@ -639,10 +627,8 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
               x[4 * c] = v.x, x[4 * c + 1] = v.y, x[4 * c + 2] = v.z, x[4 * c + 3] = v.w;
             }
           }
-          if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 128) P.dbg[kc * 8 + 2] = clock64();
           const uint32_t slot = kc % (uint32_t)kTsSlots;
           mbar_wait(bar_tfree(slot), ((kc / (uint32_t)kTsSlots) & 1u) ^ 1u);
-          if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 128) P.dbg[kc * 8 + 3] = clock64();
           tc_fence_after();
           const uint32_t a_stage = tmem_base + ((uint32_t)(q * 32) << 16) + ring0 + slot * kRingCols;
 #pragma unroll
@@ -658,7 +644,6 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
           tmem_st_wait();
           tc_fence_before();
           mbar_arrive(bar_lo(s));
-          if (P.dbg && blockIdx.x == 0 && t == 0 && kc < 128) P.dbg[kc * 8 + 4] = clock64();
           if (++s == stages) { s = 0; ph ^= 1; }
         }
       }
@@ -698,7 +683,6 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
       ew_item<true>(P, ew, b, m);
       ew_load<true>(P, ew, b, m, nt * BN);
       mbar_wait(bar_tfull(ab), aph);
-      if (P.dbg && blockIdx.x == 0 && threadIdx.x == 192 && it < 32) P.dbg[(128 + it) * 8 + 0] = clock64();
       tc_fence_after();
       for (int c0 = 0; c0 < BN; c0 += 32) {
         const int n0 = nt * BN + c0;
@@ -709,7 +693,6 @@ __global__ void __launch_bounds__(kThreadsTs, 1) k_tc_gemm_ts(const __grid_const
       }
       tc_fence_before();
       mbar_arrive(bar_tempty(ab));
-      if (P.dbg && blockIdx.x == 0 && threadIdx.x == 192 && it < 32) P.dbg[(128 + it) * 8 + 1] = clock64();
     }
     if (P.tma_out && lane == 0) tma_store_wait_all();
   }
@@ -903,11 +886,6 @@ int gemm(const GemmProblem& p, cudaStream_t stream) {
   P.alpha = p.alpha, P.accumulate = p.accumulate, P.out_bf16 = p.out_bf16;
   P.skip_lo_b_mask = p.skip_lo_b_mask;
   P.ew_S = p.ew_S, P.ew_d = p.ew_d, P.ew_coef = p.ew_coef, P.ew_eps = p.ew_eps;
-  P.dbg = ts ? g_engine_dbg : nullptr;
-  {
-    const char* e = getenv("TGPB200_ABL_GEMM");
-    P.abl = e ? atoi(e) : 0;
-  }
   // TMA-store epilogue: row-major destination, no read-modify-write, 16-byte aligned rows
   {
     const int oes = p.out_bf16 ? 2 : 4;
