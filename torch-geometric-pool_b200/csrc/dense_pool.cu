@@ -611,6 +611,108 @@ static __global__ void k_link_fix(const float* __restrict__ partial, int64_t n, 
   }
 }
 
+// Link-loss gradient from the direct residual R = A - S S^T, only when the forward took it (losses[5] != 0; every CTA
+// returns at once otherwise).  With q = ||R||^2 and cq = dL/dq:  dS += -2 cq (R + R^T) S,  dA += 2 cq R.  The identity
+// form (W + T^T and S M through Graw / P, 2 A in k_da_elementwise) subtracts terms of the size of S S^T S to leave a
+// residual-sized gradient, which float32 (and the bf16 operands) cannot resolve.  Work item = (graph, 64 rows of
+// nodes): dS rows and dA rows of the item belong to it alone, reductions in a fixed order.  FP32 pipe: a rare path,
+// where shape generality matters, not speed.
+template <typename T>
+static __global__ void __launch_bounds__(256, 1)
+    k_link_grad(const T* __restrict__ A, const T* __restrict__ S, int N, int K, int tiles_n, int64_t total,
+                const float* __restrict__ gl, const float* __restrict__ losses, float link_div, T* __restrict__ dS,
+                T* __restrict__ dA) {
+  if (losses[5] == 0.f) return;
+  const float q = losses[4], L = sqrtf(fmaxf(q, 0.f));
+  const float cq = L > 0.f ? gl[2] / (2.f * L * link_div) : 0.f;
+  if (cq == 0.f) return;
+  __shared__ float si[16][65], sj[16][65];
+  __shared__ float rs[64][65];  // (R + R^T) over the current 64 x 64 tile
+  __shared__ float sk[64][65];  // rows of the tile's S_J, 64 columns at a time
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;  // 4 x 4 micro-tile per thread
+  for (int64_t wid = blockIdx.x; wid < total; wid += gridDim.x) {
+    const int b = (int)(wid / tiles_n), i0 = (int)(wid % tiles_n) * 64;
+    const T* Sb = S + (int64_t)b * N * K;
+    const T* Ab = A + (int64_t)b * N * N;
+    for (int c0 = 0; c0 < K; c0 += 64) {  // 64 columns of dS at a time
+      float acc[4][4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+#pragma unroll
+        for (int v = 0; v < 4; ++v) acc[u][v] = 0.f;
+      for (int j0 = 0; j0 < N; j0 += 64) {
+        float p[4][4];  // (S S^T) over rows i0.. x columns j0..
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+#pragma unroll
+          for (int v = 0; v < 4; ++v) p[u][v] = 0.f;
+        for (int k0 = 0; k0 < K; k0 += 16) {
+          for (int e = threadIdx.x; e < 64 * 16; e += 256) {
+            const int r = e >> 4, k = e & 15;
+            const bool kin = k0 + k < K;
+            si[k][r] = (kin && i0 + r < N) ? to_f32<T>(Sb[(int64_t)(i0 + r) * K + k0 + k]) : 0.f;
+            sj[k][r] = (kin && j0 + r < N) ? to_f32<T>(Sb[(int64_t)(j0 + r) * K + k0 + k]) : 0.f;
+          }
+          __syncthreads();
+#pragma unroll
+          for (int k = 0; k < 16; ++k) {
+            float a[4], c[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) a[u] = si[k][ty * 4 + u], c[u] = sj[k][tx * 4 + u];
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+#pragma unroll
+              for (int v = 0; v < 4; ++v) p[u][v] = fmaf(a[u], c[v], p[u][v]);
+          }
+          __syncthreads();
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+#pragma unroll
+          for (int v = 0; v < 4; ++v) {
+            const int i = i0 + ty * 4 + u, j = j0 + tx * 4 + v;
+            float r2 = 0.f;
+            if (i < N && j < N) {
+              const float rij = to_f32<T>(Ab[(int64_t)i * N + j]) - p[u][v];
+              r2 = rij + (to_f32<T>(Ab[(int64_t)j * N + i]) - p[u][v]);
+              if (dA && c0 == 0) {
+                T* o = dA + (int64_t)b * N * N + (int64_t)i * N + j;
+                *o = from_f32<T>(fmaf(2.f * cq, rij, to_f32<T>(*o)));
+              }
+            }
+            rs[ty * 4 + u][tx * 4 + v] = r2;
+          }
+        for (int e = threadIdx.x; e < 64 * 64; e += 256) {
+          const int r = e >> 6, k = e & 63;
+          sk[r][k] = (j0 + r < N && c0 + k < K) ? to_f32<T>(Sb[(int64_t)(j0 + r) * K + c0 + k]) : 0.f;
+        }
+        __syncthreads();
+#pragma unroll 8
+        for (int j = 0; j < 64; ++j) {
+          float a[4], c[4];
+#pragma unroll
+          for (int u = 0; u < 4; ++u) a[u] = rs[ty * 4 + u][j], c[u] = sk[j][tx * 4 + u];
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+#pragma unroll
+            for (int v = 0; v < 4; ++v) acc[u][v] = fmaf(a[u], c[v], acc[u][v]);
+        }
+        __syncthreads();
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+#pragma unroll
+        for (int v = 0; v < 4; ++v) {
+          const int i = i0 + ty * 4 + u, k = c0 + tx * 4 + v;
+          if (i < N && k < K) {
+            T* o = dS + ((int64_t)b * N + i) * K + k;
+            *o = from_f32<T>(fmaf(-2.f * cq, acc[u][v], to_f32<T>(*o)));
+          }
+        }
+    }
+  }
+}
+
 // DMoN statistics of graph b = blockIdx.x, one block per graph, fixed reduction order (no atomics):
 //   c = S^T d, e = S^T 1 (cvec / evec [B, K]), 2m = sum_i d_i with d = A 1 (k_row_stats / the fused forward),
 //   dst[b] = {2m, ||c||^2, ||e||^2, spectral_b, cluster_b, 0, 0, 0}, and stats[b][7] = 2m for k_graph_bwd.
@@ -737,7 +839,8 @@ static __global__ void __launch_bounds__(512)
   } else if (loss_kind == 2) {
     float q = losses[4];
     float L = sqrtf(fmaxf(q, 0.f));
-    float cq = L > 0.f ? g_link / (2.f * L * link_div) : 0.f;  // dL/dq
+    // dL/dq; 0 when the forward took the direct residual (losses[5]): k_link_grad then adds the link terms
+    float cq = (L > 0.f && losses[5] == 0.f) ? g_link / (2.f * L * link_div) : 0.f;
     c_a2 = cq, c_num = -2.f * cq, c_m2 = cq;
     c_ent = g_ent / ent_div;
   } else if (loss_kind == 3) {  // DMoN spectral loss through t = tr(S^T A S): -gamma / 2m on the diagonal
@@ -1330,6 +1433,13 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
         launch("k_da_elementwise", k_da_elementwise<T>, (unsigned)ceil_div((int64_t)B * NN, 256), 256, 0, st, A,
                row_term, row_coef, (int64_t)B * NN, N, dA_out);
     }
+  }
+  if (loss_kind == 2 && have_a && gl) {  // link terms from the direct residual, when the forward took it
+    const int tn = (N + 63) / 64;
+    const int64_t total = (int64_t)B * tn;
+    const int64_t cap = (int64_t)tc::device_sm_count() * 8;
+    launch("k_link_grad", k_link_grad<T>, (unsigned)(total < cap ? total : cap), 256, 0, st, A, S, N, K, tn, total, gl,
+           pl.losses, link_div, dS_out, dA_out);
   }
   return launch_status();
 }
