@@ -1150,7 +1150,7 @@ static int mm(int batch, int M, int N, int npairs, const int* kd, const Mat* A, 
   p.out_bf16 = std::is_same<TC, __nv_bfloat16>::value;
   p.in_bf16 = std::is_same<T, __nv_bfloat16>::value;
   if (tc::gemm_supported(p)) {
-    if (hook.S && ocs == 1 && ors == N) {
+    if (hook.S && ocs == 1 && ors == N && aligned16(hook.S)) {  // ew_load reads S in 128-bit pieces
       p.ew_S = hook.S, p.ew_d = hook.d, p.ew_coef = hook.coef, p.ew_eps = hook.eps;
       if (hook.applied) *hook.applied = true;
     }
@@ -1178,7 +1178,6 @@ static int mm1(int batch, int M, int N, int kd, Mat A, Mat Bm, TC* out, int64_t 
 
 // How a per-graph kernel splits a [K, K] matrix over a cluster: R CTAs of `threads` threads, `rows_per` rows each,
 // with `nvec` K-vectors and the row partials in shared memory.
-static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 struct StripPlan {
   int R, rows_per, threads, rowp_floats;
   size_t smem;

@@ -532,7 +532,9 @@ static int launch_fwd(const void* x, const int64_t* node_index, const float* wei
                       const int32_t* ptr, int64_t N, int64_t nnz, int64_t K, int64_t F, int op, void* out,
                       cudaStream_t st) {
   constexpr int W = Vec<XT>::N;
-  bool vec = (F % W == 0) && (F % Vec<OT>::N == 0) && Vec<OT>::N == W;
+  // 16-byte chunks: whole rows AND 16-byte aligned bases (an unaligned view takes the scalar chunks, never the row
+  // kernels, which exist in vector form only)
+  bool vec = (F % W == 0) && (F % Vec<OT>::N == 0) && Vec<OT>::N == W && aligned16(x) && aligned16(out);
   int64_t chunks = ceil_div(F, W);
   int lpr = 1;
   while (lpr < 32 && lpr < chunks) lpr <<= 1;
@@ -562,7 +564,9 @@ static int launch_bwd(const void* x, const int64_t* node_index, const int64_t* c
                       const int32_t* order, const int32_t* ptr, const void* pool, const void* gpool, int64_t N,
                       int64_t nnz, int64_t K, int64_t F, int op, void* gx, float* gw, Workspace& ws, cudaStream_t st) {
   constexpr int W = Vec<XT>::N;
-  bool vec = (F % W == 0) && Vec<OT>::N == W;
+  const bool minmax = op == TGPB200_MAX || op == TGPB200_MIN;
+  bool vec = (F % W == 0) && Vec<OT>::N == W && aligned16(x) && aligned16(gpool) && aligned16(gx) &&
+             (!minmax || aligned16(pool));
   int32_t* first = ws.take<int32_t>((size_t)(N > 0 ? N : 1));
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (N > 0 && N <= 32768 && nnz <= 32768) {
@@ -573,7 +577,7 @@ static int launch_bwd(const void* x, const int64_t* node_index, const int64_t* c
       launch("k_first_entry", k_first_entry, (unsigned)ceil_div(nnz, 256), 256, 0, st, node_index, nnz, N, first);
   }
   float* inv_ties = nullptr;
-  if (op == TGPB200_MAX || op == TGPB200_MIN) {
+  if (minmax) {
     inv_ties = ws.take<float>((size_t)K * F);
     if (!ws.ok) return TGPB200_ERR_WORKSPACE;
     if (K * F > 0)

@@ -37,6 +37,7 @@ struct KernelParams {
   // 128 x 64 tile (measured with a cycle-counter timeline of the fp32 engine), stalling the split warps that share it.
   CUtensorMap map_out;
   int tma_out;       // 1: use map_out
+  int out_vec;       // 1: `out` is 16-byte aligned (the register-store epilogue may write 128-bit pieces)
   int epi_bufs;      // staging buffers per epilogue warp (1 or 2)
   int pack2;         // fp32 TMEM-operand engine: one 128 x 128 tile holds the products of TWO batch items with M, N <= 64
 };
@@ -188,7 +189,7 @@ __device__ __forceinline__ void store_chunk(const KernelParams& P, float (&v)[32
     }
     // every thread owns one row and moves its 32 values as 8 x 128-bit accesses
     if (m < P.M) {
-      if (!P.out_bf16 && full && (((obase + n0) & 3) == 0)) {
+      if (P.out_vec && !P.out_bf16 && full && (((obase + n0) & 3) == 0)) {
         float4* o4 = reinterpret_cast<float4*>(reinterpret_cast<float*>(P.out) + obase + n0);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
@@ -199,7 +200,7 @@ __device__ __forceinline__ void store_chunk(const KernelParams& P, float (&v)[32
           }
           o4[j] = r4;
         }
-      } else if (P.out_bf16 && full && (((obase + n0) & 7) == 0)) {
+      } else if (P.out_vec && P.out_bf16 && full && (((obase + n0) & 7) == 0)) {
         uint4* o4 = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(P.out) + obase + n0);
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
@@ -893,6 +894,7 @@ int gemm(const GemmProblem& p, cudaStream_t stream) {
     // each -- room for two 2 KB bf16 chunks, so a store can still read one while the next chunk is staged
     P.epi_bufs = bf16 ? (p.out_bf16 ? 2 : 1) : 2;
     P.tma_out = 0;
+    P.out_vec = ((uintptr_t)p.out & 15) == 0;
     if (p.out_col_stride == 1 && !p.accumulate && ((uintptr_t)p.out & 15) == 0 &&
         (p.out_row_stride * oes) % 16 == 0 && (p.out_batch_stride * oes) % 16 == 0 && p.out_row_stride >= p.N) {
       EncodeTiledFn fn = encode_fn();
