@@ -285,6 +285,32 @@ int tgpb200_dense_pool_bwd_v2(const void* adj, const void* s, const void* x, con
                               const float* graph_nodes);
 
 /* ------------------------------------------------------------------------------------------
+ * Asymmetric Cheeger Cut (TVGNN) losses of batched dense assignments (csrc/dense_acc.cu), next to the fused dense
+ * path (x_pool / adj_pool come from tgpb200_dense_pool_fwd with loss_kind 0).  adj [B,N,N] (raw), s [B,N,K] row-major
+ * of `dtype`, fp32 arithmetic, fixed-order sums; needs N >= 1, K >= 2, B <= 65535.
+ *   losses[0] = mean_b sum_ij A_ij ||S_i - S_j||_1 / (2 nnz(A_b))     replaces totvar_loss (tests/acc_oracle.py);
+ *               self loops count in nnz, an edgeless graph gives NaN
+ *   losses[1] = mean_b 1 - sum_ik f(S_ik - q_bk) / (N (K - 1))         replaces asym_norm_loss (tests/acc_oracle.py);
+ *               f(d) = (K - 1) d for d >= 0, -d otherwise; q_bk (written to `quant` [B,K], dtype) = the entry a
+ *               stable descending sort of column k puts at position N // K (N padded; -0.0 ties +0.0)
+ * `saved` (tgpb200_acc_loss_saved_bytes) carries, 256-byte aligned in this order: nnz(A_b) int64 [B], the quantile
+ * rows int32 [B,K], #{i : S_ik >= q_bk} int32 [B,K].  `workspace` (tgpb200_acc_loss_fwd_workspace_bytes) holds the
+ * per-tile partial sums of the forward; the backward needs no scratch.
+ * Backward (grad_losses = 2 device floats or NULL), c_b = g0 / (2 nnz_b B), e = g1 / (N (K - 1) B):
+ *   grad_s_ik = c_b sum_j (A_ij + A_ji) sign(S_ik - S_jk) - e f'(S_ik - q_k) (+ e sum_i f'(S_ik - q_k) at the
+ *               quantile row), f' = K - 1 on d >= 0 and -1 below;  grad_adj_ij = c_b ||S_i - S_j||_1 (grad_adj may be
+ *               NULL).  A zero g0 contributes nothing.
+ * ------------------------------------------------------------------------------------------ */
+size_t tgpb200_acc_loss_saved_bytes(int64_t B, int64_t K);
+size_t tgpb200_acc_loss_fwd_workspace_bytes(int64_t B, int64_t N, int64_t K);
+int tgpb200_acc_loss_fwd(const void* adj, const void* s, int64_t B, int64_t N, int64_t K, int dtype, float* losses,
+                         void* quant, void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes,
+                         tgpb200_stream_t stream);
+int tgpb200_acc_loss_bwd(const void* adj, const void* s, const void* saved, size_t saved_bytes,
+                         const float* grad_losses, int64_t B, int64_t N, int64_t K, int dtype, void* grad_s,
+                         void* grad_adj, tgpb200_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * Tensor-core batched product (tcgen05 / TMEM / TMA), the engine under the dense path; exported for tests
  * and for callers that need a raw S^T X / S^T A S style contraction:
  *   out[b] (M x N) = alpha * A[b] (M x Kd) * B[b] (Kd x N)  (+ out[b] when accumulate)

@@ -111,6 +111,52 @@ std::tuple<Tensor, Tensor, Tensor> stas_fused_bwd(const OptTensor& x, const OptT
   return {gx, ga, gs};
 }
 
+// (losses[2] = {total variation, balance}, quant [B, K], saved) of Asymmetric Cheeger Cut pooling
+// (totvar_loss / asym_norm_loss as restated in tests/acc_oracle.py)
+void acc_check_args(const Tensor& adj, const Tensor& s) {
+  require_cuda(s, "s");
+  require_cuda(adj, "adj");
+  TORCH_CHECK(s.dim() == 3, "acc_losses expects s of shape [B, N, K], got ", s.sizes());
+  TORCH_CHECK(adj.dim() == 3 && adj.size(0) == s.size(0) && adj.size(1) == s.size(1) && adj.size(2) == s.size(1),
+              "acc_losses expects adj of shape [B, N, N] = [", s.size(0), ", ", s.size(1), ", ", s.size(1), "], got ",
+              adj.sizes());
+  TORCH_CHECK(adj.scalar_type() == s.scalar_type(), "tgp_b200.acc_losses: adj and s must share one dtype");
+  TORCH_CHECK_VALUE(s.size(2) >= 2, "acc_losses needs K >= 2 clusters (the balance loss divides by K - 1), got K = ",
+                    s.size(2));
+  TORCH_CHECK_VALUE(s.size(1) >= 1, "acc_losses needs N >= 1 nodes");
+}
+
+std::tuple<Tensor, Tensor, Tensor> acc_losses(const Tensor& adj, const Tensor& s) {
+  acc_check_args(adj, s);
+  c10::cuda::CUDAGuard guard(s.device());
+  const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
+  Tensor saved = workspace(tgpb200_acc_loss_saved_bytes(B, K), s);
+  Tensor ws = workspace(tgpb200_acc_loss_fwd_workspace_bytes(B, N, K), s);
+  Tensor losses = at::empty({2}, s.options().dtype(at::kFloat));
+  Tensor quant = at::empty({B, K}, s.options());
+  check(tgpb200_acc_loss_fwd(adj.data_ptr(), s.data_ptr(), B, N, K, dtype_code(s), losses.data_ptr<float>(),
+                             quant.data_ptr(), saved.data_ptr(), (size_t)saved.numel(), ws.data_ptr(),
+                             (size_t)ws.numel(), stream_of(s)),
+        "acc_losses");
+  return {losses, quant, saved};
+}
+
+std::tuple<Tensor, Tensor> acc_losses_bwd(const Tensor& adj, const Tensor& s, const Tensor& saved,
+                                          const Tensor& glosses, bool need_gadj) {
+  acc_check_args(adj, s);
+  c10::cuda::CUDAGuard guard(s.device());
+  const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
+  TORCH_CHECK(glosses.numel() == 2, "acc_losses_bwd expects 2 upstream loss gradients");
+  Tensor gl = glosses.to(at::kFloat).contiguous();
+  Tensor gs = at::empty_like(s);
+  Tensor ga = need_gadj ? at::empty_like(adj) : at::empty({0}, s.options());
+  check(tgpb200_acc_loss_bwd(adj.data_ptr(), s.data_ptr(), saved.data_ptr(), (size_t)saved.numel(),
+                             gl.data_ptr<float>(), B, N, K, dtype_code(s), gs.data_ptr(),
+                             need_gadj ? ga.data_ptr() : nullptr, stream_of(s)),
+        "acc_losses_bwd");
+  return {ga, gs};
+}
+
 // CSR-by-cluster of a sparse assignment (tgp/reduce/aggr_reduce.py:13-23)
 std::tuple<Tensor, Tensor> build_csr(const Tensor& cluster_index, int64_t num_clusters) {
   require_cuda(cluster_index, "cluster_index");
@@ -174,6 +220,8 @@ TORCH_LIBRARY(tgp_b200, m) {
   m.def("stas_fused_bwd(Tensor? x, Tensor? adj, Tensor s, Tensor saved, Tensor? gx_pool, Tensor? gadj_pool, "
         "Tensor? glosses, int flags, int loss_kind, float link_div, float ent_div, bool need_gadj, "
         "Tensor? graph_nodes=None) -> (Tensor, Tensor, Tensor)");
+  m.def("acc_losses(Tensor adj, Tensor s) -> (Tensor, Tensor, Tensor)");
+  m.def("acc_losses_bwd(Tensor adj, Tensor s, Tensor saved, Tensor glosses, bool need_gadj) -> (Tensor, Tensor)");
   m.def("build_csr(Tensor cluster_index, int num_clusters) -> (Tensor, Tensor)");
   m.def("segment_reduce(Tensor x, Tensor node_index, Tensor cluster_index, Tensor? weight, Tensor order, Tensor ptr, "
         "int num_clusters, int op) -> Tensor");
@@ -184,6 +232,8 @@ TORCH_LIBRARY(tgp_b200, m) {
 TORCH_LIBRARY_IMPL(tgp_b200, CUDA, m) {
   m.impl("stas_fused", &stas_fused);
   m.impl("stas_fused_bwd", &stas_fused_bwd);
+  m.impl("acc_losses", &acc_losses);
+  m.impl("acc_losses_bwd", &acc_losses_bwd);
   m.impl("build_csr", &build_csr);
   m.impl("segment_reduce", &segment_reduce);
   m.impl("segment_reduce_bwd", &segment_reduce_bwd);

@@ -101,6 +101,10 @@ SIGNATURES = {
         [_P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _INT, _U32, _INT, _F, _F, _F, _P, _P, _P, _P, _SZ, _P, _SZ, _P,
          _P],
     ),
+    "tgpb200_acc_loss_saved_bytes": (_SZ, [_I64, _I64]),
+    "tgpb200_acc_loss_fwd_workspace_bytes": (_SZ, [_I64, _I64, _I64]),
+    "tgpb200_acc_loss_fwd": (_INT, [_P, _P, _I64, _I64, _I64, _INT, _P, _P, _P, _SZ, _P, _SZ, _P]),
+    "tgpb200_acc_loss_bwd": (_INT, [_P, _P, _P, _SZ, _P, _I64, _I64, _I64, _INT, _P, _P, _P]),
 }
 
 

@@ -349,6 +349,22 @@ def dense_pool(
     return (x_pool if x is not None else None), (adj_pool if adj is not None else None), losses
 
 
+def acc_losses(adj: Tensor, s: Tensor) -> Tensor:
+    """``[total variation, balance]`` losses of Asymmetric Cheeger Cut pooling (TVGNN), batch means, from the RAW
+    ``adj`` [B, N, N] and ``s`` [B, N, K] (padded rows zero), differentiable in both:
+
+    * total variation: ``sum_ij A_ij ||S_i - S_j||_1 / (2 nnz(A_b))`` (self loops count; an edgeless graph gives NaN);
+    * balance: ``1 - sum_ik f(S_ik - q_k) / (N (K - 1))`` with ``q_k`` the entry of rank ``N // K`` of column ``k`` in
+      a stable descending sort over the N (padded) rows and ``f(d) = (K - 1) d`` for ``d >= 0``, ``-d`` otherwise.
+
+    No ``[B, N, N, K]`` tensor is formed.  ``K < 2`` raises ``ValueError``."""
+    _require_cuda(adj, s)
+    if s.dim() == 3 and s.size(-1) < 2:
+        raise ValueError(f"acc_losses needs K >= 2 clusters, got K = {s.size(-1)}")
+    losses, _, _ = _T.acc_losses(adj.contiguous(), s.contiguous())
+    return losses
+
+
 # --------------------------------------------------------------------------- #
 # Dense -> block-diagonal sparse output, dense pre-processing
 # --------------------------------------------------------------------------- #

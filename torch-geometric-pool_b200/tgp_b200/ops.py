@@ -1,6 +1,6 @@
 """``torch.ops.tgp_b200.*``: the operators of the Reduce + Connect path as torch custom ops (SURVEY 8b).
 
-* ``stas_fused`` / ``stas_fused_bwd``, ``segment_reduce`` / ``segment_reduce_bwd``, ``build_csr`` are C++ dispatcher
+* ``stas_fused`` / ``stas_fused_bwd``, ``acc_losses`` / ``acc_losses_bwd``, ``segment_reduce`` / ``segment_reduce_bwd``, ``build_csr`` are C++ dispatcher
   ops (``csrc/torch_ops.cpp`` -> ``libtgp_b200_ops.so``: allocate with the caching allocator, take the current stream,
   call the C ABI of ``libtgp_b200.so``);
 * ``filter_relabel_edges``, ``remap_coalesce``, ``degree_norm``, ``weight_norm`` (+ their ``*_bwd``) are
@@ -76,6 +76,42 @@ def _stas_backward(ctx, gx_pool, gadj_pool, glosses, _gsaved):
 
 
 torch.library.register_autograd("tgp_b200::stas_fused", _stas_backward, setup_context=_stas_setup)
+
+
+# --------------------------------------------------------------------------------------------------------------
+# acc_losses: (losses[2] = {total variation, balance}, quant [B, K], saved) of Asymmetric Cheeger Cut pooling.
+# quant (the balance loss's per-column quantile) and saved carry no gradient.
+# --------------------------------------------------------------------------------------------------------------
+@torch.library.register_fake("tgp_b200::acc_losses")
+def _acc_losses_fake(adj, s):
+    B, N, K = s.shape
+    saved = L.load().tgpb200_acc_loss_saved_bytes(B, K)
+    return (s.new_empty((2,), dtype=torch.float32), s.new_empty((B, K)),
+            s.new_empty((max(saved, 256),), dtype=torch.uint8))
+
+
+@torch.library.register_fake("tgp_b200::acc_losses_bwd")
+def _acc_losses_bwd_fake(adj, s, saved, glosses, need_gadj):
+    return (torch.empty_like(adj) if need_gadj else s.new_empty((0,))), torch.empty_like(s)
+
+
+def _acc_setup(ctx, inputs, output):
+    adj, s = inputs
+    ctx.save_for_backward(adj, s, output[2])
+    ctx.mark_non_differentiable(output[1], output[2])
+    ctx.set_materialize_grads(False)
+
+
+def _acc_backward(ctx, glosses, _gquant, _gsaved):
+    adj, s, saved = ctx.saved_tensors
+    if glosses is None:
+        return None, None
+    need_adj = ctx.needs_input_grad[0]
+    ga, gs = _T.acc_losses_bwd(adj, s, saved, glosses, need_adj)
+    return (ga if need_adj else None), gs
+
+
+torch.library.register_autograd("tgp_b200::acc_losses", _acc_backward, setup_context=_acc_setup)
 
 
 # --------------------------------------------------------------------------------------------------------------
@@ -393,6 +429,6 @@ def _wn_backward(ctx, g, _gmx, _garg):
 
 torch.library.register_autograd("tgp_b200::weight_norm", _wn_backward, setup_context=_wn_setup)
 
-OP_NAMES = ("stas_fused", "stas_fused_bwd", "build_csr", "segment_reduce", "segment_reduce_bwd", "filter_relabel_edges",
+OP_NAMES = ("stas_fused", "stas_fused_bwd", "acc_losses", "acc_losses_bwd", "build_csr", "segment_reduce", "segment_reduce_bwd", "filter_relabel_edges",
             "filter_relabel_edges_bwd", "remap_coalesce", "remap_coalesce_bwd", "degree_norm", "degree_norm_bwd",
             "weight_norm", "weight_norm_bwd")

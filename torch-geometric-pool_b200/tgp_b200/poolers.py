@@ -1,8 +1,8 @@
 """Pooler-level orchestration of the path (what the pooler ``forward``s do after ``select``).
 
 ``mincut_pool`` / ``diff_pool`` / ``dmon_pool`` run reduce + connect + auxiliary losses + post-processing as ONE
-fused forward and ONE fused backward; ``topk_pool`` / ``cluster_pool`` chain the sparse reduce and
-the sparse connect.  ``patch_pooler`` installs the B200 operators on a reference pooler object.
+fused forward and ONE fused backward; ``acc_pool`` adds the Asymmetric Cheeger Cut losses (their own kernels) to the
+loss-free fused call; ``topk_pool`` / ``cluster_pool`` chain the sparse reduce and the sparse connect.  ``patch_pooler`` installs the B200 operators on a reference pooler object.
 """
 from __future__ import annotations
 
@@ -88,6 +88,29 @@ def dmon_pool(
     return x_pool, adj_pool, loss
 
 
+def acc_pool(
+    x: Tensor,
+    adj: Tensor,
+    s: Tensor,
+    totvar_coeff: float = 1.0,
+    balance_coeff: float = 1.0,
+    remove_self_loops: bool = True,
+    degree_norm: bool = True,
+    adj_transpose: bool = True,
+    edge_weight_norm: bool = False,
+) -> Tuple[Tensor, Tensor, Dict[str, Tensor]]:
+    """AsymCheegerCutPooling.forward batched path after select: ``S^T X`` and ``postprocess(S^T A S)`` from the fused
+    dense path (no loss there), and the total-variation and balance losses of Asymmetric Cheeger Cut pooling
+    (restated in ``tests/acc_oracle.py``) from ``functional.acc_losses`` on the raw ``adj``."""
+    x_pool, adj_pool, _ = F_.dense_pool(
+        x, adj, s, remove_self_loops=remove_self_loops, degree_norm=degree_norm, adj_transpose=adj_transpose,
+        edge_weight_norm=edge_weight_norm, loss_kind=F_.LOSS_NONE,
+    )
+    losses = F_.acc_losses(adj, s)
+    tv_key, bal_key = _ACC_KEYS
+    return x_pool, adj_pool, {tv_key: losses[0] * totvar_coeff, bal_key: losses[1] * balance_coeff}
+
+
 def sparse_pool(
     x: Tensor,
     edge_index: Tensor,
@@ -159,6 +182,10 @@ def _pooling_output_cls():
 
 
 _DMON_COEFFS = ("spectral_loss_coeff", "cluster_loss_coeff", "ortho_loss_coeff")
+# AsymCheegerCutPooling: its class name, its coefficient attributes (total variation, balance) and its loss keys
+_ACC_CLASS = "AsymCheegerCutPooling"
+_ACC_COEFFS = ("totvar_coeff", "balance_coeff")
+_ACC_KEYS = ("total_variation_loss", "balance_loss")
 _AGGR_TO_OP = {"SumAggregation": "sum", "MeanAggregation": "mean", "MaxAggregation": "max", "MinAggregation": "min"}
 
 
@@ -178,7 +205,7 @@ def _reduce_op_of(reducer) -> Optional[str]:
 
 
 def _fused_dense_forward(pooler, kind: str):
-    """``forward`` of a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` (tgp/poolers/mincut.py:210-258,
+    """``forward`` of a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` / ``AsymCheegerCutPooling`` (tgp/poolers/mincut.py:210-258,
     tgp/poolers/diffpool.py:200-237) with reduce + connect + auxiliary losses + post-processing as ONE fused
     forward / backward; select, input densification, lifting and the unbatched mode stay the reference's."""
     ref_forward = pooler.forward
@@ -200,6 +227,8 @@ def _fused_dense_forward(pooler, kind: str):
         elif kind == "dmon":
             x_pool, adj_pool, loss = dmon_pool(x, adj, so.s, mask, pooler.spectral_loss_coeff, pooler.cluster_loss_coeff,
                                                pooler.ortho_loss_coeff, **flags)
+        elif kind == "acc":
+            x_pool, adj_pool, loss = acc_pool(x, adj, so.s, *(getattr(pooler, a) for a in _ACC_COEFFS), **flags)
         else:
             x_pool, adj_pool, loss = diff_pool(x, adj, so.s, num_nodes=1, link_loss_coeff=pooler.link_loss_coeff,
                                                ent_loss_coeff=1.0, normalize_loss=pooler.normalize_loss, **flags)
@@ -222,10 +251,11 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
       same ctor attributes (the poolers read them, tgp/poolers/mincut.py:233-236);
     * ``pooler.reducer``: ``BaseReduce`` / ``AggrReduce(sum | mean | max | min)`` -> ``B200Reduce`` with the SAME
       reduction; any other reducer (learned / order-statistic aggregators) is left in place.  ``reduce_op`` overrides;
-    * ``fuse_dense``: a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` also gets the fused forward
-      (reduce + connect + losses + post-processing in one kernel chain) -- without it the patched pooler still calls
-      the reference's torch loss functions.  A ``DMoNPooling`` lacking one of ``spectral_loss_coeff``,
-      ``cluster_loss_coeff``, ``ortho_loss_coeff`` keeps the reference forward.
+    * ``fuse_dense``: a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` / ``AsymCheegerCutPooling`` also
+      gets the fused forward (reduce + connect + losses + post-processing on the device kernels) -- without it the
+      patched pooler still calls the reference's torch loss functions.  A ``DMoNPooling`` lacking one of
+      ``spectral_loss_coeff``, ``cluster_loss_coeff``, ``ortho_loss_coeff``, or an ``AsymCheegerCutPooling`` lacking
+      ``totvar_coeff`` or ``balance_coeff``, keeps the reference forward.
     """
     for attr in ("connector", "preconnector"):
         conn = getattr(pooler, attr, None)
@@ -243,8 +273,11 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
         op = reduce_op if reduce_op is not None else _reduce_op_of(reducer)
         if op is not None:
             pooler.reducer = B200Reduce(op)
-    kind = {"MinCutPooling": "mincut", "DiffPool": "diff", "DMoNPooling": "dmon"}.get(type(pooler).__name__)
+    kind = {"MinCutPooling": "mincut", "DiffPool": "diff", "DMoNPooling": "dmon", _ACC_CLASS: "acc"}.get(
+        type(pooler).__name__)
     if kind == "dmon" and not all(hasattr(pooler, a) for a in _DMON_COEFFS):
+        kind = None
+    if kind == "acc" and not all(hasattr(pooler, a) for a in _ACC_COEFFS):
         kind = None
     if fuse_dense and kind is not None and type(getattr(pooler, "connector", None)).__name__ == "B200DenseConnect":
         pooler.forward = _fused_dense_forward(pooler, kind)
