@@ -311,6 +311,37 @@ int tgpb200_acc_loss_bwd(const void* adj, const void* s, const void* saved, size
                          void* grad_adj, tgpb200_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * HOSC (higher-order spectral clustering, Duval & Malliaros 2022) losses of batched dense assignments
+ * (csrc/dense_hosc.cu), next to the fused dense path (x_pool / adj_pool come from tgpb200_dense_pool_fwd, and with
+ * hosc_ortho off the orthogonality term is losses[1] of loss_kind 1).  adj [B,N,N] (raw), s [B,N,K] row-major of
+ * `dtype` (padded rows zero), graph_nodes [B] float32 valid-node counts or NULL (= N); fp32 arithmetic, fixed-order
+ * sums; needs N >= 1, K >= 2, B <= 65535.  `terms` is a bitmask: 1 = first order, 2 = triangle motif, 4 = HOSC
+ * orthogonality; a term outside the mask is written as 0 and launches nothing (no A A product without bit 2).
+ *   d = A 1, n_k = (S^T A S)_kk, m_k = sum_i d_i S_ik^2 + eps; A_M = (A A) . A and d^M, n^M_k, m^M_k the same of A_M
+ *   losses[0] = L1 = mean_b -(1/K) sum_k n_k / m_k          losses[1] = L2 = mean_b -(1/K) sum_k n^M_k / m^M_k
+ *   losses[2] = O  = mean_b (sqrt(K) - sum_k ||S_:k||_2 / sqrt(n_b)) / (sqrt(K) - 1)
+ * (restated in tests/hosc_oracle.py; a graph without triangles gives L2 = 0).  `saved`
+ * (tgpb200_hosc_loss_saved_bytes) carries, 256-byte aligned in this order: A_M [B,N,N] in `dtype` (bit 2 only),
+ * d, d^M float [B,N], n, m, n^M, m^M, ||S_:k||^2 float [B,K].  The forward workspace holds S1 = [S | 1 | 0..],
+ * [A S | d], [A_M S | d^M] and, for bf16, the fp32 A A.
+ * Backward (grad_losses = 3 device floats g or NULL), per order alpha_k = -g / (K B m_k), beta_k = g n_k / (K B m_k^2):
+ *   grad_s = A Sa + A^T Sa + A_M Sm + A_M^T Sm + 2 d S diag(beta1) + 2 d^M S diag(beta2) - g2 S_ik / (B sqrt(n_b)
+ *            (sqrt(K) - 1) ||S_:k||)  with Sa = S diag(alpha1), Sm = S diag(alpha2) (a zero column gets 0)
+ *   grad_adj = S diag(alpha1) S^T + r 1^T + G . P + H A^T + A^T H,  P = A A, G = S diag(alpha2) S^T + r^M 1^T,
+ *            H = G . A, r_i = sum_k beta1_k S_ik^2, r^M the same of beta2 (grad_adj may be NULL)
+ * ------------------------------------------------------------------------------------------ */
+size_t tgpb200_hosc_loss_saved_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype);
+size_t tgpb200_hosc_loss_fwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype);
+int tgpb200_hosc_loss_fwd(const void* adj, const void* s, const float* graph_nodes, int64_t B, int64_t N, int64_t K,
+                          int dtype, int terms, float eps, float* losses, void* saved, size_t saved_bytes,
+                          void* workspace, size_t workspace_bytes, tgpb200_stream_t stream);
+size_t tgpb200_hosc_loss_bwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int dtype, int need_grad_adj);
+int tgpb200_hosc_loss_bwd(const void* adj, const void* s, const float* graph_nodes, const void* saved,
+                          size_t saved_bytes, const float* grad_losses, int64_t B, int64_t N, int64_t K, int dtype,
+                          int terms, void* grad_s, void* grad_adj, void* workspace, size_t workspace_bytes,
+                          tgpb200_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * Tensor-core batched product (tcgen05 / TMEM / TMA), the engine under the dense path; exported for tests
  * and for callers that need a raw S^T X / S^T A S style contraction:
  *   out[b] (M x N) = alpha * A[b] (M x Kd) * B[b] (Kd x N)  (+ out[b] when accumulate)

@@ -1,0 +1,444 @@
+// HOSC (higher-order spectral clustering) losses of batched dense assignments, next to the fused dense chain:
+//   d = A 1,  n_k = (S^T A S)_kk,  m_k = sum_i d_i S_ik^2 + eps                    (first order)
+//   A_M = (A A) . A,  d^M = A_M 1,  n^M_k = (S^T A_M S)_kk,  m^M_k = sum_i d^M_i S_ik^2 + eps   (triangle motif)
+//   L1 = mean_b -(1/K) sum_k n_k / m_k,  L2 = the same of the motif terms,
+//   O  = mean_b (sqrt(K) - sum_k ||S_:k|| / sqrt(n_b)) / (sqrt(K) - 1)             (HOSC's own orthogonality term)
+// The products run through mm() (dense.cuh): P = A A, then [A S | A 1] and [A_M S | A_M 1] as ONE product each with
+// S1 = [S | 1 | 0 ..] (multiplying by one is exact in 3xTF32 and bf16), so the degrees need no kernel of their own.
+// The backward's dS is one four-pair product A Sa + A^T Sa + A_M Sm + A_M^T Sm (Sa = S diag(alpha1), Sm = S
+// diag(alpha2), transposes read MN-major) plus k_hosc_ds_elementwise.  Every sum has a fixed order (no float atomics).
+#include <type_traits>
+
+#include "dense.cuh"
+
+namespace tgp {
+namespace {
+
+constexpr int kFirst = 1, kMotif = 2, kOrtho = 4;  // term mask bits
+constexpr int kPad = 8;                            // S1 width granule: 16 bytes of bf16 (TMA row-stride rule)
+constexpr int kMaxGridY = 65535;
+
+int s1_width(int K) { return (int)ceil_div(K + 1, kPad) * kPad; }
+
+// S1[b, i, :] = [S[b, i, :] | 1 | 0 ..]
+template <typename T>
+__global__ void k_hosc_pad(const T* __restrict__ S, int64_t rows, int K, int K1, T* __restrict__ S1) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= rows * K1) return;
+  const int64_t r = e / K1;
+  const int c = (int)(e - r * K1);
+  S1[e] = c < K ? S[r * K + c] : from_f32<T>(c == K ? 1.f : 0.f);
+}
+
+// A_M = P . A in the operand dtype (P fp32; the fp32 form writes in place over P, so no __restrict__ on P / AM)
+template <typename T>
+__global__ void k_hosc_motif(const float* P, const T* __restrict__ A, int64_t total, T* AM) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < total) AM[e] = from_f32<T>(P[e] * to_f32<T>(A[e]));
+}
+
+// Column statistics of 32 columns k0 .. k0+31 of graph b = blockIdx.y: lane = column, warp w = contiguous row segment;
+// the 8 segment partials are added in segment order.  AS1 / AMS1 are [B, N, K1] fp32 (column K = the degree).
+//   n1 = sum_i S_ik (A S)_ik, m1 = sum_i d_i S_ik^2 + eps, nM / mM the same of A_M, sq = sum_i S_ik^2.
+// Chunk 0 also copies the degrees d, d^M [B, N] for the backward.
+template <typename T>
+__global__ void __launch_bounds__(256)
+    k_hosc_stats(const T* __restrict__ S, const float* __restrict__ AS1, const float* __restrict__ AMS1, int N, int K,
+                 int K1, int terms, float eps, float* __restrict__ d, float* __restrict__ dM, float* __restrict__ n1,
+                 float* __restrict__ m1, float* __restrict__ nM, float* __restrict__ mM, float* __restrict__ sq) {
+  __shared__ float part[5][8][32];
+  const int b = blockIdx.y, t = threadIdx.x, lane = t & 31, w = t >> 5;
+  const int k = blockIdx.x * 32 + lane;
+  const bool kin = k < K;
+  const bool first = terms & kFirst, motif = terms & kMotif;
+  const int seg = (N + 7) / 8, r0 = min(N, w * seg), r1 = min(N, r0 + seg);
+  const T* Sb = S + (int64_t)b * N * K;
+  const float* Ab = first ? AS1 + (int64_t)b * N * K1 : nullptr;
+  const float* Mb = motif ? AMS1 + (int64_t)b * N * K1 : nullptr;
+  float a[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
+  if (kin)
+    for (int i = r0; i < r1; ++i) {
+      const float s = to_f32<T>(Sb[(int64_t)i * K + k]), s2 = s * s;
+      a[4] = fmaf(s, s, a[4]);
+      if (first) {
+        a[0] = fmaf(s, Ab[(int64_t)i * K1 + k], a[0]);
+        a[1] = fmaf(Ab[(int64_t)i * K1 + K], s2, a[1]);
+      }
+      if (motif) {
+        a[2] = fmaf(s, Mb[(int64_t)i * K1 + k], a[2]);
+        a[3] = fmaf(Mb[(int64_t)i * K1 + K], s2, a[3]);
+      }
+    }
+#pragma unroll
+  for (int q = 0; q < 5; ++q) part[q][w][lane] = a[q];
+  if (blockIdx.x == 0)
+    for (int i = t; i < N; i += blockDim.x) {
+      if (first) d[(int64_t)b * N + i] = Ab[(int64_t)i * K1 + K];
+      if (motif) dM[(int64_t)b * N + i] = Mb[(int64_t)i * K1 + K];
+    }
+  __syncthreads();
+  if (w == 0 && kin) {
+    float r[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
+    for (int p = 0; p < 8; ++p)
+#pragma unroll
+      for (int q = 0; q < 5; ++q) r[q] += part[q][p][lane];
+    const int64_t o = (int64_t)b * K + k;
+    n1[o] = r[0], m1[o] = r[1] + eps, nM[o] = r[2], mM[o] = r[3] + eps, sq[o] = r[4];
+  }
+}
+
+// losses = {L1, L2, O} (zero for a term outside the mask).  One block, fixed order.
+__global__ void k_hosc_finalize(const float* __restrict__ n1, const float* __restrict__ m1,
+                                const float* __restrict__ nM, const float* __restrict__ mM,
+                                const float* __restrict__ sq, const float* __restrict__ graph_nodes, int B, int N,
+                                int K, int terms, float* __restrict__ losses) {
+  __shared__ float red[32];
+  float l1 = 0.f, l2 = 0.f, o = 0.f;
+  const float rk = sqrtf((float)K);
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    float c1 = 0.f, c2 = 0.f, cn = 0.f;
+    for (int k = 0; k < K; ++k) {
+      const int64_t e = (int64_t)b * K + k;
+      if (terms & kFirst) c1 += n1[e] / m1[e];
+      if (terms & kMotif) c2 += nM[e] / mM[e];
+      if (terms & kOrtho) cn += sqrtf(sq[e]);
+    }
+    l1 -= c1 / (float)K;
+    l2 -= c2 / (float)K;
+    const float n = graph_nodes ? graph_nodes[b] : (float)N;
+    if (terms & kOrtho) o += (rk - cn / sqrtf(n)) / (rk - 1.f);
+  }
+  l1 = block_sum(l1, red);
+  l2 = block_sum(l2, red);
+  o = block_sum(o, red);
+  if (threadIdx.x == 0) losses[0] = l1 / (float)B, losses[1] = l2 / (float)B, losses[2] = o / (float)B;
+}
+
+// dL/dn_k of each order: alpha = -g / (K B m_k)
+__device__ __forceinline__ float hosc_alpha(float g, float m, int K, int B) { return -g / ((float)K * (float)B * m); }
+// dL/dm_k of each order: beta = g n_k / (K B m_k^2)
+__device__ __forceinline__ float hosc_beta(float g, float n, float m, int K, int B) {
+  return g * n / ((float)K * (float)B * m * m);
+}
+
+// Sa = S diag(alpha1), Sm = S diag(alpha2) in the operand dtype (either may be NULL)
+template <typename T>
+__global__ void k_hosc_scale(const T* __restrict__ S, const float* __restrict__ m1, const float* __restrict__ mM,
+                             const float* __restrict__ gl, int64_t total, int B, int N, int K, T* __restrict__ Sa,
+                             T* __restrict__ Sm) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= total) return;
+  const int64_t row = e / K;
+  const int64_t bk = (row / N) * K + (e - row * K);
+  const float s = to_f32<T>(S[e]);
+  if (Sa) Sa[e] = from_f32<T>(s * hosc_alpha(gl[0], m1[bk], K, B));
+  if (Sm) Sm[e] = from_f32<T>(s * hosc_alpha(gl[1], mM[bk], K, B));
+}
+
+// dS += 2 d_i S_ik beta1_k + 2 d^M_i S_ik beta2_k - g2 S_ik / (B sqrt(n_b) (sqrt(K) - 1) ||S_:k||)  (the last term is
+// zero for a zero column, as torch's norm backward gives)
+template <typename T>
+__global__ void k_hosc_ds_elementwise(const T* __restrict__ S, const float* __restrict__ d,
+                                      const float* __restrict__ dM, const float* __restrict__ n1,
+                                      const float* __restrict__ m1, const float* __restrict__ nM,
+                                      const float* __restrict__ mM, const float* __restrict__ sq,
+                                      const float* __restrict__ graph_nodes, const float* __restrict__ gl,
+                                      int64_t total, int B, int N, int K, int terms, T* __restrict__ dS) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= total) return;
+  const int64_t row = e / K;
+  const int b = (int)(row / N);
+  const int64_t bk = (int64_t)b * K + (e - row * K);
+  const float s = to_f32<T>(S[e]);
+  float v = to_f32<T>(dS[e]);
+  if (terms & kFirst) v = fmaf(2.f * d[row] * s, hosc_beta(gl[0], n1[bk], m1[bk], K, B), v);
+  if (terms & kMotif) v = fmaf(2.f * dM[row] * s, hosc_beta(gl[1], nM[bk], mM[bk], K, B), v);
+  if ((terms & kOrtho) && sq[bk] > 0.f) {
+    const float n = graph_nodes ? graph_nodes[b] : (float)N;
+    v -= gl[2] * s / ((float)B * sqrtf(n) * (sqrtf((float)K) - 1.f) * sqrtf(sq[bk]));
+  }
+  dS[e] = from_f32<T>(v);
+}
+
+// Row terms of dA, one warp per row (b, i): r_i = sum_k beta1_k S_ik^2, rM_i = sum_k beta2_k S_ik^2
+template <typename T>
+__global__ void k_hosc_rows(const T* __restrict__ S, const float* __restrict__ n1, const float* __restrict__ m1,
+                            const float* __restrict__ nM, const float* __restrict__ mM, const float* __restrict__ gl,
+                            int64_t rows, int B, int N, int K, int terms, float* __restrict__ r,
+                            float* __restrict__ rM) {
+  const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (row >= rows) return;
+  const int64_t b = row / N;
+  float a = 0.f, am = 0.f;
+  for (int k = lane; k < K; k += 32) {
+    const float s = to_f32<T>(S[row * K + k]), s2 = s * s;
+    const int64_t bk = b * K + k;
+    if (terms & kFirst) a = fmaf(hosc_beta(gl[0], n1[bk], m1[bk], K, B), s2, a);
+    if (terms & kMotif) am = fmaf(hosc_beta(gl[1], nM[bk], mM[bk], K, B), s2, am);
+  }
+  a = warp_sum(a);
+  am = warp_sum(am);
+  if (lane == 0) r[row] = a, rM[row] = am;
+}
+
+// dA = r_i (+ G_ij P_ij) and H = G . A with G = E2 + rM_i, E2 = S diag(alpha2) S^T (motif term only)
+template <typename T>
+__global__ void k_hosc_da_prep(const T* __restrict__ A, const float* __restrict__ P, const float* __restrict__ E2,
+                               const float* __restrict__ r, const float* __restrict__ rM, int64_t total, int N,
+                               T* __restrict__ H, T* __restrict__ dA) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= total) return;
+  const int64_t row = e / N;
+  float v = r[row];
+  if (P) {
+    const float g = E2[e] + rM[row];
+    v = fmaf(g, P[e], v);
+    H[e] = from_f32<T>(g * to_f32<T>(A[e]));
+  }
+  dA[e] = from_f32<T>(v);
+}
+
+template <typename T>
+struct HoscSaved {
+  T* AM;       // [B, N, N] (motif term only)
+  float* d;    // [B, N]
+  float* dM;   // [B, N]
+  float *n1, *m1, *nM, *mM, *sq;  // [B, K]
+  bool ok;
+  HoscSaved(void* p, size_t bytes, int64_t B, int64_t N, int64_t K, int terms) {
+    Workspace w(p, bytes);
+    AM = (terms & kMotif) ? w.take<T>((size_t)(B * N * N)) : nullptr;
+    d = w.take<float>((size_t)(B * N));
+    dM = w.take<float>((size_t)(B * N));
+    n1 = w.take<float>((size_t)(B * K));
+    m1 = w.take<float>((size_t)(B * K));
+    nM = w.take<float>((size_t)(B * K));
+    mM = w.take<float>((size_t)(B * K));
+    sq = w.take<float>((size_t)(B * K));
+    ok = w.ok;
+  }
+};
+
+size_t elem_size(int dtype) { return dtype == TGPB200_F32 ? 4 : 2; }
+
+size_t saved_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
+  size_t s = 2 * align_up((size_t)(B * N) * 4) + 5 * align_up((size_t)(B * K) * 4);
+  if (terms & kMotif) s += align_up((size_t)(B * N * N) * elem_size(dtype));
+  return s;
+}
+
+size_t fwd_ws_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
+  const size_t K1 = (size_t)s1_width((int)K);
+  size_t s = align_up((size_t)B * N * K1 * elem_size(dtype)) + 2 * align_up((size_t)B * N * K1 * 4);
+  if ((terms & kMotif) && dtype != TGPB200_F32) s += align_up((size_t)(B * N * N) * 4);
+  return s;
+}
+
+size_t bwd_ws_bytes(int64_t B, int64_t N, int64_t K, int dtype, bool grad_adj) {
+  size_t s = 2 * align_up((size_t)(B * N * K) * elem_size(dtype));
+  if (grad_adj) s += 2 * align_up((size_t)(B * N * N) * 4) + align_up((size_t)(B * N * N) * elem_size(dtype)) +
+                     2 * align_up((size_t)(B * N) * 4);
+  return s;
+}
+
+int hosc_check(const void* adj, const void* s, int64_t B, int64_t N, int64_t K, int dtype, int terms) {
+  if (!adj || !s || B < 0 || N < 1 || K < 2 || terms <= 0 || terms > 7) return TGPB200_ERR_INVALID;
+  if (dtype != TGPB200_F32 && dtype != TGPB200_BF16) return TGPB200_ERR_UNSUPPORTED;
+  if (B > kMaxGridY || N >= 65536 || K >= 32768) return TGPB200_ERR_UNSUPPORTED;
+  return TGPB200_OK;
+}
+
+unsigned blocks(int64_t total, int threads = 256) { return (unsigned)ceil_div(total, threads); }
+
+template <typename T>
+int hosc_fwd(const T* A, const T* S, const float* graph_nodes, int B, int N, int K, int terms, float eps,
+             float* losses, HoscSaved<T>& sv, Workspace& ws, cudaStream_t st) {
+  constexpr bool f32 = std::is_same<T, float>::value;
+  const int K1 = s1_width(K);
+  const int64_t NN = (int64_t)N * N, NK1 = (int64_t)N * K1;
+  const bool first = terms & kFirst, motif = terms & kMotif;
+  T* S1 = ws.take<T>((size_t)B * NK1);
+  float* AS1 = ws.take<float>((size_t)B * NK1);
+  float* AMS1 = ws.take<float>((size_t)B * NK1);
+  float* P = (motif && !f32) ? ws.take<float>((size_t)B * NN) : reinterpret_cast<float*>(sv.AM);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  int rc;
+  if (B > 0) {
+    const int64_t rows = (int64_t)B * N;
+    if (first || motif) launch("k_hosc_pad", k_hosc_pad<T>, blocks(rows * K1), 256, 0, st, S, rows, K, K1, S1);
+    const Mat s1{S1, NK1, K1, 1};
+    if (motif) {  // P = A A (fp32), A_M = P . A, [A_M S | d^M] = A_M S1
+      const int kd = N;
+      const Mat a{A, NN, N, 0}, at{A, NN, N, 1};
+      rc = mm<T, float>(B, N, N, 1, &kd, &a, &at, P, NN, N, 1, st, EwHook(), "k_tc_gemm:hosc:P=AA");
+      if (rc) return rc;
+      launch("k_hosc_motif", k_hosc_motif<T>, blocks((int64_t)B * NN), 256, 0, st, (const float*)P, A,
+             (int64_t)B * NN, sv.AM);
+      const Mat am{sv.AM, NN, N, 0};
+      rc = mm<T, float>(B, N, K1, 1, &kd, &am, &s1, AMS1, NK1, K1, 1, st, EwHook(), "k_tc_gemm:hosc:AMS1");
+      if (rc) return rc;
+    }
+    if (first) {  // [A S | d] = A S1
+      const int kd = N;
+      const Mat a{A, NN, N, 0};
+      rc = mm<T, float>(B, N, K1, 1, &kd, &a, &s1, AS1, NK1, K1, 1, st, EwHook(), "k_tc_gemm:hosc:AS1");
+      if (rc) return rc;
+    }
+    launch("k_hosc_stats", k_hosc_stats<T>, dim3((unsigned)ceil_div(K, 32), (unsigned)B), 256, 0, st, S,
+           (const float*)AS1, (const float*)AMS1, N, K, K1, terms, eps, sv.d, sv.dM, sv.n1, sv.m1, sv.nM, sv.mM,
+           sv.sq);
+  }
+  launch("k_hosc_finalize", k_hosc_finalize, 1, 256, 0, st, (const float*)sv.n1, (const float*)sv.m1,
+         (const float*)sv.nM, (const float*)sv.mM, (const float*)sv.sq, graph_nodes, B, N, K, terms, losses);
+  return launch_status();
+}
+
+template <typename T>
+int hosc_bwd(const T* A, const T* S, const float* graph_nodes, const float* gl, int B, int N, int K, int terms,
+             const HoscSaved<T>& sv, T* dS, T* dA, Workspace& ws, cudaStream_t st) {
+  const int64_t NN = (int64_t)N * N, NK = (int64_t)N * K;
+  const bool first = terms & kFirst, motif = terms & kMotif;
+  T* Sa = ws.take<T>((size_t)B * NK);
+  T* Sm = ws.take<T>((size_t)B * NK);
+  float *P = nullptr, *E2 = nullptr, *r = nullptr, *rM = nullptr;
+  T* H = nullptr;
+  if (dA) {
+    P = ws.take<float>((size_t)B * NN);
+    E2 = ws.take<float>((size_t)B * NN);
+    H = ws.take<T>((size_t)B * NN);
+    r = ws.take<float>((size_t)B * N);
+    rM = ws.take<float>((size_t)B * N);
+  }
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  if (B == 0) return TGPB200_OK;
+  if (!gl) {  // no upstream gradient: zero
+    cudaMemsetAsync(dS, 0, (size_t)B * NK * sizeof(T), st);
+    if (dA) cudaMemsetAsync(dA, 0, (size_t)B * NN * sizeof(T), st);
+    return launch_status();
+  }
+  int rc;
+  const int64_t total = (int64_t)B * NK;
+  if (first || motif)
+    launch("k_hosc_scale", k_hosc_scale<T>, blocks(total), 256, 0, st, S, (const float*)sv.m1, (const float*)sv.mM,
+           gl, total, B, N, K, first ? Sa : (T*)nullptr, motif ? Sm : (T*)nullptr);
+  {  // dS = A Sa + A^T Sa + A_M Sm + A_M^T Sm
+    int kd[4];
+    Mat a[4], b[4];
+    int n = 0;
+    if (first) {
+      kd[n] = N, a[n] = Mat{A, NN, N, 0}, b[n] = Mat{Sa, NK, K, 1}, ++n;
+      kd[n] = N, a[n] = Mat{A, NN, N, 1}, b[n] = Mat{Sa, NK, K, 1}, ++n;
+    }
+    if (motif) {
+      kd[n] = N, a[n] = Mat{sv.AM, NN, N, 0}, b[n] = Mat{Sm, NK, K, 1}, ++n;
+      kd[n] = N, a[n] = Mat{sv.AM, NN, N, 1}, b[n] = Mat{Sm, NK, K, 1}, ++n;
+    }
+    if (n > 0) {
+      rc = mm<T, T>(B, N, K, n, kd, a, b, dS, NK, K, 1, st, EwHook(), "k_tc_gemm:hosc:dS");
+      if (rc) return rc;
+    } else {
+      cudaMemsetAsync(dS, 0, (size_t)B * NK * sizeof(T), st);
+    }
+  }
+  launch("k_hosc_ds_elementwise", k_hosc_ds_elementwise<T>, blocks(total), 256, 0, st, S, (const float*)sv.d,
+         (const float*)sv.dM, (const float*)sv.n1, (const float*)sv.m1, (const float*)sv.nM, (const float*)sv.mM,
+         (const float*)sv.sq, graph_nodes, gl, total, B, N, K, terms, dS);
+  if (!dA) return launch_status();
+  // dA = S diag(alpha1) S^T + r 1^T + G . P + H A^T + A^T H,  G = S diag(alpha2) S^T + rM 1^T,  H = G . A
+  const int64_t rows = (int64_t)B * N;
+  launch("k_hosc_rows", k_hosc_rows<T>, blocks(rows * 32), 256, 0, st, S, (const float*)sv.n1, (const float*)sv.m1,
+         (const float*)sv.nM, (const float*)sv.mM, gl, rows, B, N, K, terms, r, rM);
+  if (motif) {
+    const int kn = N, kk = K;
+    const Mat a{A, NN, N, 0}, at{A, NN, N, 1}, sm{Sm, NK, K, 0}, s{S, NK, K, 0};
+    rc = mm<T, float>(B, N, N, 1, &kn, &a, &at, P, NN, N, 1, st, EwHook(), "k_tc_gemm:hosc:P=AA");
+    if (rc) return rc;
+    rc = mm<T, float>(B, N, N, 1, &kk, &sm, &s, E2, NN, N, 1, st, EwHook(), "k_tc_gemm:hosc:E2=SmSt");
+    if (rc) return rc;
+  }
+  launch("k_hosc_da_prep", k_hosc_da_prep<T>, blocks((int64_t)B * NN), 256, 0, st, A,
+         motif ? (const float*)P : (const float*)nullptr, (const float*)E2, (const float*)r, (const float*)rM,
+         (int64_t)B * NN, N, H, dA);
+  {  // dA += Sa S^T + H A^T + A^T H  (one accumulating call)
+    int kd[3];
+    Mat a[3], b[3];
+    int n = 0;
+    if (first) kd[n] = K, a[n] = Mat{Sa, NK, K, 0}, b[n] = Mat{S, NK, K, 0}, ++n;
+    if (motif) {
+      kd[n] = N, a[n] = Mat{H, NN, N, 0}, b[n] = Mat{A, NN, N, 0}, ++n;
+      kd[n] = N, a[n] = Mat{A, NN, N, 1}, b[n] = Mat{H, NN, N, 1}, ++n;
+    }
+    if (n > 0) {
+      rc = mm<T, T>(B, N, N, n, kd, a, b, dA, NN, N, 1, st, EwHook(), "k_tc_gemm:hosc:dA", true);
+      if (rc) return rc;
+    }
+  }
+  return launch_status();
+}
+
+}  // namespace
+}  // namespace tgp
+
+using namespace tgp;
+
+extern "C" {
+
+size_t tgpb200_hosc_loss_saved_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
+  if (B < 0 || N < 1 || K < 1) return 0;
+  return saved_bytes(B, N, K, terms, dtype);
+}
+
+size_t tgpb200_hosc_loss_fwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
+  if (B < 0 || N < 1 || K < 1) return 0;
+  return fwd_ws_bytes(B, N, K, terms, dtype);
+}
+
+size_t tgpb200_hosc_loss_bwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int dtype, int need_grad_adj) {
+  if (B < 0 || N < 1 || K < 1) return 0;
+  return bwd_ws_bytes(B, N, K, dtype, need_grad_adj != 0);
+}
+
+int tgpb200_hosc_loss_fwd(const void* adj, const void* s, const float* graph_nodes, int64_t B, int64_t N, int64_t K,
+                          int dtype, int terms, float eps, float* losses, void* saved, size_t saved_bytes,
+                          void* workspace, size_t workspace_bytes, tgpb200_stream_t stream) {
+  int rc = hosc_check(adj, s, B, N, K, dtype, terms);
+  if (rc != TGPB200_OK) return rc;
+  if (!losses) return TGPB200_ERR_INVALID;
+  Workspace ws(workspace, workspace_bytes);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == TGPB200_F32) {
+    HoscSaved<float> sv(saved, saved_bytes, B, N, K, terms);
+    if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+    return hosc_fwd<float>((const float*)adj, (const float*)s, graph_nodes, (int)B, (int)N, (int)K, terms, eps, losses,
+                           sv, ws, st);
+  }
+  HoscSaved<__nv_bfloat16> sv(saved, saved_bytes, B, N, K, terms);
+  if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+  return hosc_fwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, graph_nodes, (int)B, (int)N,
+                                 (int)K, terms, eps, losses, sv, ws, st);
+}
+
+int tgpb200_hosc_loss_bwd(const void* adj, const void* s, const float* graph_nodes, const void* saved,
+                          size_t saved_bytes, const float* grad_losses, int64_t B, int64_t N, int64_t K, int dtype,
+                          int terms, void* grad_s, void* grad_adj, void* workspace, size_t workspace_bytes,
+                          tgpb200_stream_t stream) {
+  int rc = hosc_check(adj, s, B, N, K, dtype, terms);
+  if (rc != TGPB200_OK) return rc;
+  if (!grad_s) return TGPB200_ERR_INVALID;
+  Workspace ws(workspace, workspace_bytes);
+  cudaStream_t st = (cudaStream_t)stream;
+  void* sp = const_cast<void*>(saved);
+  if (dtype == TGPB200_F32) {
+    HoscSaved<float> sv(sp, saved_bytes, B, N, K, terms);
+    if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+    return hosc_bwd<float>((const float*)adj, (const float*)s, graph_nodes, grad_losses, (int)B, (int)N, (int)K, terms,
+                           sv, (float*)grad_s, (float*)grad_adj, ws, st);
+  }
+  HoscSaved<__nv_bfloat16> sv(sp, saved_bytes, B, N, K, terms);
+  if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+  return hosc_bwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, graph_nodes, grad_losses, (int)B,
+                                 (int)N, (int)K, terms, sv, (__nv_bfloat16*)grad_s, (__nv_bfloat16*)grad_adj, ws, st);
+}
+
+}  // extern "C"

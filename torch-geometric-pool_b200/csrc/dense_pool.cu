@@ -1114,28 +1114,12 @@ static __global__ void k_cast_out(const float* __restrict__ in, T* __restrict__ 
 // ------------------------------------------------------------------------------------------
 // Host orchestration
 // ------------------------------------------------------------------------------------------
-// A GEMM operand as stored in memory (per batch item, cols contiguous):
-//   K-major : [MN extent rows][K extent cols];   MN-major: [K extent rows][MN extent cols]
-struct Mat {
-  const void* ptr;
-  int64_t bs, rs;
-  int mn;
-};
-
-// D[b] (M x N) = sum_p A_p B_p, written with (row, col) strides.  Tensor-core engine when the layout
-// satisfies the TMA constraints, FP32-pipe batched GEMM otherwise (shape generality, not a second backend:
-// both paths live in this library and compute the same product).
-struct EwHook {  // fused element-wise terms of dS (tc::GemmProblem::ew_*); *applied is set when the engine took it
-  const void* S = nullptr;
-  const float* d = nullptr;
-  const float* coef = nullptr;
-  float eps = 0.f;
-  bool* applied = nullptr;
-};
-
+// D[b] (M x N) (+)= sum_p A_p B_p (declared in dense.cuh): tensor-core engine when the layout satisfies the TMA
+// constraints, FP32-pipe batched GEMM otherwise (shape generality, not a second backend: both paths live in this
+// library and compute the same product).
 template <typename T, typename TC>
-static int mm(int batch, int M, int N, int npairs, const int* kd, const Mat* A, const Mat* Bm, TC* out, int64_t obs,
-              int64_t ors, int64_t ocs, cudaStream_t st, EwHook hook = EwHook(), const char* tag = nullptr) {
+int mm(int batch, int M, int N, int npairs, const int* kd, const Mat* A, const Mat* Bm, TC* out, int64_t obs,
+       int64_t ors, int64_t ocs, cudaStream_t st, EwHook hook, const char* tag, bool accumulate) {
   tc::GemmProblem p;
   memset(&p, 0, sizeof(p));
   p.tag = tag;
@@ -1146,7 +1130,7 @@ static int mm(int batch, int M, int N, int npairs, const int* kd, const Mat* A, 
     p.b[i] = {Bm[i].ptr, Bm[i].bs, Bm[i].rs, Bm[i].mn};
   }
   p.out = out, p.out_batch_stride = obs, p.out_row_stride = ors, p.out_col_stride = ocs;
-  p.alpha = 1.f, p.accumulate = 0;
+  p.alpha = 1.f, p.accumulate = accumulate ? 1 : 0;
   p.out_bf16 = std::is_same<TC, __nv_bfloat16>::value;
   p.in_bf16 = std::is_same<T, __nv_bfloat16>::value;
   if (tc::gemm_supported(p)) {
@@ -1158,17 +1142,25 @@ static int mm(int batch, int M, int N, int npairs, const int* kd, const Mat* A, 
   }
   if (ocs != 1) {  // transposed output: D^T = B^T A^T has unit column stride
     if (ors != 1) return TGPB200_ERR_UNSUPPORTED;
-    return mm<T, TC>(batch, N, M, npairs, kd, Bm, A, out, obs, ocs, ors, st, EwHook(), tag);
+    return mm<T, TC>(batch, N, M, npairs, kd, Bm, A, out, obs, ocs, ors, st, EwHook(), tag, accumulate);
   }
   for (int i = 0; i < npairs; ++i) {
     int64_t sAm = A[i].mn ? 1 : A[i].rs, sAk = A[i].mn ? A[i].rs : 1;
     int64_t sBk = Bm[i].mn ? Bm[i].rs : 1, sBn = Bm[i].mn ? 1 : Bm[i].rs;
     int rc = bgemm<T, T, TC>((const T*)A[i].ptr, (const T*)Bm[i].ptr, out, batch, M, N, kd[i], A[i].bs, sAm, sAk,
-                             Bm[i].bs, sBk, sBn, obs, ors, 1.f, i > 0, st);
+                             Bm[i].bs, sBk, sBn, obs, ors, 1.f, i > 0 || accumulate, st);
     if (rc) return rc;
   }
   return TGPB200_OK;
 }
+
+// the forms the other translation units call (dense_hosc.cu)
+template int mm<float, float>(int, int, int, int, const int*, const Mat*, const Mat*, float*, int64_t, int64_t, int64_t,
+                              cudaStream_t, EwHook, const char*, bool);
+template int mm<__nv_bfloat16, float>(int, int, int, int, const int*, const Mat*, const Mat*, float*, int64_t, int64_t,
+                                      int64_t, cudaStream_t, EwHook, const char*, bool);
+template int mm<__nv_bfloat16, __nv_bfloat16>(int, int, int, int, const int*, const Mat*, const Mat*, __nv_bfloat16*,
+                                              int64_t, int64_t, int64_t, cudaStream_t, EwHook, const char*, bool);
 
 template <typename T, typename TC>
 static int mm1(int batch, int M, int N, int kd, Mat A, Mat Bm, TC* out, int64_t obs, int64_t ors, int64_t ocs,

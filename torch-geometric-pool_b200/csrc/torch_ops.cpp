@@ -157,6 +157,55 @@ std::tuple<Tensor, Tensor> acc_losses_bwd(const Tensor& adj, const Tensor& s, co
   return {ga, gs};
 }
 
+// (losses[3] = {first-order cut, motif cut, HOSC orthogonality}, saved) of HOSC pooling (restated in
+// tests/hosc_oracle.py); `terms` is the bitmask of tgpb200_hosc_loss_fwd
+void hosc_check_args(const Tensor& adj, const Tensor& s, int64_t terms) {
+  require_cuda(s, "s");
+  require_cuda(adj, "adj");
+  TORCH_CHECK(s.dim() == 3, "hosc_losses expects s of shape [B, N, K], got ", s.sizes());
+  TORCH_CHECK(adj.dim() == 3 && adj.size(0) == s.size(0) && adj.size(1) == s.size(1) && adj.size(2) == s.size(1),
+              "hosc_losses expects adj of shape [B, N, N] = [", s.size(0), ", ", s.size(1), ", ", s.size(1), "], got ",
+              adj.sizes());
+  TORCH_CHECK(adj.scalar_type() == s.scalar_type(), "tgp_b200.hosc_losses: adj and s must share one dtype");
+  TORCH_CHECK_VALUE(s.size(2) >= 2, "hosc_losses needs K >= 2 clusters, got K = ", s.size(2));
+  TORCH_CHECK_VALUE(s.size(1) >= 1, "hosc_losses needs N >= 1 nodes");
+  TORCH_CHECK_VALUE(terms >= 1 && terms <= 7, "hosc_losses: terms must be a non-empty mask of 1 | 2 | 4, got ", terms);
+}
+
+std::tuple<Tensor, Tensor> hosc_losses(const Tensor& adj, const Tensor& s, const OptTensor& graph_nodes,
+                                       int64_t terms, double eps) {
+  hosc_check_args(adj, s, terms);
+  c10::cuda::CUDAGuard guard(s.device());
+  const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
+  const int dt = dtype_code(s);
+  Tensor saved = workspace(tgpb200_hosc_loss_saved_bytes(B, N, K, (int)terms, dt), s);
+  Tensor ws = workspace(tgpb200_hosc_loss_fwd_workspace_bytes(B, N, K, (int)terms, dt), s);
+  Tensor losses = at::empty({3}, s.options().dtype(at::kFloat));
+  check(tgpb200_hosc_loss_fwd(adj.data_ptr(), s.data_ptr(), graph_nodes_ptr(graph_nodes, B), B, N, K, dt, (int)terms,
+                              (float)eps, losses.data_ptr<float>(), saved.data_ptr(), (size_t)saved.numel(),
+                              ws.data_ptr(), (size_t)ws.numel(), stream_of(s)),
+        "hosc_losses");
+  return {losses, saved};
+}
+
+std::tuple<Tensor, Tensor> hosc_losses_bwd(const Tensor& adj, const Tensor& s, const OptTensor& graph_nodes,
+                                           const Tensor& saved, const Tensor& glosses, int64_t terms, bool need_gadj) {
+  hosc_check_args(adj, s, terms);
+  c10::cuda::CUDAGuard guard(s.device());
+  const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
+  const int dt = dtype_code(s);
+  TORCH_CHECK(glosses.numel() == 3, "hosc_losses_bwd expects 3 upstream loss gradients");
+  Tensor gl = glosses.to(at::kFloat).contiguous();
+  Tensor gs = at::empty_like(s);
+  Tensor ga = need_gadj ? at::empty_like(adj) : at::empty({0}, s.options());
+  Tensor ws = workspace(tgpb200_hosc_loss_bwd_workspace_bytes(B, N, K, dt, need_gadj ? 1 : 0), s);
+  check(tgpb200_hosc_loss_bwd(adj.data_ptr(), s.data_ptr(), graph_nodes_ptr(graph_nodes, B), saved.data_ptr(),
+                              (size_t)saved.numel(), gl.data_ptr<float>(), B, N, K, dt, (int)terms, gs.data_ptr(),
+                              need_gadj ? ga.data_ptr() : nullptr, ws.data_ptr(), (size_t)ws.numel(), stream_of(s)),
+        "hosc_losses_bwd");
+  return {ga, gs};
+}
+
 // CSR-by-cluster of a sparse assignment (tgp/reduce/aggr_reduce.py:13-23)
 std::tuple<Tensor, Tensor> build_csr(const Tensor& cluster_index, int64_t num_clusters) {
   require_cuda(cluster_index, "cluster_index");
@@ -222,6 +271,9 @@ TORCH_LIBRARY(tgp_b200, m) {
         "Tensor? graph_nodes=None) -> (Tensor, Tensor, Tensor)");
   m.def("acc_losses(Tensor adj, Tensor s) -> (Tensor, Tensor, Tensor)");
   m.def("acc_losses_bwd(Tensor adj, Tensor s, Tensor saved, Tensor glosses, bool need_gadj) -> (Tensor, Tensor)");
+  m.def("hosc_losses(Tensor adj, Tensor s, Tensor? graph_nodes, int terms, float eps) -> (Tensor, Tensor)");
+  m.def("hosc_losses_bwd(Tensor adj, Tensor s, Tensor? graph_nodes, Tensor saved, Tensor glosses, int terms, "
+        "bool need_gadj) -> (Tensor, Tensor)");
   m.def("build_csr(Tensor cluster_index, int num_clusters) -> (Tensor, Tensor)");
   m.def("segment_reduce(Tensor x, Tensor node_index, Tensor cluster_index, Tensor? weight, Tensor order, Tensor ptr, "
         "int num_clusters, int op) -> Tensor");
@@ -234,6 +286,8 @@ TORCH_LIBRARY_IMPL(tgp_b200, CUDA, m) {
   m.impl("stas_fused_bwd", &stas_fused_bwd);
   m.impl("acc_losses", &acc_losses);
   m.impl("acc_losses_bwd", &acc_losses_bwd);
+  m.impl("hosc_losses", &hosc_losses);
+  m.impl("hosc_losses_bwd", &hosc_losses_bwd);
   m.impl("build_csr", &build_csr);
   m.impl("segment_reduce", &segment_reduce);
   m.impl("segment_reduce_bwd", &segment_reduce_bwd);

@@ -365,6 +365,33 @@ def acc_losses(adj: Tensor, s: Tensor) -> Tensor:
     return losses
 
 
+HOSC_FIRST, HOSC_MOTIF, HOSC_ORTHO = 1, 2, 4
+
+
+def hosc_losses(adj: Tensor, s: Tensor, alpha: float, hosc_ortho: bool, graph_nodes: Optional[Tensor] = None,
+                eps: float = 1e-8) -> Tensor:
+    """``[L1, L2, O]`` losses of HOSC pooling (higher-order spectral clustering), batch means, from the RAW ``adj``
+    [B, N, N] and ``s`` [B, N, K] (padded rows zero), differentiable in both:
+
+    * first-order cut ``L1 = -(1/K) sum_k n_k / m_k`` with ``n_k = (S^T A S)_kk``, ``m_k = sum_i d_i S_ik^2 + eps``,
+      ``d = A 1``;
+    * motif cut ``L2``: the same of the triangle-motif adjacency ``A_M = (A A) * A``;
+    * ``O = (sqrt(K) - sum_k ||S_:k|| / sqrt(n_b)) / (sqrt(K) - 1)``, ``n_b = graph_nodes[b]`` (N when absent).
+
+    The HOSC loss is ``(1 - alpha) L1 + alpha L2``.  Only the terms it needs are computed: ``L1`` is 0 when
+    ``alpha == 1``, ``L2`` is 0 (and no ``A A`` product runs) when ``alpha == 0``, ``O`` is 0 unless ``hosc_ortho``.
+    ``K < 2`` raises ``ValueError``."""
+    _require_cuda(adj, s)
+    if s.dim() == 3 and s.size(-1) < 2:
+        raise ValueError(f"hosc_losses needs K >= 2 clusters, got K = {s.size(-1)}")
+    alpha = float(alpha)
+    terms = (HOSC_FIRST if alpha != 1.0 else 0) | (HOSC_MOTIF if alpha != 0.0 else 0) | (HOSC_ORTHO if hosc_ortho else 0)
+    if graph_nodes is not None:
+        graph_nodes = graph_nodes.to(torch.float32).contiguous()
+    losses, _ = _T.hosc_losses(adj.contiguous(), s.contiguous(), graph_nodes, terms, float(eps))
+    return losses
+
+
 # --------------------------------------------------------------------------- #
 # Dense -> block-diagonal sparse output, dense pre-processing
 # --------------------------------------------------------------------------- #

@@ -1,6 +1,6 @@
 """``torch.ops.tgp_b200.*``: the operators of the Reduce + Connect path as torch custom ops (SURVEY 8b).
 
-* ``stas_fused`` / ``stas_fused_bwd``, ``acc_losses`` / ``acc_losses_bwd``, ``segment_reduce`` / ``segment_reduce_bwd``, ``build_csr`` are C++ dispatcher
+* ``stas_fused`` / ``stas_fused_bwd``, ``acc_losses`` / ``acc_losses_bwd``, ``hosc_losses`` / ``hosc_losses_bwd``, ``segment_reduce`` / ``segment_reduce_bwd``, ``build_csr`` are C++ dispatcher
   ops (``csrc/torch_ops.cpp`` -> ``libtgp_b200_ops.so``: allocate with the caching allocator, take the current stream,
   call the C ABI of ``libtgp_b200.so``);
 * ``filter_relabel_edges``, ``remap_coalesce``, ``degree_norm``, ``weight_norm`` (+ their ``*_bwd``) are
@@ -112,6 +112,42 @@ def _acc_backward(ctx, glosses, _gquant, _gsaved):
 
 
 torch.library.register_autograd("tgp_b200::acc_losses", _acc_backward, setup_context=_acc_setup)
+
+
+# --------------------------------------------------------------------------------------------------------------
+# hosc_losses: (losses[3] = {first-order cut, motif cut, HOSC orthogonality}, saved) of HOSC pooling; `terms` is the
+# bitmask of the terms computed (1 first order, 2 triangle motif, 4 orthogonality).  saved carries no gradient.
+# --------------------------------------------------------------------------------------------------------------
+@torch.library.register_fake("tgp_b200::hosc_losses")
+def _hosc_losses_fake(adj, s, graph_nodes, terms, eps):
+    B, N, K = s.shape
+    saved = L.load().tgpb200_hosc_loss_saved_bytes(B, N, K, terms, L.dtype_code(s.dtype))
+    return s.new_empty((3,), dtype=torch.float32), s.new_empty((max(saved, 256),), dtype=torch.uint8)
+
+
+@torch.library.register_fake("tgp_b200::hosc_losses_bwd")
+def _hosc_losses_bwd_fake(adj, s, graph_nodes, saved, glosses, terms, need_gadj):
+    return (torch.empty_like(adj) if need_gadj else s.new_empty((0,))), torch.empty_like(s)
+
+
+def _hosc_setup(ctx, inputs, output):
+    adj, s, graph_nodes, terms, _eps = inputs
+    ctx.save_for_backward(adj, s, graph_nodes, output[1])
+    ctx.terms = terms
+    ctx.mark_non_differentiable(output[1])
+    ctx.set_materialize_grads(False)
+
+
+def _hosc_backward(ctx, glosses, _gsaved):
+    adj, s, graph_nodes, saved = ctx.saved_tensors
+    if glosses is None:
+        return None, None, None, None, None
+    need_adj = ctx.needs_input_grad[0]
+    ga, gs = _T.hosc_losses_bwd(adj, s, graph_nodes, saved, glosses, ctx.terms, need_adj)
+    return (ga if need_adj else None), gs, None, None, None
+
+
+torch.library.register_autograd("tgp_b200::hosc_losses", _hosc_backward, setup_context=_hosc_setup)
 
 
 # --------------------------------------------------------------------------------------------------------------
@@ -429,6 +465,6 @@ def _wn_backward(ctx, g, _gmx, _garg):
 
 torch.library.register_autograd("tgp_b200::weight_norm", _wn_backward, setup_context=_wn_setup)
 
-OP_NAMES = ("stas_fused", "stas_fused_bwd", "acc_losses", "acc_losses_bwd", "build_csr", "segment_reduce", "segment_reduce_bwd", "filter_relabel_edges",
+OP_NAMES = ("stas_fused", "stas_fused_bwd", "acc_losses", "acc_losses_bwd", "hosc_losses", "hosc_losses_bwd", "build_csr", "segment_reduce", "segment_reduce_bwd", "filter_relabel_edges",
             "filter_relabel_edges_bwd", "remap_coalesce", "remap_coalesce_bwd", "degree_norm", "degree_norm_bwd",
             "weight_norm", "weight_norm_bwd")

@@ -2,7 +2,7 @@
 
 ``mincut_pool`` / ``diff_pool`` / ``dmon_pool`` run reduce + connect + auxiliary losses + post-processing as ONE
 fused forward and ONE fused backward; ``acc_pool`` adds the Asymmetric Cheeger Cut losses (their own kernels) to the
-loss-free fused call; ``topk_pool`` / ``cluster_pool`` chain the sparse reduce and the sparse connect.  ``patch_pooler`` installs the B200 operators on a reference pooler object.
+loss-free fused call, ``hosc_pool`` the HOSC cut losses (their own products and kernels); ``topk_pool`` / ``cluster_pool`` chain the sparse reduce and the sparse connect.  ``patch_pooler`` installs the B200 operators on a reference pooler object.
 """
 from __future__ import annotations
 
@@ -111,6 +111,35 @@ def acc_pool(
     return x_pool, adj_pool, {tv_key: losses[0] * totvar_coeff, bal_key: losses[1] * balance_coeff}
 
 
+def hosc_pool(
+    x: Tensor,
+    adj: Tensor,
+    s: Tensor,
+    mask: Optional[Tensor] = None,
+    mu: float = 0.1,
+    alpha: float = 0.5,
+    hosc_ortho: bool = False,
+    remove_self_loops: bool = True,
+    degree_norm: bool = True,
+    adj_transpose: bool = True,
+    edge_weight_norm: bool = False,
+) -> Tuple[Tensor, Tensor, Dict[str, Tensor]]:
+    """HOSCPooling.forward batched path after select: ``S^T X`` and ``postprocess(S^T A S)`` from the fused dense path,
+    the HOSC loss ``(1 - alpha) L1 + alpha L2`` (first-order and triangle-motif cuts, restated in
+    ``tests/hosc_oracle.py``) from ``functional.hosc_losses`` on the raw ``adj``, and ``mu`` times the orthogonality
+    term: MinCut's ``orthogonality_loss`` from the fused call, or with ``hosc_ortho`` HOSC's column-norm term, whose
+    ``n_b`` is the valid node count of ``mask`` [B, N] (it stays on the device)."""
+    graph_nodes = None if mask is None else mask.sum(1).to(torch.float32)
+    x_pool, adj_pool, dl = F_.dense_pool(
+        x, adj, s, remove_self_loops=remove_self_loops, degree_norm=degree_norm, adj_transpose=adj_transpose,
+        edge_weight_norm=edge_weight_norm, loss_kind=F_.LOSS_NONE if hosc_ortho else F_.LOSS_MINCUT,
+    )
+    losses = F_.hosc_losses(adj, s, alpha, hosc_ortho, graph_nodes=graph_nodes)
+    hosc = (1.0 - alpha) * losses[0] + alpha * losses[1]
+    ortho = losses[2] if hosc_ortho else dl[1]
+    return x_pool, adj_pool, {"hosc_loss": hosc, "ortho_loss": mu * ortho}
+
+
 def sparse_pool(
     x: Tensor,
     edge_index: Tensor,
@@ -186,6 +215,9 @@ _DMON_COEFFS = ("spectral_loss_coeff", "cluster_loss_coeff", "ortho_loss_coeff")
 _ACC_CLASS = "AsymCheegerCutPooling"
 _ACC_COEFFS = ("totvar_coeff", "balance_coeff")
 _ACC_KEYS = ("total_variation_loss", "balance_loss")
+# HOSCPooling: its class name and the attributes the fused forward reads
+_HOSC_CLASS = "HOSCPooling"
+_HOSC_ATTRS = ("mu", "alpha", "hosc_ortho")
 _AGGR_TO_OP = {"SumAggregation": "sum", "MeanAggregation": "mean", "MaxAggregation": "max", "MinAggregation": "min"}
 
 
@@ -229,6 +261,8 @@ def _fused_dense_forward(pooler, kind: str):
                                                pooler.ortho_loss_coeff, **flags)
         elif kind == "acc":
             x_pool, adj_pool, loss = acc_pool(x, adj, so.s, *(getattr(pooler, a) for a in _ACC_COEFFS), **flags)
+        elif kind == "hosc":
+            x_pool, adj_pool, loss = hosc_pool(x, adj, so.s, mask, *(getattr(pooler, a) for a in _HOSC_ATTRS), **flags)
         else:
             x_pool, adj_pool, loss = diff_pool(x, adj, so.s, num_nodes=1, link_loss_coeff=pooler.link_loss_coeff,
                                                ent_loss_coeff=1.0, normalize_loss=pooler.normalize_loss, **flags)
@@ -251,11 +285,12 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
       same ctor attributes (the poolers read them, tgp/poolers/mincut.py:233-236);
     * ``pooler.reducer``: ``BaseReduce`` / ``AggrReduce(sum | mean | max | min)`` -> ``B200Reduce`` with the SAME
       reduction; any other reducer (learned / order-statistic aggregators) is left in place.  ``reduce_op`` overrides;
-    * ``fuse_dense``: a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` / ``AsymCheegerCutPooling`` also
-      gets the fused forward (reduce + connect + losses + post-processing on the device kernels) -- without it the
+    * ``fuse_dense``: a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` / ``AsymCheegerCutPooling`` /
+      ``HOSCPooling`` also gets the fused forward (reduce + connect + losses + post-processing on the device kernels) -- without it the
       patched pooler still calls the reference's torch loss functions.  A ``DMoNPooling`` lacking one of
-      ``spectral_loss_coeff``, ``cluster_loss_coeff``, ``ortho_loss_coeff``, or an ``AsymCheegerCutPooling`` lacking
-      ``totvar_coeff`` or ``balance_coeff``, keeps the reference forward.
+      ``spectral_loss_coeff``, ``cluster_loss_coeff``, ``ortho_loss_coeff``, an ``AsymCheegerCutPooling`` lacking
+      ``totvar_coeff`` or ``balance_coeff``, or a ``HOSCPooling`` lacking ``mu``, ``alpha`` or ``hosc_ortho``, keeps
+      the reference forward.
     """
     for attr in ("connector", "preconnector"):
         conn = getattr(pooler, attr, None)
@@ -273,11 +308,13 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
         op = reduce_op if reduce_op is not None else _reduce_op_of(reducer)
         if op is not None:
             pooler.reducer = B200Reduce(op)
-    kind = {"MinCutPooling": "mincut", "DiffPool": "diff", "DMoNPooling": "dmon", _ACC_CLASS: "acc"}.get(
-        type(pooler).__name__)
+    kind = {"MinCutPooling": "mincut", "DiffPool": "diff", "DMoNPooling": "dmon", _ACC_CLASS: "acc",
+            _HOSC_CLASS: "hosc"}.get(type(pooler).__name__)
     if kind == "dmon" and not all(hasattr(pooler, a) for a in _DMON_COEFFS):
         kind = None
     if kind == "acc" and not all(hasattr(pooler, a) for a in _ACC_COEFFS):
+        kind = None
+    if kind == "hosc" and not all(hasattr(pooler, a) for a in _HOSC_ATTRS):
         kind = None
     if fuse_dense and kind is not None and type(getattr(pooler, "connector", None)).__name__ == "B200DenseConnect":
         pooler.forward = _fused_dense_forward(pooler, kind)
