@@ -135,19 +135,6 @@ def test_acc_pool_and_patched_pooler_wiring(monkeypatch):
     torch.testing.assert_close(out.edge_index, ap)
 
 
-def test_pooler_without_coefficients_keeps_reference_forward():
-    import tgp_b200 as T
-
-    class Bare(H._DenseBase):
-        totvar_coeff = 1.0  # balance_coeff missing
-
-    Bare.__name__ = "AsymCheegerCutPooling"
-    pooler = Bare(selector=None, reducer=H.BaseReduce(), connector=H.DenseConnect())
-    ref = pooler.forward
-    T.patch_pooler(pooler)
-    assert pooler.forward == ref
-
-
 def test_acc_ops_fake_tensor_shapes():
     from torch._subclasses.fake_tensor import FakeTensorMode
 

@@ -1,5 +1,6 @@
 """CPU: ``patch_pooler`` on stand-ins of the reference pooler classes (tests/dropin_harness.py): operator swap,
-preserved ctor attributes, reduce op derived from the existing reducer, unsupported aggregators left alone."""
+preserved ctor attributes, reduce op derived from the existing reducer, unsupported aggregators left alone, and a
+dense pooler lacking an attribute its fused forward reads keeps the reference forward."""
 import pytest
 
 import dropin_harness as H
@@ -45,6 +46,18 @@ def test_patch_pooler_dense_gets_fused_forward():
         q.forward()
     with pytest.raises(TypeError):
         T.B200DenseConnect(sparse_output="yes")
+
+
+@pytest.mark.parametrize("name, attrs", [
+    ("DMoNPooling", {}),                                   # no loss coefficient
+    ("AsymCheegerCutPooling", {"totvar_coeff": 1.0}),      # balance_coeff missing
+    ("HOSCPooling", {"mu": 0.1, "alpha": 0.5}),            # hosc_ortho missing
+], ids=["dmon", "acc", "hosc"])
+def test_pooler_without_attributes_keeps_reference_forward(name, attrs):
+    pooler = type(name, (H._DenseBase,), attrs)(selector=None, reducer=H.BaseReduce(), connector=H.DenseConnect())
+    ref = pooler.forward
+    T.patch_pooler(pooler)
+    assert pooler.forward == ref
 
 
 def test_select_output_rejects_inverse_and_keeps_extras_on_to():

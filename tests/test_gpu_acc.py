@@ -6,18 +6,13 @@ import pytest
 import torch
 
 import acc_oracle as A
+import dense_loss_cases as C
 import dropin_harness as H
 import tgp_b200 as T
+from dense_loss_cases import DEV, FLAGSETS
 from tgp_b200 import functional as F_
 
 pytestmark = pytest.mark.gpu
-DEV = "cuda:0"
-FLAGSETS = [
-    dict(remove_self_loops=True, degree_norm=True, adj_transpose=True, edge_weight_norm=False),
-    dict(remove_self_loops=True, degree_norm=True, adj_transpose=False, edge_weight_norm=True),
-    dict(remove_self_loops=False, degree_norm=False, adj_transpose=False, edge_weight_norm=False),
-]
-SOURCES = ("x", "adj", "tv", "bal")
 COEF = {"tv": 1.7, "bal": -0.8}
 KEYS = {"tv": "total_variation_loss", "bal": "balance_loss"}
 
@@ -26,47 +21,11 @@ class AsymCheegerCutPooling(H._DenseBase):  # the restated attributes of AsymChe
     totvar_coeff, balance_coeff = 0.6, 1.4
 
 
-def _inputs(B, N, K, F, seed, ragged=True):
-    """Planted-partition graphs with communities of skewed sizes and an assignment that follows them: the cluster sizes
-    are far from balanced, so the balance loss is not a cancellation residue that float32 cannot resolve to rtol 1e-5
-    (the total variation is a sum of non-negative terms).  Graph b has n_b valid nodes (padded rows / columns zero)."""
-    g = torch.Generator().manual_seed(seed)
-    n = torch.tensor([N - (7 * b) % max(1, N // 3) if ragged else N for b in range(B)])
-    mask = torch.arange(N)[None, :] < n[:, None]
-    comm = (K * torch.rand(B, N, generator=g) ** 2).long().clamp(max=K - 1)
-    same = comm[:, :, None] == comm[:, None, :]
-    p = torch.where(same, torch.tensor(0.6), torch.tensor(0.3 / N))
-    a = (torch.rand(B, N, N, generator=g) < p).float()
-    a = torch.triu(a, 1)
-    a = (a + a.transpose(1, 2)) * torch.rand(B, N, N, generator=g).add(0.5)
-    a = (a + a.transpose(1, 2)) * 0.5 * (mask[:, :, None] & mask[:, None, :])
-    logits = 4.0 * torch.nn.functional.one_hot(comm, K).float() + torch.randn(B, N, K, generator=g)
-    s = torch.softmax(logits, -1) * mask[..., None]
-    x = torch.randn(B, N, F, generator=g) * mask[..., None]
-    return x, a, s, mask
-
-
-def _upstream(B, K, F, seed):
-    g = torch.Generator().manual_seed(seed + 100)
-    return {"x": torch.randn(B, K, F, generator=g), "adj": torch.randn(B, K, K, generator=g)}
-
-
-def _objective(xp, ap, loss, src, up):
-    if src in ("x", "adj"):
-        out = xp if src == "x" else ap
-        return (out * up[src].to(out.device, out.dtype)).sum()
-    return COEF[src] * loss[KEYS[src]]
-
-
 def _oracle(x, a, s, flags, up, dev=DEV):
     """float64 forward and the (dX, dA, dS) of each gradient source alone."""
     x64, a64, s64 = (t.to(dev, torch.float64).requires_grad_(True) for t in (x, a, s))
     xp, ap, loss = A.acc_pool(x64, a64, s64, **flags)
-    grads = {}
-    for src in SOURCES:
-        g = torch.autograd.grad(_objective(xp, ap, loss, src, up), (x64, a64, s64), retain_graph=True,
-                                allow_unused=True)
-        grads[src] = [torch.zeros_like(v) if gv is None else gv for gv, v in zip(g, (x64, a64, s64))]
+    grads = C.per_source_grads(xp, ap, loss, up, (x64, a64, s64), COEF, KEYS)
     losses = torch.stack([loss[KEYS["tv"]], loss[KEYS["bal"]]]).detach()
     qv, qi = A.quantile(s64.detach())
     return xp.detach(), ap.detach(), losses, qv, qi, grads
@@ -81,33 +40,18 @@ def _saved_rows(saved, B, K):
 def _device(x, a, s, flags, up, dtype=torch.float32):
     xd, ad, sd = (t.to(DEV, dtype).requires_grad_(True) for t in (x, a, s))
     xp, ap, loss = T.acc_pool(xd, ad, sd, **flags)
-    grads = {}
-    for src in SOURCES:
-        g = torch.autograd.grad(_objective(xp, ap, loss, src, up), (xd, ad, sd), retain_graph=True, allow_unused=True)
-        grads[src] = [torch.zeros_like(v) if gv is None else gv for gv, v in zip(g, (xd, ad, sd))]
+    grads = C.per_source_grads(xp, ap, loss, up, (xd, ad, sd), COEF, KEYS)
     losses = torch.stack([loss[KEYS["tv"]], loss[KEYS["bal"]]]).detach()
     _, quant, saved = torch.ops.tgp_b200.acc_losses(ad.detach().contiguous(), sd.detach().contiguous())
     return xp.detach(), ap.detach(), losses, quant, _saved_rows(saved, s.size(0), s.size(2)), grads
-
-
-def _check_grads(got, exp, tau, edge_weight_norm):
-    for src in SOURCES:
-        for name, gv, ev in zip(("dX", "dA", "dS"), got[src], exp[src]):
-            gv, ev = gv.double(), ev.double()
-            if name == "dA" and src == "adj" and edge_weight_norm:
-                # max-normalisation routes one term to "the" arg-max, which a symmetric adjacency ties with its mirror
-                gv, ev = 0.5 * (gv + gv.transpose(1, 2)), 0.5 * (ev + ev.transpose(1, 2))
-            bound = tau * float(ev.abs().max())
-            err = float((gv - ev).abs().max())
-            assert err <= bound, f"{src} -> {name}: max error {err:.3e} > {bound:.3e}"
 
 
 @pytest.mark.parametrize("flags", FLAGSETS)
 @pytest.mark.parametrize("shape", [(3, 256, 64, 128), (5, 200, 48, 100), (4, 100, 16, 33), (2, 96, 64, 36)])
 def test_fp32_parity(shape, flags):
     B, N, K, F = shape
-    x, a, s, mask = _inputs(B, N, K, F, seed=sum(shape))
-    up = _upstream(B, K, F, sum(shape))
+    x, a, s, mask = C.planted_partition(B, N, K, F, seed=sum(shape))
+    up = C.upstream(B, K, F, sum(shape))
     xp_e, ap_e, loss_e, qv_e, qi_e, g_e = _oracle(x, a, s, flags, up)
     xp, ap, loss, quant, rows, g = _device(x, a, s, flags, up)
     torch.testing.assert_close(loss.double(), loss_e, rtol=1e-5, atol=0.0)
@@ -115,20 +59,20 @@ def test_fp32_parity(shape, flags):
         torch.testing.assert_close(gv.double(), ev, rtol=1e-5, atol=1e-5 * float(ev.abs().max()), msg=name)
     assert torch.equal(quant, qv_e.float())  # bit for bit: the same element of S
     assert torch.equal(rows.long(), qi_e)
-    _check_grads(g, g_e, 1e-4, flags["edge_weight_norm"])
+    C.check_per_source(g, g_e, 1e-4, flags["edge_weight_norm"])
 
 
 def test_quantile_among_tied_padded_zeros():
     """Graphs with fewer valid nodes than N // K: the quantile falls among the padded zero rows (some stored as -0.0),
     and the stable sort's rank rule picks row n_b + (N // K - n_b) of them."""
     B, N, K, F = 3, 64, 4, 8
-    x, a, s, mask = _inputs(B, N, K, F, seed=4)
+    x, a, s, mask = C.planted_partition(B, N, K, F, seed=4)
     n = torch.tensor([10, 5, 64])
     mask = torch.arange(N)[None, :] < n[:, None]
     s = s * mask[..., None]
     a = a * (mask[:, :, None] & mask[:, None, :])
     s[0, 12:20, 1] = -0.0  # the selected row of graph 0, column 1 is a -0.0
-    up = _upstream(B, K, F, 4)
+    up = C.upstream(B, K, F, 4)
     _, _, loss_e, qv_e, qi_e, g_e = _oracle(x, a, s, FLAGSETS[0], up, dev="cpu")  # the CPU sort: -0.0 ties +0.0
     _, _, loss, quant, rows, g = _device(x, a, s, FLAGSETS[0], up)
     assert qi_e[0].tolist() == [16] * K and qi_e[1].tolist() == [16] * K
@@ -136,28 +80,28 @@ def test_quantile_among_tied_padded_zeros():
     assert torch.equal(quant.cpu().view(torch.int32), qv_e.float().view(torch.int32))
     assert quant[0, 1].view(torch.int32).item() == -2 ** 31
     torch.testing.assert_close(loss.cpu().double(), loss_e, rtol=1e-5, atol=0.0)
-    _check_grads({k: [t.cpu() for t in v] for k, v in g.items()}, g_e, 1e-4, False)
+    C.check_per_source({k: [t.cpu() for t in v] for k, v in g.items()}, g_e, 1e-4, False)
 
 
 def test_tie_column_rank_rule():
     s = torch.tensor([[[.5, .1], [.2, .2], [.2, .3], [.2, .9], [.1, .4]]])
     a = torch.tensor([[[0, 1, 0, 1, 0], [1, 0, 1, 0, 0], [0, 1, 0, 2, 1], [1, 0, 2, 0, 0], [0, 0, 1, 0, 1.]]])
     x = torch.randn(1, 5, 3)
-    up = _upstream(1, 2, 3, 0)
+    up = C.upstream(1, 2, 3, 0)
     _, _, loss_e, qv_e, qi_e, g_e = _oracle(x, a, s, FLAGSETS[2], up, dev="cpu")
     _, _, loss, quant, rows, g = _device(x, a, s, FLAGSETS[2], up)
     assert rows[0].tolist() == [2, 2] == qi_e[0].tolist()
     assert torch.equal(quant.cpu(), qv_e.float())
     torch.testing.assert_close(loss.cpu().double(), loss_e, rtol=1e-5, atol=1e-7)
-    _check_grads({k: [t.cpu() for t in v] for k, v in g.items()}, g_e, 1e-4, False)
+    C.check_per_source({k: [t.cpu() for t in v] for k, v in g.items()}, g_e, 1e-4, False)
 
 
 @pytest.mark.parametrize("shape", [(3, 256, 64, 128), (2, 512, 256, 64), (4, 100, 16, 32)])
 def test_bf16_parity(shape):
     B, N, K, F = shape
-    x, a, s, mask = _inputs(B, N, K, F, seed=7 + sum(shape))
+    x, a, s, mask = C.planted_partition(B, N, K, F, seed=7 + sum(shape))
     x, a, s = (t.bfloat16().float() for t in (x, a, s))  # the oracle sees the rounded operands (and their ties)
-    up = {k: v.bfloat16().float() for k, v in _upstream(B, K, F, 7).items()}
+    up = tuple(v.bfloat16().float() for v in C.upstream(B, K, F, 7))
     xp_e, ap_e, loss_e, qv_e, qi_e, g_e = _oracle(x, a, s, FLAGSETS[0], up)
     xp, ap, loss, quant, rows, g = _device(x, a, s, FLAGSETS[0], up, dtype=torch.bfloat16)
     torch.testing.assert_close(loss.double(), loss_e, rtol=2e-2, atol=0.0)
@@ -165,14 +109,14 @@ def test_bf16_parity(shape):
         torch.testing.assert_close(gv.double(), ev, rtol=2e-2, atol=2e-2 * float(ev.abs().max()), msg=name)
     assert torch.equal(quant.double(), qv_e)  # the operands are bf16 values: the selected one is exact
     assert torch.equal(rows.long(), qi_e)
-    _check_grads(g, g_e, 2e-2, False)
+    C.check_per_source(g, g_e, 2e-2, False)
 
 
 def _graph_inputs(B=6, N=256, K=64, F=128, seed=9):
-    x, a, s, mask = _inputs(B, N, K, F, seed=seed)
-    up = _upstream(B, K, F, seed)
+    x, a, s, mask = C.planted_partition(B, N, K, F, seed=seed)
+    up = C.upstream(B, K, F, seed)
     return (x.to(DEV).requires_grad_(True), a.to(DEV).requires_grad_(True), s.to(DEV).requires_grad_(True),
-            up["x"].to(DEV), up["adj"].to(DEV))
+            up[0].to(DEV), up[1].to(DEV))
 
 
 def _step(x, a, s, gx, ga):
@@ -186,51 +130,17 @@ def _step(x, a, s, gx, ga):
 
 def test_deterministic():
     x, a, s, gx, ga = _graph_inputs(B=8, seed=3)
-    runs = []
-    for _ in range(3):
-        out = _step(x, a, s, gx, ga)
-        runs.append([t.detach().clone() for t in out] + [x.grad.clone(), a.grad.clone(), s.grad.clone()])
-    for r in runs[1:]:
-        for u, v in zip(r, runs[0]):
-            assert torch.equal(u, v)
+    C.assert_deterministic(lambda: _step(x, a, s, gx, ga), [x, a, s])
 
 
 def test_graph_replay_matches_eager():
     x, a, s, gx, ga = _graph_inputs()
-    eager = [t.detach().clone() for t in _step(x, a, s, gx, ga)] + [x.grad.clone(), a.grad.clone(), s.grad.clone()]
-    graphed = T.GraphedStep(lambda: _step(x, a, s, gx, ga))
-    out = graphed.replay()
-    torch.cuda.synchronize()
-    for got, exp in zip([*out, x.grad, a.grad, s.grad], eager):
-        assert torch.equal(got.detach(), exp)
+    C.assert_replay_matches_eager(lambda: _step(x, a, s, gx, ga), [x, a, s])
 
 
 def test_patched_pooler_masked_ragged_batch():
-    g = torch.Generator().manual_seed(11)
-    B, N, K, F = 5, 96, 16, 40
-    x, a, _, mask = _inputs(B, N, K, F, seed=11)
-    wsel = torch.randn(F, K, generator=g)
-
-    def select(x, mask):  # MLPSelect: softmax(linear(x)) * mask
-        return T.SelectOutput(s=torch.softmax(x @ wsel.to(x.device), -1) * mask[..., None])
-
-    pooler = AsymCheegerCutPooling(selector=select, reducer=H.BaseReduce(),
-                                   connector=H.DenseConnect(True, True, True, False))
-    T.patch_pooler(pooler)
-    xg = x.to(DEV).requires_grad_(True)
-    out = pooler(x=xg, adj=a.to(DEV), mask=mask.to(DEV))
-    xc = x.to(DEV, torch.float64).requires_grad_(True)
-    mc = mask.to(DEV)
-    s_c = torch.softmax(xc @ wsel.to(DEV, torch.float64), -1) * mc[..., None]
-    xp_c, ap_c, loss_c = A.acc_pool(xc, a.to(DEV, torch.float64), s_c, 0.6, 1.4)
-    assert set(out.loss) == set(KEYS.values()) == set(loss_c)
-    for k in loss_c:
-        torch.testing.assert_close(out.loss[k].detach().double(), loss_c[k].detach(), rtol=1e-5, atol=1e-6, msg=k)
-    sc = lambda t: float(t.abs().max())  # noqa: E731
-    torch.testing.assert_close(out.x.detach().double(), xp_c.detach(), rtol=1e-5, atol=1e-5 * sc(xp_c))
-    (out.x.sum() + out.edge_index.sum() + sum(out.loss.values())).backward()
-    (xp_c.sum() + ap_c.sum() + sum(loss_c.values())).backward()
-    torch.testing.assert_close(xg.grad.double(), xc.grad, rtol=1e-4, atol=1e-5 * sc(xc.grad))
+    C.check_patched_pooler(AsymCheegerCutPooling, lambda x, a, s, mask: A.acc_pool(x, a, s, 0.6, 1.4), DEV,
+                           KEYS.values())
 
 
 def test_hand_values_and_edgeless_graph_on_device():
@@ -270,7 +180,7 @@ def test_argument_errors():
 def test_no_pairwise_tensor_in_memory():
     """The extra peak of a forward + backward at (64, 256, 64) stays below 2 x adj.nbytes (dA itself is one): the
     [B, N, N, K] difference tensor of the eager formulation would be 64 x adj.nbytes."""
-    x, a, s, mask = _inputs(64, 256, 64, 8, seed=1, ragged=False)
+    x, a, s, mask = C.planted_partition(64, 256, 64, 8, seed=1, ragged=False)
     a, s = a.to(DEV).requires_grad_(True), s.to(DEV).requires_grad_(True)
     torch.cuda.synchronize()
     torch.cuda.reset_peak_memory_stats()

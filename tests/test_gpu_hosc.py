@@ -4,20 +4,15 @@ pooler; the term mask (no A A product when alpha = 0); the memory bound and argu
 import pytest
 import torch
 
+import dense_loss_cases as C
 import dropin_harness as H
 import hosc_oracle as O
 import tgp_b200 as T
+from dense_loss_cases import DEV, FLAGSETS
 from tgp_b200 import _lib as L
 from tgp_b200 import functional as F_
 
 pytestmark = pytest.mark.gpu
-DEV = "cuda:0"
-FLAGSETS = [
-    dict(remove_self_loops=True, degree_norm=True, adj_transpose=True, edge_weight_norm=False),
-    dict(remove_self_loops=True, degree_norm=True, adj_transpose=False, edge_weight_norm=True),
-    dict(remove_self_loops=False, degree_norm=False, adj_transpose=False, edge_weight_norm=False),
-]
-SOURCES = ("x", "adj", "hosc", "ortho")
 COEF = {"hosc": 1.7, "ortho": -0.8}
 KEYS = {"hosc": "hosc_loss", "ortho": "ortho_loss"}
 
@@ -26,71 +21,20 @@ class HOSCPooling(H._DenseBase):  # the restated attributes of HOSCPooling
     mu, alpha, hosc_ortho = 0.2, 0.6, True
 
 
-def _inputs(B, N, K, F, seed, ragged=True):
-    """Planted-partition graphs (dense communities: many triangles) with communities of skewed sizes, an assignment that
-    follows them, and graph b with n_b valid nodes (padded rows / columns zero)."""
-    g = torch.Generator().manual_seed(seed)
-    n = torch.tensor([N - (7 * b) % max(1, N // 3) if ragged else N for b in range(B)])
-    mask = torch.arange(N)[None, :] < n[:, None]
-    comm = (K * torch.rand(B, N, generator=g) ** 2).long().clamp(max=K - 1)
-    same = comm[:, :, None] == comm[:, None, :]
-    p = torch.where(same, torch.tensor(0.6), torch.tensor(0.3 / N))
-    a = (torch.rand(B, N, N, generator=g) < p).float()
-    a = torch.triu(a, 1)
-    a = (a + a.transpose(1, 2)) * torch.rand(B, N, N, generator=g).add(0.5)
-    a = (a + a.transpose(1, 2)) * 0.5 * (mask[:, :, None] & mask[:, None, :])
-    logits = 4.0 * torch.nn.functional.one_hot(comm, K).float() + torch.randn(B, N, K, generator=g)
-    s = torch.softmax(logits, -1) * mask[..., None]
-    x = torch.randn(B, N, F, generator=g) * mask[..., None]
-    return x, a, s, mask
-
-
-def _upstream(B, K, F, seed):
-    g = torch.Generator().manual_seed(seed + 100)
-    return {"x": torch.randn(B, K, F, generator=g), "adj": torch.randn(B, K, K, generator=g)}
-
-
-def _objective(xp, ap, loss, src, up):
-    if src in ("x", "adj"):
-        out = xp if src == "x" else ap
-        return (out * up[src].to(out.device, out.dtype)).sum()
-    return COEF[src] * loss[KEYS[src]]
-
-
-def _grads(xp, ap, loss, up, leaves):
-    grads = {}
-    for src in SOURCES:
-        g = torch.autograd.grad(_objective(xp, ap, loss, src, up), leaves, retain_graph=True, allow_unused=True)
-        grads[src] = [torch.zeros_like(v) if gv is None else gv for gv, v in zip(g, leaves)]
-    return grads
-
-
 def _oracle(x, a, s, mask, alpha, hosc_ortho, flags, up):
     """float64 forward on the CPU and the (dX, dA, dS) of each gradient source alone."""
     leaves = tuple(t.double().requires_grad_(True) for t in (x, a, s))
     xp, ap, loss = O.hosc_pool(*leaves, mask, 0.3, alpha, hosc_ortho, **flags)
     losses = torch.stack([loss[KEYS["hosc"]], loss[KEYS["ortho"]]]).detach()
-    return xp.detach(), ap.detach(), losses, _grads(xp, ap, loss, up, leaves)
+    return xp.detach(), ap.detach(), losses, C.per_source_grads(xp, ap, loss, up, leaves, COEF, KEYS)
 
 
 def _device(x, a, s, mask, alpha, hosc_ortho, flags, up, dtype=torch.float32):
     leaves = tuple(t.to(DEV, dtype).requires_grad_(True) for t in (x, a, s))
     xp, ap, loss = T.hosc_pool(*leaves, mask.to(DEV), 0.3, alpha, hosc_ortho, **flags)
     losses = torch.stack([loss[KEYS["hosc"]], loss[KEYS["ortho"]]]).detach()
-    grads = _grads(xp, ap, loss, up, leaves)
+    grads = C.per_source_grads(xp, ap, loss, up, leaves, COEF, KEYS)
     return xp.detach(), ap.detach(), losses, {k: [t.cpu() for t in v] for k, v in grads.items()}
-
-
-def _check_grads(got, exp, tau, edge_weight_norm):
-    for src in SOURCES:
-        for name, gv, ev in zip(("dX", "dA", "dS"), got[src], exp[src]):
-            gv, ev = gv.double(), ev.double()
-            if name == "dA" and src == "adj" and edge_weight_norm:
-                # max-normalisation routes one term to "the" arg-max, which a symmetric adjacency ties with its mirror
-                gv, ev = 0.5 * (gv + gv.transpose(1, 2)), 0.5 * (ev + ev.transpose(1, 2))
-            bound = tau * float(ev.abs().max())
-            err = float((gv - ev).abs().max())
-            assert err <= bound, f"{src} -> {name}: max error {err:.3e} > {bound:.3e}"
 
 
 @pytest.mark.parametrize("hosc_ortho", [False, True])
@@ -99,29 +43,29 @@ def _check_grads(got, exp, tau, edge_weight_norm):
 @pytest.mark.parametrize("shape", [(3, 256, 64, 128), (5, 200, 48, 100), (4, 100, 16, 33), (2, 96, 64, 36)])
 def test_fp32_parity(shape, flags, alpha, hosc_ortho):
     B, N, K, F = shape
-    x, a, s, mask = _inputs(B, N, K, F, seed=sum(shape))
-    up = _upstream(B, K, F, sum(shape))
+    x, a, s, mask = C.planted_partition(B, N, K, F, seed=sum(shape))
+    up = C.upstream(B, K, F, sum(shape))
     xp_e, ap_e, loss_e, g_e = _oracle(x, a, s, mask, alpha, hosc_ortho, flags, up)
     xp, ap, loss, g = _device(x, a, s, mask, alpha, hosc_ortho, flags, up)
     torch.testing.assert_close(loss.cpu().double(), loss_e, rtol=1e-5, atol=0.0)
     for name, gv, ev in (("x_pool", xp, xp_e), ("adj_pool", ap, ap_e)):
         torch.testing.assert_close(gv.cpu().double(), ev, rtol=1e-5, atol=1e-5 * float(ev.abs().max()), msg=name)
-    _check_grads(g, g_e, 1e-4, flags["edge_weight_norm"])
+    C.check_per_source(g, g_e, 1e-4, flags["edge_weight_norm"])
 
 
 @pytest.mark.parametrize("hosc_ortho", [False, True])
 @pytest.mark.parametrize("shape", [(3, 256, 64, 128), (2, 512, 256, 64), (4, 100, 16, 32)])
 def test_bf16_parity(shape, hosc_ortho):
     B, N, K, F = shape
-    x, a, s, mask = _inputs(B, N, K, F, seed=7 + sum(shape))
+    x, a, s, mask = C.planted_partition(B, N, K, F, seed=7 + sum(shape))
     x, a, s = (t.bfloat16().float() for t in (x, a, s))  # the oracle sees the rounded operands
-    up = {k: v.bfloat16().float() for k, v in _upstream(B, K, F, 7).items()}
+    up = tuple(v.bfloat16().float() for v in C.upstream(B, K, F, 7))
     xp_e, ap_e, loss_e, g_e = _oracle(x, a, s, mask, 0.5, hosc_ortho, FLAGSETS[0], up)
     xp, ap, loss, g = _device(x, a, s, mask, 0.5, hosc_ortho, FLAGSETS[0], up, dtype=torch.bfloat16)
     torch.testing.assert_close(loss.cpu().double(), loss_e, rtol=2e-2, atol=0.0)
     for name, gv, ev in (("x_pool", xp, xp_e), ("adj_pool", ap, ap_e)):
         torch.testing.assert_close(gv.cpu().double(), ev, rtol=2e-2, atol=2e-2 * float(ev.abs().max()), msg=name)
-    _check_grads(g, g_e, 2e-2, False)
+    C.check_per_source(g, g_e, 2e-2, False)
 
 
 def test_raw_terms_and_hand_values_on_device():
@@ -150,10 +94,10 @@ def test_raw_terms_and_hand_values_on_device():
 
 
 def _graph_inputs(B=6, N=256, K=64, F=128, seed=9):
-    x, a, s, mask = _inputs(B, N, K, F, seed=seed)
-    up = _upstream(B, K, F, seed)
+    x, a, s, mask = C.planted_partition(B, N, K, F, seed=seed)
+    up = C.upstream(B, K, F, seed)
     return (x.to(DEV).requires_grad_(True), a.to(DEV).requires_grad_(True), s.to(DEV).requires_grad_(True),
-            mask.to(DEV), up["x"].to(DEV), up["adj"].to(DEV))
+            mask.to(DEV), up[0].to(DEV), up[1].to(DEV))
 
 
 def _step(x, a, s, mask, gx, ga):
@@ -167,55 +111,21 @@ def _step(x, a, s, mask, gx, ga):
 
 def test_deterministic():
     x, a, s, mask, gx, ga = _graph_inputs(B=8, seed=3)
-    runs = []
-    for _ in range(3):
-        out = _step(x, a, s, mask, gx, ga)
-        runs.append([t.detach().clone() for t in out] + [x.grad.clone(), a.grad.clone(), s.grad.clone()])
-    for r in runs[1:]:
-        for u, v in zip(r, runs[0]):
-            assert torch.equal(u, v)
+    C.assert_deterministic(lambda: _step(x, a, s, mask, gx, ga), [x, a, s])
 
 
 def test_graph_replay_matches_eager():
     x, a, s, mask, gx, ga = _graph_inputs()
-    eager = [t.detach().clone() for t in _step(x, a, s, mask, gx, ga)] + [x.grad.clone(), a.grad.clone(),
-                                                                         s.grad.clone()]
-    graphed = T.GraphedStep(lambda: _step(x, a, s, mask, gx, ga))
-    out = graphed.replay()
-    torch.cuda.synchronize()
-    for got, exp in zip([*out, x.grad, a.grad, s.grad], eager):
-        assert torch.equal(got.detach(), exp)
+    C.assert_replay_matches_eager(lambda: _step(x, a, s, mask, gx, ga), [x, a, s])
 
 
 def test_patched_pooler_masked_ragged_batch():
-    g = torch.Generator().manual_seed(11)
-    B, N, K, F = 5, 96, 16, 40
-    x, a, _, mask = _inputs(B, N, K, F, seed=11)
-    wsel = torch.randn(F, K, generator=g)
-
-    def select(x, mask):  # MLPSelect: softmax(linear(x)) * mask
-        return T.SelectOutput(s=torch.softmax(x @ wsel.to(x.device), -1) * mask[..., None])
-
-    pooler = HOSCPooling(selector=select, reducer=H.BaseReduce(), connector=H.DenseConnect(True, True, True, False))
-    T.patch_pooler(pooler)
-    xg = x.to(DEV).requires_grad_(True)
-    out = pooler(x=xg, adj=a.to(DEV), mask=mask.to(DEV))
-    xc = x.double().requires_grad_(True)
-    s_c = torch.softmax(xc @ wsel.double(), -1) * mask[..., None]
-    xp_c, ap_c, loss_c = O.hosc_pool(xc, a.double(), s_c, mask, 0.2, 0.6, True)
-    assert set(out.loss) == set(KEYS.values()) == set(loss_c)
-    for k in loss_c:
-        torch.testing.assert_close(out.loss[k].detach().cpu().double(), loss_c[k].detach(), rtol=1e-5, atol=1e-6,
-                                   msg=k)
-    sc = lambda t: float(t.abs().max())  # noqa: E731
-    torch.testing.assert_close(out.x.detach().cpu().double(), xp_c.detach(), rtol=1e-5, atol=1e-5 * sc(xp_c))
-    (out.x.sum() + out.edge_index.sum() + sum(out.loss.values())).backward()
-    (xp_c.sum() + ap_c.sum() + sum(loss_c.values())).backward()
-    torch.testing.assert_close(xg.grad.cpu().double(), xc.grad, rtol=1e-4, atol=1e-5 * sc(xc.grad))
+    C.check_patched_pooler(HOSCPooling, lambda x, a, s, mask: O.hosc_pool(x, a, s, mask, 0.2, 0.6, True), "cpu",
+                           KEYS.values())
 
 
 def _launched(alpha, need_adj):
-    x, a, s, mask = _inputs(2, 128, 16, 8, seed=5)
+    x, a, s, mask = C.planted_partition(2, 128, 16, 8, seed=5)
     a, s = a.to(DEV).requires_grad_(need_adj), s.to(DEV).requires_grad_(True)
     torch.cuda.synchronize()
     L.time_kernel("*")
@@ -241,7 +151,7 @@ def test_extra_memory_of_forward_and_backward():
     """With only S requiring grad, the extra peak of a forward + backward stays below 2.5 B N^2 fp32 words: A_M (saved)
     is the one N^2 buffer that lives past the forward."""
     B, N, K = 16, 512, 64
-    _, a, s, _ = _inputs(B, N, K, 8, seed=1, ragged=False)
+    _, a, s, _ = C.planted_partition(B, N, K, 8, seed=1, ragged=False)
     a, s = a.to(DEV), s.to(DEV).requires_grad_(True)
     torch.cuda.synchronize()
     torch.cuda.reset_peak_memory_stats()

@@ -146,19 +146,6 @@ def test_hosc_pool_and_patched_pooler_wiring(monkeypatch, hosc_ortho):
     torch.testing.assert_close(out.edge_index, ap)
 
 
-def test_pooler_without_attributes_keeps_reference_forward():
-    import tgp_b200 as T
-
-    class Bare(H._DenseBase):
-        mu, alpha = 0.1, 0.5  # hosc_ortho missing
-
-    Bare.__name__ = "HOSCPooling"
-    pooler = Bare(selector=None, reducer=H.BaseReduce(), connector=H.DenseConnect())
-    ref = pooler.forward
-    T.patch_pooler(pooler)
-    assert pooler.forward == ref
-
-
 def test_hosc_ops_fake_tensor_shapes():
     from torch._subclasses.fake_tensor import FakeTensorMode
 

@@ -111,23 +111,26 @@ std::tuple<Tensor, Tensor, Tensor> stas_fused_bwd(const OptTensor& x, const OptT
   return {gx, ga, gs};
 }
 
-// (losses[2] = {total variation, balance}, quant [B, K], saved) of Asymmetric Cheeger Cut pooling
-// (totvar_loss / asym_norm_loss as restated in tests/acc_oracle.py)
-void acc_check_args(const Tensor& adj, const Tensor& s) {
+// The [B, N, N] adjacency and the [B, N, K] assignment of the dense loss ops: CUDA, contiguous, one dtype, K >= 2
+// and N >= 1.  `op` names the operator in the messages; `k_reason` says why it needs two clusters (may be empty).
+void check_adj_s(const Tensor& adj, const Tensor& s, const char* op, const char* k_reason = "") {
   require_cuda(s, "s");
   require_cuda(adj, "adj");
-  TORCH_CHECK(s.dim() == 3, "acc_losses expects s of shape [B, N, K], got ", s.sizes());
+  TORCH_CHECK(s.dim() == 3, op, " expects s of shape [B, N, K], got ", s.sizes());
   TORCH_CHECK(adj.dim() == 3 && adj.size(0) == s.size(0) && adj.size(1) == s.size(1) && adj.size(2) == s.size(1),
-              "acc_losses expects adj of shape [B, N, N] = [", s.size(0), ", ", s.size(1), ", ", s.size(1), "], got ",
+              op, " expects adj of shape [B, N, N] = [", s.size(0), ", ", s.size(1), ", ", s.size(1), "], got ",
               adj.sizes());
-  TORCH_CHECK(adj.scalar_type() == s.scalar_type(), "tgp_b200.acc_losses: adj and s must share one dtype");
-  TORCH_CHECK_VALUE(s.size(2) >= 2, "acc_losses needs K >= 2 clusters (the balance loss divides by K - 1), got K = ",
-                    s.size(2));
-  TORCH_CHECK_VALUE(s.size(1) >= 1, "acc_losses needs N >= 1 nodes");
+  TORCH_CHECK(adj.scalar_type() == s.scalar_type(), "tgp_b200.", op, ": adj and s must share one dtype");
+  TORCH_CHECK_VALUE(s.size(2) >= 2, op, " needs K >= 2 clusters", k_reason, ", got K = ", s.size(2));
+  TORCH_CHECK_VALUE(s.size(1) >= 1, op, " needs N >= 1 nodes");
 }
 
+constexpr const char* kAccKReason = " (the balance loss divides by K - 1)";
+
+// (losses[2] = {total variation, balance}, quant [B, K], saved) of Asymmetric Cheeger Cut pooling
+// (totvar_loss / asym_norm_loss as restated in tests/acc_oracle.py)
 std::tuple<Tensor, Tensor, Tensor> acc_losses(const Tensor& adj, const Tensor& s) {
-  acc_check_args(adj, s);
+  check_adj_s(adj, s, "acc_losses", kAccKReason);
   c10::cuda::CUDAGuard guard(s.device());
   const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
   Tensor saved = workspace(tgpb200_acc_loss_saved_bytes(B, K), s);
@@ -143,7 +146,7 @@ std::tuple<Tensor, Tensor, Tensor> acc_losses(const Tensor& adj, const Tensor& s
 
 std::tuple<Tensor, Tensor> acc_losses_bwd(const Tensor& adj, const Tensor& s, const Tensor& saved,
                                           const Tensor& glosses, bool need_gadj) {
-  acc_check_args(adj, s);
+  check_adj_s(adj, s, "acc_losses", kAccKReason);
   c10::cuda::CUDAGuard guard(s.device());
   const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
   TORCH_CHECK(glosses.numel() == 2, "acc_losses_bwd expects 2 upstream loss gradients");
@@ -159,22 +162,10 @@ std::tuple<Tensor, Tensor> acc_losses_bwd(const Tensor& adj, const Tensor& s, co
 
 // (losses[3] = {first-order cut, motif cut, HOSC orthogonality}, saved) of HOSC pooling (restated in
 // tests/hosc_oracle.py); `terms` is the bitmask of tgpb200_hosc_loss_fwd
-void hosc_check_args(const Tensor& adj, const Tensor& s, int64_t terms) {
-  require_cuda(s, "s");
-  require_cuda(adj, "adj");
-  TORCH_CHECK(s.dim() == 3, "hosc_losses expects s of shape [B, N, K], got ", s.sizes());
-  TORCH_CHECK(adj.dim() == 3 && adj.size(0) == s.size(0) && adj.size(1) == s.size(1) && adj.size(2) == s.size(1),
-              "hosc_losses expects adj of shape [B, N, N] = [", s.size(0), ", ", s.size(1), ", ", s.size(1), "], got ",
-              adj.sizes());
-  TORCH_CHECK(adj.scalar_type() == s.scalar_type(), "tgp_b200.hosc_losses: adj and s must share one dtype");
-  TORCH_CHECK_VALUE(s.size(2) >= 2, "hosc_losses needs K >= 2 clusters, got K = ", s.size(2));
-  TORCH_CHECK_VALUE(s.size(1) >= 1, "hosc_losses needs N >= 1 nodes");
-  TORCH_CHECK_VALUE(terms >= 1 && terms <= 7, "hosc_losses: terms must be a non-empty mask of 1 | 2 | 4, got ", terms);
-}
-
 std::tuple<Tensor, Tensor> hosc_losses(const Tensor& adj, const Tensor& s, const OptTensor& graph_nodes,
                                        int64_t terms, double eps) {
-  hosc_check_args(adj, s, terms);
+  check_adj_s(adj, s, "hosc_losses");
+  TORCH_CHECK_VALUE(terms >= 1 && terms <= 7, "hosc_losses: terms must be a non-empty mask of 1 | 2 | 4, got ", terms);
   c10::cuda::CUDAGuard guard(s.device());
   const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
   const int dt = dtype_code(s);
@@ -190,7 +181,8 @@ std::tuple<Tensor, Tensor> hosc_losses(const Tensor& adj, const Tensor& s, const
 
 std::tuple<Tensor, Tensor> hosc_losses_bwd(const Tensor& adj, const Tensor& s, const OptTensor& graph_nodes,
                                            const Tensor& saved, const Tensor& glosses, int64_t terms, bool need_gadj) {
-  hosc_check_args(adj, s, terms);
+  check_adj_s(adj, s, "hosc_losses");
+  TORCH_CHECK_VALUE(terms >= 1 && terms <= 7, "hosc_losses: terms must be a non-empty mask of 1 | 2 | 4, got ", terms);
   c10::cuda::CUDAGuard guard(s.device());
   const int64_t B = s.size(0), N = s.size(1), K = s.size(2);
   const int dt = dtype_code(s);

@@ -210,14 +210,8 @@ def _pooling_output_cls():
         return PoolingOutput
 
 
-_DMON_COEFFS = ("spectral_loss_coeff", "cluster_loss_coeff", "ortho_loss_coeff")
-# AsymCheegerCutPooling: its class name, its coefficient attributes (total variation, balance) and its loss keys
-_ACC_CLASS = "AsymCheegerCutPooling"
-_ACC_COEFFS = ("totvar_coeff", "balance_coeff")
+# the loss keys of AsymCheegerCutPooling (total variation, balance)
 _ACC_KEYS = ("total_variation_loss", "balance_loss")
-# HOSCPooling: its class name and the attributes the fused forward reads
-_HOSC_CLASS = "HOSCPooling"
-_HOSC_ATTRS = ("mu", "alpha", "hosc_ortho")
 _AGGR_TO_OP = {"SumAggregation": "sum", "MeanAggregation": "mean", "MaxAggregation": "max", "MinAggregation": "min"}
 
 
@@ -236,10 +230,39 @@ def _reduce_op_of(reducer) -> Optional[str]:
     return None
 
 
-def _fused_dense_forward(pooler, kind: str):
-    """``forward`` of a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` / ``AsymCheegerCutPooling`` (tgp/poolers/mincut.py:210-258,
+def _diff_forward(pooler, x, adj, s, mask, flags):
+    x_pool, adj_pool, loss = diff_pool(x, adj, s, num_nodes=1, link_loss_coeff=pooler.link_loss_coeff,
+                                       ent_loss_coeff=1.0, normalize_loss=pooler.normalize_loss, **flags)
+    n_valid = mask.sum() if mask is not None else s.size(0) * s.size(1)  # stays on the device: no sync
+    loss["entropy_loss"] = loss["entropy_loss"] / n_valid * pooler.ent_loss_coeff
+    return x_pool, adj_pool, loss
+
+
+# The dense poolers with a fused forward, by reference class name: (the attributes the fused forward reads that must
+# exist for it to replace the reference's, ``(pooler, x, adj, s, mask, flags) -> (x_pool, adj_pool, loss)``).
+# MinCutPooling and DiffPool require none: a missing attribute raises instead of falling back.
+_FUSED_DENSE = {
+    "MinCutPooling": (
+        (), lambda p, x, adj, s, mask, flags: mincut_pool(x, adj, s, p.cut_loss_coeff, p.ortho_loss_coeff, **flags)),
+    "DiffPool": ((), _diff_forward),
+    "DMoNPooling": (
+        ("spectral_loss_coeff", "cluster_loss_coeff", "ortho_loss_coeff"),
+        lambda p, x, adj, s, mask, flags: dmon_pool(x, adj, s, mask, p.spectral_loss_coeff, p.cluster_loss_coeff,
+                                                    p.ortho_loss_coeff, **flags)),
+    "AsymCheegerCutPooling": (
+        ("totvar_coeff", "balance_coeff"),
+        lambda p, x, adj, s, mask, flags: acc_pool(x, adj, s, p.totvar_coeff, p.balance_coeff, **flags)),
+    "HOSCPooling": (
+        ("mu", "alpha", "hosc_ortho"),
+        lambda p, x, adj, s, mask, flags: hosc_pool(x, adj, s, mask, p.mu, p.alpha, p.hosc_ortho, **flags)),
+}
+
+
+def _fused_dense_forward(pooler, pool):
+    """``forward`` of a batched pooler of ``_FUSED_DENSE`` (tgp/poolers/mincut.py:210-258,
     tgp/poolers/diffpool.py:200-237) with reduce + connect + auxiliary losses + post-processing as ONE fused
-    forward / backward; select, input densification, lifting and the unbatched mode stay the reference's."""
+    forward / backward through ``pool``, its entry's function; select, input densification, lifting and the unbatched
+    mode stay the reference's."""
     ref_forward = pooler.forward
     Out = _pooling_output_cls()
 
@@ -254,20 +277,7 @@ def _fused_dense_forward(pooler, kind: str):
         c = pooler.connector
         flags = dict(remove_self_loops=c.remove_self_loops, degree_norm=c.degree_norm, adj_transpose=c.adj_transpose,
                      edge_weight_norm=c.edge_weight_norm)
-        if kind == "mincut":
-            x_pool, adj_pool, loss = mincut_pool(x, adj, so.s, pooler.cut_loss_coeff, pooler.ortho_loss_coeff, **flags)
-        elif kind == "dmon":
-            x_pool, adj_pool, loss = dmon_pool(x, adj, so.s, mask, pooler.spectral_loss_coeff, pooler.cluster_loss_coeff,
-                                               pooler.ortho_loss_coeff, **flags)
-        elif kind == "acc":
-            x_pool, adj_pool, loss = acc_pool(x, adj, so.s, *(getattr(pooler, a) for a in _ACC_COEFFS), **flags)
-        elif kind == "hosc":
-            x_pool, adj_pool, loss = hosc_pool(x, adj, so.s, mask, *(getattr(pooler, a) for a in _HOSC_ATTRS), **flags)
-        else:
-            x_pool, adj_pool, loss = diff_pool(x, adj, so.s, num_nodes=1, link_loss_coeff=pooler.link_loss_coeff,
-                                               ent_loss_coeff=1.0, normalize_loss=pooler.normalize_loss, **flags)
-            n_valid = mask.sum() if mask is not None else so.s.size(0) * so.s.size(1)  # stays on the device: no sync
-            loss["entropy_loss"] = loss["entropy_loss"] / n_valid * pooler.ent_loss_coeff
+        x_pool, adj_pool, loss = pool(pooler, x, adj, so.s, mask, flags)
         batch_pooled = B200Reduce.reduce_batch(so, batch)
         if getattr(pooler, "sparse_output", False):
             xs, ei, ew, bp = pooler._finalize_sparse_output(x_pool=x_pool, adj_pool=adj_pool, batch=batch,
@@ -285,12 +295,10 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
       same ctor attributes (the poolers read them, tgp/poolers/mincut.py:233-236);
     * ``pooler.reducer``: ``BaseReduce`` / ``AggrReduce(sum | mean | max | min)`` -> ``B200Reduce`` with the SAME
       reduction; any other reducer (learned / order-statistic aggregators) is left in place.  ``reduce_op`` overrides;
-    * ``fuse_dense``: a batched ``MinCutPooling`` / ``DiffPool`` / ``DMoNPooling`` / ``AsymCheegerCutPooling`` /
-      ``HOSCPooling`` also gets the fused forward (reduce + connect + losses + post-processing on the device kernels) -- without it the
-      patched pooler still calls the reference's torch loss functions.  A ``DMoNPooling`` lacking one of
-      ``spectral_loss_coeff``, ``cluster_loss_coeff``, ``ortho_loss_coeff``, an ``AsymCheegerCutPooling`` lacking
-      ``totvar_coeff`` or ``balance_coeff``, or a ``HOSCPooling`` lacking ``mu``, ``alpha`` or ``hosc_ortho``, keeps
-      the reference forward.
+    * ``fuse_dense``: a batched pooler whose class is in ``_FUSED_DENSE`` also gets the fused forward (reduce +
+      connect + losses + post-processing on the device kernels) -- without it the patched pooler still calls the
+      reference's torch loss functions.  A pooler lacking one of the attributes its entry requires keeps the
+      reference forward.
     """
     for attr in ("connector", "preconnector"):
         conn = getattr(pooler, attr, None)
@@ -308,14 +316,8 @@ def patch_pooler(pooler, reduce_op: Optional[str] = None, fuse_dense: bool = Tru
         op = reduce_op if reduce_op is not None else _reduce_op_of(reducer)
         if op is not None:
             pooler.reducer = B200Reduce(op)
-    kind = {"MinCutPooling": "mincut", "DiffPool": "diff", "DMoNPooling": "dmon", _ACC_CLASS: "acc",
-            _HOSC_CLASS: "hosc"}.get(type(pooler).__name__)
-    if kind == "dmon" and not all(hasattr(pooler, a) for a in _DMON_COEFFS):
-        kind = None
-    if kind == "acc" and not all(hasattr(pooler, a) for a in _ACC_COEFFS):
-        kind = None
-    if kind == "hosc" and not all(hasattr(pooler, a) for a in _HOSC_ATTRS):
-        kind = None
-    if fuse_dense and kind is not None and type(getattr(pooler, "connector", None)).__name__ == "B200DenseConnect":
-        pooler.forward = _fused_dense_forward(pooler, kind)
+    required, pool = _FUSED_DENSE.get(type(pooler).__name__, (None, None))
+    if (fuse_dense and pool is not None and all(hasattr(pooler, a) for a in required)
+            and type(getattr(pooler, "connector", None)).__name__ == "B200DenseConnect"):
+        pooler.forward = _fused_dense_forward(pooler, pool)
     return pooler
