@@ -110,20 +110,8 @@ int tgpb200_reduce_batch(const int64_t* batch, const int64_t* node_index, const 
  * *count_out (device int64) receives the number of surviving edges;
  * src_edge[j] (int32, may be NULL) = input position of output edge j (saved for backward).
  * ------------------------------------------------------------------------------------------ */
-size_t tgpb200_filter_relabel_workspace_bytes(int64_t num_edges, int64_t num_nodes);
-/* Phase 1 builds the relabel table and counts survivors; the caller reads *count_out (the one
- * unavoidable device->host word, since the reference returns exact-size tensors), allocates the
- * outputs and calls phase 2 with the SAME workspace. */
-int tgpb200_filter_relabel_count(const int64_t* row, const int64_t* col, const float* edge_weight, int64_t num_edges,
-                                 const int64_t* node_index, int64_t num_kept, int64_t num_nodes, uint32_t flags,
-                                 float eps, int64_t* count_out, void* workspace, size_t workspace_bytes,
-                                 tgpb200_stream_t stream);
-int tgpb200_filter_relabel_emit(const int64_t* row, const int64_t* col, const float* edge_weight, int64_t num_edges,
-                                int64_t num_nodes, uint32_t flags, float eps, int64_t* out_row, int64_t* out_col,
-                                float* out_weight, int32_t* src_edge, void* workspace, size_t workspace_bytes,
-                                tgpb200_stream_t stream);
-/* Single-pass form (decoupled look-back compaction): the edge list is read once.  The outputs must have capacity
- * num_edges; *count_out receives the survivor count when the stream has drained. */
+/* Decoupled look-back compaction: the edge list is read once.  The outputs must have capacity num_edges;
+ * *count_out receives the survivor count when the stream has drained. */
 size_t tgpb200_filter_relabel_onepass_workspace_bytes(int64_t num_edges, int64_t num_nodes);
 int tgpb200_filter_relabel_onepass(const int64_t* row, const int64_t* col, const float* edge_weight, int64_t num_edges,
                                    const int64_t* node_index, int64_t num_kept, int64_t num_nodes, uint32_t flags,
@@ -403,6 +391,7 @@ int tgpb200_block_diag_bwd(const void* grad_weight, const int32_t* src_pos, int6
  *   to_dense_adj:   edges -> [B, Nmax, Nmax] fp32, duplicates summed, default weight 1.0,
  *                   transpose != 0 writes A^T (src.py:442-443)                               (PyG to_dense_adj)
  * ------------------------------------------------------------------------------------------ */
+size_t tgpb200_graph_ptr_workspace_bytes(int64_t num_graphs);
 int tgpb200_graph_ptr(const int64_t* batch, int64_t num_nodes, int64_t num_graphs, int32_t* ptr, void* workspace,
                       size_t workspace_bytes, tgpb200_stream_t stream);
 int tgpb200_to_dense_batch(const void* x, const int64_t* batch, const int32_t* ptr, int64_t num_nodes, int64_t F,

@@ -25,7 +25,7 @@ def test_header_symbols_exported_and_bound():
         assert hasattr(lib, name), f"{name} declared in include/tgp_b200.h but not exported"
         assert name in L.SIGNATURES, f"{name} has no ctypes signature"
     assert sorted(L.SIGNATURES) == declared
-    assert lib.tgpb200_abi_version() >= 1
+    assert lib.tgpb200_abi_version() == 2
 
 
 def test_workspace_queries_are_pure_host_functions():
@@ -35,6 +35,7 @@ def test_workspace_queries_are_pure_host_functions():
     assert lib.tgpb200_build_csr_workspace_bytes(1000, 10) > 0
     assert lib.tgpb200_remap_coalesce_workspace_bytes(10**6, 10**5) > 20 * 10**6
     assert lib.tgpb200_dense_pool_saved_bytes(2, 16, 4) > 0
+    assert lib.tgpb200_graph_ptr_workspace_bytes(128) > 0
 
 
 def test_cpu_tensors_raise_no_fallback():

@@ -54,15 +54,22 @@ struct BlockDiagEmit {
   }
 };
 
+// Workspace layout shared by the count and emit phases: the renumbering of the kept pooled nodes with its scan, and
+// the compaction of the B K^2 entries.
 struct BlockDiagPlan {
   int* new_id;
-  int* tiles;
-  bool ok;
+  Workspace scan, tiles;
   BlockDiagPlan(Workspace& ws, int64_t B, int64_t K) {
     new_id = ws.take<int>((size_t)(B * K > 0 ? B * K : 1));
-    tiles = ws.take<int>((size_t)ceil_div(B * K * K > 0 ? B * K * K : 1, kCompactTile));
-    ok = ws.ok;
+    scan = ws.sub(scan_workspace_bytes(B * K));
+    tiles = ws.sub(compact_workspace_bytes(B * K * K));
   }
+};
+
+// Workspace of tgpb200_graph_ptr: the scan of the B + 1 graph offsets.
+struct GraphPtrLayout {
+  Workspace scan;
+  GraphPtrLayout(Workspace& ws, int64_t B) : scan(ws.sub(scan_workspace_bytes(B + 1))) {}
 };
 
 template <typename T>
@@ -117,10 +124,7 @@ using namespace tgp;
 
 extern "C" {
 
-size_t tgpb200_block_diag_workspace_bytes(int64_t B, int64_t K) {
-  int64_t n = B * K * K > 0 ? B * K * K : 1;
-  return align_up((size_t)(B * K > 0 ? B * K : 1) * 4) + compact_workspace_bytes(n) + scan_workspace_bytes(B * K) + 4096;
-}
+size_t tgpb200_block_diag_workspace_bytes(int64_t B, int64_t K) { return layout_bytes<BlockDiagPlan>(B, K); }
 
 int tgpb200_block_diag_count(const void* adj, const uint8_t* out_mask, int64_t B, int64_t K, int dtype, float eps,
                              int64_t* num_valid_out, int64_t* count_out, void* workspace, size_t workspace_bytes,
@@ -135,11 +139,11 @@ int tgpb200_block_diag_count(const void* adj, const uint8_t* out_mask, int64_t B
   }
   if (!adj) return TGPB200_ERR_INVALID;
   Workspace ws(workspace, workspace_bytes);
-  BlockDiagPlan pl(ws, B, K);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  const BlockDiagPlan pl(ws, B, K);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (out_mask) {
     launch("k_mask_to_int", k_mask_to_int, (unsigned)ceil_div(B * K, 256), 256, 0, st, out_mask, B * K, pl.new_id);
-    int rc = exclusive_scan_i32(pl.new_id, pl.new_id, B * K, nullptr, num_valid_out, ws, st);
+    int rc = exclusive_scan_i32(pl.new_id, pl.new_id, B * K, nullptr, num_valid_out, pl.scan, st);
     if (rc) return rc;
   }
   if (dtype == TGPB200_F32) {
@@ -162,8 +166,8 @@ int tgpb200_block_diag_emit(const void* adj, const uint8_t* out_mask, int64_t B,
   if (!adj || !out_row || !out_col || !out_weight) return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
-  BlockDiagPlan pl(ws, B, K);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  const BlockDiagPlan pl(ws, B, K);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   const int* new_id = out_mask ? pl.new_id : nullptr;
   if (dtype == TGPB200_F32) {
     BlockDiagPred<float> pred{(const float*)adj, out_mask, (int)K, eps};
@@ -200,17 +204,19 @@ int tgpb200_block_diag_bwd(const void* grad_weight, const int32_t* src_pos, int6
 }
 
 // ---- dense pre-processing (SURVEY 8f row 3): graph offsets, to_dense_batch, to_dense_adj
+size_t tgpb200_graph_ptr_workspace_bytes(int64_t B) { return layout_bytes<GraphPtrLayout>(B); }
+
 int tgpb200_graph_ptr(const int64_t* batch, int64_t N, int64_t B, int32_t* ptr, void* workspace, size_t workspace_bytes,
                       tgpb200_stream_t stream) {
   if (N < 0 || B <= 0 || !ptr) return TGPB200_ERR_INVALID;
+  if (N > 0 && !batch) return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
+  const GraphPtrLayout l(ws, B);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   cudaMemsetAsync(ptr, 0, (size_t)(B + 1) * sizeof(int32_t), st);
-  if (N > 0) {
-    if (!batch) return TGPB200_ERR_INVALID;
-    launch("k_graph_counts", k_graph_counts, (unsigned)ceil_div(N, 256), 256, 0, st, batch, N, B, ptr);
-  }
-  return exclusive_scan_i32(ptr, ptr, B + 1, nullptr, nullptr, ws, st);
+  if (N > 0) launch("k_graph_counts", k_graph_counts, (unsigned)ceil_div(N, 256), 256, 0, st, batch, N, B, ptr);
+  return exclusive_scan_i32(ptr, ptr, B + 1, nullptr, nullptr, l.scan, st);
 }
 
 int tgpb200_to_dense_batch(const void* x, const int64_t* batch, const int32_t* ptr, int64_t N, int64_t F, int64_t B,

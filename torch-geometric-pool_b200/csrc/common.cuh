@@ -80,7 +80,7 @@ struct Workspace {
   size_t cap;
   size_t off;
   bool ok;
-  Workspace(void* p, size_t bytes) : base(static_cast<char*>(p)), cap(bytes), off(0), ok(true) {}
+  Workspace(void* p = nullptr, size_t bytes = 0) : base(static_cast<char*>(p)), cap(bytes), off(0), ok(true) {}
   template <typename T>
   T* take(size_t n) {
     size_t bytes = align_up(n * sizeof(T));
@@ -93,7 +93,19 @@ struct Workspace {
     off += bytes;
     return r;
   }
+  // A region of `bytes` taken from this workspace, as a workspace of its own: a primitive's scratch in a layout.
+  Workspace sub(size_t bytes) { return Workspace(take<char>(bytes), bytes); }
 };
+
+// Bytes a layout carves: every workspace layout is a struct whose constructor takes all of its regions from a
+// Workspace, so its size query builds it over a null workspace (every take fails and is counted).
+template <typename Layout, typename... Args>
+inline size_t layout_bytes(Args... args) {
+  Workspace ws(nullptr, 0);
+  Layout l(ws, args...);
+  (void)l;
+  return ws.off;
+}
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 

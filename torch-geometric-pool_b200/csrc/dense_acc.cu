@@ -328,19 +328,30 @@ __global__ void __launch_bounds__(256)
   }
 }
 
+// The saved buffer, shared by the forward and the backward.
 struct AccSaved {
   long long* nnz;  // [B]
   int32_t* qidx;   // [B, K]
   int32_t* n_ge;   // [B, K]
+  AccSaved(Workspace& ws, int64_t B, int64_t K) {
+    nnz = ws.take<long long>((size_t)B);
+    qidx = ws.take<int32_t>((size_t)(B * K));
+    n_ge = ws.take<int32_t>((size_t)(B * K));
+  }
 };
 
-bool acc_saved(void* p, size_t bytes, int64_t B, int64_t K, AccSaved& o) {
-  Workspace w(p, bytes);
-  o.nnz = w.take<long long>((size_t)B);
-  o.qidx = w.take<int32_t>((size_t)(B * K));
-  o.n_ge = w.take<int32_t>((size_t)(B * K));
-  return w.ok;
-}
+// The forward workspace: per-tile partial sums of the total variation, their pair counts, per-chunk balance sums.
+struct AccFwdLayout {
+  float* tv_part;
+  unsigned long long* cnt_part;
+  float* bal_part;
+  AccFwdLayout(Workspace& ws, int64_t B, int64_t N, int64_t K) {
+    const size_t tiles = (size_t)pair_tiles(N);
+    tv_part = ws.take<float>((size_t)B * tiles);
+    cnt_part = ws.take<unsigned long long>((size_t)B * tiles);
+    bal_part = ws.take<float>((size_t)B * ceil_div(K, 32));
+  }
+};
 
 int acc_check(const void* adj, const void* s, int64_t B, int64_t N, int64_t K, int dtype) {
   if (!adj || !s || B < 0 || N < 1 || K < 2) return TGPB200_ERR_INVALID;
@@ -350,13 +361,12 @@ int acc_check(const void* adj, const void* s, int64_t B, int64_t N, int64_t K, i
 }
 
 template <typename T>
-int acc_fwd(const T* A, const T* S, int B, int N, int K, float* losses, T* quant, const AccSaved& sv, Workspace& ws,
-            cudaStream_t st) {
+int acc_fwd(const T* A, const T* S, int B, int N, int K, float* losses, T* quant, const AccSaved& sv,
+            const AccFwdLayout& l, cudaStream_t st) {
   const int tiles = pair_tiles(N), chunks = (int)ceil_div(K, 32);
-  float* tv_part = ws.take<float>((size_t)B * tiles);
-  unsigned long long* cnt_part = ws.take<unsigned long long>((size_t)B * tiles);
-  float* bal_part = ws.take<float>((size_t)B * chunks);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  float* tv_part = l.tv_part;
+  unsigned long long* cnt_part = l.cnt_part;
+  float* bal_part = l.bal_part;
   if (B > 0) {
     launch("k_acc_pair_l1", k_acc_pair_l1<T, false>, dim3(tiles, B), dim3(256), 0, st, A, S, N, K, B,
            (const float*)nullptr, (const long long*)nullptr, tv_part, cnt_part, (T*)nullptr);
@@ -390,14 +400,12 @@ extern "C" {
 
 size_t tgpb200_acc_loss_saved_bytes(int64_t B, int64_t K) {
   if (B < 0 || K < 0) return 0;
-  return align_up((size_t)B * sizeof(long long)) + 2 * align_up((size_t)(B * K) * sizeof(int32_t));
+  return layout_bytes<AccSaved>(B, K);
 }
 
 size_t tgpb200_acc_loss_fwd_workspace_bytes(int64_t B, int64_t N, int64_t K) {
   if (B < 0 || N < 1 || K < 1) return 0;
-  const size_t tiles = (size_t)pair_tiles(N);
-  return align_up((size_t)B * tiles * sizeof(float)) + align_up((size_t)B * tiles * sizeof(unsigned long long)) +
-         align_up((size_t)B * ceil_div(K, 32) * sizeof(float));
+  return layout_bytes<AccFwdLayout>(B, N, K);
 }
 
 int tgpb200_acc_loss_fwd(const void* adj, const void* s, int64_t B, int64_t N, int64_t K, int dtype, float* losses,
@@ -406,15 +414,16 @@ int tgpb200_acc_loss_fwd(const void* adj, const void* s, int64_t B, int64_t N, i
   int rc = acc_check(adj, s, B, N, K, dtype);
   if (rc != TGPB200_OK) return rc;
   if (!losses || !quant) return TGPB200_ERR_INVALID;
-  AccSaved sv;
-  if (!acc_saved(saved, saved_bytes, B, K, sv)) return TGPB200_ERR_WORKSPACE;
-  Workspace ws(workspace, workspace_bytes);
+  Workspace sw(saved, saved_bytes), ws(workspace, workspace_bytes);
+  const AccSaved sv(sw, B, K);
+  const AccFwdLayout l(ws, B, N, K);
+  if (!sw.ok || !ws.ok) return TGPB200_ERR_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == TGPB200_F32)
-    return acc_fwd<float>((const float*)adj, (const float*)s, (int)B, (int)N, (int)K, losses, (float*)quant, sv, ws,
+    return acc_fwd<float>((const float*)adj, (const float*)s, (int)B, (int)N, (int)K, losses, (float*)quant, sv, l,
                           st);
   return acc_fwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, (int)B, (int)N, (int)K, losses,
-                                (__nv_bfloat16*)quant, sv, ws, st);
+                                (__nv_bfloat16*)quant, sv, l, st);
 }
 
 int tgpb200_acc_loss_bwd(const void* adj, const void* s, const void* saved, size_t saved_bytes,
@@ -423,8 +432,9 @@ int tgpb200_acc_loss_bwd(const void* adj, const void* s, const void* saved, size
   int rc = acc_check(adj, s, B, N, K, dtype);
   if (rc != TGPB200_OK) return rc;
   if (!grad_s) return TGPB200_ERR_INVALID;
-  AccSaved sv;
-  if (!acc_saved(const_cast<void*>(saved), saved_bytes, B, K, sv)) return TGPB200_ERR_WORKSPACE;
+  Workspace sw(const_cast<void*>(saved), saved_bytes);
+  const AccSaved sv(sw, B, K);
+  if (!sw.ok) return TGPB200_ERR_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == TGPB200_F32)
     return acc_bwd<float>((const float*)adj, (const float*)s, grad_losses, (int)B, (int)N, (int)K, sv,

@@ -199,47 +199,60 @@ __global__ void k_hosc_da_prep(const T* __restrict__ A, const float* __restrict_
   dA[e] = from_f32<T>(v);
 }
 
+// The saved buffer, shared by the forward and the backward.
 template <typename T>
 struct HoscSaved {
   T* AM;       // [B, N, N] (motif term only)
   float* d;    // [B, N]
   float* dM;   // [B, N]
   float *n1, *m1, *nM, *mM, *sq;  // [B, K]
-  bool ok;
-  HoscSaved(void* p, size_t bytes, int64_t B, int64_t N, int64_t K, int terms) {
-    Workspace w(p, bytes);
-    AM = (terms & kMotif) ? w.take<T>((size_t)(B * N * N)) : nullptr;
-    d = w.take<float>((size_t)(B * N));
-    dM = w.take<float>((size_t)(B * N));
-    n1 = w.take<float>((size_t)(B * K));
-    m1 = w.take<float>((size_t)(B * K));
-    nM = w.take<float>((size_t)(B * K));
-    mM = w.take<float>((size_t)(B * K));
-    sq = w.take<float>((size_t)(B * K));
-    ok = w.ok;
+  HoscSaved(Workspace& ws, int64_t B, int64_t N, int64_t K, int terms) {
+    AM = (terms & kMotif) ? ws.take<T>((size_t)(B * N * N)) : nullptr;
+    d = ws.take<float>((size_t)(B * N));
+    dM = ws.take<float>((size_t)(B * N));
+    n1 = ws.take<float>((size_t)(B * K));
+    m1 = ws.take<float>((size_t)(B * K));
+    nM = ws.take<float>((size_t)(B * K));
+    mM = ws.take<float>((size_t)(B * K));
+    sq = ws.take<float>((size_t)(B * K));
   }
 };
 
-size_t elem_size(int dtype) { return dtype == TGPB200_F32 ? 4 : 2; }
+// The forward workspace: S padded to K1 columns, the products A S1 and A_M S1, and the fp32 A A of bf16 runs (fp32
+// runs build it in the saved A_M).
+template <typename T>
+struct HoscFwdLayout {
+  T* S1;
+  float *AS1, *AMS1, *P;
+  HoscFwdLayout(Workspace& ws, int64_t B, int64_t N, int64_t K, int terms) {
+    const size_t NK1 = (size_t)N * s1_width((int)K);
+    S1 = ws.take<T>((size_t)B * NK1);
+    AS1 = ws.take<float>((size_t)B * NK1);
+    AMS1 = ws.take<float>((size_t)B * NK1);
+    P = ((terms & kMotif) && !std::is_same<T, float>::value) ? ws.take<float>((size_t)(B * N * N)) : nullptr;
+  }
+};
 
-size_t saved_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
-  size_t s = 2 * align_up((size_t)(B * N) * 4) + 5 * align_up((size_t)(B * K) * 4);
-  if (terms & kMotif) s += align_up((size_t)(B * N * N) * elem_size(dtype));
-  return s;
-}
+// The backward workspace: the scaled assignments, and the terms of the adjacency gradient when it is asked for.
+template <typename T>
+struct HoscBwdLayout {
+  T *Sa, *Sm, *H;
+  float *P, *E2, *r, *rM;
+  HoscBwdLayout(Workspace& ws, int64_t B, int64_t N, int64_t K, bool need_grad_adj) {
+    Sa = ws.take<T>((size_t)(B * N * K));
+    Sm = ws.take<T>((size_t)(B * N * K));
+    P = need_grad_adj ? ws.take<float>((size_t)(B * N * N)) : nullptr;
+    E2 = need_grad_adj ? ws.take<float>((size_t)(B * N * N)) : nullptr;
+    H = need_grad_adj ? ws.take<T>((size_t)(B * N * N)) : nullptr;
+    r = need_grad_adj ? ws.take<float>((size_t)(B * N)) : nullptr;
+    rM = need_grad_adj ? ws.take<float>((size_t)(B * N)) : nullptr;
+  }
+};
 
-size_t fwd_ws_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
-  const size_t K1 = (size_t)s1_width((int)K);
-  size_t s = align_up((size_t)B * N * K1 * elem_size(dtype)) + 2 * align_up((size_t)B * N * K1 * 4);
-  if ((terms & kMotif) && dtype != TGPB200_F32) s += align_up((size_t)(B * N * N) * 4);
-  return s;
-}
-
-size_t bwd_ws_bytes(int64_t B, int64_t N, int64_t K, int dtype, bool grad_adj) {
-  size_t s = 2 * align_up((size_t)(B * N * K) * elem_size(dtype));
-  if (grad_adj) s += 2 * align_up((size_t)(B * N * N) * 4) + align_up((size_t)(B * N * N) * elem_size(dtype)) +
-                     2 * align_up((size_t)(B * N) * 4);
-  return s;
+// Bytes of a HOSC layout for the operand dtype.
+template <template <typename> class Layout, typename... Args>
+size_t hosc_layout_bytes(int dtype, Args... args) {
+  return dtype == TGPB200_F32 ? layout_bytes<Layout<float>>(args...) : layout_bytes<Layout<__nv_bfloat16>>(args...);
 }
 
 int hosc_check(const void* adj, const void* s, int64_t B, int64_t N, int64_t K, int dtype, int terms) {
@@ -253,16 +266,14 @@ unsigned blocks(int64_t total, int threads = 256) { return (unsigned)ceil_div(to
 
 template <typename T>
 int hosc_fwd(const T* A, const T* S, const float* graph_nodes, int B, int N, int K, int terms, float eps,
-             float* losses, HoscSaved<T>& sv, Workspace& ws, cudaStream_t st) {
+             float* losses, const HoscSaved<T>& sv, const HoscFwdLayout<T>& l, cudaStream_t st) {
   constexpr bool f32 = std::is_same<T, float>::value;
   const int K1 = s1_width(K);
   const int64_t NN = (int64_t)N * N, NK1 = (int64_t)N * K1;
   const bool first = terms & kFirst, motif = terms & kMotif;
-  T* S1 = ws.take<T>((size_t)B * NK1);
-  float* AS1 = ws.take<float>((size_t)B * NK1);
-  float* AMS1 = ws.take<float>((size_t)B * NK1);
-  float* P = (motif && !f32) ? ws.take<float>((size_t)B * NN) : reinterpret_cast<float*>(sv.AM);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  T* S1 = l.S1;
+  float *AS1 = l.AS1, *AMS1 = l.AMS1;
+  float* P = (motif && !f32) ? l.P : reinterpret_cast<float*>(sv.AM);
   int rc;
   if (B > 0) {
     const int64_t rows = (int64_t)B * N;
@@ -296,21 +307,11 @@ int hosc_fwd(const T* A, const T* S, const float* graph_nodes, int B, int N, int
 
 template <typename T>
 int hosc_bwd(const T* A, const T* S, const float* graph_nodes, const float* gl, int B, int N, int K, int terms,
-             const HoscSaved<T>& sv, T* dS, T* dA, Workspace& ws, cudaStream_t st) {
+             const HoscSaved<T>& sv, T* dS, T* dA, const HoscBwdLayout<T>& l, cudaStream_t st) {
   const int64_t NN = (int64_t)N * N, NK = (int64_t)N * K;
   const bool first = terms & kFirst, motif = terms & kMotif;
-  T* Sa = ws.take<T>((size_t)B * NK);
-  T* Sm = ws.take<T>((size_t)B * NK);
-  float *P = nullptr, *E2 = nullptr, *r = nullptr, *rM = nullptr;
-  T* H = nullptr;
-  if (dA) {
-    P = ws.take<float>((size_t)B * NN);
-    E2 = ws.take<float>((size_t)B * NN);
-    H = ws.take<T>((size_t)B * NN);
-    r = ws.take<float>((size_t)B * N);
-    rM = ws.take<float>((size_t)B * N);
-  }
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  T *Sa = l.Sa, *Sm = l.Sm, *H = l.H;
+  float *P = l.P, *E2 = l.E2, *r = l.r, *rM = l.rM;
   if (B == 0) return TGPB200_OK;
   if (!gl) {  // no upstream gradient: zero
     cudaMemsetAsync(dS, 0, (size_t)B * NK * sizeof(T), st);
@@ -386,17 +387,17 @@ extern "C" {
 
 size_t tgpb200_hosc_loss_saved_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
   if (B < 0 || N < 1 || K < 1) return 0;
-  return saved_bytes(B, N, K, terms, dtype);
+  return hosc_layout_bytes<HoscSaved>(dtype, B, N, K, terms);
 }
 
 size_t tgpb200_hosc_loss_fwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int terms, int dtype) {
   if (B < 0 || N < 1 || K < 1) return 0;
-  return fwd_ws_bytes(B, N, K, terms, dtype);
+  return hosc_layout_bytes<HoscFwdLayout>(dtype, B, N, K, terms);
 }
 
 size_t tgpb200_hosc_loss_bwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int dtype, int need_grad_adj) {
   if (B < 0 || N < 1 || K < 1) return 0;
-  return bwd_ws_bytes(B, N, K, dtype, need_grad_adj != 0);
+  return hosc_layout_bytes<HoscBwdLayout>(dtype, B, N, K, need_grad_adj != 0);
 }
 
 int tgpb200_hosc_loss_fwd(const void* adj, const void* s, const float* graph_nodes, int64_t B, int64_t N, int64_t K,
@@ -405,18 +406,20 @@ int tgpb200_hosc_loss_fwd(const void* adj, const void* s, const float* graph_nod
   int rc = hosc_check(adj, s, B, N, K, dtype, terms);
   if (rc != TGPB200_OK) return rc;
   if (!losses) return TGPB200_ERR_INVALID;
-  Workspace ws(workspace, workspace_bytes);
+  Workspace sw(saved, saved_bytes), ws(workspace, workspace_bytes);
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == TGPB200_F32) {
-    HoscSaved<float> sv(saved, saved_bytes, B, N, K, terms);
-    if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+    const HoscSaved<float> sv(sw, B, N, K, terms);
+    const HoscFwdLayout<float> l(ws, B, N, K, terms);
+    if (!sw.ok || !ws.ok) return TGPB200_ERR_WORKSPACE;
     return hosc_fwd<float>((const float*)adj, (const float*)s, graph_nodes, (int)B, (int)N, (int)K, terms, eps, losses,
-                           sv, ws, st);
+                           sv, l, st);
   }
-  HoscSaved<__nv_bfloat16> sv(saved, saved_bytes, B, N, K, terms);
-  if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+  const HoscSaved<__nv_bfloat16> sv(sw, B, N, K, terms);
+  const HoscFwdLayout<__nv_bfloat16> l(ws, B, N, K, terms);
+  if (!sw.ok || !ws.ok) return TGPB200_ERR_WORKSPACE;
   return hosc_fwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, graph_nodes, (int)B, (int)N,
-                                 (int)K, terms, eps, losses, sv, ws, st);
+                                 (int)K, terms, eps, losses, sv, l, st);
 }
 
 int tgpb200_hosc_loss_bwd(const void* adj, const void* s, const float* graph_nodes, const void* saved,
@@ -426,19 +429,20 @@ int tgpb200_hosc_loss_bwd(const void* adj, const void* s, const float* graph_nod
   int rc = hosc_check(adj, s, B, N, K, dtype, terms);
   if (rc != TGPB200_OK) return rc;
   if (!grad_s) return TGPB200_ERR_INVALID;
-  Workspace ws(workspace, workspace_bytes);
+  Workspace sw(const_cast<void*>(saved), saved_bytes), ws(workspace, workspace_bytes);
   cudaStream_t st = (cudaStream_t)stream;
-  void* sp = const_cast<void*>(saved);
   if (dtype == TGPB200_F32) {
-    HoscSaved<float> sv(sp, saved_bytes, B, N, K, terms);
-    if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+    const HoscSaved<float> sv(sw, B, N, K, terms);
+    const HoscBwdLayout<float> l(ws, B, N, K, grad_adj != nullptr);
+    if (!sw.ok || !ws.ok) return TGPB200_ERR_WORKSPACE;
     return hosc_bwd<float>((const float*)adj, (const float*)s, graph_nodes, grad_losses, (int)B, (int)N, (int)K, terms,
-                           sv, (float*)grad_s, (float*)grad_adj, ws, st);
+                           sv, (float*)grad_s, (float*)grad_adj, l, st);
   }
-  HoscSaved<__nv_bfloat16> sv(sp, saved_bytes, B, N, K, terms);
-  if (!sv.ok) return TGPB200_ERR_WORKSPACE;
+  const HoscSaved<__nv_bfloat16> sv(sw, B, N, K, terms);
+  const HoscBwdLayout<__nv_bfloat16> l(ws, B, N, K, grad_adj != nullptr);
+  if (!sw.ok || !ws.ok) return TGPB200_ERR_WORKSPACE;
   return hosc_bwd<__nv_bfloat16>((const __nv_bfloat16*)adj, (const __nv_bfloat16*)s, graph_nodes, grad_losses, (int)B,
-                                 (int)N, (int)K, terms, sv, (__nv_bfloat16*)grad_s, (__nv_bfloat16*)grad_adj, ws, st);
+                                 (int)N, (int)K, terms, sv, (__nv_bfloat16*)grad_s, (__nv_bfloat16*)grad_adj, l, st);
 }
 
 }  // extern "C"

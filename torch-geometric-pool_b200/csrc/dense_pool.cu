@@ -1189,15 +1189,16 @@ static StripPlan strip_plan(int K, int nvec, int64_t elems_for_512 = 2048) {
   return p;
 }
 
+// The saved buffer, shared by the forward and the backward.  Operand-dtype regions are carved at fp32 width for every
+// dtype: the size query takes no dtype.
 template <typename T>
 struct DensePlan {
   T* Tt;  // T = S^T A  [B, K, N]
   float *Araw, *M, *d, *ss, *a2, *ent, *dvec, *stats, *losses, *link_partial;
   float *dm_c, *dm_e, *dm_st;  // DMoN: c = S^T d, e = S^T 1 [B, K], per-graph terms [B, 8] (k_dmon_stats)
   int32_t* argmax;
-  bool ok;
   DensePlan(Workspace& ws, int64_t B, int64_t N, int64_t K) {
-    Tt = ws.take<T>((size_t)B * N * K);
+    Tt = reinterpret_cast<T*>(ws.take<float>((size_t)B * N * K));
     Araw = ws.take<float>((size_t)B * K * K);
     M = ws.take<float>((size_t)B * K * K);
     d = ws.take<float>((size_t)B * N);
@@ -1212,24 +1213,36 @@ struct DensePlan {
     dm_c = ws.take<float>((size_t)B * K);
     dm_e = ws.take<float>((size_t)B * K);
     dm_st = ws.take<float>((size_t)B * 8);
-    ok = ws.ok;
   }
 };
 
-static size_t dense_saved_bytes(int64_t B, int64_t N, int64_t K) {
-  size_t f = sizeof(float);
-  return align_up((size_t)B * K * N * f) + align_up((size_t)B * K * K * f) * 2 + align_up((size_t)B * N * f) * 4 +
-         align_up((size_t)B * K * f) + align_up((size_t)B * 8 * f) + align_up(8 * f) + align_up((size_t)B * 4) +
-         align_up((size_t)B * ((N + 63) / 64) * ((N + 63) / 64) * f) + align_up((size_t)B * K * f) * 2 +
-         align_up((size_t)B * 8 * f) + 4096;
-}
+// The backward workspace.  U (the product S Graw behind dA) only when the adjacency gradient is asked for; the
+// operand-dtype regions at fp32 width, as in DensePlan.
+template <typename T>
+struct DenseBwdLayout {
+  float *Graw, *P, *coef, *uv, *rvec, *coef_r;
+  T *W, *U, *Gt, *Pt;
+  DenseBwdLayout(Workspace& ws, int64_t B, int64_t N, int64_t K, bool need_grad_adj) {
+    const size_t KK = (size_t)B * K * K, NK = (size_t)B * N * K;
+    Graw = ws.take<float>(KK);
+    P = ws.take<float>(KK);
+    coef = ws.take<float>((size_t)B * 4);
+    W = reinterpret_cast<T*>(ws.take<float>(NK));
+    U = need_grad_adj ? reinterpret_cast<T*>(ws.take<float>(NK)) : nullptr;
+    Gt = reinterpret_cast<T*>(ws.take<float>(KK));  // Graw / P in the operand dtype (bf16 runs)
+    Pt = reinterpret_cast<T*>(ws.take<float>(KK));
+    uv = ws.take<float>((size_t)B * 2 * K);  // DMoN (k_dmon_bwd)
+    rvec = ws.take<float>((size_t)B * N);
+    coef_r = ws.take<float>((size_t)B * 4);
+  }
+};
 
 template <typename T>
 static int dense_fwd(const T* A, const T* S, const T* X, int B, int N, int K, int F, uint32_t flags, int loss_kind,
                      float eps, float link_div, float ent_div, const float* graph_nodes, T* Xpool, T* Apool,
                      float* losses_out, Workspace& saved, cudaStream_t st) {
-  DensePlan<T> pl(saved, B, N, K);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  const DensePlan<T> pl(saved, B, N, K);
+  if (!saved.ok) return TGPB200_ERR_WORKSPACE;
   int rc;
   int64_t NK = (int64_t)N * K, NN = (int64_t)N * N, NF = (int64_t)N * F, KK = (int64_t)K * K, KF = (int64_t)K * F;
   const Mat Smn{S, NK, K, 1};  // S read with the node index as the contraction dim
@@ -1319,20 +1332,12 @@ static int dense_bwd(const T* A, const T* S, const T* X, const T* gXpool, const 
                      int N, int K, int F, uint32_t flags, int loss_kind, float eps, float link_div, float ent_div,
                      const float* graph_nodes, T* dS_out, T* dX_out, T* dA_out, Workspace& saved, Workspace& ws,
                      cudaStream_t st) {
-  DensePlan<T> pl(saved, B, N, K);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  const DensePlan<T> pl(saved, B, N, K);
+  const DenseBwdLayout<T> l(ws, B, N, K, dA_out != nullptr);
+  if (!saved.ok || !ws.ok) return TGPB200_ERR_WORKSPACE;
   int64_t NK = (int64_t)N * K, NN = (int64_t)N * N, NF = (int64_t)N * F, KK = (int64_t)K * K, KF = (int64_t)K * F;
-  float* Graw = ws.take<float>((size_t)B * KK);
-  float* P = ws.take<float>((size_t)B * KK);
-  float* coef = ws.take<float>((size_t)B * 4);
-  T* W = ws.take<T>((size_t)B * NK);
-  T* U = ws.take<T>((size_t)B * NK);
-  T* Gt = ws.take<T>((size_t)B * KK);  // Graw / P in the operand dtype (bf16 runs)
-  T* Pt = ws.take<T>((size_t)B * KK);
-  float* uv = ws.take<float>((size_t)B * 2 * K);  // DMoN (k_dmon_bwd)
-  float* rvec = ws.take<float>((size_t)B * N);
-  float* coef_r = ws.take<float>((size_t)B * 4);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  float *Graw = l.Graw, *P = l.P, *coef = l.coef, *uv = l.uv, *rvec = l.rvec, *coef_r = l.coef_r;
+  T *W = l.W, *U = l.U, *Gt = l.Gt, *Pt = l.Pt;
   int rc;
   if (B == 0) return TGPB200_OK;
   const bool have_a = A != nullptr;
@@ -1441,13 +1446,12 @@ using namespace tgp;
 
 extern "C" {
 
-size_t tgpb200_dense_pool_saved_bytes(int64_t B, int64_t N, int64_t K) { return dense_saved_bytes(B, N, K); }
+size_t tgpb200_dense_pool_saved_bytes(int64_t B, int64_t N, int64_t K) {
+  return layout_bytes<DensePlan<float>>(B, N, K);
+}
 
 size_t tgpb200_dense_pool_bwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int need_grad_adj) {
-  size_t f = sizeof(float);
-  (void)need_grad_adj;
-  return 4 * align_up((size_t)B * K * K * f) + align_up((size_t)B * 4 * f) + 2 * align_up((size_t)B * N * K * f) +
-         align_up((size_t)B * 2 * K * f) + align_up((size_t)B * N * f) + align_up((size_t)B * 4 * f) + 8192;
+  return layout_bytes<DenseBwdLayout<float>>(B, N, K, need_grad_adj != 0);
 }
 
 // Batched product with the shape-general fallback (tensor-core engine when the operand layout satisfies the TMA

@@ -190,8 +190,8 @@ inline size_t scan_workspace_bytes(int64_t n) {
   return align_up(((size_t)ceil_div(n > 0 ? n : 1, kScanTile) + 2) * sizeof(unsigned long long));
 }
 
-// out may alias in.  total32/total64 (device) receive the grand total when non-null.
-inline int exclusive_scan_i32(const int* in, int* out, int64_t n, int* total32, int64_t* total64, Workspace& ws,
+// out may alias in.  total32/total64 (device) receive the grand total when non-null.  ws: scan_workspace_bytes(n).
+inline int exclusive_scan_i32(const int* in, int* out, int64_t n, int* total32, int64_t* total64, Workspace ws,
                               cudaStream_t stream) {
   int nt = (int)ceil_div(n > 0 ? n : 1, kScanTile);
   unsigned long long* state = ws.take<unsigned long long>((size_t)nt + 2);
@@ -265,18 +265,23 @@ inline size_t compact_workspace_bytes(int64_t n) {
   return align_up((size_t)ceil_div(n > 0 ? n : 1, kCompactTile) * sizeof(int));
 }
 
-// Phase 1: per-tile survivor counts -> exclusive tile offsets in `counts`, grand total to total32/total64.
+// Phase 1: per-tile survivor counts -> exclusive tile offsets kept in `ws` (compact_workspace_bytes(n)), grand total
+// to total32/total64.
 template <typename Pred>
-inline int compact_count(Pred pred, int64_t n, int* counts, int* total32, int64_t* total64, cudaStream_t stream) {
+inline int compact_count(Pred pred, int64_t n, Workspace ws, int* total32, int64_t* total64, cudaStream_t stream) {
   int nt = (int)ceil_div(n > 0 ? n : 1, kCompactTile);
+  int* counts = ws.take<int>((size_t)nt);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   launch("k_compact_count", k_compact_count<Pred>, nt, kCompactThreads, 0, stream, pred, n, counts);
   launch("k_scan_spine", k_scan_spine, 1, 1024, 0, stream, counts, nt, total32, total64);
   return launch_status();
 }
-// Phase 2: write survivors (counts must hold the offsets produced by compact_count on the same input).
+// Phase 2: write survivors (ws must be the region compact_count ran on, over the same input).
 template <typename Pred, typename Emit>
-inline int compact_emit(Pred pred, Emit emit, int64_t n, const int* counts, cudaStream_t stream) {
+inline int compact_emit(Pred pred, Emit emit, int64_t n, Workspace ws, cudaStream_t stream) {
   int nt = (int)ceil_div(n > 0 ? n : 1, kCompactTile);
+  const int* counts = ws.take<int>((size_t)nt);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (n > 0) launch("k_compact_emit", k_compact_emit<Pred, Emit>, nt, kCompactThreads, 0, stream, pred, emit, n, counts);
   return launch_status();
 }
@@ -413,7 +418,7 @@ static int compact_onepass_on(Pred pred, Emit emit, int64_t n, int64_t* count_ou
 }
 
 template <typename Pred, typename Emit>
-static int compact_onepass(Pred pred, Emit emit, int64_t n, int64_t* count_out, Workspace& ws, cudaStream_t stream) {
+static int compact_onepass(Pred pred, Emit emit, int64_t n, int64_t* count_out, Workspace ws, cudaStream_t stream) {
   unsigned long long* state = ws.take<unsigned long long>(compact_onepass_state_words(n));
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   return compact_onepass_on(pred, emit, n, count_out, state, false, stream);
@@ -429,7 +434,6 @@ constexpr int kSortThreads = 256;
 #endif
 constexpr int kSortItems = TGPB200_SORT_ITEMS;
 constexpr int kSortTile = kSortThreads * kSortItems;
-constexpr int kSortMaxBins = 2048;  // histogram rows reserved per tile in the workspace (a pass uses kRadixBins)
 
 // Measured on B200 (20 M 39-bit keys): a 10-bit pass costs 1.55x an 8-bit pass (2 KB x 8 warp counters and the staging
 // buffer halve the occupancy), so 4 x 10-bit passes lose to 5 x 8-bit passes.
@@ -568,9 +572,10 @@ constexpr size_t radix_scatter_smem() {
   return (sizeof(KeyT) + 4) * kSortTile + sizeof(int) * (kSortThreads / 32 + 2) * kRadixBins;
 }
 
+// the [bins][tiles] histogram and the scan of it
 inline size_t radix_sort_workspace_bytes(int64_t n) {
   int64_t nt = ceil_div(n > 0 ? n : 1, kSortTile);
-  return align_up((size_t)nt * kSortMaxBins * sizeof(int)) + scan_workspace_bytes(nt * kSortMaxBins);
+  return align_up((size_t)nt * kRadixBins * sizeof(int)) + scan_workspace_bytes(nt * kRadixBins);
 }
 
 // NOTE: internal linkage on purpose.  The kernels above are `static` (one copy per translation unit), so the
@@ -578,7 +583,7 @@ inline size_t radix_sort_workspace_bytes(int64_t n) {
 // across units and leave the other units' kernel copies without the > 48 KB shared-memory opt-in.
 template <typename KeyT>
 static int radix_pass(const KeyT* kin, const uint32_t* vin, KeyT* kout, uint32_t* vout, int64_t n,
-                      const int64_t* n_dev, int shift, int* hist, int nt, Workspace& ws, cudaStream_t stream) {
+                      const int64_t* n_dev, int shift, int* hist, int nt, Workspace scan_ws, cudaStream_t stream) {
   static bool smem_attr_set = false;  // per instantiation: > 48 KB dynamic shared memory needs the opt-in
   if (!smem_attr_set) {
     smem_attr_set = true;
@@ -592,7 +597,7 @@ static int radix_pass(const KeyT* kin, const uint32_t* vin, KeyT* kout, uint32_t
     hist = nullptr;
   } else {
     launch("k_radix_hist", k_radix_hist<KeyT>, nt, kSortThreads, 0, stream, kin, n, n_dev, shift, hist, nt);
-    int rc = exclusive_scan_i32(hist, hist, (int64_t)nt * kRadixBins, nullptr, nullptr, ws, stream);
+    int rc = exclusive_scan_i32(hist, hist, (int64_t)nt * kRadixBins, nullptr, nullptr, scan_ws, stream);
     if (rc != TGPB200_OK) return rc;
   }
   if (vin == nullptr)
@@ -607,24 +612,23 @@ static int radix_pass(const KeyT* kin, const uint32_t* vin, KeyT* kout, uint32_t
 // Sorts n pairs by the low `key_bits` bits of the key (n_dev, when given, is a device-side count <= n: the launch
 // covers the capacity n and tiles past the count do nothing).  The first pass takes the payload as
 // iota when vals0 == nullptr.  Buffers (keys0, vals0) and (keys1, vals1) ping-pong; returns
-// (via *result_in_1) which pair holds the result.  keys0 is overwritten.
+// (via *result_in_1) which pair holds the result.  keys0 is overwritten.  ws: radix_sort_workspace_bytes(n).
 template <typename KeyT>
 static int radix_sort_pairs(KeyT* keys0, uint32_t* vals0_or_null, uint32_t* vals0_buf, KeyT* keys1, uint32_t* vals1,
-                            int64_t n, int key_bits, bool* result_in_1, Workspace& ws, cudaStream_t stream,
+                            int64_t n, int key_bits, bool* result_in_1, Workspace ws, cudaStream_t stream,
                             const int64_t* n_dev = nullptr) {
   int nt = (int)ceil_div(n > 0 ? n : 1, kSortTile);
   const int passes = radix_passes(key_bits);
   int* hist = ws.take<int>((size_t)nt * kRadixBins);
+  const Workspace scan_ws = ws.sub(scan_workspace_bytes((int64_t)nt * kRadixBins));  // every pass scans on it anew
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
-  size_t mark2 = ws.off;
   KeyT* kin = keys0;
   KeyT* kout = keys1;
   const uint32_t* vin = vals0_or_null;
   uint32_t* vout = vals1;
   bool in1 = false;
   for (int p = 0; p < passes; ++p) {
-    ws.off = mark2;
-    int rc = radix_pass<KeyT>(kin, vin, kout, vout, n, n_dev, kRadixBits * p, hist, nt, ws, stream);
+    int rc = radix_pass<KeyT>(kin, vin, kout, vout, n, n_dev, kRadixBits * p, hist, nt, scan_ws, stream);
     if (rc != TGPB200_OK) return rc;
     in1 = !in1;
     KeyT* tk = kin;

@@ -610,10 +610,12 @@ struct BucketPlan {
   int* hoff;
   int64_t* hub_members;
   int* long_list;
-  int* tile_counts;
+  Workspace scan;   // voff (plan call), hoff (count call)
+  Workspace hubs;   // compaction of the hub members
+  Workspace sort;   // the hub edges
+  Workspace tiles;  // compaction of the virtual entries (count / emit calls)
   int64_t V;  // virtual capacity E + N
   int ntiles;
-  bool ok;
   BucketPlan(Workspace& ws, int64_t E, int64_t N, int64_t K) {
     V = E + N;
     ntiles = (int)ceil_div(V > 0 ? V : 1, kBkTile);
@@ -645,8 +647,10 @@ struct BucketPlan {
     hoff = ws.take<int>(n + 1);
     hub_members = ws.take<int64_t>(1);
     long_list = ws.take<int>(e / kBkLongRun + 2);
-    tile_counts = ws.take<int>((size_t)ceil_div(v, kCompactTile) + 1);
-    ok = ws.ok;
+    scan = ws.sub(scan_workspace_bytes(N + 1));
+    hubs = ws.sub(compact_onepass_workspace_bytes(N));
+    sort = ws.sub(radix_sort_workspace_bytes(E));
+    tiles = ws.sub(compact_workspace_bytes((int64_t)v));
   }
 };
 
@@ -657,11 +661,7 @@ using namespace tgp;
 extern "C" {
 
 size_t tgpb200_bucket_coalesce_workspace_bytes(int64_t E, int64_t N, int64_t K) {
-  const size_t n = (size_t)(N > 0 ? N : 1), e = (size_t)(E > 0 ? E : 1), v = n + e;
-  return 8 * align_up((n + 1) * 4) + 256 + 5 * align_up((v / kBkTile + 4) * 4) + align_up((size_t)(K / 32 + 1) * 4) +
-         align_up((size_t)(K > 0 ? K : 1) * 4) + 2 * 256 + 6 * align_up(v * 4) + align_up(e * 4) + 2 * align_up(e * 8) +
-         2 * align_up(e * 4) + align_up((e / kBkLongRun + 2) * 4) + align_up((v / kCompactTile + 2) * 4) +
-         2 * scan_workspace_bytes(N + 1) + radix_sort_workspace_bytes(E) + compact_onepass_workspace_bytes(N) + 8192;
+  return layout_bytes<BucketPlan>(E, N, K);
 }
 
 // Phase 0: virtual layout of the coarse rows.  plan_out (device int64[4]) = {virtual entries, hub edges, hub rows, 0}.
@@ -676,7 +676,7 @@ int tgpb200_bucket_coalesce_plan(const int64_t* row, int64_t E, const int64_t* c
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
   BucketPlan pl(ws, E, N, K);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   cudaMemsetAsync(pl.rs, 0, (size_t)N * 4, st);
   cudaMemsetAsync(pl.re, 0, (size_t)N * 4, st);
   cudaMemsetAsync(pl.hubbits, 0, (size_t)(K / 32 + 1) * 4, st);
@@ -684,7 +684,7 @@ int tgpb200_bucket_coalesce_plan(const int64_t* row, int64_t E, const int64_t* c
   if (E > 0)
     launch("k_fine_row_spans", k_fine_row_spans, (unsigned)ceil_div(ceil_div(E, 4), 256), 256, 0, st, row, E, N, pl.rs, pl.re);
   launch("k_member_cost", k_member_cost, (unsigned)ceil_div(N + 1, 256), 256, 0, st, order, pl.rs, pl.re, N, pl.voff);
-  int rc = exclusive_scan_i32(pl.voff, pl.voff, N + 1, nullptr, reinterpret_cast<int64_t*>(pl.plan), ws, st);
+  int rc = exclusive_scan_i32(pl.voff, pl.voff, N + 1, nullptr, reinterpret_cast<int64_t*>(pl.plan), pl.scan, st);
   if (rc != TGPB200_OK) return rc;
   launch("k_member_rows", k_member_rows, (unsigned)ceil_div(N, 256), 256, 0, st, order, ptr, cluster_index, pl.voff, pl.rs,
          pl.re, N, K, pl.mrowoff, pl.mcrow, pl.hubbits, pl.plan);
@@ -709,7 +709,7 @@ int tgpb200_bucket_coalesce_count(const int64_t* row, const int64_t* col, const 
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
   BucketPlan pl(ws, E, N, K);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (virt_cap < 0 || virt_cap > pl.V) virt_cap = pl.V;
   if (hub_cap < 0 || hub_cap > E) hub_cap = E;
   const bool weighted = edge_weight != nullptr;
@@ -738,15 +738,15 @@ int tgpb200_bucket_coalesce_count(const int64_t* row, const int64_t* col, const 
       HubMemPred pred{order, pl.mcrow, pl.rs, pl.re, pl.hubbits};
       HubMemEmit emit{pl.hm_v, pl.hm_c, pl.hoff};
       cudaMemsetAsync(pl.hoff, 0, (size_t)(N + 1) * sizeof(int), st);
-      int rc = compact_onepass(pred, emit, N, pl.hub_members, ws, st);
+      int rc = compact_onepass(pred, emit, N, pl.hub_members, pl.hubs, st);
       if (rc != TGPB200_OK) return rc;
-      rc = exclusive_scan_i32(pl.hoff, pl.hoff, N + 1, nullptr, pl.hub_count, ws, st);
+      rc = exclusive_scan_i32(pl.hoff, pl.hoff, N + 1, nullptr, pl.hub_count, pl.scan, st);
       if (rc != TGPB200_OK) return rc;
       launch("k_hub_edges", k_hub_edges, (unsigned)ceil_div(hub_cap, 256), 256, 0, st, col, cluster_index, pl.rs, pl.hm_v,
              pl.hm_c, pl.hoff, pl.hub_members, pl.hub_count, N, K, cb, pl.hk0, pl.hv0);
       bool in1 = false;
-      rc = radix_sort_pairs<unsigned long long>(pl.hk0, pl.hv0, pl.hv0, pl.hk1, pl.hv1, hub_cap, 2 * cb, &in1, ws, st,
-                                                pl.hub_count);
+      rc = radix_sort_pairs<unsigned long long>(pl.hk0, pl.hv0, pl.hv0, pl.hk1, pl.hv1, hub_cap, 2 * cb, &in1, pl.sort,
+                                                st, pl.hub_count);
       if (rc != TGPB200_OK) return rc;
       HubRunArgs H;
       H.ks = in1 ? pl.hk1 : pl.hk0, H.perm = in1 ? pl.hv1 : pl.hv0, H.n_dev = pl.hub_count, H.w = edge_weight;
@@ -762,7 +762,7 @@ int tgpb200_bucket_coalesce_count(const int64_t* row, const int64_t* col, const 
     }
   }
   VirtPred vp{pl.t_row};
-  return compact_count(vp, virt_cap, pl.tile_counts, nullptr, count_out, st);
+  return compact_count(vp, virt_cap, pl.tiles, nullptr, count_out, st);
 }
 
 // Phase 2: write the coarse edge list (int64 at the boundary).  edge_slot / run_len / run_aux as in
@@ -777,12 +777,12 @@ int tgpb200_bucket_coalesce_emit(int64_t E, int64_t N, int64_t K, int weighted, 
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
   BucketPlan pl(ws, E, N, K);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (virt_cap < 0 || virt_cap > pl.V) virt_cap = pl.V;
   VirtPred vp{pl.t_row};
   VirtEmit ve{pl.t_row, pl.t_col, pl.t_len, pl.t_w, pl.t_aux, out_row, out_col, weighted ? out_weight : nullptr,
               run_aux, run_len, edge_slot ? pl.tpos2out : nullptr};
-  int rc = compact_emit(vp, ve, virt_cap, pl.tile_counts, st);
+  int rc = compact_emit(vp, ve, virt_cap, pl.tiles, st);
   if (rc != TGPB200_OK) return rc;
   if (edge_slot && E > 0)
     launch("k_slot_fixup", k_slot_fixup, (unsigned)ceil_div(ceil_div(E, 4), 256), 256, 0, st, pl.slot_tmp, pl.tpos2out, E, edge_slot);

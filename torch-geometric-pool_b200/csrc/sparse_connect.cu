@@ -223,18 +223,17 @@ template <typename KeyT>
 struct CoalescePlan {
   KeyT *keys0, *keys1;
   uint32_t *vals0, *vals1;
-  int* tile_counts;
   float* comb;
-  bool ok;
+  Workspace sort, tiles;
   CoalescePlan(Workspace& ws, int64_t E) {
-    size_t n = (size_t)E;
+    size_t n = (size_t)(E > 0 ? E : 1);
     keys0 = ws.take<KeyT>(n);
     keys1 = ws.take<KeyT>(n);
     vals0 = ws.take<uint32_t>(n);
     vals1 = ws.take<uint32_t>(n);
     comb = ws.take<float>(n);
-    tile_counts = ws.take<int>((size_t)ceil_div(E, kCompactTile));
-    ok = ws.ok;
+    sort = ws.sub(radix_sort_workspace_bytes(E));
+    tiles = ws.sub(compact_workspace_bytes(E));
   }
 };
 
@@ -243,17 +242,17 @@ static int remap_coalesce_count_impl(const int64_t* row, const int64_t* col, con
                                      const int64_t* cluster, int64_t N, int64_t K, int op, uint32_t flags, float eps,
                                      int64_t* count_out, Workspace& ws, cudaStream_t st) {
   CoalescePlan<KeyT> pl(ws, E);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   unsigned grid = (unsigned)ceil_div(E, 256);
   const int cb = coarse_col_bits(K);
   launch("k_remap_keys", k_remap_keys<KeyT>, grid, 256, 0, st, row, col, cluster, E, N, K, cb, pl.keys0);
   int bits = 2 * cb;
   bool in1 = false;
-  int rc = radix_sort_pairs<KeyT>(pl.keys0, nullptr, pl.vals0, pl.keys1, pl.vals1, E, bits, &in1, ws, st);
+  int rc = radix_sort_pairs<KeyT>(pl.keys0, nullptr, pl.vals0, pl.keys1, pl.vals1, E, bits, &in1, pl.sort, st);
   if (rc != TGPB200_OK) return rc;
   RunCountPred<KeyT> pred{in1 ? pl.keys1 : pl.keys0, in1 ? pl.vals1 : pl.vals0, w, pl.comb, E, cb, op,
                           (flags & TGPB200_REMOVE_SELF_LOOPS) != 0, eps};
-  return compact_count(pred, E, pl.tile_counts, nullptr, count_out, st);
+  return compact_count(pred, E, pl.tiles, nullptr, count_out, st);
 }
 
 template <typename KeyT>
@@ -261,7 +260,7 @@ static int remap_coalesce_emit_impl(int64_t E, int64_t K, bool weighted, uint32_
                                     int64_t* out_col, float* out_w, int32_t* edge_slot, int32_t* run_len,
                                     Workspace& ws, cudaStream_t st) {
   CoalescePlan<KeyT> pl(ws, E);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   const int cb = coarse_col_bits(K);
   int bits = 2 * cb;
   bool in1 = (radix_passes(bits) & 1) != 0;
@@ -270,7 +269,7 @@ static int remap_coalesce_emit_impl(int64_t E, int64_t K, bool weighted, uint32_
   if (edge_slot) cudaMemsetAsync(edge_slot, 0xff, (size_t)E * sizeof(int32_t), st);
   RunEmitPred<KeyT> pred{ks, weighted ? pl.comb : nullptr, cb, (flags & TGPB200_REMOVE_SELF_LOOPS) != 0, eps};
   RunEmit2<KeyT> emit{ks, perm, E, out_row, out_col, weighted ? out_w : nullptr, run_len, edge_slot};
-  return compact_emit(pred, emit, E, pl.tile_counts, st);
+  return compact_emit(pred, emit, E, pl.tiles, st);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -505,11 +504,26 @@ struct ValOfArray {
   __device__ float operator()(int64_t i) const { return a[i]; }
 };
 
-static size_t det_segment_sum_workspace_bytes(int64_t n, int64_t K) {
-  size_t m = (size_t)(n > 0 ? n : 1);
-  return 6 * align_up(m * sizeof(uint32_t)) + radix_sort_workspace_bytes(n) +
-         2 * align_up((size_t)(K + 1) * sizeof(double)) + align_up((m / kDsTile + 2) * sizeof(double)) + 1024;
-}
+// Scratch of one det_segment_sum of n values into K segments: the run bounds and tile sums of the prefix passes, and
+// for unsorted keys the 32-bit keys, the values in position order and the stable sort that groups them.
+struct DetSumScratch {
+  double *pb, *pe, *tiles;
+  uint32_t *keys0, *keys1, *vals0, *vals1;
+  float* ev;
+  Workspace sort;
+  DetSumScratch(Workspace& ws, int64_t n, int64_t K) {
+    const size_t m = (size_t)(n > 0 ? n : 1);
+    pb = ws.take<double>((size_t)(K > 0 ? K : 0) + 1);
+    pe = ws.take<double>((size_t)(K > 0 ? K : 0) + 1);
+    tiles = ws.take<double>(m / kDsTile + 2);
+    keys0 = ws.take<uint32_t>(m);
+    keys1 = ws.take<uint32_t>(m);
+    vals0 = ws.take<uint32_t>(m);
+    vals1 = ws.take<uint32_t>(m);
+    ev = ws.take<float>(m);
+    sort = ws.sub(radix_sort_workspace_bytes(n));
+  }
+};
 
 // tiles_ready: `tiles` already holds the per-tile sums (a producer kernel with the tile layout of k_dsum_reduce)
 template <typename KeyF, typename ValF>
@@ -532,56 +546,42 @@ struct val_is_costly : std::false_type {};
 template <typename V>
 struct val_is_costly<V, std::void_t<decltype(V::kCostly)>> : std::integral_constant<bool, V::kCostly> {};
 
-// keys0 (32-bit, invalid keys = K) and ev (values in position order) are ready: group by key, then prefix sums.
+// s.keys0 (32-bit, invalid keys = K) and s.ev (values in position order) are ready: group by key, then prefix sums.
 // The values themselves ride through the stable sort as its 32-bit payload: no index payload, no gather afterwards
-// (a random 4-byte gather over 100 M values cost 1.5 ms, as much as two sort passes).  keys0 is overwritten.
-static int grouped_sums_of(uint32_t* keys0, float* ev, int64_t n, const int64_t* n_dev, int64_t K, double* pb, double* pe,
-                           double* tiles, float* out, Workspace& ws, cudaStream_t st) {
-  const size_t m = (size_t)(n > 0 ? n : 1);
-  uint32_t* keys1 = ws.take<uint32_t>(m);
-  uint32_t* vals0 = ws.take<uint32_t>(m);
-  uint32_t* vals1 = ws.take<uint32_t>(m);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+// (a random 4-byte gather over 100 M values cost 1.5 ms, as much as two sort passes).  s.keys0 is overwritten.
+static int grouped_sums_of(const DetSumScratch& s, int64_t n, const int64_t* n_dev, int64_t K, float* out,
+                           cudaStream_t st) {
   bool in1 = false;
-  int rc = radix_sort_pairs<uint32_t>(keys0, reinterpret_cast<uint32_t*>(ev), vals0, keys1, vals1, n,
-                                      key_bits_for_u64((uint64_t)K), &in1, ws, st, n_dev);
+  int rc = radix_sort_pairs<uint32_t>(s.keys0, reinterpret_cast<uint32_t*>(s.ev), s.vals0, s.keys1, s.vals1, n,
+                                      key_bits_for_u64((uint64_t)K), &in1, s.sort, st, n_dev);
   if (rc != TGPB200_OK) return rc;
-  const float* sv = reinterpret_cast<const float*>(in1 ? vals1 : vals0);
-  prefix_run_sums(KeyOfArray32{in1 ? keys1 : keys0}, ValOfArray{sv}, n, n_dev, K, pb, pe, tiles, out, st);
+  const float* sv = reinterpret_cast<const float*>(in1 ? s.vals1 : s.vals0);
+  prefix_run_sums(KeyOfArray32{in1 ? s.keys1 : s.keys0}, ValOfArray{sv}, n, n_dev, K, s.pb, s.pe, s.tiles, out, st);
   return launch_status();
 }
 
+// s: carved for at least n values and K segments.
 template <typename KeyF, typename ValF>
 static int det_segment_sum(KeyF key, ValF val, int64_t n, const int64_t* n_dev, int64_t K, bool keys_sorted, float* out,
-                           Workspace& ws, cudaStream_t st) {
+                           const DetSumScratch& s, cudaStream_t st) {
   if (K <= 0) return TGPB200_OK;
-  const size_t m = (size_t)(n > 0 ? n : 1);
-  double* pb = ws.take<double>((size_t)K + 1);
-  double* pe = ws.take<double>((size_t)K + 1);
-  double* tiles = ws.take<double>(m / kDsTile + 2);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (n <= 0) {
     cudaMemsetAsync(out, 0, (size_t)K * sizeof(float), st);
     return launch_status();
   }
   if (keys_sorted) {
     if constexpr (val_is_costly<ValF>::value) {
-      float* ev = ws.take<float>(m);
-      if (!ws.ok) return TGPB200_ERR_WORKSPACE;
-      launch("k_eval_vals", k_eval_vals<ValF>, (unsigned)ceil_div(n, 256), 256, 0, st, val, n, n_dev, ev);
-      prefix_run_sums(key, ValOfArray{ev}, n, n_dev, K, pb, pe, tiles, out, st);
+      launch("k_eval_vals", k_eval_vals<ValF>, (unsigned)ceil_div(n, 256), 256, 0, st, val, n, n_dev, s.ev);
+      prefix_run_sums(key, ValOfArray{s.ev}, n, n_dev, K, s.pb, s.pe, s.tiles, out, st);
     } else {
-      prefix_run_sums(key, val, n, n_dev, K, pb, pe, tiles, out, st);
+      prefix_run_sums(key, val, n, n_dev, K, s.pb, s.pe, s.tiles, out, st);
     }
     return launch_status();
   }
-  uint32_t* keys0 = ws.take<uint32_t>(m);
-  float* ev = ws.take<float>(m);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   const unsigned grid = (unsigned)ceil_div(n, 256);
-  launch("k_fill_keys32", k_fill_keys32<KeyF>, grid, 256, 0, st, key, n, n_dev, K, keys0);
-  launch("k_eval_vals", k_eval_vals<ValF>, grid, 256, 0, st, val, n, n_dev, ev);
-  return grouped_sums_of(keys0, ev, n, n_dev, K, pb, pe, tiles, out, ws, st);
+  launch("k_fill_keys32", k_fill_keys32<KeyF>, grid, 256, 0, st, key, n, n_dev, K, s.keys0);
+  launch("k_eval_vals", k_eval_vals<ValF>, grid, 256, 0, st, val, n, n_dev, s.ev);
+  return grouped_sums_of(s, n, n_dev, K, out, st);
 }
 
 static __global__ void k_rows_sorted(const int64_t* __restrict__ row, int64_t E, int32_t* __restrict__ sorted_out) {
@@ -699,6 +699,21 @@ static __global__ void k_deg_bwd_apply(const int64_t* __restrict__ row, const in
   gw[e] = gout[e] * dr * dc + gdeg;
 }
 
+// Workspace shared by the edge-normalisation entry points (tgpb200_edge_norm_workspace_bytes(E, K)): the two sides
+// of the degree backward, the sums over the E edges by row and by column, and the weight-norm backward's sum of the
+// per-node values by graph (its K is max(pooled nodes, graphs)).
+struct EdgeNormLayout {
+  float *part_row, *part_col;  // [K]
+  DetSumScratch row, col;      // E values, K segments
+  DetSumScratch nodes;         // K values, K segments
+  EdgeNormLayout(Workspace& ws, int64_t E, int64_t K)
+      : part_row(ws.take<float>((size_t)(K > 0 ? K : 1))),
+        part_col(ws.take<float>((size_t)(K > 0 ? K : 1))),
+        row(ws, E, K),
+        col(ws, E, K),
+        nodes(ws, K, K) {}
+};
+
 static __global__ void k_wn_max(const int64_t* __restrict__ row, const float* __restrict__ w,
                                 const int64_t* __restrict__ batch, int64_t E, const int64_t* __restrict__ E_dev,
                                 int64_t G, float* __restrict__ mx) {
@@ -745,64 +760,9 @@ using namespace tgp;
 
 extern "C" {
 
-size_t tgpb200_filter_relabel_workspace_bytes(int64_t E, int64_t N) {
-  return align_up((size_t)(N > 0 ? N : 1) * sizeof(int32_t)) + align_up((size_t)(N / 32 + 1) * 4) +
-         compact_workspace_bytes(E) + 1024;
-}
-
-struct KeptPlan {
-  int32_t* table;
-  uint32_t* bits;
-  int* tile_counts;
-  bool ok;
-  KeptPlan(Workspace& ws, int64_t E, int64_t N) {
-    table = ws.take<int32_t>((size_t)(N > 0 ? N : 1));
-    bits = ws.take<uint32_t>((size_t)(N / 32 + 1));
-    tile_counts = ws.take<int>((size_t)ceil_div(E > 0 ? E : 1, kCompactTile));
-    ok = ws.ok;
-  }
-};
-
-int tgpb200_filter_relabel_count(const int64_t* row, const int64_t* col, const float* edge_weight, int64_t E,
-                                 const int64_t* node_index, int64_t kept, int64_t N, uint32_t flags, float eps,
-                                 int64_t* count_out, void* workspace, size_t workspace_bytes,
-                                 tgpb200_stream_t stream) {
-  if (E < 0 || kept < 0 || N < 0 || E >= INT32_MAX || N >= INT32_MAX || !count_out) return TGPB200_ERR_INVALID;
-  if (E > 0 && (!row || !col)) return TGPB200_ERR_INVALID;
-  if (kept > 0 && !node_index) return TGPB200_ERR_INVALID;
-  cudaStream_t st = (cudaStream_t)stream;
-  Workspace ws(workspace, workspace_bytes);
-  KeptPlan pl(ws, E, N);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
-  cudaMemsetAsync(pl.table, 0xff, (size_t)(N > 0 ? N : 1) * sizeof(int32_t), st);
-  cudaMemsetAsync(pl.bits, 0, (size_t)(N / 32 + 1) * sizeof(uint32_t), st);
-  if (kept > 0)
-    launch("k_build_table", k_build_table, (unsigned)ceil_div(kept, 256), 256, 0, st, node_index, kept, N, pl.table, pl.bits);
-  KeptPred pred{row, col, edge_weight, pl.table, pl.bits, N, (flags & TGPB200_REMOVE_SELF_LOOPS) != 0, eps};
-  return compact_count(pred, E, pl.tile_counts, nullptr, count_out, st);
-}
-
-int tgpb200_filter_relabel_emit(const int64_t* row, const int64_t* col, const float* edge_weight, int64_t E,
-                                int64_t N, uint32_t flags, float eps, int64_t* out_row, int64_t* out_col,
-                                float* out_weight, int32_t* src_edge, void* workspace, size_t workspace_bytes,
-                                tgpb200_stream_t stream) {
-  if (E < 0 || N < 0 || E >= INT32_MAX) return TGPB200_ERR_INVALID;
-  if (E == 0) return TGPB200_OK;
-  if (!row || !col || !out_row || !out_col) return TGPB200_ERR_INVALID;
-  if (edge_weight && !out_weight) return TGPB200_ERR_INVALID;
-  Workspace ws(workspace, workspace_bytes);
-  KeptPlan pl(ws, E, N);
-  if (!pl.ok) return TGPB200_ERR_WORKSPACE;
-  KeptPred pred{row, col, edge_weight, pl.table, pl.bits, N, (flags & TGPB200_REMOVE_SELF_LOOPS) != 0, eps};
-  KeptEmit emit{out_row, out_col, edge_weight ? out_weight : nullptr, src_edge};
-  return compact_emit(pred, emit, E, pl.tile_counts, (cudaStream_t)stream);
-}
-
 size_t tgpb200_remap_coalesce_workspace_bytes(int64_t E, int64_t K) {
-  (void)K;
-  size_t n = (size_t)(E > 0 ? E : 1);
-  return 2 * align_up(n * 8) + 7 * align_up((n + 1) * 4) + radix_sort_workspace_bytes(E) + scan_workspace_bytes(E) +
-         compact_workspace_bytes(E) + 4096;
+  if (2 * coarse_col_bits(K) <= 32) return layout_bytes<CoalescePlan<uint32_t>>(E);
+  return layout_bytes<CoalescePlan<uint64_t>>(E);
 }
 
 int tgpb200_remap_coalesce_count(const int64_t* row, const int64_t* col, const float* edge_weight, int64_t E,
@@ -840,10 +800,19 @@ int tgpb200_remap_coalesce_emit(int64_t E, int64_t K, int weighted, uint32_t fla
                                             run_len, ws, st);
 }
 
-size_t tgpb200_filter_relabel_onepass_workspace_bytes(int64_t E, int64_t N) {
-  return align_up((size_t)(N > 0 ? N : 1) * sizeof(int32_t)) + align_up((size_t)(N / 32 + 1) * 4) +
-         compact_onepass_workspace_bytes(E) + 1024;
-}
+// Workspace of tgpb200_filter_relabel_onepass: the relabel table, the kept-node bits and the compaction's tile states.
+struct KeptLayout {
+  int32_t* table;
+  uint32_t* bits;
+  unsigned long long* state;
+  KeptLayout(Workspace& ws, int64_t E, int64_t N) {
+    table = ws.take<int32_t>((size_t)(N > 0 ? N : 1));
+    bits = ws.take<uint32_t>((size_t)(N / 32 + 1));
+    state = ws.take<unsigned long long>(compact_onepass_state_words(E));
+  }
+};
+
+size_t tgpb200_filter_relabel_onepass_workspace_bytes(int64_t E, int64_t N) { return layout_bytes<KeptLayout>(E, N); }
 
 // Single-pass form: the edge list is read once; outputs have capacity E and *count_out gets the survivor count.
 int tgpb200_filter_relabel_onepass(const int64_t* row, const int64_t* col, const float* edge_weight, int64_t E,
@@ -857,12 +826,12 @@ int tgpb200_filter_relabel_onepass(const int64_t* row, const int64_t* col, const
   if (kept > 0 && !node_index) return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
-  int32_t* table = ws.take<int32_t>((size_t)(N > 0 ? N : 1));
-  uint32_t* bits = ws.take<uint32_t>((size_t)(N / 32 + 1));
+  const KeptLayout l(ws, E, N);
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  int32_t* table = l.table;
+  uint32_t* bits = l.bits;
+  unsigned long long* state = l.state;
   const size_t state_words = compact_onepass_state_words(E);
-  unsigned long long* state = ws.take<unsigned long long>(state_words);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   const bool small = N <= kSmallNodes && kept <= kSmallNodes && state_words <= 4096;
   if (small) {
     launch("k_kept_init_small", k_kept_init_small, 1, kSmallThreads, 0, st, node_index, (int)kept, (int)N, table, bits, state,
@@ -911,10 +880,17 @@ int tgpb200_filter_relabel_bwd(const float* grad_out, const int32_t* src_edge, i
   return launch_status();
 }
 
+// Workspace of tgpb200_coalesce_bwd: the tie counts of MAX / MIN runs (the other ops need none).
+struct CoalesceBwdLayout {
+  int* ties;
+  CoalesceBwdLayout(Workspace& ws, int64_t num_out, int op) {
+    ties = (op == TGPB200_MAX || op == TGPB200_MIN) ? ws.take<int>((size_t)(num_out > 0 ? num_out : 1)) : nullptr;
+  }
+};
+
 size_t tgpb200_coalesce_bwd_workspace_bytes(int64_t E, int64_t num_out, int op) {
   (void)E;
-  if (op == TGPB200_MAX || op == TGPB200_MIN) return align_up((size_t)(num_out > 0 ? num_out : 1) * sizeof(int)) + 256;
-  return 256;
+  return layout_bytes<CoalesceBwdLayout>(num_out, op);
 }
 
 int tgpb200_coalesce_bwd(const float* edge_weight, const float* out_weight, const float* grad_out,
@@ -928,11 +904,11 @@ int tgpb200_coalesce_bwd(const float* edge_weight, const float* out_weight, cons
   if (op >= TGPB200_MAX && (!edge_weight || !out_weight)) return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
-  int* ties = nullptr;
+  const CoalesceBwdLayout l(ws, num_out, op);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  int* ties = l.ties;
   unsigned grid = (unsigned)ceil_div(E, 256);
-  if (op == TGPB200_MAX || op == TGPB200_MIN) {
-    ties = ws.take<int>((size_t)(num_out > 0 ? num_out : 1));
-    if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  if (ties) {
     cudaMemsetAsync(ties, 0, (size_t)(num_out > 0 ? num_out : 1) * sizeof(int), st);
     launch("k_coalesce_ties", k_coalesce_ties, grid, 256, 0, st, edge_weight, out_weight, edge_slot, E, ties);
   }
@@ -950,11 +926,7 @@ int tgpb200_coalesce_bwd(const float* edge_weight, const float* out_weight, cons
   return launch_status();
 }
 
-size_t tgpb200_edge_norm_workspace_bytes(int64_t E, int64_t K) {
-  // two segmented sums (row side, column side) + two [K] partial vectors
-  return 2 * det_segment_sum_workspace_bytes(E, K) + 3 * align_up((size_t)(K > 0 ? K : 1) * sizeof(float)) +
-         det_segment_sum_workspace_bytes(K, K) + 1024;
-}
+size_t tgpb200_edge_norm_workspace_bytes(int64_t E, int64_t K) { return layout_bytes<EdgeNormLayout>(E, K); }
 
 int tgpb200_rows_sorted(const int64_t* row, int64_t E, int32_t* sorted_out, tgpb200_stream_t stream) {
   if (E < 0 || !sorted_out) return TGPB200_ERR_INVALID;
@@ -975,7 +947,9 @@ int tgpb200_degree_accumulate(const int64_t* row, const float* w, int64_t E, con
   if (K == 0) return TGPB200_OK;
   if (!deg || (E > 0 && !row)) return TGPB200_ERR_INVALID;
   Workspace ws(workspace, workspace_bytes);
-  return det_segment_sum(KeyOfArray64{row}, DegVal{w}, E, E_dev, K, rows_sorted != 0, deg, ws, (cudaStream_t)stream);
+  const EdgeNormLayout l(ws, E, K);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  return det_segment_sum(KeyOfArray64{row}, DegVal{w}, E, E_dev, K, rows_sorted != 0, deg, l.row, (cudaStream_t)stream);
 }
 
 int tgpb200_degree_apply(const int64_t* row, const int64_t* col, const float* w, const float* deg, int64_t E,
@@ -1005,34 +979,27 @@ int tgpb200_degree_bwd_accumulate(const int64_t* row, const int64_t* col, const 
   if (!grad_dinv || (E > 0 && (!row || !col || !deg || !grad_out))) return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
-  float* part_row = ws.take<float>((size_t)K);
-  float* part_col = ws.take<float>((size_t)K);
+  const EdgeNormLayout l(ws, E, K);
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   int rc;
   if (rows_sorted && E > 0) {
-    const size_t m = (size_t)E;
-    double* pb = ws.take<double>((size_t)K + 1);
-    double* pe = ws.take<double>((size_t)K + 1);
-    double* tiles = ws.take<double>(m / kDsTile + 2);
-    float* ev_row = ws.take<float>(m);
-    float* ev_col = ws.take<float>(m);
-    uint32_t* keys0 = ws.take<uint32_t>(m);
-    if (!ws.ok) return TGPB200_ERR_WORKSPACE;
     launch("k_deg_bwd_prepare", k_deg_bwd_prepare, (unsigned)ceil_div(E, kDsTile), kDsThreads, 0, st, row, col, w, deg,
-           grad_out, E, E_dev, K, eps, ev_row, ev_col, keys0, tiles);
-    prefix_run_sums(KeyOfArray64{row}, ValOfArray{ev_row}, E, E_dev, K, pb, pe, tiles, part_row, st, true);
-    // the column side is a scatter by `col`: grouped through the stable sort (pb / pe / tiles are reused in stream order)
-    rc = grouped_sums_of(keys0, ev_col, E, E_dev, K, pb, pe, tiles, part_col, ws, st);
+           grad_out, E, E_dev, K, eps, l.row.ev, l.col.ev, l.col.keys0, l.row.tiles);
+    prefix_run_sums(KeyOfArray64{row}, ValOfArray{l.row.ev}, E, E_dev, K, l.row.pb, l.row.pe, l.row.tiles, l.part_row,
+                    st, true);
+    // the column side is a scatter by `col`: grouped through the stable sort
+    rc = grouped_sums_of(l.col, E, E_dev, K, l.part_col, st);
     if (rc != TGPB200_OK) return rc;
   } else {
     rc = det_segment_sum(KeyOfArray64{row}, DegBwdVal{col, w, deg, grad_out, K, eps}, E, E_dev, K, rows_sorted != 0,
-                         part_row, ws, st);
+                         l.part_row, l.row, st);
     if (rc != TGPB200_OK) return rc;
     // the column side is a scatter by `col`: always grouped through the stable sort
-    rc = det_segment_sum(KeyOfArray64{col}, DegBwdVal{row, w, deg, grad_out, K, eps}, E, E_dev, K, false, part_col, ws, st);
+    rc = det_segment_sum(KeyOfArray64{col}, DegBwdVal{row, w, deg, grad_out, K, eps}, E, E_dev, K, false, l.part_col,
+                         l.col, st);
     if (rc != TGPB200_OK) return rc;
   }
-  launch("k_add_vec", k_add_vec, (unsigned)ceil_div(K, 256), 256, 0, st, part_row, part_col, K, grad_dinv);
+  launch("k_add_vec", k_add_vec, (unsigned)ceil_div(K, 256), 256, 0, st, l.part_row, l.part_col, K, grad_dinv);
   return launch_status();
 }
 
@@ -1113,11 +1080,12 @@ int tgpb200_weight_norm_bwd(const int64_t* row, const float* w, const int64_t* b
     return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
-  float* node_acc = ws.take<float>((size_t)(K > 0 ? K : 1));
+  const EdgeNormLayout l(ws, E, K > G ? K : G);  // the query's K covers both the pooled nodes and the graphs
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
-  int rc = det_segment_sum(KeyOfArray64{row}, ProdVal{grad_out, w}, E, E_dev, K, rows_sorted != 0, node_acc, ws, st);
+  float* node_acc = l.part_row;
+  int rc = det_segment_sum(KeyOfArray64{row}, ProdVal{grad_out, w}, E, E_dev, K, rows_sorted != 0, node_acc, l.row, st);
   if (rc != TGPB200_OK) return rc;
-  rc = det_segment_sum(KeyOfArray64{batch_pooled}, ArrVal{node_acc}, K, nullptr, G, false, graph_acc, ws, st);
+  rc = det_segment_sum(KeyOfArray64{batch_pooled}, ArrVal{node_acc}, K, nullptr, G, false, graph_acc, l.nodes, st);
   if (rc != TGPB200_OK) return rc;
   launch("k_wn_bwd_apply", k_wn_bwd_apply, (unsigned)ceil_div(E, 256), 256, 0, st, row, w, batch_pooled, max_in, arg_in,
          grad_out, graph_acc, E, E_dev, G, grad_w);

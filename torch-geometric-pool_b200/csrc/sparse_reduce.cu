@@ -559,16 +559,40 @@ static int launch_fwd(const void* x, const int64_t* node_index, const float* wei
   return launch_status();
 }
 
+// Workspace of tgpb200_build_csr: the sort keys, the payload buffer that is not `order`, the sort and the scan of ptr.
+struct CsrLayout {
+  uint32_t *keys0, *keys1, *valsA;
+  Workspace sort, scan;
+  CsrLayout(Workspace& ws, int64_t nnz, int64_t K) {
+    const size_t n = (size_t)(nnz > 0 ? nnz : 1);
+    keys0 = ws.take<uint32_t>(n);
+    keys1 = ws.take<uint32_t>(n);
+    valsA = ws.take<uint32_t>(n);
+    sort = ws.sub(radix_sort_workspace_bytes(nnz));
+    scan = ws.sub(scan_workspace_bytes(K + 1));
+  }
+};
+
+// Workspace of tgpb200_segment_reduce_bwd: node -> first entry, and the tie counts of MAX / MIN.
+struct ReduceBwdLayout {
+  int32_t* first;
+  float* inv_ties;
+  ReduceBwdLayout(Workspace& ws, int64_t N, int64_t K, int64_t F, int op) {
+    first = ws.take<int32_t>((size_t)(N > 0 ? N : 1));
+    inv_ties = (op == TGPB200_MAX || op == TGPB200_MIN) ? ws.take<float>((size_t)(K * F > 0 ? K * F : 1)) : nullptr;
+  }
+};
+
 template <typename XT, typename OT>
 static int launch_bwd(const void* x, const int64_t* node_index, const int64_t* cluster_index, const float* weight,
                       const int32_t* order, const int32_t* ptr, const void* pool, const void* gpool, int64_t N,
-                      int64_t nnz, int64_t K, int64_t F, int op, void* gx, float* gw, Workspace& ws, cudaStream_t st) {
+                      int64_t nnz, int64_t K, int64_t F, int op, void* gx, float* gw, const ReduceBwdLayout& l,
+                      cudaStream_t st) {
   constexpr int W = Vec<XT>::N;
   const bool minmax = op == TGPB200_MAX || op == TGPB200_MIN;
   bool vec = (F % W == 0) && Vec<OT>::N == W && aligned16(x) && aligned16(gpool) && aligned16(gx) &&
              (!minmax || aligned16(pool));
-  int32_t* first = ws.take<int32_t>((size_t)(N > 0 ? N : 1));
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  int32_t* first = l.first;
   if (N > 0 && N <= 32768 && nnz <= 32768) {
     first = nullptr;  // the backward kernels search the (cache-resident) sorted node_index themselves: one launch less
   } else {
@@ -576,10 +600,8 @@ static int launch_bwd(const void* x, const int64_t* node_index, const int64_t* c
     if (nnz > 0)
       launch("k_first_entry", k_first_entry, (unsigned)ceil_div(nnz, 256), 256, 0, st, node_index, nnz, N, first);
   }
-  float* inv_ties = nullptr;
+  float* inv_ties = l.inv_ties;
   if (minmax) {
-    inv_ties = ws.take<float>((size_t)K * F);
-    if (!ws.ok) return TGPB200_ERR_WORKSPACE;
     if (K * F > 0)
       launch("k_count_ties", k_count_ties<XT, OT>, (unsigned)ceil_div(K * F, 256), 256, 0, st, (const XT*)x, node_index, weight, order, ptr,
                                                                           (const OT*)pool, N, K, F, inv_ties);
@@ -617,42 +639,37 @@ using namespace tgp;
 
 extern "C" {
 
-int tgpb200_abi_version(void) { return 1; }
+int tgpb200_abi_version(void) { return 2; }
 
-size_t tgpb200_build_csr_workspace_bytes(int64_t nnz, int64_t K) {
-  size_t n = (size_t)(nnz > 0 ? nnz : 1);
-  return 4 * align_up(n * sizeof(uint32_t)) + radix_sort_workspace_bytes(nnz) + scan_workspace_bytes(K + 1) + 1024;
-}
+size_t tgpb200_build_csr_workspace_bytes(int64_t nnz, int64_t K) { return layout_bytes<CsrLayout>(nnz, K); }
 
 int tgpb200_build_csr(const int64_t* cluster_index, int64_t nnz, int64_t K, int32_t* order, int32_t* ptr,
                       void* workspace, size_t workspace_bytes, tgpb200_stream_t stream) {
   if (nnz < 0 || K < 0 || nnz >= INT32_MAX || K >= INT32_MAX || !ptr || (nnz > 0 && (!cluster_index || !order)))
     return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
-  Workspace ws(workspace, workspace_bytes);
-  size_t n = (size_t)(nnz > 0 ? nnz : 1);
-  uint32_t* keys0 = ws.take<uint32_t>(n);
-  uint32_t* keys1 = ws.take<uint32_t>(n);
-  uint32_t* valsA = ws.take<uint32_t>(n);
-  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (nnz > 0 && K == 0) return TGPB200_ERR_INVALID;
+  Workspace ws(workspace, workspace_bytes);
+  const CsrLayout l(ws, nnz, K);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (nnz <= kCsrSmallNnz && K <= kCsrSmallK) {
     launch("k_build_csr_small", k_build_csr_small, 1, kCsrSmallThreads, 0, st, cluster_index, (int)nnz, (int)K, order, ptr);
     return launch_status();
   }
   cudaMemsetAsync(ptr, 0, (size_t)(K + 1) * sizeof(int32_t), st);
   if (nnz > 0) {
-    launch("k_cluster_keys_count", k_cluster_keys_count, (unsigned)ceil_div(nnz, 256), 256, 0, st, cluster_index, nnz, K, keys0, ptr);
+    launch("k_cluster_keys_count", k_cluster_keys_count, (unsigned)ceil_div(nnz, 256), 256, 0, st, cluster_index, nnz, K,
+           l.keys0, ptr);
     int bits = key_bits_for(K - 1);
     int passes = radix_passes(bits);
     // choose buffers so the final payload lands in `order`
-    uint32_t* vals1 = (passes & 1) ? (uint32_t*)order : valsA;
-    uint32_t* vals0 = (passes & 1) ? valsA : (uint32_t*)order;
+    uint32_t* vals1 = (passes & 1) ? (uint32_t*)order : l.valsA;
+    uint32_t* vals0 = (passes & 1) ? l.valsA : (uint32_t*)order;
     bool in1 = false;
-    int rc = radix_sort_pairs<uint32_t>(keys0, nullptr, vals0, keys1, vals1, nnz, bits, &in1, ws, st);
+    int rc = radix_sort_pairs<uint32_t>(l.keys0, nullptr, vals0, l.keys1, vals1, nnz, bits, &in1, l.sort, st);
     if (rc != TGPB200_OK) return rc;
   }
-  int rc = exclusive_scan_i32(ptr, ptr, K + 1, nullptr, nullptr, ws, st);
+  int rc = exclusive_scan_i32(ptr, ptr, K + 1, nullptr, nullptr, l.scan, st);
   return rc != TGPB200_OK ? rc : launch_status();
 }
 
@@ -674,9 +691,7 @@ int tgpb200_segment_reduce_fwd(const void* x, const int64_t* node_index, const f
 
 size_t tgpb200_segment_reduce_bwd_workspace_bytes(int64_t N, int64_t nnz, int64_t K, int64_t F, int op) {
   (void)nnz;
-  size_t b = align_up((size_t)(N > 0 ? N : 1) * sizeof(int32_t)) + 256;  // node -> first entry
-  if (op == TGPB200_MAX || op == TGPB200_MIN) b += align_up((size_t)(K * F > 0 ? K * F : 1) * sizeof(float));
-  return b;
+  return layout_bytes<ReduceBwdLayout>(N, K, F, op);
 }
 
 int tgpb200_segment_reduce_bwd(const void* x, const int64_t* node_index, const int64_t* cluster_index,
@@ -691,12 +706,14 @@ int tgpb200_segment_reduce_bwd(const void* x, const int64_t* node_index, const i
   if ((op == TGPB200_MAX || op == TGPB200_MIN) && (!x_pool || !order)) return TGPB200_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
   Workspace ws(workspace, workspace_bytes);
+  const ReduceBwdLayout l(ws, N, K, F, op);
+  if (!ws.ok) return TGPB200_ERR_WORKSPACE;
   if (x_dtype == TGPB200_F32 && out_dtype == TGPB200_F32)
     return launch_bwd<float, float>(x, node_index, cluster_index, weight, order, ptr, x_pool, grad_pool, N, nnz, K, F,
-                                    op, grad_x, grad_weight, ws, st);
+                                    op, grad_x, grad_weight, l, st);
   if (x_dtype == TGPB200_BF16 && out_dtype == TGPB200_BF16)
     return launch_bwd<__nv_bfloat16, __nv_bfloat16>(x, node_index, cluster_index, weight, order, ptr, x_pool, grad_pool,
-                                                    N, nnz, K, F, op, grad_x, grad_weight, ws, st);
+                                                    N, nnz, K, F, op, grad_x, grad_weight, l, st);
   return TGPB200_ERR_UNSUPPORTED;
 }
 

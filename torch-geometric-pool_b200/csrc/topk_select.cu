@@ -76,17 +76,36 @@ struct NodeEmit {
   }
 };
 
+// Workspace of tgpb200_topk_select: the (graph, score) sort, the selection ranks, the graph offsets with their scan,
+// and the two compactions (rank -> selected, selected -> outputs).
+struct TopkLayout {
+  uint64_t *keys0, *keys1;
+  uint32_t *vals0, *vals1;
+  int* sel_rank;
+  int* ptr;
+  Workspace sort, scan, tiles1, tiles2;
+  TopkLayout(Workspace& ws, int64_t N, int64_t G) {
+    const size_t n = (size_t)(N > 0 ? N : 1);
+    keys0 = ws.take<uint64_t>(n);
+    keys1 = ws.take<uint64_t>(n);
+    vals0 = ws.take<uint32_t>(n);
+    vals1 = ws.take<uint32_t>(n);
+    sel_rank = ws.take<int>(n);
+    ptr = ws.take<int>((size_t)(G > 0 ? G : 0) + 2);
+    sort = ws.sub(radix_sort_workspace_bytes(N));
+    scan = ws.sub(scan_workspace_bytes(G + 1));
+    tiles1 = ws.sub(compact_workspace_bytes(N));
+    tiles2 = ws.sub(compact_workspace_bytes(N));
+  }
+};
+
 }  // namespace tgp
 
 using namespace tgp;
 
 extern "C" {
 
-size_t tgpb200_topk_select_workspace_bytes(int64_t N, int64_t G) {
-  size_t n = (size_t)(N > 0 ? N : 1);
-  return 2 * align_up(n * 8) + 3 * align_up(n * 4) + align_up((size_t)(G + 2) * 4) + radix_sort_workspace_bytes(N) +
-         scan_workspace_bytes(G + 1) + 2 * compact_workspace_bytes(N) + 4096;
-}
+size_t tgpb200_topk_select_workspace_bytes(int64_t N, int64_t G) { return layout_bytes<TopkLayout>(N, G); }
 
 int tgpb200_topk_select(const float* score, const int64_t* batch, int64_t N, int64_t G, float ratio,
                         int64_t* node_index, int64_t* cluster_index, int64_t* count_out, void* workspace,
@@ -99,39 +118,36 @@ int tgpb200_topk_select(const float* score, const int64_t* batch, int64_t N, int
   }
   if (!score || !node_index || !cluster_index) return TGPB200_ERR_INVALID;
   Workspace ws(workspace, workspace_bytes);
-  size_t n = (size_t)N;
-  uint64_t* keys0 = ws.take<uint64_t>(n);
-  uint64_t* keys1 = ws.take<uint64_t>(n);
-  uint32_t* vals0 = ws.take<uint32_t>(n);
-  uint32_t* vals1 = ws.take<uint32_t>(n);
-  int* sel_rank = ws.take<int>(n);
-  int* ptr = ws.take<int>((size_t)G + 2);
-  int* tiles1 = ws.take<int>((size_t)ceil_div(N, kCompactTile));
-  int* tiles2 = ws.take<int>((size_t)ceil_div(N, kCompactTile));
+  const TopkLayout l(ws, N, G);
   if (!ws.ok) return TGPB200_ERR_WORKSPACE;
+  const size_t n = (size_t)N;
+  uint64_t *keys0 = l.keys0, *keys1 = l.keys1;
+  uint32_t *vals0 = l.vals0, *vals1 = l.vals1;
+  int* sel_rank = l.sel_rank;
+  int* ptr = l.ptr;
   unsigned grid = (unsigned)ceil_div(N, 256);
   cudaMemsetAsync(ptr, 0, (size_t)(G + 1) * sizeof(int), st);
   launch("k_topk_count", k_topk_count, grid, 256, 0, st, batch, N, G, ptr);
-  int rc = exclusive_scan_i32(ptr, ptr, G + 1, nullptr, nullptr, ws, st);
+  int rc = exclusive_scan_i32(ptr, ptr, G + 1, nullptr, nullptr, l.scan, st);
   if (rc) return rc;
   launch("k_topk_keys", k_topk_keys, grid, 256, 0, st, score, batch, N, G, keys0);
   int gbits = 0;
   while (((int64_t)1 << gbits) < G) ++gbits;
   bool in1 = false;
-  rc = radix_sort_pairs<uint64_t>(keys0, nullptr, vals0, keys1, vals1, N, 32 + gbits, &in1, ws, st);
+  rc = radix_sort_pairs<uint64_t>(keys0, nullptr, vals0, keys1, vals1, N, 32 + gbits, &in1, l.sort, st);
   if (rc) return rc;
   cudaMemsetAsync(sel_rank, 0xff, n * sizeof(int), st);
   RankPred rp{in1 ? keys1 : keys0, in1 ? vals1 : vals0, ptr, ratio};
   RankEmit re{sel_rank};
-  rc = compact_count(rp, N, tiles1, nullptr, nullptr, st);
+  rc = compact_count(rp, N, l.tiles1, nullptr, nullptr, st);
   if (rc) return rc;
-  rc = compact_emit(rp, re, N, tiles1, st);
+  rc = compact_emit(rp, re, N, l.tiles1, st);
   if (rc) return rc;
   NodePred np{sel_rank};
   NodeEmit ne{node_index, cluster_index};
-  rc = compact_count(np, N, tiles2, nullptr, count_out, st);
+  rc = compact_count(np, N, l.tiles2, nullptr, count_out, st);
   if (rc) return rc;
-  return compact_emit(np, ne, N, tiles2, st);
+  return compact_emit(np, ne, N, l.tiles2, st);
 }
 
 }  // extern "C"

@@ -40,9 +40,6 @@ SIGNATURES = {
         [_P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _INT, _INT, _INT, _P, _P, _P, _SZ, _P],
     ),
     "tgpb200_reduce_batch": (_INT, [_P, _P, _P, _P, _I64, _P, _P]),
-    "tgpb200_filter_relabel_workspace_bytes": (_SZ, [_I64, _I64]),
-    "tgpb200_filter_relabel_count": (_INT, [_P, _P, _P, _I64, _P, _I64, _I64, _U32, _F, _P, _P, _SZ, _P]),
-    "tgpb200_filter_relabel_emit": (_INT, [_P, _P, _P, _I64, _I64, _U32, _F, _P, _P, _P, _P, _P, _SZ, _P]),
     "tgpb200_filter_relabel_onepass_workspace_bytes": (_SZ, [_I64, _I64]),
     "tgpb200_filter_relabel_onepass": (_INT, [_P, _P, _P, _I64, _P, _I64, _I64, _U32, _F, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "tgpb200_filter_relabel_bwd": (_INT, [_P, _P, _I64, _P, _I64, _P, _P]),
@@ -79,6 +76,7 @@ SIGNATURES = {
     "tgpb200_block_diag_count": (_INT, [_P, _P, _I64, _I64, _INT, _F, _P, _P, _P, _SZ, _P]),
     "tgpb200_block_diag_emit": (_INT, [_P, _P, _I64, _I64, _INT, _F, _P, _P, _P, _P, _P, _SZ, _P]),
     "tgpb200_block_diag_bwd": (_INT, [_P, _P, _I64, _I64, _INT, _P, _P]),
+    "tgpb200_graph_ptr_workspace_bytes": (_SZ, [_I64]),
     "tgpb200_graph_ptr": (_INT, [_P, _I64, _I64, _P, _P, _SZ, _P]),
     "tgpb200_to_dense_batch": (_INT, [_P, _P, _P, _I64, _I64, _I64, _I64, _INT, _P, _P, _P]),
     "tgpb200_to_dense_adj": (_INT, [_P, _P, _P, _P, _P, _I64, _I64, _I64, _INT, _P, _P]),

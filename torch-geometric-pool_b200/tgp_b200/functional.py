@@ -460,7 +460,7 @@ def finalize_sparse_output(x_pool: Tensor, adj_pool: Tensor, batch: Optional[Ten
 
 def graph_ptr(batch: Tensor, num_graphs: int) -> Tensor:
     ptr = torch.empty(num_graphs + 1, dtype=torch.int32, device=batch.device)
-    ws = L.workspace(4096 + 4 * (num_graphs + 2), batch.device)
+    ws = L.workspace(L.load().tgpb200_graph_ptr_workspace_bytes(num_graphs), batch.device)
     L.call("tgpb200_graph_ptr", L.ptr(batch.contiguous()), batch.numel(), num_graphs, L.ptr(ptr), L.ptr(ws), ws.numel(),
            L.stream())
     return ptr
