@@ -331,16 +331,22 @@ static __global__ void k_coalesce_bwd(const float* __restrict__ w, const float* 
 // Deterministic segmented sums (degree / normalisation partials): no floating-point atomics.
 //   out[k] = sum of val(i) over the positions i with key(i) == k, k in [0, K)
 // For a non-decreasing key sequence (coarse edge lists are row-sorted: the cluster path sorts them, the kept-node
-// path keeps the order of a row-sorted input) the sum of a key's run is the difference of two values of ONE
-// running prefix sum over all positions, carried in double precision with a fixed reduce-then-scan structure
-// (tile sums -> sequential spine -> tile down-sweep): bitwise reproducible, perfectly load-balanced whatever the
-// run lengths (a power-law hub row is just a long run), and accurate to ~1e-16 of the total, i.e. far below the
-// fp32 rounding of the result.  Other key sequences are first grouped with the stable radix sort.
+// path keeps the order of a row-sorted input) a key's positions form one run, and a SEGMENTED scan in double
+// precision sums every run on its own: a position starts a segment where its key differs from the one before, and
+// the running sum restarts there.  Fixed reduce-then-scan structure (tile summaries -> sequential spine -> tile
+// down-sweep): bitwise reproducible, perfectly load-balanced whatever the run lengths (a power-law hub row is just a
+// long run), and every partial sum holds values of one run only, so the error of out[k] is bounded by its own
+// sum of |values| (|err| <= ~n_k 2^-53 sum|values| before the final rounding to fp32), whatever precedes it in the
+// sequence.  Other key sequences are first grouped with the stable radix sort.
 // `n_dev`, when given, is the device-side element count (<= the launch capacity n).
+//
+// (flag, value) pairs combine as  a . b = (a.f | b.f, b.f ? b.v : a.v + b.v): the flag says that a segment starts
+// inside the span, the value is the sum from the span's last segment start (or from its beginning) to its end.
 // ------------------------------------------------------------------------------------------
 constexpr int kDsThreads = 256;
 constexpr int kDsItems = 8;
 constexpr int kDsTile = kDsThreads * kDsItems;
+constexpr int kDsWarps = kDsThreads / 32;
 
 struct KeyOfArray64 {
   const int64_t* k;
@@ -351,134 +357,196 @@ struct KeyOfArray32 {
   __device__ int64_t operator()(int64_t i) const { return (int64_t)k[i]; }
 };
 
-// exclusive scan of one double per thread over the block (fixed shape); *total = block sum
-__device__ __forceinline__ double block_exclusive_scan_d(double v, double* smem /* >= 33 */, double* total) {
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  double inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    double t = __shfl_up_sync(kFull, inc, o);
-    if (lane >= o) inc += t;
-  }
-  __syncthreads();
-  if (lane == 31) smem[w] = inc;
-  __syncthreads();
-  if (w == 0) {
-    double s = lane < nw ? smem[lane] : 0.0;
-    double si = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      double t = __shfl_up_sync(kFull, si, o);
-      if (lane >= o) si += t;
-    }
-    smem[lane] = si - s;
-    if (lane == 31) smem[32] = si;
-  }
-  __syncthreads();
-  if (total) *total = smem[32];
-  return smem[w] + inc - v;
+// key at position i, -1 when i is past the end or the key is outside [0, K)
+template <typename KeyF>
+__device__ __forceinline__ int64_t dsum_key(KeyF key, int64_t i, int64_t n, int64_t K) {
+  if (i < 0 || i >= n) return -1;
+  const int64_t k = key(i);
+  return (k < 0 || k >= K) ? -1 : k;
 }
 
-// Tile layout of both passes: warp w of the block owns the 256 consecutive positions [tile + 256 w, +256) and reads
+// Tile layout of all passes: warp w of the block owns the 256 consecutive positions [tile + 256 w, +256) and reads
 // them in 8 rounds of 32 (round r, lane l -> position 256 w + 32 r + l): every load is a full coalesced line.
+// Segmented inclusive scan over the warp's positions, round after round.  k: keys (-1 = none), v: values (0 where
+// k = -1), k_before: key of the position before the window (lane 0; -1 if none).  inc[r] is the sum from the latest
+// segment start in the window at or before the position (from the window's start if there is none, fl[r] = false);
+// any / tail: the window's summary.  The segment starts of a round are one ballot: lane l adds the partial of lane
+// l - o unless a segment starts in lanes (l - o, l].
+__device__ __forceinline__ void dsum_warp_scan(const int64_t (&k)[kDsItems], const double (&v)[kDsItems],
+                                               int64_t k_before, double (&inc)[kDsItems], bool (&fl)[kDsItems],
+                                               bool& any, double& tail) {
+  const int lane = threadIdx.x & 31;
+  any = false;
+  tail = 0.0;
+#pragma unroll
+  for (int r = 0; r < kDsItems; ++r) {
+    int64_t prev = __shfl_up_sync(kFull, k[r], 1);
+    const int64_t last_prev = __shfl_sync(kFull, r > 0 ? k[r > 0 ? r - 1 : 0] : k_before, r > 0 ? 31 : 0);
+    if (lane == 0) prev = last_prev;
+    const unsigned heads = __ballot_sync(kFull, k[r] >= 0 && k[r] != prev);
+    double x = v[r];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const double t = __shfl_up_sync(kFull, x, o);
+      if (lane >= o && ((heads >> (lane - o + 1)) & ((1u << o) - 1u)) == 0u) x = t + x;
+    }
+    const bool f = (heads & ((2u << lane) - 1u)) != 0u;  // a segment starts in lanes [0, lane]
+    inc[r] = f ? x : tail + x;
+    fl[r] = f || any;
+    const double x31 = __shfl_sync(kFull, x, 31);
+    tail = heads ? x31 : tail + x31;
+    any = any || heads != 0u;
+  }
+}
+
+// Summary of one tile (keys / values in the tile layout, k_before = key before the warp's window): per warp, whether
+// a segment starts in its window and the sum of the values from the last such start (from the window's start if
+// none); the warps folded in warp order.  Shared by every producer of tile summaries, so they agree bit for bit.
+__device__ __forceinline__ void dsum_tile_summary(const int64_t (&k)[kDsItems], const double (&v)[kDsItems],
+                                                  int64_t k_before, double* __restrict__ tile_sums,
+                                                  uint32_t* __restrict__ tile_flags) {
+  __shared__ double s_tail[kDsWarps];
+  __shared__ int s_any[kDsWarps];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  unsigned last = 0;  // 1 + window position of the thread's last segment start, 0 if none
+#pragma unroll
+  for (int r = 0; r < kDsItems; ++r) {
+    int64_t prev = __shfl_up_sync(kFull, k[r], 1);
+    const int64_t last_prev = __shfl_sync(kFull, r > 0 ? k[r > 0 ? r - 1 : 0] : k_before, r > 0 ? 31 : 0);
+    if (lane == 0) prev = last_prev;
+    if (k[r] >= 0 && k[r] != prev) last = (unsigned)(r * 32 + lane) + 1u;
+  }
+  const unsigned head = __reduce_max_sync(kFull, last);
+  double s = 0.0;
+#pragma unroll
+  for (int r = 0; r < kDsItems; ++r)
+    if ((unsigned)(r * 32 + lane) + 1u >= head) s += v[r];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
+  if (lane == 0) {
+    s_tail[w] = s;
+    s_any[w] = head != 0u;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    bool a = false;
+    double t = 0.0;
+    for (int q = 0; q < kDsWarps; ++q) {
+      t = s_any[q] ? s_tail[q] : t + s_tail[q];
+      a = a || s_any[q];
+    }
+    tile_sums[blockIdx.x] = t;
+    tile_flags[blockIdx.x] = a ? 1u : 0u;
+  }
+}
+
 template <typename KeyF, typename ValF>
 static __global__ void __launch_bounds__(kDsThreads)
     k_dsum_reduce(KeyF key, ValF val, int64_t n, const int64_t* __restrict__ n_dev, int64_t K,
-                  double* __restrict__ tile_sums) {
-  __shared__ double red[33];
+                  double* __restrict__ tile_sums, uint32_t* __restrict__ tile_flags) {
   if (n_dev) n = min(n, *n_dev);
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t wbase = (int64_t)blockIdx.x * kDsTile + (int64_t)w * (32 * kDsItems);
-  double s = 0.0;
+  int64_t k[kDsItems];
+  double v[kDsItems];
 #pragma unroll
   for (int r = 0; r < kDsItems; ++r) {
     const int64_t i = wbase + r * 32 + lane;
-    if (i < n) {
-      const int64_t k = key(i);
-      if (k >= 0 && k < K) s += (double)val(i);
-    }
+    k[r] = dsum_key(key, i, n, K);
+    v[r] = k[r] >= 0 ? (double)val(i) : 0.0;
   }
-  double tot;
-  block_exclusive_scan_d(s, red, &tot);
-  if (threadIdx.x == 0) tile_sums[blockIdx.x] = tot;
+  const int64_t k_before = lane == 0 ? dsum_key(key, wbase - 1, n, K) : -1;
+  dsum_tile_summary(k, v, k_before, tile_sums, tile_flags);
 }
 
-// one block: exclusive scan of the tile sums in place, tile after tile in a fixed order
-static __global__ void k_dsum_spine(double* __restrict__ tile_sums, int nt) {
-  __shared__ double red[33];
+// one block: segmented exclusive scan of the tile summaries in place (tile_sums[t] becomes the running sum of the
+// segment open at the start of tile t), 1024 tiles per round, rounds in order with the carry between them
+static __global__ void __launch_bounds__(1024) k_dsum_spine(double* __restrict__ tile_sums,
+                                                            const uint32_t* __restrict__ tile_flags, int nt) {
+  __shared__ double s_tail[32], s_in[32];
+  __shared__ int s_any[32];
+  __shared__ double s_carry;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   double carry = 0.0;
   for (int start = 0; start < nt; start += blockDim.x) {
     const int i = start + threadIdx.x;
-    const double v = i < nt ? tile_sums[i] : 0.0;
-    double tot;
-    const double ex = block_exclusive_scan_d(v, red, &tot);
-    if (i < nt) tile_sums[i] = carry + ex;
-    carry += tot;
+    double x = i < nt ? tile_sums[i] : 0.0;
+    const unsigned heads = __ballot_sync(kFull, i < nt && tile_flags[i] != 0u);
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const double t = __shfl_up_sync(kFull, x, o);
+      if (lane >= o && ((heads >> (lane - o + 1)) & ((1u << o) - 1u)) == 0u) x = t + x;
+    }
+    const bool f = (heads & ((2u << lane) - 1u)) != 0u;
+    if (lane == 31) {
+      s_tail[w] = x;
+      s_any[w] = heads != 0u;
+    }
+    __syncthreads();
+    if (w == 0) {  // running sum entering every warp: the round's carry, then the warps before it in order
+      double y = s_tail[lane];
+      const unsigned wh = __ballot_sync(kFull, s_any[lane] != 0);
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const double t = __shfl_up_sync(kFull, y, o);
+        if (lane >= o && ((wh >> (lane - o + 1)) & ((1u << o) - 1u)) == 0u) y = t + y;
+      }
+      const double ye = __shfl_up_sync(kFull, y, 1);
+      const bool fe = (wh & ((1u << lane) - 1u)) != 0u;  // a segment starts in the warps before this one
+      s_in[lane] = lane == 0 ? carry : (fe ? ye : carry + ye);
+      if (lane == 31) s_carry = wh ? y : carry + y;
+    }
+    __syncthreads();
+    const double c = s_in[w];
+    const double incl = f ? x : c + x;
+    const double before = __shfl_up_sync(kFull, incl, 1);
+    if (i < nt) tile_sums[i] = lane == 0 ? c : before;
+    carry = s_carry;
     __syncthreads();
   }
 }
 
-// down-sweep: running prefix at every position; a run's first position stores its prefix in pb[key], its last
-// position the prefix after it in pe[key]
+// down-sweep: segmented running sum at every position; the last position of a key's run writes the run's sum
 template <typename KeyF, typename ValF>
 static __global__ void __launch_bounds__(kDsThreads)
     k_dsum_down(KeyF key, ValF val, int64_t n, const int64_t* __restrict__ n_dev, int64_t K,
-                const double* __restrict__ tile_off, double* __restrict__ pb, double* __restrict__ pe) {
-  __shared__ double wsum[kDsThreads / 32];
+                const double* __restrict__ tile_off, float* __restrict__ out) {
+  __shared__ double s_tail[kDsWarps];
+  __shared__ int s_any[kDsWarps];
   if (n_dev) n = min(n, *n_dev);
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t wbase = (int64_t)blockIdx.x * kDsTile + (int64_t)w * (32 * kDsItems);
   int64_t k[kDsItems];
   double v[kDsItems], inc[kDsItems];
+  bool fl[kDsItems];
 #pragma unroll
   for (int r = 0; r < kDsItems; ++r) {
     const int64_t i = wbase + r * 32 + lane;
-    k[r] = i < n ? key(i) : -1;
-    if (k[r] < 0 || k[r] >= K) k[r] = -1;
+    k[r] = dsum_key(key, i, n, K);
     v[r] = k[r] >= 0 ? (double)val(i) : 0.0;
   }
-  // keys just outside the warp's window (raw values: only compared for inequality with valid keys)
-  const int64_t k_before = (lane == 0 && wbase > 0 && wbase - 1 < n) ? key(wbase - 1) : -1;
-  const int64_t k_after = (lane == 31 && wbase + 32 * kDsItems < n) ? key(wbase + 32 * kDsItems) : -1;
-  double wtot = 0.0;
-#pragma unroll
-  for (int r = 0; r < kDsItems; ++r) {  // inclusive prefix over the warp's positions, round after round
-    double x = v[r];
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      double t = __shfl_up_sync(kFull, x, o);
-      if (lane >= o) x += t;
-    }
-    inc[r] = wtot + x;
-    wtot += __shfl_sync(kFull, x, 31);
+  // keys just outside the warp's window
+  const int64_t k_before = lane == 0 ? dsum_key(key, wbase - 1, n, K) : -1;
+  const int64_t k_after = lane == 31 ? dsum_key(key, wbase + 32 * kDsItems, n, K) : -1;
+  bool any;
+  double tail;
+  dsum_warp_scan(k, v, k_before, inc, fl, any, tail);
+  if (lane == 0) {
+    s_tail[w] = tail;
+    s_any[w] = any;
   }
-  if (lane == 0) wsum[w] = wtot;
   __syncthreads();
-  double off = tile_off[blockIdx.x];
-  for (int q = 0; q < w; ++q) off += wsum[q];
+  double c = tile_off[blockIdx.x];  // running sum entering the warp's window
+  for (int q = 0; q < w; ++q) c = s_any[q] ? s_tail[q] : c + s_tail[q];
 #pragma unroll
   for (int r = 0; r < kDsItems; ++r) {
-    int64_t prev = __shfl_up_sync(kFull, k[r], 1);
     int64_t next = __shfl_down_sync(kFull, k[r], 1);
-    const int64_t last_prev = __shfl_sync(kFull, r > 0 ? k[r > 0 ? r - 1 : 0] : k_before, r > 0 ? 31 : 0);
     const int64_t first_next =
         __shfl_sync(kFull, r + 1 < kDsItems ? k[r + 1 < kDsItems ? r + 1 : r] : k_after, r + 1 < kDsItems ? 0 : 31);
-    if (lane == 0) prev = last_prev;
     if (lane == 31) next = first_next;
     const int64_t kk = k[r];
-    if (kk >= 0) {
-      if (prev != kk) pb[kk] = off + inc[r] - v[r];
-      if (next != kk) pe[kk] = off + inc[r];
-    }
+    if (kk >= 0 && next != kk) out[kk] = (float)(fl[r] ? inc[r] : c + inc[r]);
   }
-}
-
-static __global__ void k_dsum_finish(const double* __restrict__ pb, const double* __restrict__ pe, int64_t K,
-                                     float* __restrict__ out) {
-  int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (k >= K) return;
-  const double b = pb[k];
-  out[k] = (b == b) ? (float)(pe[k] - b) : 0.f;  // pb is NaN-filled: keys without a run sum to 0
 }
 
 template <typename KeyF>
@@ -492,7 +560,7 @@ static __global__ void k_fill_keys32(KeyF key, int64_t n, const int64_t* __restr
 }
 
 // grouped (unsorted-key) path: the values are evaluated once in position order (coalesced operand reads) and carried
-// into key order as the payload of the stable sort; the prefix passes read them linearly
+// into key order as the payload of the stable sort; the scan passes read them linearly
 template <typename ValF>
 static __global__ void k_eval_vals(ValF val, int64_t n, const int64_t* __restrict__ n_dev, float* __restrict__ out) {
   if (n_dev) n = min(n, *n_dev);
@@ -504,18 +572,19 @@ struct ValOfArray {
   __device__ float operator()(int64_t i) const { return a[i]; }
 };
 
-// Scratch of one det_segment_sum of n values into K segments: the run bounds and tile sums of the prefix passes, and
-// for unsorted keys the 32-bit keys, the values in position order and the stable sort that groups them.
+// Scratch of one det_segment_sum of n values: the tile summaries of the scan passes, and for unsorted keys the 32-bit
+// keys, the values in position order and the stable sort that groups them.  Nothing in it is per segment: the sums
+// go straight to `out`.
 struct DetSumScratch {
-  double *pb, *pe, *tiles;
+  double* tiles;
+  uint32_t* tile_flags;
   uint32_t *keys0, *keys1, *vals0, *vals1;
   float* ev;
   Workspace sort;
-  DetSumScratch(Workspace& ws, int64_t n, int64_t K) {
+  DetSumScratch(Workspace& ws, int64_t n) {
     const size_t m = (size_t)(n > 0 ? n : 1);
-    pb = ws.take<double>((size_t)(K > 0 ? K : 0) + 1);
-    pe = ws.take<double>((size_t)(K > 0 ? K : 0) + 1);
     tiles = ws.take<double>(m / kDsTile + 2);
+    tile_flags = ws.take<uint32_t>(m / kDsTile + 2);
     keys0 = ws.take<uint32_t>(m);
     keys1 = ws.take<uint32_t>(m);
     vals0 = ws.take<uint32_t>(m);
@@ -525,28 +594,29 @@ struct DetSumScratch {
   }
 };
 
-// tiles_ready: `tiles` already holds the per-tile sums (a producer kernel with the tile layout of k_dsum_reduce)
+// tiles_ready: `tiles` / `tile_flags` already hold the tile summaries (a producer kernel with the tile layout of
+// k_dsum_reduce that calls dsum_tile_summary)
 template <typename KeyF, typename ValF>
-static void prefix_run_sums(KeyF key, ValF val, int64_t n, const int64_t* n_dev, int64_t K, double* pb, double* pe,
-                            double* tiles, float* out, cudaStream_t st, bool tiles_ready = false) {
+static void segmented_run_sums(KeyF key, ValF val, int64_t n, const int64_t* n_dev, int64_t K, double* tiles,
+                               uint32_t* tile_flags, float* out, cudaStream_t st, bool tiles_ready = false) {
   const int nt = (int)ceil_div(n, kDsTile);
-  cudaMemsetAsync(pb, 0xff, (size_t)K * sizeof(double), st);
+  cudaMemsetAsync(out, 0, (size_t)K * sizeof(float), st);  // keys without a run sum to 0
   if (!tiles_ready)
-    launch("k_dsum_reduce", k_dsum_reduce<KeyF, ValF>, nt, kDsThreads, 0, st, key, val, n, n_dev, K, tiles);
-  launch("k_dsum_spine", k_dsum_spine, 1, 1024, 0, st, tiles, nt);
-  launch("k_dsum_down", k_dsum_down<KeyF, ValF>, nt, kDsThreads, 0, st, key, val, n, n_dev, K, tiles, pb, pe);
-  launch("k_dsum_finish", k_dsum_finish, (unsigned)ceil_div(K, 256), 256, 0, st, pb, pe, K, out);
+    launch("k_dsum_reduce", k_dsum_reduce<KeyF, ValF>, nt, kDsThreads, 0, st, key, val, n, n_dev, K, tiles,
+           tile_flags);
+  launch("k_dsum_spine", k_dsum_spine, 1, 1024, 0, st, tiles, tile_flags, nt);
+  launch("k_dsum_down", k_dsum_down<KeyF, ValF>, nt, kDsThreads, 0, st, key, val, n, n_dev, K, tiles, out);
 }
 
 // A value functor that gathers (`static constexpr bool kCostly = true`) is evaluated ONCE into a float array and the
-// two prefix passes read the array: the degree backward's dependent gather deg[other[e]] otherwise runs in both the
+// two scan passes read the array: the degree backward's dependent gather deg[other[e]] otherwise runs in both the
 // tile-sum and the down-sweep pass (ncu: down-sweep 1.37 ms against 0.45 ms for the plain-array form on 100 M edges).
 template <typename V, typename = void>
 struct val_is_costly : std::false_type {};
 template <typename V>
 struct val_is_costly<V, std::void_t<decltype(V::kCostly)>> : std::integral_constant<bool, V::kCostly> {};
 
-// s.keys0 (32-bit, invalid keys = K) and s.ev (values in position order) are ready: group by key, then prefix sums.
+// s.keys0 (32-bit, invalid keys = K) and s.ev (values in position order) are ready: group by key, then run sums.
 // The values themselves ride through the stable sort as its 32-bit payload: no index payload, no gather afterwards
 // (a random 4-byte gather over 100 M values cost 1.5 ms, as much as two sort passes).  s.keys0 is overwritten.
 static int grouped_sums_of(const DetSumScratch& s, int64_t n, const int64_t* n_dev, int64_t K, float* out,
@@ -556,11 +626,12 @@ static int grouped_sums_of(const DetSumScratch& s, int64_t n, const int64_t* n_d
                                       key_bits_for_u64((uint64_t)K), &in1, s.sort, st, n_dev);
   if (rc != TGPB200_OK) return rc;
   const float* sv = reinterpret_cast<const float*>(in1 ? s.vals1 : s.vals0);
-  prefix_run_sums(KeyOfArray32{in1 ? s.keys1 : s.keys0}, ValOfArray{sv}, n, n_dev, K, s.pb, s.pe, s.tiles, out, st);
+  segmented_run_sums(KeyOfArray32{in1 ? s.keys1 : s.keys0}, ValOfArray{sv}, n, n_dev, K, s.tiles, s.tile_flags, out,
+                     st);
   return launch_status();
 }
 
-// s: carved for at least n values and K segments.
+// s: carved for at least n values.
 template <typename KeyF, typename ValF>
 static int det_segment_sum(KeyF key, ValF val, int64_t n, const int64_t* n_dev, int64_t K, bool keys_sorted, float* out,
                            const DetSumScratch& s, cudaStream_t st) {
@@ -572,9 +643,9 @@ static int det_segment_sum(KeyF key, ValF val, int64_t n, const int64_t* n_dev, 
   if (keys_sorted) {
     if constexpr (val_is_costly<ValF>::value) {
       launch("k_eval_vals", k_eval_vals<ValF>, (unsigned)ceil_div(n, 256), 256, 0, st, val, n, n_dev, s.ev);
-      prefix_run_sums(key, ValOfArray{s.ev}, n, n_dev, K, s.pb, s.pe, s.tiles, out, st);
+      segmented_run_sums(key, ValOfArray{s.ev}, n, n_dev, K, s.tiles, s.tile_flags, out, st);
     } else {
-      prefix_run_sums(key, val, n, n_dev, K, s.pb, s.pe, s.tiles, out, st);
+      segmented_run_sums(key, val, n, n_dev, K, s.tiles, s.tile_flags, out, st);
     }
     return launch_status();
   }
@@ -626,14 +697,14 @@ struct ArrVal {
 // Both sides of the degree backward from ONE pass over the edges (row-sorted input): the row-side values
 // g w dinv[col], the column-side values g w dinv[row] and the 32-bit column keys of the grouped sum.  Same products in
 // the same order as DegBwdVal, so the sums are bit-identical to the two-functor form (3 kernels, each edge read 3 x).
-// It also leaves the row-side tile sums behind (one k_dsum_reduce pass less).
+// It also leaves the row-side tile summaries behind (one k_dsum_reduce pass less).
 static __global__ void __launch_bounds__(kDsThreads)
     k_deg_bwd_prepare(const int64_t* __restrict__ row, const int64_t* __restrict__ col, const float* __restrict__ w,
                       const float* __restrict__ deg, const float* __restrict__ gout, int64_t E,
                       const int64_t* __restrict__ E_dev, int64_t K, float eps, float* __restrict__ ev_row,
-                      float* __restrict__ ev_col, uint32_t* __restrict__ keys_col, double* __restrict__ tile_sums) {
-  // tile layout and summation order of k_dsum_reduce, so tile_sums are the row-side tile sums bit for bit
-  __shared__ double red[33];
+                      float* __restrict__ ev_col, uint32_t* __restrict__ keys_col, double* __restrict__ tile_sums,
+                      uint32_t* __restrict__ tile_flags) {
+  // tile layout, keys and values of k_dsum_reduce over (row, ev_row), so the summaries agree with it bit for bit
   if (E_dev) E = min(E, *E_dev);
   const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
   const int64_t wbase = (int64_t)blockIdx.x * kDsTile + (int64_t)wp * (32 * kDsItems);
@@ -652,21 +723,23 @@ static __global__ void __launch_bounds__(kDsThreads)
     dr[k] = (r[k] >= 0 && r[k] < K) ? __ldg(deg + r[k]) : 0.f;
     dc[k] = (c[k] >= 0 && c[k] < K) ? __ldg(deg + c[k]) : 0.f;
   }
-  double s = 0.0;
+  int64_t kr[kDsItems];
+  double vr[kDsItems];
 #pragma unroll
   for (int k = 0; k < kDsItems; ++k) {
     const int64_t e = wbase + k * 32 + lane;
-    if (e >= E) continue;
     const bool okr = r[k] >= 0 && r[k] < K, okc = c[k] >= 0 && c[k] < K;
-    const float vr = okc ? g[k] * dinv_of(dc[k], eps) : 0.f;  // keyed by row, opposite endpoint = col
-    ev_row[e] = vr;
-    ev_col[e] = okr ? g[k] * dinv_of(dr[k], eps) : 0.f;       // keyed by col, opposite endpoint = row
+    kr[k] = okr ? r[k] : -1;
+    vr[k] = 0.0;
+    if (e >= E) continue;
+    const float v = okc ? g[k] * dinv_of(dc[k], eps) : 0.f;  // keyed by row, opposite endpoint = col
+    ev_row[e] = v;
+    ev_col[e] = okr ? g[k] * dinv_of(dr[k], eps) : 0.f;      // keyed by col, opposite endpoint = row
     keys_col[e] = okc ? (uint32_t)c[k] : (uint32_t)K;
-    if (okr) s += (double)vr;
+    if (okr) vr[k] = (double)v;
   }
-  double tot;
-  block_exclusive_scan_d(s, red, &tot);
-  if (threadIdx.x == 0) tile_sums[blockIdx.x] = tot;
+  const int64_t k_before = lane == 0 ? dsum_key(KeyOfArray64{row}, wbase - 1, E, K) : -1;
+  dsum_tile_summary(kr, vr, k_before, tile_sums, tile_flags);
 }
 
 static __global__ void k_deg_apply(const int64_t* __restrict__ row, const int64_t* __restrict__ col,
@@ -704,14 +777,14 @@ static __global__ void k_deg_bwd_apply(const int64_t* __restrict__ row, const in
 // per-node values by graph (its K is max(pooled nodes, graphs)).
 struct EdgeNormLayout {
   float *part_row, *part_col;  // [K]
-  DetSumScratch row, col;      // E values, K segments
-  DetSumScratch nodes;         // K values, K segments
+  DetSumScratch row, col;      // E values each
+  DetSumScratch nodes;         // K values
   EdgeNormLayout(Workspace& ws, int64_t E, int64_t K)
       : part_row(ws.take<float>((size_t)(K > 0 ? K : 1))),
         part_col(ws.take<float>((size_t)(K > 0 ? K : 1))),
-        row(ws, E, K),
-        col(ws, E, K),
-        nodes(ws, K, K) {}
+        row(ws, E),
+        col(ws, E),
+        nodes(ws, K) {}
 };
 
 static __global__ void k_wn_max(const int64_t* __restrict__ row, const float* __restrict__ w,
@@ -984,9 +1057,9 @@ int tgpb200_degree_bwd_accumulate(const int64_t* row, const int64_t* col, const 
   int rc;
   if (rows_sorted && E > 0) {
     launch("k_deg_bwd_prepare", k_deg_bwd_prepare, (unsigned)ceil_div(E, kDsTile), kDsThreads, 0, st, row, col, w, deg,
-           grad_out, E, E_dev, K, eps, l.row.ev, l.col.ev, l.col.keys0, l.row.tiles);
-    prefix_run_sums(KeyOfArray64{row}, ValOfArray{l.row.ev}, E, E_dev, K, l.row.pb, l.row.pe, l.row.tiles, l.part_row,
-                    st, true);
+           grad_out, E, E_dev, K, eps, l.row.ev, l.col.ev, l.col.keys0, l.row.tiles, l.row.tile_flags);
+    segmented_run_sums(KeyOfArray64{row}, ValOfArray{l.row.ev}, E, E_dev, K, l.row.tiles, l.row.tile_flags,
+                       l.part_row, st, true);
     // the column side is a scatter by `col`: grouped through the stable sort
     rc = grouped_sums_of(l.col, E, E_dev, K, l.part_col, st);
     if (rc != TGPB200_OK) return rc;
