@@ -330,6 +330,47 @@ int tgpb200_hosc_loss_bwd(const void* adj, const void* s, const float* graph_nod
                           tgpb200_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * HOSC losses on a sparse adjacency (csrc/hosc_sparse.cu): the losses of tgpb200_hosc_loss_fwd with A given as nnz
+ * coalesced edges over the padded layout of B graphs of N rows (node i of graph b is row b N + i), so that memory is
+ * O(nnz + B N K) and no [B, N, N] array exists.  row / col int64 [nnz] sorted by (row, col), duplicates summed,
+ * weight float32 [nnz] (any sign, zero kept); row_ptr int32 [B N + 1] the row CSR of these edges, col_ptr int32
+ * [B N + 1] and col_order int32 [nnz] the column CSR (edge ids by column, ascending row inside a column: a stable
+ * sort by col).  Directed edges and self loops are ordinary input.  s [B, N, K] row-major of `dtype` (padded rows
+ * zero), graph_nodes [B] float32 or NULL (= N); needs N >= 1, K >= 2, B <= 65535, B N and nnz below 2^31.
+ *   P_e = (A A)_ij = sum_{k in out(i) ∩ in(j)} w_ik w_kj,  wM_e = P_e w_e  (A_M = (A A) . A on A's pattern)
+ * is a per-edge intersection of the sorted row list of i and column list of j (one warp per edge, one block per edge
+ * whose shorter lists exceed 1024 entries); [A S | d] and [A_M S | d^M] are segment reduces of S1 = [S | 1 | 0 ..]
+ * (K1 = K + 1 rounded up to 8 columns).  Every sum has a fixed order: the results are bitwise deterministic.
+ * `terms` as in tgpb200_hosc_loss_fwd: a term outside the mask is written as 0, and without bit 2 no motif kernel runs.
+ * `as1` (float [B, N, K1], always written) returns [A S | d]: its first K columns are the A S of the pooled
+ * adjacency S^T A S.  `saved` (tgpb200_hosc_sparse_loss_saved_bytes) carries, 256-byte aligned in this order:
+ * P, wM float [nnz] (bit 2 only), d, d^M float [B N], n, m, n^M, m^M, ||S_:k||^2 float [B, K].  The forward
+ * workspace holds S1, [A_M S | d^M], the 32-bit endpoints, the column lists and the heavy-edge queue.
+ * Backward (grad_losses = 3 device floats; grad_as1 = float [B, N, K1] cotangent of as1 or NULL):
+ *   grad_s = A Sa + A^T (Sa + grad_as1[:, :K]) + A_M Sm + A_M^T Sm + the elementwise terms of tgpb200_hosc_loss_bwd
+ *   grad_weight[e] = <U_i, S1_j> + gM_e P_e + sum_{k in out(i) ∩ out(j)} H_ik w_jk + sum_{k in in(i) ∩ in(j)} w_ki H_kj
+ *     U_i = [Sa_i + grad_as1_i[:K] | r_i + grad_as1_iK | ..],  gM_e = <Sm_i, S_j> + r^M_i,  H_e = gM_e w_e
+ *   (Sa, Sm, r, r^M as in tgpb200_hosc_loss_bwd; grad_weight may be NULL).  Size queries measure exactly what their
+ * entry point carves; a short buffer returns TGPB200_ERR_WORKSPACE before anything is enqueued.
+ * ------------------------------------------------------------------------------------------ */
+size_t tgpb200_hosc_sparse_loss_saved_bytes(int64_t B, int64_t N, int64_t K, int64_t nnz, int terms);
+size_t tgpb200_hosc_sparse_loss_fwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int64_t nnz, int terms,
+                                                    int dtype);
+int tgpb200_hosc_sparse_loss_fwd(const int64_t* row, const int64_t* col, const float* weight, const int32_t* row_ptr,
+                                 const int32_t* col_ptr, const int32_t* col_order, const void* s,
+                                 const float* graph_nodes, int64_t B, int64_t N, int64_t K, int64_t nnz, int dtype,
+                                 int terms, float eps, float* losses, float* as1, void* saved, size_t saved_bytes,
+                                 void* workspace, size_t workspace_bytes, tgpb200_stream_t stream);
+size_t tgpb200_hosc_sparse_loss_bwd_workspace_bytes(int64_t B, int64_t N, int64_t K, int64_t nnz, int terms, int dtype,
+                                                    int has_grad_as1, int need_grad_weight);
+int tgpb200_hosc_sparse_loss_bwd(const int64_t* row, const int64_t* col, const float* weight, const int32_t* row_ptr,
+                                 const int32_t* col_ptr, const int32_t* col_order, const void* s,
+                                 const float* graph_nodes, const void* saved, size_t saved_bytes,
+                                 const float* grad_losses, const float* grad_as1, int64_t B, int64_t N, int64_t K,
+                                 int64_t nnz, int dtype, int terms, void* grad_s, float* grad_weight, void* workspace,
+                                 size_t workspace_bytes, tgpb200_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * Tensor-core batched product (tcgen05 / TMEM / TMA), the engine under the dense path; exported for tests
  * and for callers that need a raw S^T X / S^T A S style contraction:
  *   out[b] (M x N) = alpha * A[b] (M x Kd) * B[b] (Kd x N)  (+ out[b] when accumulate)

@@ -198,6 +198,77 @@ std::tuple<Tensor, Tensor> hosc_losses_bwd(const Tensor& adj, const Tensor& s, c
   return {ga, gs};
 }
 
+// The coalesced edge list (row, col, weight), its row CSR and column CSR, and s [B, N, K] of the sparse HOSC ops
+void check_sparse_hosc(const Tensor& row, const Tensor& col, const Tensor& weight, const Tensor& row_ptr,
+                       const Tensor& col_ptr, const Tensor& col_order, const Tensor& s, int64_t terms) {
+  require_cuda(s, "s");
+  for (const Tensor* t : {&row, &col, &weight, &row_ptr, &col_ptr, &col_order}) require_cuda(*t, "edge list / CSR");
+  TORCH_CHECK(s.dim() == 3, "hosc_losses_sparse expects s of shape [B, N, K], got ", s.sizes());
+  TORCH_CHECK_VALUE(s.size(2) >= 2, "hosc_losses_sparse needs K >= 2 clusters, got K = ", s.size(2));
+  TORCH_CHECK_VALUE(s.size(1) >= 1, "hosc_losses_sparse needs N >= 1 nodes");
+  TORCH_CHECK_VALUE(terms >= 1 && terms <= 7, "hosc_losses_sparse: terms must be a non-empty mask of 1 | 2 | 4, got ",
+                    terms);
+  const int64_t nnz = row.numel(), R = s.size(0) * s.size(1);
+  TORCH_CHECK(row.scalar_type() == at::kLong && col.scalar_type() == at::kLong && col.numel() == nnz,
+              "hosc_losses_sparse: row / col must be int64 [nnz]");
+  TORCH_CHECK(weight.scalar_type() == at::kFloat && weight.numel() == nnz, "hosc_losses_sparse: weight must be float32 [nnz]");
+  TORCH_CHECK(row_ptr.scalar_type() == at::kInt && col_ptr.scalar_type() == at::kInt && col_order.scalar_type() == at::kInt &&
+                  row_ptr.numel() == R + 1 && col_ptr.numel() == R + 1 && col_order.numel() >= nnz,
+              "hosc_losses_sparse: row_ptr / col_ptr must be int32 [B N + 1] and col_order int32 [nnz]");
+}
+
+// (losses[3] = {first-order cut, motif cut, HOSC orthogonality}, as1 = [A S | A 1 | 0..] [B, N, K1], saved) of HOSC
+// pooling on a sparse adjacency; `terms` is the bitmask of tgpb200_hosc_sparse_loss_fwd
+std::tuple<Tensor, Tensor, Tensor> hosc_losses_sparse(const Tensor& row, const Tensor& col, const Tensor& weight,
+                                                      const Tensor& row_ptr, const Tensor& col_ptr,
+                                                      const Tensor& col_order, const Tensor& s,
+                                                      const OptTensor& graph_nodes, int64_t terms, double eps) {
+  check_sparse_hosc(row, col, weight, row_ptr, col_ptr, col_order, s, terms);
+  c10::cuda::CUDAGuard guard(s.device());
+  const int64_t B = s.size(0), N = s.size(1), K = s.size(2), nnz = row.numel(), K1 = (K + 8) / 8 * 8;
+  const int dt = dtype_code(s);
+  Tensor saved = workspace(tgpb200_hosc_sparse_loss_saved_bytes(B, N, K, nnz, (int)terms), s);
+  Tensor ws = workspace(tgpb200_hosc_sparse_loss_fwd_workspace_bytes(B, N, K, nnz, (int)terms, dt), s);
+  Tensor losses = at::empty({3}, s.options().dtype(at::kFloat));
+  Tensor as1 = at::empty({B, N, K1}, s.options().dtype(at::kFloat));
+  check(tgpb200_hosc_sparse_loss_fwd((const int64_t*)ptr(row), (const int64_t*)ptr(col), (const float*)ptr(weight),
+                                     row_ptr.data_ptr<int32_t>(), col_ptr.data_ptr<int32_t>(),
+                                     (const int32_t*)ptr(col_order), s.data_ptr(), graph_nodes_ptr(graph_nodes, B), B,
+                                     N, K, nnz, dt, (int)terms, (float)eps, losses.data_ptr<float>(),
+                                     as1.data_ptr<float>(), saved.data_ptr(), (size_t)saved.numel(), ws.data_ptr(),
+                                     (size_t)ws.numel(), stream_of(s)),
+        "hosc_losses_sparse");
+  return {losses, as1, saved};
+}
+
+std::tuple<Tensor, Tensor> hosc_losses_sparse_bwd(const Tensor& row, const Tensor& col, const Tensor& weight,
+                                                  const Tensor& row_ptr, const Tensor& col_ptr, const Tensor& col_order,
+                                                  const Tensor& s, const OptTensor& graph_nodes, const Tensor& saved,
+                                                  const Tensor& glosses, const OptTensor& gas1, int64_t terms,
+                                                  bool need_gweight) {
+  check_sparse_hosc(row, col, weight, row_ptr, col_ptr, col_order, s, terms);
+  c10::cuda::CUDAGuard guard(s.device());
+  const int64_t B = s.size(0), N = s.size(1), K = s.size(2), nnz = row.numel();
+  const int dt = dtype_code(s);
+  TORCH_CHECK(glosses.numel() == 3, "hosc_losses_sparse_bwd expects 3 upstream loss gradients");
+  Tensor gl = glosses.to(at::kFloat).contiguous();
+  const bool has_gas = gas1.has_value() && gas1->defined();
+  Tensor ga = has_gas ? gas1->to(at::kFloat).contiguous() : Tensor();
+  Tensor gs = at::empty_like(s);
+  Tensor gw = at::empty({need_gweight ? nnz : 0}, s.options().dtype(at::kFloat));
+  Tensor ws = workspace(tgpb200_hosc_sparse_loss_bwd_workspace_bytes(B, N, K, nnz, (int)terms, dt, has_gas ? 1 : 0,
+                                                                     need_gweight ? 1 : 0), s);
+  check(tgpb200_hosc_sparse_loss_bwd((const int64_t*)ptr(row), (const int64_t*)ptr(col), (const float*)ptr(weight),
+                                     row_ptr.data_ptr<int32_t>(), col_ptr.data_ptr<int32_t>(),
+                                     (const int32_t*)ptr(col_order), s.data_ptr(), graph_nodes_ptr(graph_nodes, B),
+                                     saved.data_ptr(), (size_t)saved.numel(), gl.data_ptr<float>(),
+                                     has_gas ? ga.data_ptr<float>() : nullptr, B, N, K, nnz, dt, (int)terms,
+                                     gs.data_ptr(), need_gweight ? (float*)ptr(gw) : nullptr, ws.data_ptr(),
+                                     (size_t)ws.numel(), stream_of(s)),
+        "hosc_losses_sparse_bwd");
+  return {gw, gs};
+}
+
 // CSR-by-cluster of a sparse assignment (tgp/reduce/aggr_reduce.py:13-23)
 std::tuple<Tensor, Tensor> build_csr(const Tensor& cluster_index, int64_t num_clusters) {
   require_cuda(cluster_index, "cluster_index");
@@ -266,6 +337,11 @@ TORCH_LIBRARY(tgp_b200, m) {
   m.def("hosc_losses(Tensor adj, Tensor s, Tensor? graph_nodes, int terms, float eps) -> (Tensor, Tensor)");
   m.def("hosc_losses_bwd(Tensor adj, Tensor s, Tensor? graph_nodes, Tensor saved, Tensor glosses, int terms, "
         "bool need_gadj) -> (Tensor, Tensor)");
+  m.def("hosc_losses_sparse(Tensor row, Tensor col, Tensor weight, Tensor row_ptr, Tensor col_ptr, Tensor col_order, "
+        "Tensor s, Tensor? graph_nodes, int terms, float eps) -> (Tensor, Tensor, Tensor)");
+  m.def("hosc_losses_sparse_bwd(Tensor row, Tensor col, Tensor weight, Tensor row_ptr, Tensor col_ptr, "
+        "Tensor col_order, Tensor s, Tensor? graph_nodes, Tensor saved, Tensor glosses, Tensor? gas1, int terms, "
+        "bool need_gweight) -> (Tensor, Tensor)");
   m.def("build_csr(Tensor cluster_index, int num_clusters) -> (Tensor, Tensor)");
   m.def("segment_reduce(Tensor x, Tensor node_index, Tensor cluster_index, Tensor? weight, Tensor order, Tensor ptr, "
         "int num_clusters, int op) -> Tensor");
@@ -280,6 +356,8 @@ TORCH_LIBRARY_IMPL(tgp_b200, CUDA, m) {
   m.impl("acc_losses_bwd", &acc_losses_bwd);
   m.impl("hosc_losses", &hosc_losses);
   m.impl("hosc_losses_bwd", &hosc_losses_bwd);
+  m.impl("hosc_losses_sparse", &hosc_losses_sparse);
+  m.impl("hosc_losses_sparse_bwd", &hosc_losses_sparse_bwd);
   m.impl("build_csr", &build_csr);
   m.impl("segment_reduce", &segment_reduce);
   m.impl("segment_reduce_bwd", &segment_reduce_bwd);

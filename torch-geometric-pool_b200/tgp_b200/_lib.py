@@ -108,6 +108,17 @@ SIGNATURES = {
     "tgpb200_hosc_loss_fwd": (_INT, [_P, _P, _P, _I64, _I64, _I64, _INT, _INT, _F, _P, _P, _SZ, _P, _SZ, _P]),
     "tgpb200_hosc_loss_bwd_workspace_bytes": (_SZ, [_I64, _I64, _I64, _INT, _INT]),
     "tgpb200_hosc_loss_bwd": (_INT, [_P, _P, _P, _P, _SZ, _P, _I64, _I64, _I64, _INT, _INT, _P, _P, _P, _SZ, _P]),
+    "tgpb200_hosc_sparse_loss_saved_bytes": (_SZ, [_I64, _I64, _I64, _I64, _INT]),
+    "tgpb200_hosc_sparse_loss_fwd_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64, _INT, _INT]),
+    "tgpb200_hosc_sparse_loss_fwd": (
+        _INT,
+        [_P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I64, _INT, _INT, _F, _P, _P, _P, _SZ, _P, _SZ, _P],
+    ),
+    "tgpb200_hosc_sparse_loss_bwd_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64, _INT, _INT, _INT, _INT]),
+    "tgpb200_hosc_sparse_loss_bwd": (
+        _INT,
+        [_P, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P, _P, _I64, _I64, _I64, _I64, _INT, _INT, _P, _P, _P, _SZ, _P],
+    ),
 }
 
 

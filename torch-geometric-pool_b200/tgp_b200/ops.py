@@ -1,6 +1,7 @@
 """``torch.ops.tgp_b200.*``: the operators of the Reduce + Connect path as torch custom ops (SURVEY 8b).
 
-* ``stas_fused`` / ``stas_fused_bwd``, ``acc_losses`` / ``acc_losses_bwd``, ``hosc_losses`` / ``hosc_losses_bwd``, ``segment_reduce`` / ``segment_reduce_bwd``, ``build_csr`` are C++ dispatcher
+* ``stas_fused`` / ``stas_fused_bwd``, ``acc_losses`` / ``acc_losses_bwd``, ``hosc_losses`` / ``hosc_losses_bwd``,
+  ``hosc_losses_sparse`` / ``hosc_losses_sparse_bwd``, ``segment_reduce`` / ``segment_reduce_bwd``, ``build_csr`` are C++ dispatcher
   ops (``csrc/torch_ops.cpp`` -> ``libtgp_b200_ops.so``: allocate with the caching allocator, take the current stream,
   call the C ABI of ``libtgp_b200.so``);
 * ``filter_relabel_edges``, ``remap_coalesce``, ``degree_norm``, ``weight_norm`` (+ their ``*_bwd``) are
@@ -148,6 +149,48 @@ def _hosc_backward(ctx, glosses, _gsaved):
 
 
 torch.library.register_autograd("tgp_b200::hosc_losses", _hosc_backward, setup_context=_hosc_setup)
+
+
+# --------------------------------------------------------------------------------------------------------------
+# hosc_losses_sparse: (losses[3], as1 = [A S | A 1 | 0..] [B, N, K1] fp32, saved) of HOSC pooling on a coalesced
+# sparse adjacency (row-sorted edges, row CSR, column CSR); differentiable in `weight` and `s`, and as1 carries the
+# cotangent of the connect's A S back.  saved carries no gradient.
+# --------------------------------------------------------------------------------------------------------------
+@torch.library.register_fake("tgp_b200::hosc_losses_sparse")
+def _hosc_losses_sparse_fake(row, col, weight, row_ptr, col_ptr, col_order, s, graph_nodes, terms, eps):
+    B, N, K = s.shape
+    saved = L.load().tgpb200_hosc_sparse_loss_saved_bytes(B, N, K, row.numel(), terms)
+    return (s.new_empty((3,), dtype=torch.float32), s.new_empty((B, N, (K + 8) // 8 * 8), dtype=torch.float32),
+            s.new_empty((max(saved, 256),), dtype=torch.uint8))
+
+
+@torch.library.register_fake("tgp_b200::hosc_losses_sparse_bwd")
+def _hosc_losses_sparse_bwd_fake(row, col, weight, row_ptr, col_ptr, col_order, s, graph_nodes, saved, glosses, gas1,
+                                 terms, need_gweight):
+    return weight.new_empty((row.numel() if need_gweight else 0,)), torch.empty_like(s)
+
+
+def _hosc_sparse_setup(ctx, inputs, output):
+    row, col, weight, row_ptr, col_ptr, col_order, s, graph_nodes, terms, _eps = inputs
+    ctx.save_for_backward(row, col, weight, row_ptr, col_ptr, col_order, s, graph_nodes, output[2])
+    ctx.terms = terms
+    ctx.mark_non_differentiable(output[2])
+    ctx.set_materialize_grads(False)
+
+
+def _hosc_sparse_backward(ctx, glosses, gas1, _gsaved):
+    row, col, weight, row_ptr, col_ptr, col_order, s, graph_nodes, saved = ctx.saved_tensors
+    if glosses is None and gas1 is None:
+        return (None,) * 10
+    if glosses is None:
+        glosses = torch.zeros(3, dtype=torch.float32, device=s.device)
+    need_w = ctx.needs_input_grad[2]
+    gw, gs = _T.hosc_losses_sparse_bwd(row, col, weight, row_ptr, col_ptr, col_order, s, graph_nodes, saved, glosses,
+                                       gas1, ctx.terms, need_w)
+    return (None, None, gw if need_w else None, None, None, None, gs, None, None, None)
+
+
+torch.library.register_autograd("tgp_b200::hosc_losses_sparse", _hosc_sparse_backward, setup_context=_hosc_sparse_setup)
 
 
 # --------------------------------------------------------------------------------------------------------------
@@ -465,6 +508,7 @@ def _wn_backward(ctx, g, _gmx, _garg):
 
 torch.library.register_autograd("tgp_b200::weight_norm", _wn_backward, setup_context=_wn_setup)
 
-OP_NAMES = ("stas_fused", "stas_fused_bwd", "acc_losses", "acc_losses_bwd", "hosc_losses", "hosc_losses_bwd", "build_csr", "segment_reduce", "segment_reduce_bwd", "filter_relabel_edges",
+OP_NAMES = ("stas_fused", "stas_fused_bwd", "acc_losses", "acc_losses_bwd", "hosc_losses", "hosc_losses_bwd",
+            "hosc_losses_sparse", "hosc_losses_sparse_bwd", "build_csr", "segment_reduce", "segment_reduce_bwd", "filter_relabel_edges",
             "filter_relabel_edges_bwd", "remap_coalesce", "remap_coalesce_bwd", "degree_norm", "degree_norm_bwd",
             "weight_norm", "weight_norm_bwd")

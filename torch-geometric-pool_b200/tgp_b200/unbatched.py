@@ -12,6 +12,10 @@ twins ``sparse_mincut_loss`` / ``unbatched_orthogonality_loss`` / ``sparse_link_
 
 The losses reuse ``W`` (``tr(S^T A S) = sum_i <S_i, W_i>``), so they cost no extra pass over the edges and no
 ``[E, K]`` temporaries.
+
+HOSC's motif cut needs ``A_M = (A A) . A`` on A's pattern: ``hosc_losses_unbatched`` coalesces the edge list into the
+padded ``[B, Nmax]`` node layout and runs ``torch.ops.tgp_b200.hosc_losses_sparse`` (csrc/hosc_sparse.cu), whose
+per-edge list intersection builds the triangle weights from the edge list; memory stays ``O(E + B Nmax K)``.
 """
 from __future__ import annotations
 
@@ -23,6 +27,7 @@ from torch import Tensor
 
 from . import _lib as L
 from . import functional as F_
+from . import ops as O
 
 EPS = 1e-8
 
@@ -189,6 +194,86 @@ def mincut_pool_unbatched(x: Tensor, edge_index: Tensor, edge_weight: Optional[T
     x_pool = _BmmTN.apply(s3.contiguous(), x3.contiguous())
     loss = {"cut_loss": sparse_mincut_loss(edge_index, s, edge_weight, b, num_graphs=B, _as=w_as) * cut_loss_coeff,
             "ortho_loss": unbatched_orthogonality_loss(s, b, num_graphs=B, _s3=s3.contiguous()) * ortho_loss_coeff}
+    adj_pool = postprocess_adj_pool_dense(raw, remove_self_loops=remove_self_loops, degree_norm=degree_norm,
+                                          adj_transpose=False, edge_weight_norm=edge_weight_norm)
+    return x_pool, adj_pool, loss
+
+
+def _hosc_sparse(edge_index: Tensor, edge_weight: Optional[Tensor], s: Tensor, batch: Optional[Tensor], alpha: float,
+                 hosc_ortho: bool, num_graphs: Optional[int], max_num_nodes: Optional[int], eps: float):
+    """(losses [3], as1 = [A S | A 1 | 0..] [B, Nmax, K1] fp32, s3 [B, Nmax, K], batch, B, Nmax) of the sparse HOSC
+    op.  One ``remap_coalesce`` maps node i of graph b to row ``b Nmax + (i - ptr[b])`` of the padded layout and sums
+    duplicates (``to_dense_adj``); it keeps self loops and every run, zero-weight ones included (they still have a
+    gradient), and carries the edge gradient back to the input edges."""
+    F_._require_cuda(edge_index, edge_weight, s, batch)
+    F_._validate_edge_index(edge_index)
+    if s.dim() != 2:
+        raise ValueError(f"hosc_losses_unbatched expects s of shape [N, K], got {tuple(s.shape)}")
+    N, K = s.shape
+    if K < 2:
+        raise ValueError(f"hosc_losses_unbatched needs K >= 2 clusters, got K = {K}")
+    dev = s.device
+    batch, B = _graphs_of(batch, N, num_graphs, dev)
+    batch = batch.contiguous()
+    ptr = F_.graph_ptr(batch, B)
+    counts = ptr[1:] - ptr[:-1]
+    if max_num_nodes is None:
+        max_num_nodes = int(counts.max().item()) if N > 0 else 1
+    nmax = max(int(max_num_nodes), 1)
+    R = B * nmax
+    slot = batch * nmax + (torch.arange(N, device=dev) - ptr.long()[batch])
+    ei = edge_index.contiguous()
+    w = F_._as_f32_weight(edge_weight)
+    if w is None:
+        w = torch.ones(ei.size(1), dtype=torch.float32, device=dev)
+    need_grad = w.requires_grad and torch.is_grad_enabled()
+    csr = F_.build_csr(slot, R) if ei.size(1) > 0 and F_.rows_sorted(ei) else (None, None)
+    # eps = -1 keeps every run: the filter drops |w| <= eps, and |w| >= 0 > -1
+    ei_c, w_c, _, _, _, _ = O.remap_coalesce(ei[0], ei[1], w, slot, csr[0], csr[1], N, R, L.SUM, 0, -1.0, False,
+                                             need_grad)
+    row, col = ei_c[0], ei_c[1]
+    _, row_ptr = F_.build_csr(row, R)
+    col_order, col_ptr = F_.build_csr(col, R)  # stable: ascending row inside every column
+    s3, _ = F_.to_dense_batch(s, batch, B, nmax)
+    s3 = s3.contiguous()
+    alpha = float(alpha)
+    terms = ((F_.HOSC_FIRST if alpha != 1.0 else 0) | (F_.HOSC_MOTIF if alpha != 0.0 else 0)
+             | (F_.HOSC_ORTHO if hosc_ortho else 0))
+    losses, as1, _ = O._T.hosc_losses_sparse(row, col, w_c, row_ptr, col_ptr, col_order, s3, counts.float(), terms,
+                                             float(eps))
+    return losses, as1, s3, batch, B, nmax
+
+
+def hosc_losses_unbatched(edge_index: Tensor, edge_weight: Optional[Tensor], s: Tensor, batch: Optional[Tensor] = None,
+                          alpha: float = 0.5, hosc_ortho: bool = False, num_graphs: Optional[int] = None,
+                          max_num_nodes: Optional[int] = None, eps: float = EPS) -> Tensor:
+    """``[L1, L2, O]`` of HOSC pooling from a sparse adjacency and ``s [N, K]``: the values of
+    ``functional.hosc_losses(to_dense_adj(edge_index, batch, edge_weight), to_dense_batch(s, batch)[0])`` with
+    ``n_b`` each graph's own node count, without any ``[B, Nmax, Nmax]`` tensor.  Duplicates add up, self loops count,
+    directed edges are taken as given.  ``L1`` is 0 when ``alpha == 1``, ``L2`` is 0 (and no motif kernel runs) when
+    ``alpha == 0``, ``O`` is 0 unless ``hosc_ortho``.  Differentiable in ``s`` and ``edge_weight``; ``K < 2`` raises
+    ``ValueError``."""
+    return _hosc_sparse(edge_index, edge_weight, s, batch, alpha, hosc_ortho, num_graphs, max_num_nodes, eps)[0]
+
+
+def hosc_pool_unbatched(x: Tensor, edge_index: Tensor, edge_weight: Optional[Tensor], s: Tensor,
+                        batch: Optional[Tensor] = None, num_graphs: Optional[int] = None, mu: float = 0.1,
+                        alpha: float = 0.5, hosc_ortho: bool = False, remove_self_loops: bool = True,
+                        degree_norm: bool = True, edge_weight_norm: bool = False) -> Tuple[Tensor, Tensor, Dict]:
+    """Unbatched HOSC pooling after select: ``x_pool = S^T X`` [B, K, F], ``adj_pool`` = post-processed ``S^T A S``
+    [B, K, K] and ``{"hosc_loss": (1 - alpha) L1 + alpha L2, "ortho_loss": mu * O}`` (MinCut's orthogonality term
+    without ``hosc_ortho``).  The connect's ``A S`` is the first K columns of the loss op's ``[A S | A 1]``: the
+    adjacency is multiplied by ``S`` once."""
+    from .connect import postprocess_adj_pool_dense
+
+    losses, as1, s3, b, B, nmax = _hosc_sparse(edge_index, edge_weight, s, batch, alpha, hosc_ortho, num_graphs, None,
+                                               EPS)
+    K = s.size(1)
+    raw = _BmmTN.apply(s3, as1[..., :K].to(s.dtype).contiguous())
+    x3, _ = F_.to_dense_batch(x, b, B, nmax)
+    x_pool = _BmmTN.apply(s3, x3.contiguous())
+    ortho = losses[2] if hosc_ortho else unbatched_orthogonality_loss(s, b, num_graphs=B, _s3=s3)
+    loss = {"hosc_loss": (1.0 - alpha) * losses[0] + alpha * losses[1], "ortho_loss": mu * ortho}
     adj_pool = postprocess_adj_pool_dense(raw, remove_self_loops=remove_self_loops, degree_norm=degree_norm,
                                           adj_transpose=False, edge_weight_norm=edge_weight_norm)
     return x_pool, adj_pool, loss
